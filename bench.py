@@ -1,7 +1,11 @@
 #!/usr/bin/env python
 """bench.py -- lnlike evals/sec of the batched likelihood hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes the lnL vector of the last timed step as DIR/lnl.npy (float64).  Every input
+(networks, mock observation, live points) comes from fixed seeds and the CPU oracle, never from the build
+being measured, so two builds run with the same arguments can be compared file by file.
 
 One "step" = one pass of the whole hot path (emulator MLP -> broadening tail -> chi2) over a
 batch of B synthetic live points of config C2 (SURVEY.md §8d: LinNet 4-256-256-256-14172,
@@ -183,21 +187,27 @@ class ClockSampler(threading.Thread):
 
 
 # --------------------------------------------------------------------------- config
-def build_c2_on_gpu(precision):
-    """C2 with the mock observation generated by the CUDA path itself (no oracle involved)."""
-    import torch
+def build_c2():
+    """C2 with the mock observation from the CPU oracle: the inputs do not depend on the build being measured."""
+    from oracle import payne_oracle as O
     from thepayne_b200 import synth
-    from thepayne_b200.engine import engine_from_config
+    return synth.config_c2(O.model_fn)
 
-    def model_fn(cfg, theta):
-        n = len(cfg.obs_wave)
-        cfg.obs_flux, cfg.obs_eflux = np.ones(n), np.ones(n)
-        eng = engine_from_config(cfg, precision=precision)
-        fl, mg, _ = eng.model_batch(torch.from_numpy(np.ascontiguousarray(theta)).cuda())
-        out = (fl.cpu().numpy(), None if mg is None else mg.cpu().numpy())
-        eng.close()
-        return out
-    return synth.config_c2(model_fn)
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write every array as <path>/<name>.npy in float64, DUMP_MAX_BYTES at most in all.  An array over its share is
+    replaced by a fixed sample of its elements (seed 0, in index order): the same positions for every run of the
+    same shape."""
+    os.makedirs(path, exist_ok=True)
+    keep = DUMP_MAX_BYTES // max(1, len(arrays)) // 8
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.size > keep:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def bench_config(B, D_out, n_obs):
@@ -267,10 +277,8 @@ def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    from oracle import payne_oracle as O
-    from thepayne_b200 import synth
     kind = reference_kind()
-    cfg = synth.config_c2(O.model_fn)
+    cfg = build_c2()
     cores = os.cpu_count() or 1
     pool = CpuPool(cfg, cores, kind)
     B = args.batch
@@ -289,9 +297,11 @@ def run_reference(args):
         pool.run(theta[:S])
     tot = 0.0
     for i in range(args.steps):
-        _, dt = pool.run(theta[:S])
+        lnl, dt = pool.run(theta[:S])
         tot += dt
     pool.close()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'lnl': lnl})
     v = S * args.steps / tot
     sample = ('%d of the %d points per step x %d steps, scalar lnlikefn per point, %d procs x 1 thread; '
               'implementation: %s' % (S, B, args.steps, cores,
@@ -320,7 +330,12 @@ def run_ours(args):
         os.environ.setdefault('MASTER_ADDR', '127.0.0.1')
         dist.init_process_group('nccl', device_id=torch.device('cuda', local))
     B, K, W = args.batch, args.steps, args.warmup
-    cfg = build_c2_on_gpu(args.precision)
+    cfg = build_c2()
+    # A throw-away engine evaluates the truth once before the timed engine is made.  Without it the timed engine, then
+    # the first on the device, ran 0.2 % slower per step (one B200 at 1000 W: 0.8551 against 0.8534 ms, alternated runs).
+    warm = engine_from_config(cfg, precision=args.precision)
+    warm.model_batch(torch.from_numpy(np.ascontiguousarray(cfg.theta_true[None, :])).cuda())
+    warm.close()
     eng = engine_from_config(cfg, precision=args.precision)
     eng.set('max_batch', args.slab)
     theta_h = np.ascontiguousarray(cfg.draw(B, seed=1234 + rank))    # rank 0: the reference arm's batch
@@ -405,6 +420,8 @@ def run_ours(args):
                    'sm_mhz': [float(a[1].item()) for a in allr]}
         ms = max(float(a[0].item()) for a in allr)
     n_finite = int(torch.isfinite(out).sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'lnl': out.cpu().numpy()})
 
     # per-kernel device time (CUDA events on the launching stream inside the library)
     eng.set('timing', 1)
@@ -605,7 +622,10 @@ def main():
     ap.add_argument('--cpu-seconds', type=float, default=12.0)
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-extra', action='store_true', help='skip the C3/C4/C5 extra lines')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the lnL of the last timed step to DIR/lnl.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

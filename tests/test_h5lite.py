@@ -6,8 +6,6 @@ import pytest
 
 from thepayne_b200 import annio, h5lite, synth
 
-REF_DEMO = '/root/reference/demo/demodata.h5'
-
 
 def _sample():
     rng = np.random.default_rng(3)
@@ -49,19 +47,6 @@ def test_rejects_what_it_cannot_read(tmp_path):
     p.write_bytes(bytes(good))
     with pytest.raises(IOError, match='superblock version 2'):
         h5lite.read(str(p))
-
-
-@pytest.mark.skipif(not os.path.exists(REF_DEMO), reason='reference tree not mounted')
-def test_reads_a_file_written_by_h5py():
-    """demo/demodata.h5 ships with the reference and was written by h5py/libhdf5."""
-    d = h5lite.read(REF_DEMO)
-    assert sorted(d) == ['phot/filter', 'phot/phot', 'spec/flux', 'spec/wave']
-    w, f = d['spec/wave'], d['spec/flux']
-    assert w.dtype == np.float64 and w.shape == f.shape == (25600,)
-    assert np.all(np.diff(w) > 0) and 5100 < w[0] < w[-1] < 5400
-    assert np.all((f > 0) & (f < 1.2))
-    assert d['phot/filter'].dtype.kind == 'S' and d['phot/filter'][0] == b'2MASS_H'
-    assert d['phot/phot'].shape == d['phot/filter'].shape
 
 
 def test_specnet_and_photnet_through_h5(tmp_path):

@@ -110,3 +110,19 @@ def test_legacy_network_containers_round_trip(tmp_path):
             assert all(np.array_equal(a, b) for a, b in zip(net.weights + net.biases, back.weights + back.biases))
             assert np.array_equal(back.wavelength, net.wavelength) and np.array_equal(back.xmax, net.xmax)
             assert annio.load_specnet(p, NNtype=nntype).D_out == net.D_out
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 .npy files; an output over the size cap becomes the same seeded sample on every
+    run, so that two builds compare the same positions."""
+    import bench
+    a = np.linspace(-5.0, 5.0, 100, dtype=np.float32)
+    bench.dump_outputs(str(tmp_path / 'a'), {'lnl': a[:10]})
+    got = np.load(tmp_path / 'a' / 'lnl.npy')
+    assert got.dtype == np.float64 and np.array_equal(got, a[:10])
+    monkeypatch.setattr(bench, 'DUMP_MAX_BYTES', 8 * 64)
+    for d in 'bc':
+        bench.dump_outputs(str(tmp_path / d), {'lnl': a, 'flux': a})
+    b = [np.load(tmp_path / 'b' / n) for n in ('lnl.npy', 'flux.npy')]
+    assert all(x.size == 32 for x in b) and np.all(np.diff(b[0]) > 0) and np.isin(b[0], a).all()
+    assert np.array_equal(b[0], np.load(tmp_path / 'c' / 'lnl.npy'))

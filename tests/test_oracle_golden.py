@@ -8,6 +8,18 @@ from conftest import load_case
 from oracle import goldens, payne_oracle as O
 
 
+@pytest.fixture(autouse=True, scope='module')
+def _minting_threads():
+    """The fixtures were minted with torch on 8 CPU threads of an AVX-512 host, and MKL's fp32 sgemm sums in an order
+    that follows the thread count: pinned to 8, the oracle's emulator reproduces them bit for bit on AVX-512 hosts of
+    any core count (16 threads differ by up to 1.5e-8 relative in flux, beyond the 1e-9 checked here)."""
+    import torch
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.mark.parametrize('name', list(goldens.CASES))
 def test_oracle_matches_reference(name):
     cfg, g = load_case(name)
