@@ -224,6 +224,12 @@ int payne_ctx_set(PayneCtx* ctx, const char* key, int64_t value);
 int payne_gemm_test(const float* A_host, const float* W_host, const float* bias_host, int M, int N, int K,
                     int precision, int device, float* C_host);
 
+/* Kernel unit-test hook: y = irfft(rfft(x) * H) through the runtime-planned shared-memory FFT convolution of
+ * the fused tails (csrc/fft.cuh), one CTA.  x, y: N = 2^log2N real samples, log2N in [5, 15]; H: the N/2 + 1
+ * real transfer-function values at frequencies 0 .. N/2 (the hook applies the 1/(N/2) of the inverse).
+ * HOST buffers in and out.  Synchronous. */
+int payne_fft_test(const float* x_host, int log2N, const float* H_host, int device, float* y_host);
+
 /* Per-kernel device time of the most recent payne_lnlike_batch call on this context,
  * measured with CUDA events on the launching stream when timing is enabled
  * (payne_ctx_set(ctx,"timing",1)).  which: 0 = emulator GEMM stages, 1 = fused tail,

@@ -23,7 +23,7 @@ PREC = {'parity': 0, 'x3': 0, 'tf32': 1, 'bf16': 2, 'simt': 3, 'fp32': 3, '3xtf3
 
 EXPORTS = ['payne_abi_version', 'payne_last_error', 'payne_ctx_create', 'payne_ctx_destroy',
            'payne_lnlike_batch', 'payne_lnlike_batch_host', 'payne_model_batch', 'payne_ann_eval',
-           'payne_ctx_query', 'payne_ctx_set', 'payne_ctx_last_ms', 'payne_gemm_test',
+           'payne_ctx_query', 'payne_ctx_set', 'payne_ctx_last_ms', 'payne_gemm_test', 'payne_fft_test',
            'payne_ctx_attach_continuum', 'payne_ctx_set_lsf',
            'payne_gather_create', 'payne_gather_connect', 'payne_lnlike_batch_gather', 'payne_gather_flush']
 GATHER_HANDLE_BYTES = 128
@@ -114,6 +114,8 @@ def load():
     lib.payne_ctx_last_ms.argtypes = [vp, C.c_int]
     lib.payne_gemm_test.restype = C.c_int
     lib.payne_gemm_test.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]
+    lib.payne_fft_test.restype = C.c_int
+    lib.payne_fft_test.argtypes = [vp, C.c_int, vp, C.c_int, vp]
     _lib = lib
     return lib
 

@@ -64,5 +64,8 @@ int launch_tail_general(int l2, int grid, size_t smem_bytes, cudaStream_t st, co
 bool probe_tail_lsf(size_t smem_bytes, int* ctas_per_sm);
 int launch_tail_lsf(int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const LsfParams& L);
 int launch_continuum(int grid, cudaStream_t st, const ContParams& C);
+// unit-test convolution: y = irfft(rfft(x) * H) of 2^log2N real samples (device buffers; H[0..N/2] without the
+// 1/M; tw = the N/2-entry twiddle table of the tails), one CTA on the default stream
+int launch_fft_test(const float* x, int log2N, const float* H, const float2* tw, float* y);
 
 }  // namespace payne

@@ -1373,6 +1373,32 @@ int payne_gemm_test(const float* A_host, const float* W_host, const float* bias_
   return rc;
 }
 
+int payne_fft_test(const float* x_host, int log2N, const float* H_host, int device, float* y_host) {
+  if (!x_host || !H_host || !y_host || log2N < 5 || log2N > 15) return fail(PAYNE_E_INVALID, "bad argument");
+  CU_TRY(cudaSetDevice(device));
+  const int N = 1 << log2N;
+  std::vector<float2> tw(N / 2);                       // the tails' table (build_tail) for an N-sample transform
+  for (int e = 0; e < N / 2; ++e) tw[e] = unit_round(-2.0 * 3.14159265358979323846 * (double)e / (double)N);
+  float *dx = nullptr, *dH = nullptr, *dy = nullptr;
+  float2* dtw = nullptr;
+  int rc = PAYNE_OK;
+  if (cudaMalloc((void**)&dx, (size_t)N * 4) != cudaSuccess || cudaMalloc((void**)&dy, (size_t)N * 4) != cudaSuccess ||
+      cudaMalloc((void**)&dH, (size_t)(N / 2 + 1) * 4) != cudaSuccess ||
+      cudaMalloc((void**)&dtw, (size_t)(N / 2) * sizeof(float2)) != cudaSuccess)
+    rc = fail(PAYNE_E_NOMEM, "fft_test alloc");
+  if (!rc) {
+    cudaMemcpy(dx, x_host, (size_t)N * 4, cudaMemcpyHostToDevice);
+    cudaMemcpy(dH, H_host, (size_t)(N / 2 + 1) * 4, cudaMemcpyHostToDevice);
+    cudaMemcpy(dtw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice);
+    rc = payne::launch_fft_test(dx, log2N, dH, dtw, dy);
+    if (rc) fail(rc, "fft_test launch failed");
+    if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(PAYNE_E_CUDA, cudaGetErrorString(cudaGetLastError()));
+    if (!rc) cudaMemcpy(y_host, dy, (size_t)N * 4, cudaMemcpyDeviceToHost);
+  }
+  if (dx) cudaFree(dx); if (dy) cudaFree(dy); if (dH) cudaFree(dH); if (dtw) cudaFree(dtw);
+  return rc;
+}
+
 double payne_ctx_last_ms(PayneCtx* c, int which) {
   if (!c || which < 0 || which > 2 || !c->timing) return -1.0;
   if (!c->ms_valid) {

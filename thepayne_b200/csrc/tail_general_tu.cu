@@ -1,5 +1,6 @@
 // Translation unit of the general-grid fused tail (tail_general.cuh), the LSF-vector tail (tail_lsf.cuh) and
-// the continuum-emulator multiply (continuum.cuh); see launchers.h.
+// the continuum-emulator multiply (continuum.cuh) and the unit-test hook of the runtime-planned FFT (fft.cuh);
+// see launchers.h.
 #include "launchers.h"
 
 namespace payne {
@@ -48,6 +49,41 @@ int launch_tail_lsf(int grid, size_t smem, cudaStream_t st, const TailParams& T,
 
 int launch_continuum(int grid, cudaStream_t st, const ContParams& C) {
   continuum_kernel<0><<<grid, 256, 0, st>>>(C);
+  return cudaGetLastError() == cudaSuccess ? PAYNE_OK : PAYNE_E_CUDA;
+}
+
+// The runtime-planned convolution of fft.cuh on its own (payne_fft_test): one CTA packs x into the swizzled
+// complex layout the tails use, runs forward -> filter -> inverse and unpacks the result in natural order.
+struct TableH {
+  const float* h;
+  float invM;
+  __device__ __forceinline__ float operator()(int k) const { return __ldg(h + k) * invM; }
+};
+
+__global__ void __launch_bounds__(kNT) fft_test_kernel(const float* __restrict__ x, int log2N,
+                                                       const float* __restrict__ H, const float2* __restrict__ tw,
+                                                       float* __restrict__ y) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float2* z = reinterpret_cast<float2*>(smem_raw);
+  const int tid = threadIdx.x, log2M = log2N - 1, M = 1 << log2M;
+  for (int m = tid; m < M; m += kNT) z[swz(m)] = make_float2(x[2 * m], x[2 * m + 1]);
+  __syncthreads();
+  const Twiddles twr{tw, log2N};
+  FftPlan plan; plan.make(log2M);
+  fft_forward(z, log2M, plan, twr, tid, kNT);
+  filter_pairs(z, log2M, plan, twr, TableH{H, 1.0f / (float)M}, tid, kNT);
+  fft_inverse(z, log2M, plan, twr, tid, kNT);
+  for (int m = tid; m < M; m += kNT) {
+    const float2 v = z[swz(m)];
+    y[2 * m] = v.x; y[2 * m + 1] = v.y;
+  }
+}
+
+int launch_fft_test(const float* x, int log2N, const float* H, const float2* tw, float* y) {
+  const size_t smem = (size_t)4 << log2N;              // N/2 complex points of 8 bytes
+  if (cudaFuncSetAttribute(fft_test_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+    return PAYNE_E_CUDA;
+  fft_test_kernel<<<1, kNT, smem>>>(x, log2N, H, tw, y);
   return cudaGetLastError() == cudaSuccess ? PAYNE_OK : PAYNE_E_CUDA;
 }
 
