@@ -212,8 +212,13 @@ inline int tc_launch_hidden_stack(const TcWeights* tcw, float* const* bias, int 
     if (tcw[1 + l].N != H || tcw[1 + l].K != H || !tcw[1 + l].xplane[0]) return PAYNE_E_UNSUPPORTED;
   TcStackCache& C = *cache;
   const long long rows = a0->rows >= M ? a0->rows : M;
-  const bool hit = C.valid && C.a0 == a0->plane[0] && C.a1 == a1->plane[0] && C.w0 == tcw[1].xplane[0] && C.rows == rows &&
-                   C.lda == a0->ld && C.H == H && C.layers == layers;
+  const void* key[6 + 3 * kStackMaxLayers] = {};
+  for (int p = 0; p < 3; ++p) {
+    key[p] = a0->plane[p]; key[3 + p] = a1->plane[p];
+    for (int l = 0; l < layers; ++l) key[6 + 3 * l + p] = tcw[1 + l].xplane[p];
+  }
+  bool hit = C.valid && C.rows == rows && C.lda == a0->ld && C.H == H && C.layers == layers;
+  for (int i = 0; i < 6 + 3 * kStackMaxLayers && hit; ++i) hit = C.ptr[i] == key[i];
   if (!hit) {
     C.valid = false;
     for (int p = 0; p < 3; ++p) {
@@ -224,7 +229,8 @@ inline int tc_launch_hidden_stack(const TcWeights* tcw, float* const* bias, int 
         if (make_tmap(&C.maps.b[l][p], W.xplane[p], W.N, H, W.Kp, 64, 2)) return PAYNE_E_CUDA;
       }
     }
-    C.a0 = a0->plane[0]; C.a1 = a1->plane[0]; C.w0 = tcw[1].xplane[0]; C.rows = rows; C.lda = a0->ld; C.H = H; C.layers = layers;
+    for (int i = 0; i < 6 + 3 * kStackMaxLayers; ++i) C.ptr[i] = key[i];
+    C.rows = rows; C.lda = a0->ld; C.H = H; C.layers = layers;
     C.valid = true;
   }
   static unsigned long long attr_set = 0;

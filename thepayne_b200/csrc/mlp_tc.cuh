@@ -792,8 +792,8 @@ inline void tc_free_acts(TcActs* a) {
 // loads half of the weight tile and TMA-multicasts it to both).  Measured on B200 (C2, B=4096) it
 // removes 25 % of the L2 reads and changes the time by < 1 %: the kernel was never short of operand
 // bandwidth -- ncu's source view put ~75 % of its instructions in the old row-loop epilogue, and the
-// TMA-store epilogue (not multicast) is what lifted the tensor pipe from 40 % to 73 %.  Kept, tested,
-// off by default.
+// TMA-store epilogue (not multicast) is what lifted the tensor pipe from 40 % to 73 %.  Kept, off by
+// default; bit-identical to the default path (tests/test_gpu_emulator_shapes.py runs it in a subprocess).
 inline bool tc_multicast_enabled() {
   static int v = -1;
   if (v < 0) { const char* e = getenv("PAYNE_GEMM_MULTICAST"); v = (e && e[0] == '1') ? 1 : 0; }
@@ -827,8 +827,10 @@ inline int tc_launch_impl(const TcActs& A, int K, const TcWeights& W, const floa
   const long long mrows = grouped ? grp->groups * grp->a_grows : ((cache && map_rows >= M) ? map_rows : M);
   TcMaps local;
   TcMaps& T = cache ? cache->maps : local;
-  const bool hit = cache && cache->variant == kVariant && cache->a0 == A.plane[0] && cache->out == out0 &&
-                   cache->rows == mrows && cache->lda == A.ld && cache->ldc == ldc;
+  const void* key[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, out0};
+  for (int p = 0; p < Cfg::kPlanes; ++p) { key[p] = A.plane[p]; key[3 + p] = MODE == kModeX3 ? W.xplane[p] : W.plane[p]; }
+  bool hit = cache && cache->variant == kVariant && cache->rows == mrows && cache->lda == A.ld && cache->ldc == ldc;
+  for (int i = 0; i < 7 && hit; ++i) hit = cache->ptr[i] == key[i];
   if (!hit) {
     if (cache) cache->variant = -1;
     for (int p = 0; p < Cfg::kPlanes; ++p) {
@@ -842,7 +844,8 @@ inline int tc_launch_impl(const TcActs& A, int K, const TcWeights& W, const floa
       if (int rc = make_tmap_out(&T.c, out0, orows, out_cols > 0 ? out_cols : W.N, ldc)) return rc;
     } else T.c = T.a[0];
     if (cache) {
-      cache->a0 = A.plane[0]; cache->out = out0; cache->rows = mrows; cache->lda = A.ld; cache->ldc = ldc;
+      for (int i = 0; i < 7; ++i) cache->ptr[i] = key[i];
+      cache->rows = mrows; cache->lda = A.ld; cache->ldc = ldc;
       cache->variant = kVariant;
     }
   }

@@ -31,9 +31,11 @@ struct TcMaps {
 // the driver costs several microseconds of host time per launch, which is what bounds the latency
 // of small batches.  The maps cover `rows` (the allocated row count), not the batch: rows past the
 // batch are computed on stale data and land in workspace rows nobody reads.
+// The key holds every pointer the maps encode: a workspace that grows frees and reallocates all activation planes, and
+// the allocator may hand one of them back at its old address while the others move.
 struct TcMapCache {
   TcMaps maps;
-  const void* a0 = nullptr; const void* out = nullptr;
+  const void* ptr[7] = {};   // A planes 0-2, weight planes 0-2, output (unused planes of the mode: null)
   long long rows = 0, lda = 0, ldc = 0;
   int variant = -1;
 };
@@ -54,7 +56,7 @@ struct TcStackArgs {
 };
 struct TcStackCache {
   TcStackMaps maps;
-  const void* a0 = nullptr; const void* a1 = nullptr; const void* w0 = nullptr;
+  const void* ptr[6 + 3 * kStackMaxLayers] = {};   // every plane the maps encode (both buffers, every layer's weights)
   long long rows = 0, lda = 0;
   int H = 0, layers = 0;
   bool valid = false;
