@@ -21,6 +21,9 @@
  *                                                          Payne/predict/predictspec.py:96-102,122-134,208-226
  *   payne_ctx_set_lsf       getspec(inst_R=<vector>)       Payne/predict/predictspec.py:265-286 ->
  *                           smoothspec(smoothtype='lsf')   Payne/utils/smoothing.py:126-150,482-586
+ *   payne_ctx_create_stars, payne_*_stars   one context for the observations of many stars that share the
+ *                           emulators and the parameter layout (likelihood.__init__ per star; a survey fits
+ *                           thousands of stars with one emulator): every point of a batch names its star.
  *
  * Conventions: plain pointers and sizes only; every function returns 0 on success or a
  * negative PAYNE_E_* code and never throws; payne_last_error() gives the message of the
@@ -44,7 +47,7 @@
 extern "C" {
 #endif
 
-#define PAYNE_ABI_VERSION 5
+#define PAYNE_ABI_VERSION 6
 
 enum {
   PAYNE_OK = 0,
@@ -143,23 +146,46 @@ typedef struct PayneCtx PayneCtx;
 int payne_abi_version(void);
 const char* payne_last_error(void);
 
-/* spec / phot may be NULL when the corresponding runbool is 0. device = CUDA ordinal. */
+/* spec / phot may be NULL when the corresponding runbool is 0. device = CUDA ordinal.
+ * Same as payne_ctx_create_stars(spec, phot, obs, 1, layout, device, out). */
 int payne_ctx_create(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs,
                      const PayneLayout* layout, int device, PayneCtx** out);
+
+/* Observation set: obs is an array of n_stars PayneObs, HOST pointers, copied.  Every star must have the same nb
+ * (= phot->nb when phot_bool).  Star k keeps its own n_obs, wavelength range, sort order and Chebyshev
+ * normalisation (polycalc on its own wave, fitutils.py:13-14).  The emulators, the parameter layout and every table
+ * built from the emulator grid are shared.  A single-star context is the case n_stars = 1.
+ * On a context of several stars, payne_ctx_set_lsf (the LSF vector is per observed pixel) and payne_gather_create
+ * (the fused all-gather has no star argument) return PAYNE_E_UNSUPPORTED; payne_ctx_attach_continuum works. */
+int payne_ctx_create_stars(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs,
+                           int32_t n_stars, const PayneLayout* layout, int device, PayneCtx** out);
 void payne_ctx_destroy(PayneCtx* ctx);
 
-/* theta_dev: [B, ld] fp64 row-major on the device.  lnl_dev: [B] fp64. */
+/* theta_dev: [B, ld] fp64 row-major on the device.  lnl_dev: [B] fp64.
+ * star_dev: [B] int32 on the device, the star of every row of theta; NULL = star 0 for every row, which a context of
+ * several stars refuses (PAYNE_E_INVALID).  A row whose star lies outside [0, n_stars) cannot be checked without a
+ * synchronise: it gets lnL NaN, no model row and sets status bit 2; the other rows are not affected.
+ * payne_lnlike_batch = payne_lnlike_batch_stars with star_dev = NULL. */
 int payne_lnlike_batch(PayneCtx* ctx, const double* theta_dev, int64_t B, int64_t ld,
                        double* lnl_dev, void* stream);
+int payne_lnlike_batch_stars(PayneCtx* ctx, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                             double* lnl_dev, void* stream);
 
-/* Same with HOST buffers: copies theta in, runs, copies lnL out, synchronises. */
+/* Same with HOST buffers: copies theta (and star) in, runs, copies lnL out, synchronises.  A star index outside
+ * [0, n_stars) returns PAYNE_E_INVALID before anything is launched or written. */
 int payne_lnlike_batch_host(PayneCtx* ctx, const double* theta_host, int64_t B, int64_t ld,
                             double* lnl_host);
+int payne_lnlike_batch_stars_host(PayneCtx* ctx, const double* theta_host, const int32_t* star_host, int64_t B,
+                                  int64_t ld, double* lnl_host);
 
 /* Model spectrum on the observed grid and magnitudes; either output may be NULL.
- * flux_dev: [B, n_obs] fp64, mags_dev: [B, nb] fp64, lnl_dev: [B] fp64 or NULL. */
+ * flux_dev: [B, n_obs] fp64, mags_dev: [B, nb] fp64, lnl_dev: [B] fp64 or NULL.
+ * _stars: flux_dev: [B, ld_flux], ld_flux >= the largest n_obs; row p gets the first n_obs[star[p]] entries, the
+ * rest are not written.  payne_model_batch = payne_model_batch_stars with star_dev = NULL, ld_flux = n_obs. */
 int payne_model_batch(PayneCtx* ctx, const double* theta_dev, int64_t B, int64_t ld,
                       double* flux_dev, double* mags_dev, double* lnl_dev, void* stream);
+int payne_model_batch_stars(PayneCtx* ctx, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                            double* flux_dev, int64_t ld_flux, double* mags_dev, double* lnl_dev, void* stream);
 
 /* Continuum emulator (HOST pointers, copied): any PayneSpecNet the spectrum emulator could be; its
  * `wavelength` is the continuum's own grid.  From then on every model spectrum is multiplied, right after
@@ -202,10 +228,12 @@ int payne_lnlike_batch_gather(PayneCtx* ctx, const double* theta_dev, int64_t B,
                               double** gathered_prev);
 int payne_gather_flush(PayneCtx* ctx, void* stream, double** gathered_last);
 
-/* Introspection for benches/tests: key is one of "n_ann","n_obs","nfft1","launches",
+/* Introspection for benches/tests: key is one of "n_ann","n_obs" (the largest star's),"n_stars","n_obs_total"
+ * (observed pixels of all stars),"nfft1","launches",
  * "grid_loguniform","fast_tail","max_batch","sm_count","tail_grid","precision","continuum","lsf","legacy_tc"
  * (a leaky-ReLU stack whose output layer runs on the tensor cores),"status"
- * (bit0: a point needed a larger transform than the shared-memory carve-out; bit1: a peer of the gather never arrived).
+ * (bit0: a point needed a larger transform than the shared-memory carve-out; bit1: a peer of the gather never arrived;
+ * bit2: a point named a star outside [0, n_stars)).
  * Returns the value or -1. */
 int64_t payne_ctx_query(PayneCtx* ctx, const char* key);
 /* Runtime switches: "precision" (PAYNE_PREC_*), "max_batch" (workspace slab, points), "timing" (0/1,

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PAYNE_LIB_PATH: development override (an instrumented build of the same sources)
 LIB_PATH = os.environ.get('PAYNE_LIB_PATH') or os.path.join(HERE, 'libpayne_b200.so')
 
-ABI_VERSION = 5          # PAYNE_ABI_VERSION of include/payne_b200.h the ctypes structs below mirror
+ABI_VERSION = 6          # PAYNE_ABI_VERSION of include/payne_b200.h the ctypes structs below mirror
 NPAR = 13
 MAX_POLY = 16
 PAR_INDEX = {
@@ -25,7 +25,9 @@ EXPORTS = ['payne_abi_version', 'payne_last_error', 'payne_ctx_create', 'payne_c
            'payne_lnlike_batch', 'payne_lnlike_batch_host', 'payne_model_batch', 'payne_ann_eval',
            'payne_ctx_query', 'payne_ctx_set', 'payne_ctx_last_ms', 'payne_gemm_test', 'payne_fft_test',
            'payne_ctx_attach_continuum', 'payne_ctx_set_lsf',
-           'payne_gather_create', 'payne_gather_connect', 'payne_lnlike_batch_gather', 'payne_gather_flush']
+           'payne_gather_create', 'payne_gather_connect', 'payne_lnlike_batch_gather', 'payne_gather_flush',
+           'payne_ctx_create_stars', 'payne_lnlike_batch_stars', 'payne_lnlike_batch_stars_host',
+           'payne_model_batch_stars']
 GATHER_HANDLE_BYTES = 128
 
 _f = C.POINTER(C.c_float)
@@ -84,6 +86,15 @@ def load():
     lib.payne_ctx_create.restype = C.c_int
     lib.payne_ctx_create.argtypes = [C.POINTER(PayneSpecNet), C.POINTER(PaynePhotNet), C.POINTER(PayneObs),
                                      C.POINTER(PayneLayout), C.c_int, C.POINTER(vp)]
+    lib.payne_ctx_create_stars.restype = C.c_int
+    lib.payne_ctx_create_stars.argtypes = [C.POINTER(PayneSpecNet), C.POINTER(PaynePhotNet), C.POINTER(PayneObs),
+                                           C.c_int32, C.POINTER(PayneLayout), C.c_int, C.POINTER(vp)]
+    lib.payne_lnlike_batch_stars.restype = C.c_int
+    lib.payne_lnlike_batch_stars.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, vp]
+    lib.payne_lnlike_batch_stars_host.restype = C.c_int
+    lib.payne_lnlike_batch_stars_host.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp]
+    lib.payne_model_batch_stars.restype = C.c_int
+    lib.payne_model_batch_stars.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, vp, vp]
     lib.payne_ctx_destroy.restype = None
     lib.payne_ctx_destroy.argtypes = [vp]
     lib.payne_lnlike_batch.restype = C.c_int

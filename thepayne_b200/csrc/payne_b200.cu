@@ -165,6 +165,11 @@ struct PayneCtx {
   payne::LsfParams lsf{};
   size_t lsf_smem = 0;
   int lsf_grid = 0;
+  // observation set: n_stars observations back to back in the tail's and photometry's arrays (obs_star.cuh)
+  int n_stars = 1, n_obs_max = 0;
+  long long n_obs_total = 0;
+  std::vector<payne::ObsStar> stars;    // host copy of the records
+  payne::ObsStar* stars_dev = nullptr;
   // photometry
   bool has_phot = false;
   payne::PhotParams phot{};
@@ -193,6 +198,8 @@ struct PayneCtx {
   long long stage_cap = 0, stage_ld = 0;
   double *theta_pin = nullptr, *lnl_pin = nullptr, *theta_stage = nullptr, *lnl_stage = nullptr;
   double* lnl_map = nullptr;       // device view of lnl_pin (zero-copy result: the tail writes lnL straight to the host)
+  long long star_cap = 0;
+  int *star_pin = nullptr, *star_stage = nullptr;   // star indices of the *_stars_host entry
   // device allocations to free
   std::vector<void*> owned;
   // timing
@@ -234,6 +241,36 @@ int upload_owned(PayneCtx* c, T** dst, const T* src, size_t n) {
   int rc = upload(dst, src, n);
   if (rc == PAYNE_OK && *dst) c->owned.push_back((void*)*dst);
   return rc;
+}
+
+// One star's observation (fitargs of likelihood.py:84-112) appended to the context's concatenated arrays, and its
+// record: pixel offset and count, wavelength range, sort order.  The Chebyshev abscissa is normalised on the
+// star's own grid (polycalc, fitutils.py:13-14).
+struct ObsArrays {
+  std::vector<double> w, lnw, ot, inv_s, x;   // wavelength, ln wavelength, flux / eflux, 1 / eflux, Chebyshev abscissa
+  std::vector<double> q, otm1;                // fast tail: grid position (ln w - ln w_0) / dlnw, (flux - 1) / eflux
+};
+int append_star_obs(const PayneObs* obs, double lnw0, double inv_dlnw, ObsArrays& A, payne::ObsStar* rec) {
+  const int no = obs->n_obs;
+  if (no < 1) return fail(PAYNE_E_INVALID, "n_obs must be >= 1");
+  if (!obs->wave || !obs->flux || !obs->eflux) return fail(PAYNE_E_INVALID, "null observation array");
+  const double* ow = obs->wave;
+  const double omin = *std::min_element(ow, ow + no);
+  const double omax = *std::max_element(ow, ow + no);
+  rec->off = (int)A.w.size(); rec->n_obs = no; rec->obs_min = omin; rec->obs_max = omax; rec->sorted = 1;
+  for (int j = 0; j < no; ++j) {
+    const double lnw = std::log(ow[j]);
+    A.w.push_back(ow[j]);
+    A.lnw.push_back(lnw);
+    A.ot.push_back(obs->flux[j] / obs->eflux[j]);
+    A.inv_s.push_back(1.0 / obs->eflux[j]);
+    const double x = ow[j] - omin;                     // fitutils.py:13-14
+    A.x.push_back(2.0 * (x / (omax - omin)) - 1.0);
+    A.q.push_back((lnw - lnw0) * inv_dlnw);
+    A.otm1.push_back((obs->flux[j] - 1.0) / obs->eflux[j]);
+    if (!std::isfinite(ow[j]) || (j > 0 && ow[j] < ow[j - 1])) rec->sorted = 0;
+  }
+  return PAYNE_OK;
 }
 
 // Per-dataset tables of the fused tail: emulator grid, stage-1 regrid tables, rotation-kernel table,
@@ -355,27 +392,29 @@ int build_tail(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs) {
   c->tail_smem = l2 >= 16 ? (size_t)2 * N1 : (size_t)4 * N1;
   if (l2 > 16) return fail(PAYNE_E_UNSUPPORTED, "emulator grids above 65536 pixels are not supported");
 
-  // ---- observation
-  const int no = obs->n_obs;
-  if (no < 1) return fail(PAYNE_E_INVALID, "n_obs must be >= 1");
-  std::vector<double> ow(obs->wave, obs->wave + no), lnw(no), ot(no), inv_s(no), ox(no);
-  const double omin = *std::min_element(ow.begin(), ow.end());
-  const double omax = *std::max_element(ow.begin(), ow.end());
-  for (int j = 0; j < no; ++j) {
-    lnw[j] = std::log(ow[j]);
-    inv_s[j] = 1.0 / obs->eflux[j];
-    ot[j] = obs->flux[j] / obs->eflux[j];
-    const double x = ow[j] - omin;                     // fitutils.py:13-14
-    ox[j] = 2.0 * (x / (omax - omin)) - 1.0;
+  // ---- observation: every star's arrays back to back, one record per star
+  {
+    FastGrid& F = c->fast;
+    const double dlnw = (std::log(w[n - 1]) - std::log(w[0])) / (double)(n - 1);
+    F.dlnw = dlnw; F.inv_dlnw = 1.0 / dlnw;
   }
+  ObsArrays A;
+  for (int k = 0; k < c->n_stars; ++k) {
+    rc = append_star_obs(&obs[k], T.lnw0, c->fast.inv_dlnw, A, &c->stars[k]);
+    if (rc) return rc;
+    c->n_obs_max = std::max(c->n_obs_max, obs[k].n_obs);
+  }
+  const size_t no = A.w.size();
+  if (no > (size_t)std::numeric_limits<int>::max()) return fail(PAYNE_E_INVALID, "more than 2^31 - 1 observed pixels in all");
+  c->n_obs_total = (long long)no;
   double *d1, *d2, *d3, *d4, *d5;
-  rc = upload_owned(c, &d1, ow.data(), no); if (rc) return rc;
-  rc = upload_owned(c, &d2, lnw.data(), no); if (rc) return rc;
-  rc = upload_owned(c, &d3, ot.data(), no); if (rc) return rc;
-  rc = upload_owned(c, &d4, inv_s.data(), no); if (rc) return rc;
-  rc = upload_owned(c, &d5, ox.data(), no); if (rc) return rc;
-  T.n_obs = no; T.obs_w = d1; T.obs_lnw = d2; T.obs_ot = d3; T.obs_inv_s = d4; T.obs_x = d5;
-  T.obs_min = omin; T.obs_max = omax;
+  rc = upload_owned(c, &d1, A.w.data(), no); if (rc) return rc;
+  rc = upload_owned(c, &d2, A.lnw.data(), no); if (rc) return rc;
+  rc = upload_owned(c, &d3, A.ot.data(), no); if (rc) return rc;
+  rc = upload_owned(c, &d4, A.inv_s.data(), no); if (rc) return rc;
+  rc = upload_owned(c, &d5, A.x.data(), no); if (rc) return rc;
+  T.n_obs = obs[0].n_obs; T.obs_w = d1; T.obs_lnw = d2; T.obs_ot = d3; T.obs_inv_s = d4; T.obs_x = d5;
+  T.obs_min = c->stars[0].obs_min; T.obs_max = c->stars[0].obs_max;
   for (int i = 0; i < PAYNE_NPAR; ++i) { T.col[i] = c->lay.col[i]; T.fixed[i] = c->lay.fixed[i]; }
   T.n_poly = c->lay.modpoly_bool ? c->lay.n_poly : 0;
   for (int i = 0; i < PAYNE_MAX_POLY; ++i) T.poly_col[i] = c->lay.poly_col[i];
@@ -386,8 +425,7 @@ int build_tail(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs) {
   // ---- analytic regrid constants for the fast tail, verified against the exact tables
   {
     FastGrid& F = c->fast;
-    const double dlnw = (std::log(w[n - 1]) - std::log(w[0])) / (double)(n - 1);
-    F.dlnw = dlnw; F.inv_dlnw = 1.0 / dlnw;
+    const double dlnw = F.dlnw;
     F.f_num = n - 1; F.f_den = N1 - 1;
     F.f_incj = (int)((2LL * kNT * F.f_num) / F.f_den);       // forward regrid walks in pairs
     F.f_incr = (int)((2LL * kNT * F.f_num) % F.f_den);
@@ -415,18 +453,11 @@ int build_tail(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs) {
       worst = std::max(worst, std::fabs(((double)k + ta) - ((double)back[i].x + (double)te)));
     }
     c->use_fast = (worst < 2e-7) && l2 >= 10 && l2 <= 16;
-    std::vector<double> oq(no), oot(no);
-    for (int j = 0; j < no; ++j) {
-      oq[j] = (lnw[j] - T.lnw0) * F.inv_dlnw;
-      oot[j] = (obs->flux[j] - 1.0) / obs->eflux[j];
-    }
     double *dq, *dot;
-    rc = upload_owned(c, &dq, oq.data(), no); if (rc) return rc;
-    rc = upload_owned(c, &dot, oot.data(), no); if (rc) return rc;
+    rc = upload_owned(c, &dq, A.q.data(), no); if (rc) return rc;
+    rc = upload_owned(c, &dot, A.otm1.data(), no); if (rc) return rc;
     F.obs_q = dq; F.obs_otm1 = dot;
-    F.obs_sorted = 1;
-    for (int j = 0; j < no; ++j)
-      if (!std::isfinite(ow[j]) || (j > 0 && ow[j] < ow[j - 1])) F.obs_sorted = 0;
+    F.obs_sorted = c->stars[0].sorted;
     for (int set = 0; set < 2; ++set)
       for (int ip = 0; ip < 4; ++ip)
         for (int q = 0; q < 16; ++q) {
@@ -617,7 +648,9 @@ int build_spec(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs, bool emu
 
 int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs) {
   using namespace payne;
-  if (p->nb != obs->nb) return fail(PAYNE_E_INVALID, "photometry net and observation disagree on nb");
+  for (int k = 0; k < c->n_stars; ++k)
+    if (p->nb != obs[k].nb)
+      return fail(PAYNE_E_INVALID, "photometry net and observation of star " + std::to_string(k) + " disagree on nb");
   const int nb = p->nb, H = p->H;
   PhotParams& P = c->phot;
   P.nb = nb; P.H = H;
@@ -636,10 +669,18 @@ int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs) {
   rc = upload_owned(c, &d6, p->b3, (size_t)nb); if (rc) return rc;
   P.w1 = d1; P.b1 = d2; P.w2t = d3; P.b2 = d4; P.w3 = d5; P.b3 = d6;
   for (int i = 0; i < 6; ++i) { P.xmin[i] = p->xmin[i]; P.xmax[i] = p->xmax[i]; }
+  // every star's magnitudes and errors back to back (star k at k * nb)
+  std::vector<double> mag, err;
+  for (int k = 0; k < c->n_stars; ++k) {
+    if (nb > 0 && (!obs[k].phot_mag || !obs[k].phot_err)) return fail(PAYNE_E_INVALID, "null photometry array");
+    mag.insert(mag.end(), obs[k].phot_mag, obs[k].phot_mag + nb);
+    err.insert(err.end(), obs[k].phot_err, obs[k].phot_err + nb);
+    c->stars[k].phot_off = k * nb;
+  }
   double *h1, *h2, *h3;
   rc = upload_owned(c, &h1, p->hiav, (size_t)nb * 5); if (rc) return rc;
-  rc = upload_owned(c, &h2, obs->phot_mag, (size_t)nb); if (rc) return rc;
-  rc = upload_owned(c, &h3, obs->phot_err, (size_t)nb); if (rc) return rc;
+  rc = upload_owned(c, &h2, mag.data(), mag.size()); if (rc) return rc;
+  rc = upload_owned(c, &h3, err.data(), err.size()); if (rc) return rc;
   P.hiav = h1; P.obs_mag = h2; P.obs_err = h3;
   for (int i = 0; i < PAYNE_NPAR; ++i) { P.col[i] = c->lay.col[i]; P.fixed[i] = c->lay.fixed[i]; }
   P.photscale = c->lay.photscale_bool;
@@ -775,11 +816,20 @@ int run_mlp(PayneCtx* c, const payne::EncodeParams& E, const double* x, long lon
 
 __global__ void gather_wait_kernel(const unsigned long long* flags, unsigned long long wait_for, int world, int* status);
 
-int run_batch(PayneCtx* c, const double* theta, long long B, long long ld, double* flux_out,
-              double* mags_out, double* lnl, cudaStream_t st) {
+// A context of several stars needs every point's star: the entries without a star array mean star 0 throughout.
+int need_star_array(const PayneCtx* c, const int32_t* star, const char* entry) {
+  if (!star && c->n_stars > 1)
+    return fail(PAYNE_E_INVALID, "this context holds " + std::to_string(c->n_stars) + " stars: pass every point's star to " + entry);
+  return PAYNE_OK;
+}
+
+// star: [B] star index of every point (null: star 0); flux_out rows are ld_flux apart
+int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, long long ld, double* flux_out,
+              long long ld_flux, double* mags_out, double* lnl, cudaStream_t st) {
   using namespace payne;
   if (B <= 0) return PAYNE_OK;
   if (ld < c->lay.ndim) return fail(PAYNE_E_INVALID, "ld < ndim");
+  if (flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
   int rc = ensure_workspace(c, B);
   if (rc) return rc;
   rc = order_after_previous(c, st);
@@ -801,7 +851,9 @@ int run_batch(PayneCtx* c, const double* theta, long long B, long long ld, doubl
       T.theta = th; T.ld = ld; T.flux = c->flux; T.ldf = c->ldf; T.B = nb;
       T.chi2_sed = c->has_phot ? c->chi2_sed : nullptr;
       T.lnl = lnl ? lnl + p0 : nullptr;
-      T.model_out = flux_out ? flux_out + p0 * T.n_obs : nullptr;
+      T.model_out = flux_out ? flux_out + p0 * ld_flux : nullptr;
+      T.ld_flux = ld_flux;
+      T.star = star ? star + p0 : nullptr;
       T.status = c->status;
       if (gather_here) {
         // all-gather fused into the tail (tail.cuh store_lnl / gather_exit): this slab's slice of every peer's buffer
@@ -851,6 +903,8 @@ int run_batch(PayneCtx* c, const double* theta, long long B, long long ld, doubl
       PhotParams P = c->phot;
       P.theta = th; P.ld = ld; P.B = nb; P.chi2_sed = c->chi2_sed;
       P.mags_out = mags_out ? mags_out + p0 * P.nb : nullptr;
+      P.star = star ? star + p0 : nullptr;
+      P.status = c->status;
       phot_kernel<<<(nb + kPhotTile - 1) / kPhotTile, kPhotThreads, c->phot_smem, st>>>(P);
       c->launches++;
     }
@@ -899,8 +953,17 @@ const char* payne_last_error(void) { return g_err.c_str(); }
 
 int payne_ctx_create(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs,
                      const PayneLayout* layout, int device, PayneCtx** out) {
+  return payne_ctx_create_stars(spec, phot, obs, 1, layout, device, out);
+}
+
+int payne_ctx_create_stars(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs, int32_t n_stars,
+                           const PayneLayout* layout, int device, PayneCtx** out) {
   if (!out || !layout || !obs) return fail(PAYNE_E_INVALID, "null argument");
   *out = nullptr;
+  if (n_stars < 1) return fail(PAYNE_E_INVALID, "n_stars must be >= 1");
+  if (layout->phot_bool)
+    for (int k = 1; k < n_stars; ++k)
+      if (obs[k].nb != obs[0].nb) return fail(PAYNE_E_INVALID, "every star must have the same nb (star " + std::to_string(k) + ")");
   if (layout->spec_bool && !spec) return fail(PAYNE_E_INVALID, "spec_bool set but no spectrum net");
   if (layout->phot_bool && !phot) return fail(PAYNE_E_INVALID, "phot_bool set but no photometry net");
   if (!layout->spec_bool && !layout->phot_bool) return fail(PAYNE_E_INVALID, "nothing to fit");
@@ -917,6 +980,8 @@ int payne_ctx_create(const PayneSpecNet* spec, const PaynePhotNet* phot, const P
   { const char* e = getenv("PAYNE_GEMM_STACK"); c->use_stack = !(e && e[0] == '0'); }
   c->device = device; c->sm_count = prop.multiProcessorCount; c->lay = *layout;
   c->has_spec = layout->spec_bool != 0; c->has_phot = layout->phot_bool != 0;
+  c->n_stars = n_stars;
+  c->stars.assign(n_stars, payne::ObsStar{});
   int rc = PAYNE_OK;
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) rc = fail(PAYNE_E_CUDA, "stream");
   if (!rc && (cudaStreamCreateWithFlags(&c->side, cudaStreamNonBlocking) != cudaSuccess ||
@@ -928,6 +993,11 @@ int payne_ctx_create(const PayneSpecNet* spec, const PaynePhotNet* phot, const P
   if (!rc) cudaMemset(c->status, 0, sizeof(int));
   if (!rc && c->has_spec) rc = build_spec(c, spec, obs);
   if (!rc && c->has_phot) rc = build_phot(c, phot, obs);
+  if (!rc) rc = upload_owned(c, &c->stars_dev, c->stars.data(), c->stars.size());
+  if (!rc) {
+    c->tail.stars = c->phot.stars = c->stars_dev;
+    c->tail.n_stars = c->phot.n_stars = n_stars;
+  }
   if (rc) { std::string keep = g_err; payne_ctx_destroy(c); g_err = keep; return rc; }
   *out = c;
   return PAYNE_OK;
@@ -943,7 +1013,8 @@ void payne_ctx_destroy(PayneCtx* c) {
   drop(c->flux); drop(c->hA); drop(c->hB); drop(c->chi2_sed); drop(c->fast.points); drop(c->rscale);
   c->fast.points = nullptr; drop(c->status);
   payne::tc_free_acts_x(&c->actA); payne::tc_free_acts_x(&c->actB);
-  drop(c->theta_stage); drop(c->lnl_stage);
+  drop(c->theta_stage); drop(c->lnl_stage); drop(c->star_stage);
+  if (c->star_pin) cudaFreeHost(c->star_pin);
   for (int r = 0; r < 16; ++r)
     if (c->g_opened[r]) { cudaIpcCloseMemHandle(c->g_peer_buf[r]); cudaIpcCloseMemHandle(c->g_peer_flag[r]); }
   drop(c->g_buf); drop(c->g_flag); drop(c->g_done);
@@ -960,28 +1031,62 @@ void payne_ctx_destroy(PayneCtx* c) {
 
 int payne_lnlike_batch(PayneCtx* c, const double* theta_dev, int64_t B, int64_t ld, double* lnl_dev,
                        void* stream) {
+  return payne_lnlike_batch_stars(c, theta_dev, nullptr, B, ld, lnl_dev, stream);
+}
+
+int payne_lnlike_batch_stars(PayneCtx* c, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                             double* lnl_dev, void* stream) {
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   if (B == 0) return PAYNE_OK;                       // an empty batch may come with null buffers
   if (!theta_dev || !lnl_dev) return fail(PAYNE_E_INVALID, "null argument");
+  int rc = need_star_array(c, star_dev, "payne_lnlike_batch_stars");
+  if (rc) return rc;
   DeviceGuard dg(c->device);
-  return run_batch(c, theta_dev, B, ld, nullptr, nullptr, lnl_dev, (cudaStream_t)stream);
+  return run_batch(c, theta_dev, star_dev, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream);
 }
 
 int payne_model_batch(PayneCtx* c, const double* theta_dev, int64_t B, int64_t ld, double* flux_dev,
                       double* mags_dev, double* lnl_dev, void* stream) {
+  return payne_model_batch_stars(c, theta_dev, nullptr, B, ld, flux_dev, c ? c->n_obs_max : 0, mags_dev, lnl_dev, stream);
+}
+
+int payne_model_batch_stars(PayneCtx* c, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                            double* flux_dev, int64_t ld_flux, double* mags_dev, double* lnl_dev, void* stream) {
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   if (B == 0) return PAYNE_OK;
   if (!theta_dev) return fail(PAYNE_E_INVALID, "null argument");
+  int rc = need_star_array(c, star_dev, "payne_model_batch_stars");
+  if (rc) return rc;
   DeviceGuard dg(c->device);
-  return run_batch(c, theta_dev, B, ld, flux_dev, mags_dev, lnl_dev, (cudaStream_t)stream);
+  return run_batch(c, theta_dev, star_dev, B, ld, flux_dev, ld_flux, mags_dev, lnl_dev, (cudaStream_t)stream);
 }
 
 int payne_lnlike_batch_host(PayneCtx* c, const double* theta_host, int64_t B, int64_t ld, double* lnl_host) {
+  return payne_lnlike_batch_stars_host(c, theta_host, nullptr, B, ld, lnl_host);
+}
+
+int payne_lnlike_batch_stars_host(PayneCtx* c, const double* theta_host, const int32_t* star_host, int64_t B, int64_t ld,
+                                  double* lnl_host) {
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   if (B == 0) return PAYNE_OK;
   if (!theta_host || !lnl_host) return fail(PAYNE_E_INVALID, "null argument");
   if (B <= 0) return PAYNE_OK;
+  int rc = need_star_array(c, star_host, "payne_lnlike_batch_stars_host");
+  if (rc) return rc;
+  if (star_host)
+    for (int64_t i = 0; i < B; ++i)
+      if (star_host[i] < 0 || star_host[i] >= c->n_stars)
+        return fail(PAYNE_E_INVALID, "star index " + std::to_string(star_host[i]) + " of point " + std::to_string(i) +
+                    " outside [0, " + std::to_string(c->n_stars) + ")");
   DeviceGuard dg(c->device);
+  if (star_host && B > c->star_cap) {
+    if (c->star_pin) cudaFreeHost(c->star_pin);
+    if (c->star_stage) cudaFree(c->star_stage);
+    c->star_pin = c->star_stage = nullptr; c->star_cap = 0;
+    CU_TRY(cudaMallocHost((void**)&c->star_pin, (size_t)B * sizeof(int)));
+    CU_TRY(cudaMalloc((void**)&c->star_stage, (size_t)B * sizeof(int)));
+    c->star_cap = B;
+  }
   if (B > c->stage_cap || ld != c->stage_ld) {
     if (c->theta_pin) cudaFreeHost(c->theta_pin);
     if (c->lnl_pin) cudaFreeHost(c->lnl_pin);
@@ -1003,7 +1108,12 @@ int payne_lnlike_batch_host(PayneCtx* c, const double* theta_host, int64_t B, in
   std::memcpy(c->theta_pin, theta_host, (size_t)B * ld * sizeof(double));
   CU_TRY(cudaMemcpyAsync(c->theta_stage, c->theta_pin, (size_t)B * ld * sizeof(double),
                          cudaMemcpyHostToDevice, c->stream));
-  int rc = run_batch(c, c->theta_stage, B, ld, nullptr, nullptr, c->lnl_map ? c->lnl_map : c->lnl_stage, c->stream);
+  if (star_host) {
+    std::memcpy(c->star_pin, star_host, (size_t)B * sizeof(int));
+    CU_TRY(cudaMemcpyAsync(c->star_stage, c->star_pin, (size_t)B * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+  }
+  rc = run_batch(c, c->theta_stage, star_host ? c->star_stage : nullptr, B, ld, nullptr, 0, nullptr,
+                 c->lnl_map ? c->lnl_map : c->lnl_stage, c->stream);
   if (rc) return rc;
   if (!c->lnl_map)
     CU_TRY(cudaMemcpyAsync(c->lnl_pin, c->lnl_stage, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost,
@@ -1088,6 +1198,7 @@ int payne_gather_create(PayneCtx* c, int world, int rank, int64_t slots, void* h
   if (!c || !handles_out) return fail(PAYNE_E_INVALID, "null argument");
   if (world < 1 || world > 16 || rank < 0 || rank >= world || slots < 1) return fail(PAYNE_E_INVALID, "bad world / rank / slots");
   if (c->g_buf) return fail(PAYNE_E_INVALID, "gather already created on this context");
+  if (c->n_stars > 1) return fail(PAYNE_E_UNSUPPORTED, "the fused all-gather has no star argument: not available on a context of several stars");
   DeviceGuard dg(c->device);
   c->g_world = world; c->g_rank = rank; c->g_slots = slots; c->g_seq = 0;
   { const char* e = getenv("PAYNE_GATHER_FUSED"); c->g_fuse = !(e && e[0] == '0'); }
@@ -1144,7 +1255,7 @@ int payne_lnlike_batch_gather(PayneCtx* c, const double* theta_dev, int64_t B, i
   c->g_active = true; c->g_fused = false;
   c->g_wait_for = (unsigned long long)s; c->g_raise_to = (unsigned long long)(s + 1);
   c->g_bufoff = (size_t)(s % 3) * per;
-  int rc = run_batch(c, theta_dev, B, ld, nullptr, nullptr, mine, st);
+  int rc = run_batch(c, theta_dev, nullptr, B, ld, nullptr, 0, nullptr, mine, st);
   c->g_active = false;
   if (rc) return rc;
   if (gathered_prev) *gathered_prev = s > 0 ? c->g_buf + (size_t)((s - 1) % 3) * per : nullptr;
@@ -1251,6 +1362,7 @@ int payne_ctx_set_lsf(PayneCtx* c, const double* lsf_host, int64_t n) {
   using namespace payne;
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   if (!c->has_spec) return fail(PAYNE_E_INVALID, "context has no spectrum emulator");
+  if (c->n_stars > 1) return fail(PAYNE_E_UNSUPPORTED, "the LSF vector is per observed pixel: not available on a context of several stars");
   DeviceGuard dg(c->device);
   CU_TRY(cudaDeviceSynchronize());
   if (!lsf_host) { c->lsf_on = false; return PAYNE_OK; }
@@ -1280,7 +1392,9 @@ int64_t payne_ctx_query(PayneCtx* c, const char* key) {
   if (!c || !key) return -1;
   std::string k(key);
   if (k == "n_ann") return c->D_out;
-  if (k == "n_obs") return c->tail.n_obs;
+  if (k == "n_obs") return c->n_obs_max;
+  if (k == "n_stars") return c->n_stars;
+  if (k == "n_obs_total") return c->n_obs_total;
   if (k == "nfft1") return c->has_spec ? (1LL << c->tail.log2N1) : 0;
   if (k == "launches") return c->launches;
   if (k == "grid_loguniform") return c->grid_loguniform;

@@ -13,6 +13,7 @@
 #include <cuda_runtime.h>
 #include <math_constants.h>
 #include "../../include/payne_b200.h"
+#include "obs_star.cuh"
 
 namespace payne {
 
@@ -24,7 +25,7 @@ struct PhotParams {
   const float *w1, *b1, *w2t, *b2, *w3, *b3;   // w2t[b][h_in][h_out] (transposed on the host)
   double xmin[6], xmax[6];
   const double* hiav;        // [nb,5]
-  const double *obs_mag, *obs_err;
+  const double *obs_mag, *obs_err;   // [n_stars, nb]
   int col[PAYNE_NPAR];
   double fixed[PAYNE_NPAR];
   int photscale;
@@ -33,6 +34,12 @@ struct PhotParams {
   double* chi2_sed;          // [B] or null
   double* mags_out;          // [B, nb] or null
   int B;
+  // observation set (obs_star.cuh): star of every point of this slab (null: star 0); a point whose star lies outside
+  // [0, n_stars) gets chi2 NaN, no magnitudes row, and status bit 2
+  const int* star;
+  const ObsStar* stars;
+  int n_stars;
+  int* status;
 };
 
 __device__ __forceinline__ double phot_par(const PhotParams& P, const double* th, int which) {
@@ -49,6 +56,7 @@ phot_kernel(const __grid_constant__ PhotParams P) {
   __shared__ double zin[kPhotTile][6];
   __shared__ double aux[kPhotTile][4];   // logt, av, rv(for hiav), scale term
   __shared__ double chi[kPhotTile];
+  __shared__ int moff[kPhotTile];        // the point's star: first of its magnitudes (-1: no such star)
   const int tid = threadIdx.x;
   const int p0 = blockIdx.x * kPhotTile;
   const double log10_tsun = log10(5770.0);
@@ -57,6 +65,9 @@ phot_kernel(const __grid_constant__ PhotParams P) {
     const int p = p0 + tid;
     chi[tid] = 0.0;
     if (p < P.B) {
+      const int k = star_of(P.star, P.n_stars, p);
+      moff[tid] = k < 0 ? -1 : P.stars[k].phot_off;
+      if (k < 0) { chi[tid] = CUDART_NAN; atomicOr(P.status, 4); }
       const double* th = P.theta + (long long)p * P.ld;
       const double teff = phot_par(P, th, PAYNE_P_TEFF);
       const double logt = log10(teff);
@@ -116,7 +127,7 @@ phot_kernel(const __grid_constant__ PhotParams P) {
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
       const int p = p0 + q;
-      if (lane == 0 && p < P.B) {
+      if (lane == 0 && p < P.B && moff[q] >= 0) {
         double BC = s + (double)__ldg(P.b3 + b);
         if (aux[q][2] != 0.0) {                                  // highred.py:19-25
           const double* c = P.hiav + b * 5;
@@ -125,7 +136,7 @@ phot_kernel(const __grid_constant__ PhotParams P) {
         }
         const double m = aux[q][3] - BC;
         if (P.mags_out) P.mags_out[(long long)p * P.nb + b] = m;
-        const double d = m - P.obs_mag[b], e = P.obs_err[b];
+        const double d = m - P.obs_mag[moff[q] + b], e = P.obs_err[moff[q] + b];
         chi[q] += (d * d) / (e * e);
       }
     }

@@ -18,6 +18,7 @@
 #pragma once
 #include <math_constants.h>
 #include "fft.cuh"
+#include "obs_star.cuh"
 #include "../../include/payne_b200.h"
 
 namespace payne {
@@ -47,7 +48,7 @@ struct TailParams {
   int log2tw;
   const float2* twpass[16]; // [log2 M] compact per-pass twiddle tables of the compile-time plans (fft_ct.cuh)
   int max_log2N;          // largest FFT the shared-memory carve-out holds
-  // observation
+  // observation: the stars' arrays back to back (obs_star.cuh); n_obs / obs_min / obs_max are star 0's
   int n_obs;
   const double* obs_w;      // [n_obs] wavelength
   const double* obs_lnw;    // [n_obs] ln wavelength
@@ -71,7 +72,7 @@ struct TailParams {
   int flux_is_depth;        // rows hold f - 1 (tensor-core path) instead of f
   const double* chi2_sed;   // [B] or null
   double* lnl;              // [B] or null
-  double* model_out;        // [B, n_obs] or null
+  double* model_out;        // [B, ld_flux] or null: row p holds the first n_obs of p's star
   int* status;              // device flag: bit0 = a point needed a larger FFT than the carve-out
   int B;
   int gauss_stencil;        // fast tail: instrumental broadening as a real-space stencil when the kernel is compact
@@ -89,6 +90,12 @@ struct TailParams {
   unsigned long long* g_flag[16];    // rank r's flag word of this rank
   unsigned long long g_raise;        // 0: this launch does not finish the step (a slab before the last one)
   int* g_done;                       // CTA counter (zero between launches)
+  // Observation set (payne_ctx_create_stars): star of every point of this slab (null: star 0) and the per-star
+  // records.  A point whose star lies outside [0, n_stars) gets lnL NaN, no model row, and status bit 2.
+  const int* star;
+  const ObsStar* stars;
+  int n_stars;
+  long long ld_flux;                 // model_out row stride
 };
 
 // lnL of point p: local result and, with the fused gather on, the copy in every peer's buffer
@@ -120,6 +127,12 @@ struct PointSetup {
   float taper_a;        // exp(-a k^2)
   float hdu;
   int do_rot, use_inst, bad, i0, i1, log2N2, clean;
+};
+
+// The point's star: observed pixels [off, off + n) of the concatenated arrays (0 pixels for an invalid star).
+// (Not in PointSetup: the fast tails' per-point record keeps the layout its kernels were tuned with.)
+struct ObsSlice {
+  int off, n;
 };
 
 __device__ __forceinline__ double get_par(const TailParams& P, const double* th, int which) {
@@ -251,7 +264,16 @@ __device__ __forceinline__ float depth_of(float v, bool is_depth, bool fill_nan)
   return is_depth ? v : v - 1.f;
 }
 
-static __device__ void tail_setup(const TailParams& P, const double* th, PointSetup& S) {
+static __device__ void tail_setup(const TailParams& P, const double* th, int p, PointSetup& S, ObsSlice& obs) {
+  const int k = star_of(P.star, P.n_stars, p);
+  if (k < 0) {                                    // no observation to compare with: NaN, nothing written
+    S.bad = 1; S.use_inst = 0; S.do_rot = 0;
+    obs.off = 0; obs.n = 0;
+    atomicOr(P.status, 4);
+    return;
+  }
+  const ObsStar& st = P.stars[k];
+  obs.off = st.off; obs.n = st.n_obs;
   const double vrot = get_par(P, th, PAYNE_P_VROT);
   const double vrad = get_par(P, th, PAYNE_P_VRAD);
   const double instR = get_par(P, th, PAYNE_P_INSTR);
@@ -273,8 +295,8 @@ static __device__ void tail_setup(const TailParams& P, const double* th, PointSe
   S.log2N2 = 0; S.i0 = 0; S.i1 = P.n - 1;
   if (!S.use_inst || S.bad) return;
   // mask_wave (smoothing.py:631-647): wlim * (1 + 20/width * [-1, 1]), strict inequalities
-  const double lo = P.obs_min * (1.0 + 20.0 / Rs * -1.0);
-  const double hi = P.obs_max * (1.0 + 20.0 / Rs * 1.0);
+  const double lo = st.obs_min * (1.0 + 20.0 / Rs * -1.0);
+  const double hi = st.obs_max * (1.0 + 20.0 / Rs * 1.0);
   const int n = P.n;
   // first index with w*D > lo
   int g0 = (int)ceil((log(lo) - S.lnD - P.lnw0) * P.inv_dlnw);

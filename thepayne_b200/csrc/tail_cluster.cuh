@@ -267,7 +267,7 @@ __device__ __forceinline__ void convolve_regrid(float2* z, uint32_t zb, unsigned
 // Observed pixels whose bracketing sample k = floor(position) lies in this CTA's quarter (pixels left of the
 // grid count for CTA 0, right of it for CTA 3: they make the residual NaN, smoothing.py:289).  Pixels
 // [jlo, jhi) are scanned; ownership is tested per pixel, so any superset of the owned pixels is correct.
-template <bool POLY, class ZV>
+template <bool POLY, bool STARS, class ZV>
 __device__ __forceinline__ double final_pass_part(const TailParams& P, const FastGrid& F, const PointSetup& S,
                                                   const FastSetup& FS, const ZV& zv, int tid, int p, int N2,
                                                   int rank, int log2nq, int jlo, int jhi) {
@@ -282,6 +282,7 @@ __device__ __forceinline__ double final_pass_part(const TailParams& P, const Fas
   const float hdu = S.hdu;
   const double q0 = FS.q0, scale = FS.scale;
   const double* __restrict__ otab = POLY ? P.obs_ot : F.obs_otm1;
+  const int off = obs_lo<STARS>(FS.obs);
   double acc = 0.0;
   constexpr int U = 4;
 #pragma unroll 1
@@ -326,7 +327,7 @@ __device__ __forceinline__ double final_pass_part(const TailParams& P, const Fas
         double m = ((okm >> u) & 1u) ? 1.0 + (double)d[u] : nan;
         if (P.n_poly) m *= cv[u];
         if ((minem >> u) & 1u) {
-          if (P.model_out) P.model_out[(long long)p * P.n_obs + j0 + u * kNT] = m;
+          if (P.model_out) P.model_out[(long long)p * P.ld_flux + (j0 + u * kNT - off)] = m;
           const double r = fma(m, is[u], -ot[u]);
           acc = fma(r, r, acc);
         }
@@ -347,7 +348,7 @@ __device__ __forceinline__ double final_pass_part(const TailParams& P, const Fas
 
 // One cluster of four CTAs owns one live point at a time.  LOG2N1 in {15, 16}; every CTA holds N1/8 complex
 // points (32 / 64 KB) plus its own copy of the rotation-table window.
-template <int LOG2N1>
+template <int LOG2N1, bool STARS>
 __global__ void __launch_bounds__(kNT, 3)
 tail_cluster_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -394,7 +395,7 @@ tail_cluster_kernel(const __grid_constant__ TailParams P, const __grid_constant_
     if (S.bad) {
       if (rank == 0) {
         if (P.model_out)
-          for (int j = tid; j < P.n_obs; j += kNT) P.model_out[(long long)p * P.n_obs + j] = nan;
+          for (int j = tid; j < obs_hi<STARS>(P, FS.obs) - obs_lo<STARS>(FS.obs); j += kNT) P.model_out[(long long)p * P.ld_flux + j] = nan;
         if (tid == 0 && P.lnl) store_lnl(P, p, nan);
       }
       cl::cluster_sync();
@@ -439,16 +440,16 @@ tail_cluster_kernel(const __grid_constant__ TailParams P, const __grid_constant_
         else
           cl::convolve_regrid<LOG2MQ - 1>(z, zb, rank, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den, FS.s_invden, F.c_native, S.clean != 0, 12);
         const cl::ZCluster zc{zf, zb, (int)rank, log2nq2};
-        int jlo = 0, jhi = P.n_obs;
-        if (F.obs_sorted) {
+        int jlo = obs_lo<STARS>(FS.obs), jhi = obs_hi<STARS>(P, FS.obs);   // the point's star
+        if (STARS ? FS.jcut[0] >= 0 : F.obs_sorted != 0) {
           if (rank > 0) jlo = FS.jcut[rank - 1];
           if (rank < cl::kCluster - 1) jhi = FS.jcut[rank];
         }
 #ifdef PAYNE_CLUSTER_PROF
         prof_t = clock64();
 #endif
-        if (P.n_poly == 0 && P.model_out == nullptr) acc = cl::final_pass_part<false>(P, F, S, FS, zc, tid, p, N2, (int)rank, log2nq2, jlo, jhi);
-        else acc = cl::final_pass_part<true>(P, F, S, FS, zc, tid, p, N2, (int)rank, log2nq2, jlo, jhi);
+        if (P.n_poly == 0 && P.model_out == nullptr) acc = cl::final_pass_part<false, STARS>(P, F, S, FS, zc, tid, p, N2, (int)rank, log2nq2, jlo, jhi);
+        else acc = cl::final_pass_part<true, STARS>(P, F, S, FS, zc, tid, p, N2, (int)rank, log2nq2, jlo, jhi);
         CL_PROF(22);
       } else if (rank == 0) {
         // small masks (N2 <= N1/4 fits one CTA's buffer): CTA 0 alone, runtime-planned transform
@@ -459,13 +460,14 @@ tail_cluster_kernel(const __grid_constant__ TailParams P, const __grid_constant_
         fft_forward(z, log2N2 - 1, plan, twr, tid, kNT);
         filter_pairs(z, log2N2 - 1, plan, twr, H, tid, kNT);
         fft_inverse(z, log2N2 - 1, plan, twr, tid, kNT);
-        acc = (P.n_poly == 0 && P.model_out == nullptr) ? final_pass<false>(P, F, S, FS, zs, tid, p, N2)
-                                                        : final_pass<true>(P, F, S, FS, zs, tid, p, N2);
+        acc = (P.n_poly == 0 && P.model_out == nullptr) ? final_pass<false, STARS>(P, F, S, FS, zs, tid, p, N2)
+                                                        : final_pass<true, STARS>(P, F, S, FS, zs, tid, p, N2);
       }
     } else {
       // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289); pixels split evenly
       const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
-      const int jlo = (int)((long long)P.n_obs * rank / cl::kCluster), jhi = (int)((long long)P.n_obs * (rank + 1) / cl::kCluster);
+      const int off = obs_lo<STARS>(FS.obs), no = obs_hi<STARS>(P, FS.obs) - off;
+      const int jlo = off + (int)((long long)no * rank / cl::kCluster), jhi = off + (int)((long long)no * (rank + 1) / cl::kCluster);
       for (int j = jlo + tid; j < jhi; j += kNT) {
         const double x = __ldg(P.obs_w + j);
         double m;
@@ -479,7 +481,7 @@ tail_cluster_kernel(const __grid_constant__ TailParams P, const __grid_constant_
           m = 1.0 + ((b - a) / (wb - wa) * (x - wa) + a);
         }
         if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-        if (P.model_out) P.model_out[(long long)p * P.n_obs + j] = m;
+        if (P.model_out) P.model_out[(long long)p * P.ld_flux + (j - off)] = m;
         const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
         acc += r * r;
       }

@@ -36,10 +36,18 @@ bool probe_tail_cluster(int l2, size_t bytes, int* ctas_per_sm, int* max_cluster
   switch (l2) {
 #define X(L)                                                                                                      \
     case L: {                                                                                                     \
-      e1 = cudaFuncSetAttribute(tail_cluster_kernel<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); \
-      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, tail_cluster_kernel<L>, kNT, bytes);        \
-      cudaLaunchConfig_t cfg = cluster_config(tail_cluster_kernel<L>, cl::kCluster, bytes, nullptr, &attr);       \
-      e3 = cudaOccupancyMaxActiveClusters(max_clusters, tail_cluster_kernel<L>, &cfg);                            \
+      e1 = cudaFuncSetAttribute(tail_cluster_kernel<L, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); \
+      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, tail_cluster_kernel<L, false>, kNT, bytes); \
+      cudaLaunchConfig_t cfg = cluster_config(tail_cluster_kernel<L, false>, cl::kCluster, bytes, nullptr, &attr); \
+      e3 = cudaOccupancyMaxActiveClusters(max_clusters, tail_cluster_kernel<L, false>, &cfg);                     \
+      if (e1 == cudaSuccess && e2 == cudaSuccess && e3 == cudaSuccess) {   /* the multi-star instantiation alike */ \
+        int o2 = 0, c2 = 0;                                                                                       \
+        e1 = cudaFuncSetAttribute(tail_cluster_kernel<L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); \
+        e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o2, tail_cluster_kernel<L, true>, kNT, bytes);        \
+        e3 = cudaOccupancyMaxActiveClusters(&c2, tail_cluster_kernel<L, true>, &cfg);                             \
+        if (o2 < *ctas_per_sm) *ctas_per_sm = o2;                                                                 \
+        if (c2 < *max_clusters) *max_clusters = c2;                                                               \
+      }                                                                                                           \
       break;                                                                                                      \
     }
     PAYNE_CLUSTER_SIZES(X)
@@ -56,8 +64,9 @@ int launch_tail_cluster(int l2, int n_clusters, size_t smem, cudaStream_t st, co
   switch (l2) {
 #define X(L)                                                                                                        \
     case L: {                                                                                                       \
-      cudaLaunchConfig_t cfg = cluster_config(tail_cluster_kernel<L>, n_clusters * cl::kCluster, smem, st, &attr);  \
-      e = cudaLaunchKernelEx(&cfg, tail_cluster_kernel<L>, T, F);                                                   \
+      cudaLaunchConfig_t cfg = cluster_config(tail_cluster_kernel<L, false>, n_clusters * cl::kCluster, smem, st, &attr); \
+      e = T.n_stars > 1 ? cudaLaunchKernelEx(&cfg, tail_cluster_kernel<L, true>, T, F)                              \
+                        : cudaLaunchKernelEx(&cfg, tail_cluster_kernel<L, false>, T, F);                            \
       break;                                                                                                        \
     }
     PAYNE_CLUSTER_SIZES(X)

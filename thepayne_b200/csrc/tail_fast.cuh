@@ -58,7 +58,8 @@ struct FastGrid {
   float* scratch;                     // [grid, N1/2] second half of split transforms (N1 = 65536)
   TwConst twc;
   // (behind twc: the constant-bank offsets of the fields above are what the single-CTA kernel was tuned with)
-  int obs_sorted;                     // observed wavelengths are non-decreasing (cluster tail: pixel ranges per CTA)
+  int obs_sorted;                     // single-star context: observed wavelengths are non-decreasing (cluster tail:
+                                      // pixel ranges per CTA; a context of several stars decides per star, jcut[0])
   int cluster;                        // the cluster tail (tail_cluster.cuh) is in use: tail_setup fills FastSetup::jcut
   // dynamic point scheduling of tail_fast_kernel: CTA b starts with point b and takes further points from this
   // counter (reset to work_start = the tail's grid size by tail_setup_kernel); null = static round robin
@@ -76,11 +77,13 @@ struct FastSetup {
       double st_inv2s2;               // 1 / (2 sigma_px^2)
     };
     // cluster tail (contexts that have it never take the stencil, st_R = 0): first observed pixel at or beyond
-    // sample (r+1) N2/4 (sorted pixels).  Shares the stencil's bytes: the record sits in static shared memory
-    // and every 16 bytes of it come out of the rotation-table window.
+    // sample (r+1) N2/4 (the star's pixels sorted; jcut[0] = -1: not sorted, every CTA scans the star's pixels).
+    // Shares the stencil's bytes: the record sits in static shared memory and every 16 bytes of it come out of
+    // the rotation-table window.
     int jcut[3];
   };
   double q0, scale;                   // final: p = (obs_q - q0) * scale
+  ObsSlice obs;                       // the point's star (fills the record's padding: sizeof(FastPoint) stays 320)
 };
 
 // Per-point setup, computed by tail_setup_kernel (one thread per point) ahead of the tail so that
@@ -221,28 +224,38 @@ __device__ __forceinline__ void regrid_back(float* row, const ZV& zv, const Fast
   }
 }
 
+// The point's observed pixels [obs_lo, obs_hi).  STARS = false: a single-star context (launch-time specialisation),
+// whose bounds are the kernel parameters' -- the per-point record is not consulted and the loops compile as they
+// did before observation sets existed (measured: reading the bounds from the record cost 0.6 % of the C2 tail).
+template <bool STARS>
+__device__ __forceinline__ int obs_lo(const ObsSlice& o) { return STARS ? o.off : 0; }
+template <bool STARS>
+__device__ __forceinline__ int obs_hi(const TailParams& P, const ObsSlice& o) { return STARS ? o.off + o.n : P.n_obs; }
+
 // Observed pixels with a continuum polynomial and / or model output (m = (1 + d) chebval(x), r = m / sigma -
 // flux / sigma; fitutils.py:11-20, likelihood.py:95-97): four pixels per trip like the plain path, loads grouped
 // (positions -> samples -> depth; then the per-pixel constants -> Clenshaw on four abscissae at once ->
 // residuals).  It lives in its own instantiation of the kernel (POLY = true): the plain path sits at its 80-register
 // cap and any code beside it changes its allocation (measured: +0.5 % with this loop behind a call).
-template <class ZV>
+template <bool STARS, class ZV>
 __device__ __forceinline__ double final_pass_poly(const TailParams& P, const FastGrid& F, const PointSetup& S,
                                                   const FastSetup& FS, const ZV& zv, int tid, int p, int N2) {
   const double nan = CUDART_NAN;
   const double pmax = (double)(N2 - 1);
   const float hdu = S.hdu;
   const double q0 = FS.q0, scale = FS.scale;
+  const int off = obs_lo<STARS>(FS.obs), jend = obs_hi<STARS>(P, FS.obs);   // the point's star: pixels [off, jend)
+  double* mrow = P.model_out ? P.model_out + (long long)p * P.ld_flux : nullptr;
   double acc = 0.0;
   constexpr int U = 4;
 #pragma unroll 1
-  for (int j0 = tid; j0 < P.n_obs; j0 += U * kNT) {
+  for (int j0 = off + tid; j0 < jend; j0 += U * kNT) {
     float d[U];
     unsigned okm = 0;
     {
       double q[U];
 #pragma unroll
-      for (int u = 0; u < U; ++u) q[u] = (j0 + u * kNT < P.n_obs) ? __ldcg(F.obs_q + j0 + u * kNT) : -1.0;
+      for (int u = 0; u < U; ++u) q[u] = (j0 + u * kNT < jend) ? __ldcg(F.obs_q + j0 + u * kNT) : -1.0;
       float g0[U], g1[U], dl[U];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
@@ -259,7 +272,7 @@ __device__ __forceinline__ double final_pass_poly(const TailParams& P, const Fas
     double is[U], ot[U], x[U], cv[U];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
-      const bool in = j0 + u * kNT < P.n_obs;
+      const bool in = j0 + u * kNT < jend;
       is[u] = in ? __ldcg(P.obs_inv_s + j0 + u * kNT) : 0.0;
       ot[u] = in ? __ldcg(P.obs_ot + j0 + u * kNT) : 0.0;
       x[u] = (in && P.n_poly) ? __ldcg(P.obs_x + j0 + u * kNT) : 0.0;
@@ -269,8 +282,8 @@ __device__ __forceinline__ double final_pass_poly(const TailParams& P, const Fas
     for (int u = 0; u < U; ++u) {
       double m = ((okm >> u) & 1u) ? 1.0 + (double)d[u] : nan;
       if (P.n_poly) m *= cv[u];
-      if (j0 + u * kNT < P.n_obs) {
-        if (P.model_out) P.model_out[(long long)p * P.n_obs + j0 + u * kNT] = m;
+      if (j0 + u * kNT < jend) {
+        if (mrow) mrow[j0 + u * kNT - off] = m;
         const double r = fma(m, is[u], -ot[u]);
         acc = fma(r, r, acc);
       }
@@ -280,7 +293,7 @@ __device__ __forceinline__ double final_pass_poly(const TailParams& P, const Fas
 }
 
 // observed pixels, continuum, residuals; returns this thread's partial chi2
-template <bool POLY, class ZV>
+template <bool POLY, bool STARS, class ZV>
 __device__ __forceinline__ double final_pass(const TailParams& P, const FastGrid& F, const PointSetup& S,
                                              const FastSetup& FS, const ZV& zv, int tid, int p, int N2) {
   const double nan = CUDART_NAN;
@@ -292,13 +305,14 @@ __device__ __forceinline__ double final_pass(const TailParams& P, const FastGrid
     // four pixels per trip: the twelve per-pixel constants are requested together, then the eight
     // shared-memory samples, then the arithmetic (the phase is latency-bound at 24 warps per SM)
     constexpr int U = 4;
+    const int jend = obs_hi<STARS>(P, FS.obs);                // the point's star: pixels [obs_lo, jend)
 #pragma unroll 1
-    for (int j0 = tid; j0 < P.n_obs; j0 += U * kNT) {
+    for (int j0 = obs_lo<STARS>(FS.obs) + tid; j0 < jend; j0 += U * kNT) {
       double q[U], is[U], ot[U];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int j = j0 + u * kNT;
-        const bool in = j < P.n_obs;
+        const bool in = j < jend;
         q[u] = in ? __ldcg(F.obs_q + j) : -1.0;          // -1 -> outside the grid -> contributes through `in` only
         is[u] = in ? __ldcg(P.obs_inv_s + j) : 0.0;
         ot[u] = in ? __ldcg(F.obs_otm1 + j) : 0.0;
@@ -318,11 +332,11 @@ __device__ __forceinline__ double final_pass(const TailParams& P, const FastGrid
         const float d = fmaf(interp_w(dl[u], hdu), g1[u] - g0[u], g0[u]);
         double r = fma((double)d, is[u], -ot[u]);
         if (!ok[u]) r = nan;
-        if (j0 + u * kNT < P.n_obs) acc = fma(r, r, acc);
+        if (j0 + u * kNT < jend) acc = fma(r, r, acc);
       }
     }
   } else {
-    acc = final_pass_poly(P, F, S, FS, zv, tid, p, N2);
+    acc = final_pass_poly<STARS>(P, F, S, FS, zv, tid, p, N2);
   }
   return acc;
 }
@@ -344,7 +358,8 @@ static __device__ __noinline__ void discard_lines(const float* row, int n, int t
 // LOG2N1 <= 15: the whole transform sits in shared memory (3 CTAs/SM up to 2^14).
 // LOG2N1 == 16: split transform, half in shared memory (128 KB), half in the scratch line.
 // POLY: continuum polynomial and / or model output in the final pass (the host picks the instantiation).
-template <int LOG2N1, bool POLY>
+// STARS: a context of several stars (obs_lo / obs_hi).
+template <int LOG2N1, bool POLY, bool STARS>
 __global__ void __launch_bounds__(kNT, LOG2N1 <= 14 ? PAYNE_TAIL_MINB : 1)
 tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -393,7 +408,7 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
 #endif
     if (S.bad) {
       if (P.model_out)
-        for (int j = tid; j < P.n_obs; j += kNT) P.model_out[(long long)p * P.n_obs + j] = nan;
+        for (int j = tid; j < obs_hi<STARS>(P, FS.obs) - obs_lo<STARS>(FS.obs); j += kNT) P.model_out[(long long)p * P.ld_flux + j] = nan;
       if (tid == 0 && P.lnl) store_lnl(P, p, nan);
       __syncthreads();
       continue;
@@ -465,7 +480,7 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
           stage_regrid(S, row, zp, tid, N2, FS.s_num, FS.s_den, i0, FS.s_invden, F.c_native, FS.s_incj, FS.s_incr);
           __syncthreads();
           ct_convolve_split<LOG2MH>(z, reinterpret_cast<float2*>(gline), tw, F.twc, H, tid);
-          acc = final_pass<POLY>(P, F, S, FS, zp, tid, p, N2);
+          acc = final_pass<POLY, STARS>(P, F, S, FS, zp, tid, p, N2);
         }
       } else {
         constexpr int LA = LOG2N1 > 15 ? 15 : LOG2N1;       // largest all-in-smem transform
@@ -485,13 +500,14 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
             ct_convolve_regrid<(LA >= 10 ? LA - 2 : 8)>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den,
                                                          FS.s_invden, F.c_native, S.clean != 0);
         }
-        if (!(P.debug_skip & 16)) acc = final_pass<POLY>(P, F, S, FS, zs, tid, p, N2);
+        if (!(P.debug_skip & 16)) acc = final_pass<POLY, STARS>(P, F, S, FS, zs, tid, p, N2);
       }
     } else {
       // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289)
       const int n = P.n;
       const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
-      for (int j = tid; j < P.n_obs; j += kNT) {
+      const int off = obs_lo<STARS>(FS.obs), jend = obs_hi<STARS>(P, FS.obs);
+      for (int j = off + tid; j < jend; j += kNT) {
         const double x = __ldg(P.obs_w + j);
         double m;
         if (!(x >= wlo && x <= whi)) m = nan;
@@ -504,7 +520,7 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
           m = 1.0 + ((b - a) / (wb - wa) * (x - wa) + a);
         }
         if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-        if (P.model_out) P.model_out[(long long)p * P.n_obs + j] = m;
+        if (P.model_out) P.model_out[(long long)p * P.ld_flux + (j - off)] = m;
         const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
         acc += r * r;
       }
@@ -542,7 +558,7 @@ tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ 
   if (p == 0 && F.work_counter) *F.work_counter = F.work_start;
   PointSetup S{};
   FastSetup FS{};
-  tail_setup(P, P.theta + (long long)p * P.ld, S);
+  tail_setup(P, P.theta + (long long)p * P.ld, p, S, FS.obs);
   if (!S.bad && S.use_inst) {
     const int nM = S.i1 - S.i0 + 1, N2 = 1 << S.log2N2;
     FS.s_num = nM - 1; FS.s_den = N2 - 1;
@@ -556,7 +572,8 @@ tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ 
     // must fit the shared-memory transform buffer (no split transforms) and fill whole chunks
     const double spx = sqrt(S.sig_px2);
     const int R = (int)ceil(kStSigmas * spx);
-    if (PAYNE_WITH_STENCIL && P.gauss_stencil && !P.rows_may_nan && spx >= kStMinSigmaPx && R <= kStMaxR && S.log2N2 >= 11 && S.log2N2 <= 15 &&
+    // (the stencil's final pass walks the pixels of a single-star context: off with several stars)
+    if (PAYNE_WITH_STENCIL && P.gauss_stencil && P.n_stars == 1 && !P.rows_may_nan && spx >= kStMinSigmaPx && R <= kStMaxR && S.log2N2 >= 11 && S.log2N2 <= 15 &&
         F.win_floats >= kStSideFloats) {
       const int E = (R + 2) / 2;                       // offsets 2e-1, 2e, 2e+1 must cover [-R, R]
       FS.st_R = R;
@@ -565,17 +582,19 @@ tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ 
       FS.st_inv2s2 = 0.5 / S.sig_px2;
     }
     if (F.cluster) FS.st_R = 0;
-    if (F.cluster && F.obs_sorted) {
+    if (F.cluster && P.stars[star_of(P.star, P.n_stars, p)].sorted) {
       // tail_cluster.cuh: CTA r of the cluster serves the observed pixels whose position falls into quarter r
       for (int r = 0; r < 3; ++r) {
         const double thr = (double)((long long)(r + 1) << (S.log2N2 - 2));
-        int a = 0, b = P.n_obs;                          // first j with (obs_q[j] - q0) * scale >= thr
+        int a = FS.obs.off, b = FS.obs.off + FS.obs.n;   // first j of the star with (obs_q[j] - q0) * scale >= thr
         while (a < b) {
           const int mid = (a + b) >> 1;
           if ((__ldg(F.obs_q + mid) - FS.q0) * FS.scale >= thr) b = mid; else a = mid + 1;
         }
         FS.jcut[r] = a;
       }
+    } else if (F.cluster) {
+      FS.jcut[0] = -1;
     }
   }
   out->S = S;

@@ -33,6 +33,7 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
   float2* z = reinterpret_cast<float2*>(smem_raw);
   float* zf = reinterpret_cast<float*>(smem_raw);
   __shared__ PointSetup S;
+  __shared__ ObsSlice SL;
   __shared__ double red[kTailThreads / 32];
   const int tid = threadIdx.x;
   const TwTab tw{P.tw, P.log2tw, P.twpass};
@@ -41,11 +42,11 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
   for (int p = blockIdx.x; p < P.B; p += gridDim.x) {
     const double* th = P.theta + (long long)p * P.ld;
     float* row = P.flux + (long long)p * P.ldf;
-    if (tid == 0) tail_setup(P, th, S);
+    if (tid == 0) tail_setup(P, th, p, S, SL);
     __syncthreads();
     if (S.bad) {
       if (P.model_out)
-        for (int j = tid; j < P.n_obs; j += kTailThreads) P.model_out[(long long)p * P.n_obs + j] = nan;
+        for (int j = tid; j < SL.n; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
       if (tid == 0 && P.lnl) P.lnl[p] = nan;
       __syncthreads();
       continue;
@@ -98,7 +99,8 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
       convolve_any<LOG2N1>(z, S.log2N2, tw, TC, H, tid);
       // ---------------- onto the observed pixels, continuum, chi2
       const double pmax = (double)(N2 - 1);
-      for (int j = tid; j < P.n_obs; j += kTailThreads) {
+      const int off = SL.off, jend = off + SL.n;            // the point's star
+      for (int j = off + tid; j < jend; j += kTailThreads) {
         const double pp = (__ldg(P.obs_lnw + j) - S.u0) * S.inv_du;
         double m;
         if (!(pp >= 0.0 && pp <= pmax)) m = nan;            // smoothing.py:289 left/right = nan
@@ -110,7 +112,7 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
           m = 1.0 + (double)(g0 + t * (g1 - g0));
         }
         if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-        if (P.model_out) P.model_out[(long long)p * P.n_obs + j] = m;
+        if (P.model_out) P.model_out[(long long)p * P.ld_flux + (j - off)] = m;
         const double r = m * (double)__ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
         acc += r * r;
       }
@@ -118,7 +120,8 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
       // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289)
       const int n = P.n;
       const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
-      for (int j = tid; j < P.n_obs; j += kTailThreads) {
+      const int off = SL.off, jend = off + SL.n;
+      for (int j = off + tid; j < jend; j += kTailThreads) {
         const double x = __ldg(P.obs_w + j);
         double m;
         if (!(x >= wlo && x <= whi)) m = nan;
@@ -131,7 +134,7 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
           m = 1.0 + ((b - a) / (wb - wa) * (x - wa) + a);
         }
         if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-        if (P.model_out) P.model_out[(long long)p * P.n_obs + j] = m;
+        if (P.model_out) P.model_out[(long long)p * P.ld_flux + (j - off)] = m;
         const double r = m * (double)__ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
         acc += r * r;
       }

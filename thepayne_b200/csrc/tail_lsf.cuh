@@ -86,7 +86,8 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
     const double* th = P.theta + (long long)p * P.ld;
     float* row = P.flux + (long long)p * P.ldf;
     if (tid == 0) {
-      tail_setup(P, th, S);             // Inst_R is absent in this mode: Doppler, rotation and polynomial only
+      ObsSlice obs;                     // (star 0 throughout: the LSF vector is refused on several stars)
+      tail_setup(P, th, p, S, obs);            // Inst_R is absent in this mode: Doppler, rotation and polynomial only
       const double D = S.D;
       const double lo = P.obs_min + 20.0 * 100.0 * -1.0, hi = P.obs_max + 20.0 * 100.0 * 1.0;   // smoothing.py:128, 643
       int i0 = n, i1 = -1;
@@ -105,7 +106,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
     const int i0 = sh_i0, i1 = sh_i1, nM = i1 - i0 + 1;
     if (S.bad || nM < 17) {
       if (P.model_out)
-        for (int j = tid; j < P.n_obs; j += kTailThreads) P.model_out[(long long)p * P.n_obs + j] = nan;
+        for (int j = tid; j < P.n_obs; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
       if (tid == 0 && P.lnl) P.lnl[p] = nan;
       __syncthreads();
       continue;
@@ -193,7 +194,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
     if (log2nx < 5 || log2nx > L.log2nx_max) {
       if (tid == 0) { if (log2nx > L.log2nx_max) atomicOr(P.status, 1); if (P.lnl) P.lnl[p] = nan; }
       if (P.model_out)
-        for (int j = tid; j < P.n_obs; j += kTailThreads) P.model_out[(long long)p * P.n_obs + j] = nan;
+        for (int j = tid; j < P.n_obs; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
       __syncthreads();
       continue;
     }
@@ -232,7 +233,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
       for (int j = tid; j < P.n_obs; j += kTailThreads) {
         double m = 1.0 + np_interp(__ldg(P.obs_w + j), lamf, convf, nx);
         if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-        if (P.model_out) P.model_out[(long long)p * P.n_obs + j] = m;
+        if (P.model_out) P.model_out[(long long)p * P.ld_flux + j] = m;
         const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
         acc += r * r;
       }

@@ -6,6 +6,10 @@ device-memory / stream provider; the arithmetic all happens inside libpayne_b200
 The parameter-vector convention is the reference's (Payne/fitting/likelihood.py:35-72): a
 row of ``theta`` holds the free parameters in ``fitpars_i`` order, fixed ones come from
 ``fixedpars``, and spectral parameters that are neither are NaN.
+
+One context may hold the observations of many stars (``stars=[...]``): the emulators, the
+parameter layout and the fixed parameters are shared, and every row of a batch names its star.
+A single-star engine is the case of one star.
 """
 from __future__ import annotations
 
@@ -71,7 +75,17 @@ def _specnet_struct(spec, keep):
 class Engine:
     def __init__(self, spec=None, phot=None, obs_wave=None, obs_flux=None, obs_eflux=None,
                  obs_phot=None, fitpars_i=(), fixedpars=None, runbools=(True, False, False, False, False),
-                 precision='parity', device=None):
+                 precision='parity', device=None, stars=None):
+        """``stars``: instead of ``obs_wave``, ``obs_flux``, ``obs_eflux`` and ``obs_phot``, a list of
+        ``{'wave', 'flux', 'eflux', 'phot': {band: (mag, err)}}``, one per star; ``lnlike_batch`` and
+        ``model_batch`` then take the star index of every row."""
+        if stars is None:
+            stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot}]
+        elif any(v is not None for v in (obs_wave, obs_flux, obs_eflux, obs_phot)):
+            raise ValueError('give either stars=[...] or obs_wave / obs_flux / obs_eflux / obs_phot, not both')
+        stars = list(stars)
+        if not stars:
+            raise ValueError('stars is empty')
         self.lib = _lib.load()
         if not torch.cuda.is_available():
             raise _lib.PayneError('no CUDA device: thepayne_b200 has no CPU fallback')
@@ -103,19 +117,22 @@ class Engine:
                 raise ValueError('spec_bool set but no spectrum emulator given')
             sp = _specnet_struct(spec, keep)
             self.D_in, self.D_out = int(sp.D_in), int(sp.D_out)
-        ob = _lib.PayneObs()
-        self.n_obs = 0
+        self.n_stars = len(stars)
+        obs = (_lib.PayneObs * self.n_stars)()
+        self.n_obs_star = [0] * self.n_stars
         if spec_bool:
-            ow, of, oe = _f64(obs_wave), _f64(obs_flux), _f64(obs_eflux)
-            if not (len(ow) == len(of) == len(oe)):
-                raise ValueError('observed wave/flux/eflux lengths differ')
-            keep += [ow, of, oe]
-            ob.n_obs, ob.wave, ob.flux, ob.eflux = len(ow), _pd(ow), _pd(of), _pd(oe)
-            self.n_obs = len(ow)
+            for k, st in enumerate(stars):
+                ow, of, oe = _f64(st['wave']), _f64(st['flux']), _f64(st['eflux'])
+                if not (len(ow) == len(of) == len(oe)):
+                    raise ValueError('observed wave/flux/eflux lengths differ (star %d)' % k)
+                keep += [ow, of, oe]
+                obs[k].n_obs, obs[k].wave, obs[k].flux, obs[k].eflux = len(ow), _pd(ow), _pd(of), _pd(oe)
+                self.n_obs_star[k] = len(ow)
+        self.n_obs = max(self.n_obs_star)          # the largest star's
         ph = None
         self.bands = []
         if phot_bool:
-            if phot is None or obs_phot is None:
+            if phot is None or any(st.get('phot') is None for st in stars):
                 raise ValueError('phot_bool set but no photometry emulator / observation given')
             self.bands = list(phot.bands)
             ph = _lib.PaynePhotNet()
@@ -127,16 +144,17 @@ class Engine:
             pxmin, pxmax, hiav = _f64(phot.xmin), _f64(phot.xmax), _f64(phot.hiav)
             keep += [pxmin, pxmax, hiav]
             ph.xmin, ph.xmax, ph.hiav = _pd(pxmin), _pd(pxmax), _pd(hiav)
-            mag = _f64([obs_phot[b][0] for b in self.bands])
-            err = _f64([obs_phot[b][1] for b in self.bands])
-            keep += [mag, err]
-            ob.nb, ob.phot_mag, ob.phot_err = len(self.bands), _pd(mag), _pd(err)
+            for k, st in enumerate(stars):
+                mag = _f64([st['phot'][b][0] for b in self.bands])
+                err = _f64([st['phot'][b][1] for b in self.bands])
+                keep += [mag, err]
+                obs[k].nb, obs[k].phot_mag, obs[k].phot_err = len(self.bands), _pd(mag), _pd(err)
         self.nb = len(self.bands)
 
         ctx = C.c_void_p()
-        _lib.check(self.lib.payne_ctx_create(C.byref(sp) if sp is not None else None,
-                                              C.byref(ph) if ph is not None else None,
-                                              C.byref(ob), C.byref(lay), self.device, C.byref(ctx)))
+        _lib.check(self.lib.payne_ctx_create_stars(C.byref(sp) if sp is not None else None,
+                                                    C.byref(ph) if ph is not None else None,
+                                                    obs, self.n_stars, C.byref(lay), self.device, C.byref(ctx)))
         self._ctx = ctx
         del keep
 
@@ -190,38 +208,66 @@ class Engine:
             raise ValueError('theta has %d columns, layout expects %d' % (theta.shape[1], self.ndim))
         return theta.contiguous()
 
-    def lnlike_batch(self, theta):
+    def _star_dev(self, star, B, dev):
+        if star is None:
+            return None
+        if not (isinstance(star, torch.Tensor) and star.is_cuda and star.dtype == torch.int32):
+            raise ValueError('with a CUDA theta, star must be an int32 CUDA tensor')
+        if star.shape != (B,) or star.device != dev:
+            raise ValueError('star must be [%d] on %s' % (B, dev))
+        return star.contiguous()
+
+    def lnlike_batch(self, theta, star=None):
         """theta: [B, ndim] float64.  CUDA tensor -> CUDA tensor [B] (stream-ordered, no sync);
-        numpy / CPU tensor -> numpy [B] through the host-buffer entry point."""
+        numpy / CPU tensor -> numpy [B] through the host-buffer entry point.  ``star``: [B] star index of
+        every row, an int32 CUDA tensor with a CUDA theta, anything numpy takes otherwise (None: star 0,
+        which only a single-star engine accepts).  On the device a row with an index outside
+        [0, n_stars) gets NaN and sets status bit 2; the host path refuses such an index."""
         if isinstance(theta, torch.Tensor) and theta.is_cuda:
             th = self._theta_dev(theta)
+            sv = self._star_dev(star, th.shape[0], th.device)
             out = torch.empty(th.shape[0], dtype=torch.float64, device=th.device)
             st = torch.cuda.current_stream(th.device).cuda_stream
-            _lib.check(self.lib.payne_lnlike_batch(self._ctx, th.data_ptr(), th.shape[0], th.shape[1],
-                                                   out.data_ptr(), st))
+            _lib.check(self.lib.payne_lnlike_batch_stars(self._ctx, th.data_ptr(),
+                                                         sv.data_ptr() if sv is not None else None,
+                                                         th.shape[0], th.shape[1], out.data_ptr(), st))
             return out
         th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
         if th.ndim != 2 or th.shape[1] != self.ndim:
             raise ValueError('theta must be [B, %d]' % self.ndim)
+        sv = None
+        if star is not None:
+            if isinstance(star, torch.Tensor):
+                star = star.cpu().numpy()
+            sv = np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind'))
+            if sv.shape != (th.shape[0],):
+                raise ValueError('star must be [%d]' % th.shape[0])
         out = np.empty(th.shape[0], dtype=np.float64)
-        _lib.check(self.lib.payne_lnlike_batch_host(self._ctx, th.ctypes.data, th.shape[0], th.shape[1],
-                                                    out.ctypes.data))
+        _lib.check(self.lib.payne_lnlike_batch_stars_host(self._ctx, th.ctypes.data,
+                                                          sv.ctypes.data if sv is not None else None,
+                                                          th.shape[0], th.shape[1], out.ctypes.data))
         return out
 
-    def model_batch(self, theta, want_flux=True, want_mags=True):
-        """Model spectra [B, n_obs], magnitudes [B, nb] and lnL [B] as CUDA float64 tensors."""
+    def model_batch(self, theta, star=None, want_flux=True, want_mags=True):
+        """Model spectra [B, n_obs], magnitudes [B, nb] and lnL [B] as CUDA float64 tensors.  With several
+        stars, n_obs is the largest star's: row p holds the first ``n_obs_star[star[p]]`` pixels, the rest
+        stay NaN.  ``star`` as in ``lnlike_batch`` (numpy is copied to the device)."""
         dev = torch.device('cuda', self.device)
         if not isinstance(theta, torch.Tensor):
             theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
         th = self._theta_dev(theta.to(dev))
         B = th.shape[0]
-        flux = torch.empty((B, self.n_obs), dtype=torch.float64, device=dev) if (want_flux and self.n_obs) else None
+        if star is not None and not isinstance(star, torch.Tensor):
+            star = torch.from_numpy(np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind')))
+        sv = self._star_dev(star.to(dev) if star is not None else None, B, dev)
+        flux = torch.full((B, self.n_obs), float('nan'), dtype=torch.float64, device=dev) \
+            if (want_flux and self.n_obs) else None
         mags = torch.empty((B, self.nb), dtype=torch.float64, device=dev) if (want_mags and self.nb) else None
         lnl = torch.empty(B, dtype=torch.float64, device=dev)
         st = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(self.lib.payne_model_batch(
-            self._ctx, th.data_ptr(), B, th.shape[1],
-            flux.data_ptr() if flux is not None else None,
+        _lib.check(self.lib.payne_model_batch_stars(
+            self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None, B, th.shape[1],
+            flux.data_ptr() if flux is not None else None, self.n_obs,
             mags.data_ptr() if mags is not None else None, lnl.data_ptr(), st))
         return flux, mags, lnl
 

@@ -42,6 +42,10 @@ class FitPayne(object):
 
     # ------------------------------------------------------------------ input dictionary -> fit setup
     def run(self, *args, **kwargs):
+        return self(self._setup(*args, **kwargs))
+
+    def _setup(self, *args, **kwargs):
+        """The user dictionary -> ``indicts`` (fitargs, fitpars, sampler, priordict, runbools)."""
         self.verbose = kwargs.get('verbose', True)
         if 'inputdict' not in kwargs:
             print('NO USER DEFINED INPUT DICT, NOTHING TO FIT!')
@@ -112,10 +116,9 @@ class FitPayne(object):
             if isinstance(self.priordict[kk], dict) and 'fixed' in self.priordict[kk]:
                 fa['fixedpars'][kk] = self.priordict[kk]['fixed']
                 self.fitpars_bool[kk] = False
-        return self({'fitargs': fa, 'fitpars': [self.fitpars, self.fitpars_bool], 'sampler': self.samplerdict,
-                     'priordict': self.priordict,
-                     'runbools': [self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool,
-                                  self.carbon_bool]})
+        return {'fitargs': fa, 'fitpars': [self.fitpars, self.fitpars_bool], 'sampler': self.samplerdict,
+                'priordict': self.priordict,
+                'runbools': [self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool]}
 
     def __call__(self, indicts):
         return self.run_dynesty(indicts)
@@ -123,15 +126,24 @@ class FitPayne(object):
     def run_dynesty(self, indicts):
         """Name kept from the reference (fitstar.py:236-258); the sampler is the batched one."""
         fitargs, fitpars, runbools = indicts['fitargs'], indicts['fitpars'], indicts['runbools']
-        self.ndim = sum(1 for pp in fitpars[0] if fitpars[1][pp])
-        self.priorobj = self.prior(fitargs, indicts['priordict'], fitpars, runbools)
+        self._prepare(indicts)
         self.likeobj = self.likelihood(fitargs, fitpars, runbools, verbose=False,
                                        precision=getattr(self, 'precision', 'parity'),
                                        device=getattr(self, 'device', None))
+        self._check_sampler(indicts)
+        return self._runsampler(indicts['sampler'])
+
+    def _prepare(self, indicts):
+        """Dimension and prior object of the fit (everything but the likelihood)."""
+        fitpars = indicts['fitpars']
+        self.ndim = sum(1 for pp in fitpars[0] if fitpars[1][pp])
+        self.priorobj = self.prior(indicts['fitargs'], indicts['priordict'], fitpars, indicts['runbools'])
+
+    @staticmethod
+    def _check_sampler(indicts):
         kind = indicts['sampler'].get('samplertype', 'Static')
         if kind != 'Static':
             raise NotImplementedError("samplertype %r: only the static sampler is batched" % kind)
-        return self._runsampler(indicts['sampler'])
 
     # ------------------------------------------------------------------ output file (fitstar.py:219-227)
     def _initoutput(self, parnames):

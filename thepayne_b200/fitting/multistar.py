@@ -1,0 +1,283 @@
+"""Fitting many stars at once: one engine for all their observations, and their samplers in lock-step.
+
+A survey fits thousands of stars with the same emulator.  Between two stars only the observation changes
+(wavelengths, fluxes, errors, magnitudes); the emulator weights, the parameter layout and every table built
+from the emulator grid stay the same.  A single star's sampler hands over a few hundred points per call, which
+leaves the GPU latency-bound; the points of many stars together make one full-size batch.
+
+``StarSetLikelihood`` builds one ``Engine`` holding every star's observation.  ``star(k)`` is a view with the
+interface of ``likelihood.likelihood`` for star k, so ``BatchedLnProb`` and ``BatchedNestedSampler`` work on it
+unchanged.
+
+``FitPayneMany().run(inputdicts=[...])`` is ``FitPayne.run`` for a list of input dictionaries: each star gets its
+fitargs, prior, sampler and output file exactly as ``FitPayne.run`` makes them, and the samplers run in their own
+threads.  Every sampler's likelihood call goes to a ``LockstepBatcher``; once every unfinished sampler has posted
+its points, the batcher makes ONE ``lnlike_batch(theta, star)`` call, concatenated in star order, and hands back
+the slices.  A sampler that finishes or raises leaves the barrier.  Each sampler sees exactly the values a
+separate ``FitPayne`` run would give it, so its output file is the same byte for byte.
+"""
+from __future__ import annotations
+
+import threading
+
+import numpy as np
+
+from ..engine import Engine
+from .fitstar import FitPayne
+from .genmod import GenMod
+from .likelihood import free_parameters
+
+
+def _same(a, b):
+    if a is b:
+        return True
+    if isinstance(a, (str, int, float)) and isinstance(b, (str, int, float)):
+        return a == b
+    return False
+
+
+class StarSetLikelihood(object):
+    """The likelihoods of several stars that share emulators, free parameters, fixed parameters and bands.
+
+    ``fitargs_list``: one ``fitargs`` per star (as ``FitPayne.run`` builds them).  ``fitpars`` / ``runbools``:
+    one value for every star, or a list with one per star (they must then agree)."""
+
+    def __init__(self, fitargs_list, fitpars, runbools, precision='parity', device=None):
+        fitargs_list = list(fitargs_list)
+        if not fitargs_list:
+            raise ValueError('no stars')
+        S = len(fitargs_list)
+        fp_list = list(fitpars) if _is_per_star(fitpars, S) else [fitpars] * S
+        rb_list = list(runbools) if isinstance(runbools[0], (list, tuple)) else [runbools] * S
+        if len(rb_list) != S:
+            raise ValueError('runbools: one list for all stars or one per star')
+        fa0, free0, rb0 = fitargs_list[0], free_parameters(fp_list[0]), [bool(b) for b in rb_list[0][:5]]
+        for k in range(1, S):
+            fa = fitargs_list[k]
+            if [bool(b) for b in rb_list[k][:5]] != rb0:
+                raise ValueError('star %d: runbools differ from star 0' % k)
+            if free_parameters(fp_list[k]) != free0:
+                raise ValueError('star %d: free parameters differ from star 0' % k)
+            for key in ('specANNpath', 'photANNpath'):
+                if not _same(fa.get(key), fa0.get(key)):
+                    raise ValueError('star %d: %s differs from star 0' % (k, key))
+            if fa.get('NNtype', 'LinNet') != fa0.get('NNtype', 'LinNet'):
+                raise ValueError('star %d: NNtype differs from star 0' % k)
+            if dict(fa.get('fixedpars', {})) != dict(fa0.get('fixedpars', {})):
+                raise ValueError('star %d: fixedpars differ from star 0' % k)
+            if rb0[1] and set(fa['obs_phot'].keys()) != set(fa0['obs_phot'].keys()):
+                raise ValueError('star %d: photometric bands differ from star 0' % k)
+        self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool = rb0
+        if self.carbon_bool:
+            raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
+        self.n_stars = S
+        self.fitargs_list = fitargs_list
+        self.fixedpars = fa0['fixedpars']
+        self.precision = precision
+        self.GM = GenMod(precision=precision)            # the emulators, as likelihood.__init__ loads them
+        if self.spec_bool:
+            self.GM._initspecnn(nnpath=fa0['specANNpath'], NNtype=fa0.get('NNtype', 'LinNet'), carbon_bool=False)
+        if self.phot_bool:
+            self.GM._initphotnn(fa0['obs_phot'].keys(), nnpath=fa0['photANNpath'])
+        self.fitpars_i = free0
+        self.ndim = len(free0)
+        stars = [{'wave': fa.get('obs_wave_fit'), 'flux': fa.get('obs_flux_fit'), 'eflux': fa.get('obs_eflux_fit'),
+                  'phot': fa.get('obs_phot')} for fa in fitargs_list]
+        self.engine = Engine(spec=self.GM.PP.anns.model if self.spec_bool else None,
+                             phot=self.GM.fppsed.net if self.phot_bool else None, stars=stars,
+                             fitpars_i=self.fitpars_i, fixedpars=self.fixedpars,
+                             runbools=[self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
+                             precision=precision, device=device)
+        self.ncalls = 0                                   # lnlike_batch calls made on the engine
+
+    def lnlike_batch(self, theta, star):
+        """theta [B, ndim] and star [B] (CUDA tensors or numpy, as ``Engine.lnlike_batch``) -> lnL [B]."""
+        self.ncalls += 1
+        return self.engine.lnlike_batch(theta, star)
+
+    def star(self, k):
+        """Star k with the interface of ``likelihood.likelihood``."""
+        if not 0 <= k < self.n_stars:
+            raise IndexError('star %d of %d' % (k, self.n_stars))
+        return StarView(self, k)
+
+
+def _is_per_star(fitpars, S):
+    # [names, flags] for all stars vs a list of S such pairs
+    return len(fitpars) == S and all(isinstance(f, (list, tuple)) and len(f) == 2 and isinstance(f[1], dict)
+                                     for f in fitpars)
+
+
+class StarView(object):
+    """One star of a ``StarSetLikelihood``: ``lnlikefn``, ``lnlike_batch(theta)``, ``parsdict``, ``fitpars_i``,
+    ``ndim``, ``fixedpars`` as in ``likelihood.likelihood``."""
+
+    def __init__(self, owner, k):
+        self.owner, self.k = owner, int(k)
+        self.fitpars_i, self.ndim, self.fixedpars = owner.fitpars_i, owner.ndim, owner.fixedpars
+        self.fitargs = owner.fitargs_list[self.k]
+        self.parsdict = {}
+
+    def _set_parsdict(self, pars):
+        self.parsdict = {pp: vv for pp, vv in zip(self.fitpars_i, pars)}
+        for kk in self.fixedpars.keys():
+            self.parsdict[kk] = self.fixedpars[kk]
+
+    def _lnlike(self, theta):
+        if hasattr(theta, 'is_cuda') and theta.is_cuda:
+            import torch
+            star = torch.full((theta.shape[0],), self.k, dtype=torch.int32, device=theta.device)
+        else:
+            star = np.full(len(theta), self.k, dtype=np.int32)
+        return self.owner.lnlike_batch(theta, star)
+
+    def lnlikefn(self, pars):
+        self._set_parsdict(pars)
+        th = np.asarray(pars, dtype=np.float64).reshape(1, self.ndim)
+        return float(self._lnlike(th)[0])
+
+    def lnlike_batch(self, theta):
+        out = self._lnlike(theta)
+        last = theta[-1]
+        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
+        return out
+
+
+class _Released(Exception):
+    """The batcher stopped (its likelihood raised) while this participant waited."""
+
+
+class LockstepBatcher(object):
+    """Barrier that turns the likelihood calls of n participants into one call.
+
+    ``fn(theta_cat, star_cat) -> values`` with ``theta_cat`` the posted arrays concatenated in participant order
+    and ``star_cat`` the participant index of every row.  ``call(k, theta)`` posts and blocks until every
+    participant that has not left has posted too, then returns participant k's slice.  ``leave(k)``: k makes no
+    more calls.  If ``fn`` raises, every waiting participant raises that exception."""
+
+    def __init__(self, fn, n):
+        self.fn = fn
+        self.cv = threading.Condition()
+        self.active = set(range(n))
+        self.pending = {}
+        self.results = {}
+        self.error = None
+        self.ncalls = 0
+        self.batch_sizes = []
+
+    def call(self, k, theta):
+        theta = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
+        with self.cv:
+            if self.error is not None:
+                raise _Released() from self.error
+            if k not in self.active or k in self.pending:
+                raise RuntimeError('participant %d cannot post now' % k)
+            self.pending[k] = theta
+            self._run_if_complete()
+            while k not in self.results:
+                if self.error is not None:
+                    raise _Released() from self.error
+                self.cv.wait()
+            return self.results.pop(k)
+
+    def leave(self, k):
+        with self.cv:
+            self.active.discard(k)
+            self._run_if_complete()
+
+    def _run_if_complete(self):
+        # (lock held) every participant still active has posted: one call for all of them
+        if not self.pending or not self.active.issubset(self.pending.keys()):
+            return
+        ks = sorted(self.pending)
+        theta = np.concatenate([self.pending[k] for k in ks], axis=0)
+        star = np.concatenate([np.full(len(self.pending[k]), k, dtype=np.int32) for k in ks])
+        try:
+            out = np.asarray(self.fn(theta, star))
+        except BaseException as e:                      # noqa: B036 -- handed to every waiting thread
+            self.error = e
+            self.pending.clear()
+            self.cv.notify_all()
+            return
+        self.ncalls += 1
+        self.batch_sizes.append(len(theta))
+        o = 0
+        for k in ks:
+            n = len(self.pending[k])
+            self.results[k] = out[o:o + n]
+            o += n
+        self.pending.clear()
+        self.cv.notify_all()
+
+
+class _BatchedStarView(StarView):
+    """A star's view whose batched calls go through the lock-step batcher."""
+
+    def __init__(self, owner, k, batcher):
+        super().__init__(owner, k)
+        self.batcher = batcher
+
+    def lnlike_batch(self, theta):
+        out = self.batcher.call(self.k, theta)
+        last = theta[-1]
+        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
+        return out
+
+
+class FitPayneMany(object):
+    """``FitPayne`` for many stars sharing one emulator: one engine, samplers in lock-step (module docstring)."""
+
+    def run(self, *args, **kwargs):
+        """``inputdicts=[inputdict, ...]``, each as ``FitPayne.run(inputdict=...)`` takes it (its own ``output``
+        file and ``sampler`` settings).  Returns the list of samplers in star order.  ``precision`` and
+        ``device`` come from the first dictionary."""
+        if 'inputdicts' not in kwargs:
+            raise IOError('NO USER DEFINED INPUT DICTS, NOTHING TO FIT!')
+        inputdicts = list(kwargs['inputdicts'])
+        verbose = kwargs.get('verbose', True)
+        fits, indicts = [], []
+        for d in inputdicts:
+            f = FitPayne()
+            ind = f._setup(inputdict=d, verbose=verbose)
+            f._prepare(ind)
+            f._check_sampler(ind)
+            fits.append(f)
+            indicts.append(ind)
+        self.fits = fits
+        self.likeobj = StarSetLikelihood([ind['fitargs'] for ind in indicts], [ind['fitpars'] for ind in indicts],
+                                         [ind['runbools'] for ind in indicts], precision=fits[0].precision,
+                                         device=fits[0].device)
+        self.batcher = LockstepBatcher(self.likeobj.lnlike_batch, len(fits))
+        for k, f in enumerate(fits):
+            f.likeobj = _BatchedStarView(self.likeobj, k, self.batcher)
+        samplers, errors = run_lockstep([lambda f=f, ind=ind: f._runsampler(ind['sampler'])
+                                         for f, ind in zip(fits, indicts)], self.batcher)
+        for e in errors:
+            if e is not None:
+                raise e
+        return samplers
+
+
+def run_lockstep(jobs, batcher):
+    """Run ``jobs[k]()`` in thread k; job k's batched calls go through ``batcher`` as participant k.  Returns
+    (results, exceptions) in job order once every thread has ended.  A job that returns or raises leaves the
+    barrier, so the others never wait for it."""
+    results, errors = [None] * len(jobs), [None] * len(jobs)
+
+    def body(k):
+        try:
+            results[k] = jobs[k]()
+        except _Released as e:
+            errors[k] = e.__cause__ if e.__cause__ is not None else e
+        except BaseException as e:                      # noqa: B036 -- re-raised by the caller
+            errors[k] = e
+        finally:
+            batcher.leave(k)
+
+    threads = [threading.Thread(target=body, args=(k,), name='lockstep-%d' % k, daemon=True)
+               for k in range(len(jobs))]
+    for t in threads:
+        t.start()
+    for t in threads:
+        t.join()
+    return results, errors

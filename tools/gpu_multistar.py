@@ -1,0 +1,149 @@
+"""Measurement: one multi-star call against K single-star calls (observation sets, payne_ctx_create_stars).
+
+Workload: the C2 emulator (LinNet 4-256-256-256-14172, SURVEY §8d) with K stars.  Each star has its own observed
+grid inside the emulator coverage; the grids differ in range and n_obs (3000 .. 7000 pixels).  For every K and
+per-star batch b three cases are timed:
+
+  multi    one payne_lnlike_batch_stars call of K*b points (stars concatenated, as FitPayneMany makes them);
+  singles  K payne_lnlike_batch calls of b points each, on K single-star contexts, one stream;
+  ceiling  one single-star call of K*b points (star 0's context): the rate the GPU reaches at that size.
+
+Device time: CUDA events around the case, median over --reps repetitions.  Host-entry time: a host clock around
+the case and a device synchronise (what a sampler waiting for its lnL sees), median.  Inputs are drawn once per
+(K, b); every case is warmed up before it is timed.  The GPU name and power limit are read in the same run.
+
+usage: python tools/gpu_multistar.py [--out DIR] [--ks 1,4,16,64] [--bs 64,128,256,512] [--reps 30]
+Prints one line per (K, b) and the GPU record; with --out DIR it also writes every row to DIR/multistar.json.
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+from thepayne_b200 import synth  # noqa: E402
+from thepayne_b200.engine import Engine  # noqa: E402
+
+FIT = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot', 'Inst_R']
+
+
+def gpu_info():
+    info = {'name': torch.cuda.get_device_name(0)}
+    try:
+        out = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'],
+                             capture_output=True, text=True, timeout=30).stdout.strip().split('\n')[0]
+        info['nvidia_smi'] = out
+    except Exception as e:                              # noqa: BLE001 -- recorded, not fatal
+        info['nvidia_smi'] = 'unavailable: %s' % e
+    return info
+
+
+def make_stars(spec, K, seed=1):
+    w = spec.wavelength
+    a, b = w[0], w[-1]
+    span = b - a
+    rng = np.random.default_rng(seed)
+    stars = []
+    for k in range(K):
+        lo = a + span * (0.04 + 0.10 * rng.random())
+        hi = b - span * (0.04 + 0.10 * rng.random())
+        n = int(rng.integers(3000, 7001))
+        g = np.linspace(lo, hi, n)
+        stars.append({'wave': g, 'flux': 1.0 + 0.02 * rng.standard_normal(n), 'eflux': np.full(n, 0.02), 'phot': None})
+    return stars
+
+
+def draw(B, seed):
+    box = synth._BOX
+    rng = np.random.default_rng(seed)
+    lo = np.array([box[p][0] for p in FIT])
+    hi = np.array([box[p][1] for p in FIT])
+    return lo + (hi - lo) * rng.random((B, len(FIT)))
+
+
+def time_case(fn, reps, warm=3):
+    for _ in range(warm):
+        fn()
+    torch.cuda.synchronize()
+    dev, host = [], []
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(reps):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        e0.record()
+        fn()
+        e1.record()
+        torch.cuda.synchronize()
+        host.append((time.perf_counter() - t0) * 1e3)
+        dev.append(e0.elapsed_time(e1))
+    return float(np.median(dev)), float(np.median(host)), float(np.min(dev))
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument('--out', default=None, help='directory for multistar.json (default: print only)')
+    ap.add_argument('--ks', default='1,4,16,64')
+    ap.add_argument('--bs', default='64,128,256,512')
+    ap.add_argument('--reps', type=int, default=30)
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit('gpu_multistar.py measures on the GPU: no CUDA device')
+    ks = [int(v) for v in args.ks.split(',')]
+    bs = [int(v) for v in args.bs.split(',')]
+    wave, rsig = synth.ann_wavegrid(5130.0, 5340.0, 50000.0)              # C2 (synth.config_c2)
+    spec = synth.make_specnet(4, 256, wave, rsig, seed=0)
+    kw = dict(spec=spec, fitpars_i=FIT, fixedpars={}, runbools=[True, False, False, False, False], precision='parity')
+    Kmax = max(ks)
+    all_stars = make_stars(spec, Kmax)
+    singles = [Engine(obs_wave=s['wave'], obs_flux=s['flux'], obs_eflux=s['eflux'], **kw) for s in all_stars]
+    rows = []
+    for K in ks:
+        multi = Engine(stars=all_stars[:K], **kw)
+        for b in bs:
+            th = torch.from_numpy(draw(K * b, seed=K * 1000 + b)).cuda()
+            star = torch.repeat_interleave(torch.arange(K, dtype=torch.int32), b).cuda()
+            parts = [th[k * b:(k + 1) * b] for k in range(K)]
+            res = {'K': K, 'b': b, 'points': K * b}
+            res['multi_dev_ms'], res['multi_host_ms'], res['multi_dev_min_ms'] = time_case(
+                lambda: multi.lnlike_batch(th, star), args.reps)
+            res['singles_dev_ms'], res['singles_host_ms'], res['singles_dev_min_ms'] = time_case(
+                lambda: [singles[k].lnlike_batch(parts[k]) for k in range(K)], args.reps)
+            res['ceiling_dev_ms'], res['ceiling_host_ms'], res['ceiling_dev_min_ms'] = time_case(
+                lambda: singles[0].lnlike_batch(th), args.reps)
+            # same answers: the multi-star call against the K single-star calls
+            got = multi.lnlike_batch(th, star)
+            ref = torch.cat([singles[k].lnlike_batch(parts[k]) for k in range(K)])
+            torch.cuda.synchronize()
+            res['bit_identical'] = bool(torch.equal(torch.nan_to_num(got, nan=1.5), torch.nan_to_num(ref, nan=1.5)))
+            res['speedup_host'] = res['singles_host_ms'] / res['multi_host_ms']
+            res['speedup_dev'] = res['singles_dev_ms'] / res['multi_dev_ms']
+            res['multi_over_ceiling_dev'] = res['multi_dev_ms'] / res['ceiling_dev_ms']
+            res['multi_Mevals_s'] = K * b / res['multi_host_ms'] / 1e3
+            rows.append(res)
+            print('K=%3d b=%4d  multi %.3f ms dev / %.3f ms host | %d singles %.3f / %.3f | ceiling %.3f / %.3f | '
+                  'x%.2f host  x%.2f dev  multi/ceiling %.3f  %s' % (
+                      K, b, res['multi_dev_ms'], res['multi_host_ms'], K, res['singles_dev_ms'], res['singles_host_ms'],
+                      res['ceiling_dev_ms'], res['ceiling_host_ms'], res['speedup_host'], res['speedup_dev'],
+                      res['multi_over_ceiling_dev'], 'bit-identical' if res['bit_identical'] else 'DIFFERENT'),
+                  flush=True)
+        multi.close()
+    for e in singles:
+        e.close()
+    doc = {'gpu': gpu_info(), 'workload': 'C2 emulator LinNet 4-256-256-256-14172, per-star n_obs 3000-7000, parity',
+           'reps': args.reps, 'rows': rows}
+    if args.out:
+        os.makedirs(args.out, exist_ok=True)
+        with open(os.path.join(args.out, 'multistar.json'), 'w') as f:
+            json.dump(doc, f, indent=1)
+    print(json.dumps(doc['gpu']))
+
+
+if __name__ == '__main__':
+    main()
