@@ -239,11 +239,9 @@ int64_t payne_ctx_query(PayneCtx* ctx, const char* key);
 /* Runtime switches: "precision" (PAYNE_PREC_*), "max_batch" (workspace slab, points), "timing" (0/1,
  * see payne_ctx_last_ms), "fast_tail" (0 forces the general-grid tail), "gemm_stack" (0: one launch per hidden layer instead of
  * one cluster launch for lin2..lin5; bit-identical), "tail_cluster" (transforms above
- * 16384 samples spread over a cluster of four CTAs: default 1 for 65536-sample transforms, 0 for 32768), "debug_skip" (profiling aid:
- * switches phases of the fused tail off, results are then meaningless; see csrc/tail.cuh).
+ * 16384 samples spread over a cluster of four CTAs: default 1 for 65536-sample transforms, 0 for 32768).
  * Environment, read once: PAYNE_TAIL_CLUSTER=0 (never use the cluster tail) / 1 (also for 32768-sample transforms), PAYNE_ROT_WINDOW=0 (no shared-memory slice of the rotation-kernel table),
- * PAYNE_GEMM_PDL=0 (no programmatic dependent launch along the layer chain), PAYNE_GEMM_STACK=0 (see "gemm_stack"),
- * PAYNE_GEMM_MULTICAST=1 (experimental GEMM variant: 2-CTA weight multicast; bit-exact, same speed). */
+ * PAYNE_GEMM_PDL=0 (no programmatic dependent launch along the layer chain), PAYNE_GEMM_STACK=0 (see "gemm_stack"). */
 int payne_ctx_set(PayneCtx* ctx, const char* key, int64_t value);
 
 /* Kernel unit-test hook: C[M,N] = A[M,K] . W[N,K]^T + bias[N] through the tensor-core GEMM of

@@ -29,9 +29,8 @@ its padded pitch, the output map sized to the workspace rows).  Labels 6 to 8 ha
 (payne_b200.cu leaves them NaN): there the library returns NaN spectra and NaN lnL without a status bit, which the test
 pins.
 
-Also here: the 2-CTA weight multicast (PAYNE_GEMM_MULTICAST=1) and PDL off (PAYNE_GEMM_PDL=0), both read once per
-process, run in a subprocess and must match the default bit for bit; and the tensor-map caches across a workspace
-that grows between two calls.
+Also here: PDL off (PAYNE_GEMM_PDL=0), read once per process, runs in a subprocess and must match the default bit for
+bit; and the tensor-map caches across a workspace that grows between two calls.
 """
 import math
 import os
@@ -417,9 +416,9 @@ def _run_variant(tmp_path, env_key, env_val):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('env_key,env_val', [('PAYNE_GEMM_MULTICAST', '1'), ('PAYNE_GEMM_PDL', '0')])
+@pytest.mark.parametrize('env_key,env_val', [('PAYNE_GEMM_PDL', '0')])
 def test_env_variants_are_bit_identical(tmp_path, env_key, env_val):
-    """Same MMAs in the same K order: multicasting the weight tile or launching without PDL changes no bit."""
+    """Same MMAs in the same K order: launching without PDL changes no bit."""
     got = _run_variant(tmp_path, env_key, env_val)
     ref = variant_outputs()
     assert sorted(got) == sorted(ref)

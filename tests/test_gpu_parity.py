@@ -326,33 +326,6 @@ def test_fuzz_far_points_sit_at_the_float32_noise_floor(seed, cfgs):
     assert gpu_fuzz.run(seed=seed, ncfg=max(cfgs) + 1, verbose=False, only=cfgs) == 0
 
 
-def test_gauss_stencil_agrees_with_fft_stage():
-    """Instrumental broadening as a real-space stencil (compact kernels) against the FFT convolution it
-    replaces, on the same points: the two are the same circular convolution (tail_stencil.cuh)."""
-    for name in ['c2', 'mini_joint', 'mid']:
-        cfg, g = load_case(name)
-        eng = _engine(cfg, 'parity')
-        th = torch.from_numpy(np.ascontiguousarray(np.vstack([g['theta'], cfg.draw(64, seed=8)]))).cuda()
-        eng.set('gauss_stencil', 1)                  # opt-in path (the FFT is the default: it is as fast)
-        if eng.query('gauss_stencil') != 1:
-            eng.close()
-            pytest.skip('library built without -DPAYNE_WITH_STENCIL=1 (the default: the stencil is no faster than '
-                        'the FFT stage and its shared memory comes out of the rotation-table window)')
-        fa, _, la = eng.model_batch(th)
-        la2 = eng.lnlike_batch(th)
-        eng.set('gauss_stencil', 0)
-        fb, _, lb = eng.model_batch(th)
-        fa, fb, la, lb, la2 = [t.cpu().numpy() for t in (fa, fb, la, lb, la2)]
-        assert np.array_equal(np.isnan(fa), np.isnan(fb)) and np.array_equal(np.isnan(la), np.isnan(lb))
-        fin = np.isfinite(fb)
-        assert np.max(np.abs(fa[fin] - fb[fin])) < 1.5e-7
-        ok = np.isfinite(lb)
-        assert np.all(np.abs(la[ok] - lb[ok]) <= np.maximum(1e-3, 1e-8 * np.abs(lb[ok])))
-        np.testing.assert_array_equal(np.nan_to_num(la, nan=7.0), np.nan_to_num(la2, nan=7.0))
-        assert eng.query('status') == 0
-        eng.close()
-
-
 @pytest.mark.parametrize('name', ['mini_smlp', 'mini_yst'])
 def test_legacy_output_layer_on_tensor_cores(name):
     """SMLP / YST1 in parity mode: hidden layers on CUDA cores, the wide output layer as a row-scaled

@@ -17,7 +17,7 @@ HDR = os.path.join(os.path.dirname(HERE), 'include', 'payne_b200.h')
 
 _GEMM = ['mlp_tc.cuh', 'mlp_simt.cuh']
 _FFT = ['fft.cuh', 'fft_ct.cuh', 'tail.cuh', 'obs_star.cuh']
-_FAST = _FFT + ['tail_fast.cuh', 'tail_stencil.cuh', 'tail_general.cuh']
+_FAST = _FFT + ['tail_fast.cuh', 'tail_general.cuh']
 # translation unit -> the headers whose change alters its object code
 UNITS = {
     'payne_b200.cu': ['mlp_simt.cuh', 'mlp_tc_types.h'] + _FAST + ['launchers.h', 'phot.cuh', 'continuum.cuh', 'tail_lsf.cuh'],

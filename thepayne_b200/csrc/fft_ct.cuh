@@ -577,30 +577,6 @@ __device__ __forceinline__ void ct_convolve_regrid(float2* z, const TwTab& tw, c
 #endif
 }
 
-// The same in two halves around the filter stage, for callers that choose between filter instantiations at run time
-// without duplicating the passes: ct_convolve_regrid_fwd; ct_filter_pairs<LOG2M>(z, tw, H, tid); ct_convolve_inv.
-template <int LOG2M>
-__device__ __forceinline__ void ct_convolve_regrid_fwd(float2* z, const TwTab& tw, const TwConst& tc, int tid,
-                                                       const float* row, int num, int den, float invden, float c,
-                                                       bool clean) {
-  if (clean) ct_pass0_regrid<LOG2M, true>(z, tw, tc, tid, row, num, den, invden, c);
-  else ct_pass0_regrid<LOG2M, false>(z, tw, tc, tid, row, num, den, invden, c);
-#if PAYNE_SHARED_PASSES
-  ct_fwd_mid_shared<LOG2M>(tw, tid);
-#else
-  ct_fft_forward_rest<LOG2M>(z, tw, tc, tid);
-#endif
-}
-template <int LOG2M>
-__device__ __forceinline__ void ct_convolve_inv(float2* z, const TwTab& tw, const TwConst& tc, int tid) {
-#if PAYNE_SHARED_PASSES
-  ct_inv_mid_shared<LOG2M>(tw, tid);
-  ct_fft_inverse_last<LOG2M>(z, tw, tc, tid);
-#else
-  ct_fft_inverse<LOG2M>(z, tw, tc, tid);
-#endif
-}
-
 template <int LOG2M, class HF>
 __device__ __forceinline__ void ct_convolve(float2* z, const TwTab& tw, const TwConst& tc, const HF& H, int tid) {
   ct_fft_forward<LOG2M>(z, tw, tc, tid);

@@ -71,23 +71,6 @@ __device__ __forceinline__ void tma_load_2d(const CUtensorMap* map, uint64_t* ba
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
 }
-// Same, delivered to the same CTA-relative offset (data and mbarrier signal) of every CTA in mask.
-__device__ __forceinline__ void tma_load_2d_mc(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster "
-      "[%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask) : "memory");
-}
-__device__ __forceinline__ void mma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
@@ -285,16 +268,12 @@ struct TcGemmArgs {
   long long a_grows, b_grows, out_gstride;
 };
 
-// MC = 1: the CTAs of a 2-CTA cluster work on the SAME weight tile for two different row tiles;
-// each loads half of the weight rows and TMA-multicasts them to both, so the weight operand
-// crosses L2->SMEM once per pair (measured: -25 % L2 reads, no change in time; see tc_multicast_enabled).
-template <int BN, int MODE, int EPI, int MC>
+template <int BN, int MODE, int EPI>
 __global__ void __launch_bounds__(TcThreads<MODE, EPI>::value, 1)
 tc_gemm_kernel(const __grid_constant__ TcMaps T, const __grid_constant__ TcGemmArgs G) {
   using Cfg = TcCfg<BN, MODE>;
   static_assert(Cfg::kPatchBytes > 0 || (EPI == 1 && MODE == kModeX3), "this epilogue needs its staging block");
   constexpr int NS = Cfg::kStages, NP = Cfg::kPlanes;
-  const uint32_t crank = MC ? ptx::cluster_ctarank() : 0u;
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* base = (unsigned char*)(((uintptr_t)smem_dyn + 1023) & ~(uintptr_t)1023);
   unsigned char* stages = base;
@@ -309,27 +288,24 @@ tc_gemm_kernel(const __grid_constant__ TcMaps T, const __grid_constant__ TcGemmA
   float* sscale = sbias + BN;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int num_m_true = (G.M + kBM - 1) / kBM, num_n = (G.N + BN - 1) / BN;
-  // with MC the two CTAs of a cluster walk pair-tiles in lockstep: row tile 2*mp + crank
-  const int num_m = MC ? (num_m_true + 1) / 2 : num_m_true;
+  const int num_m = (G.M + kBM - 1) / kBM, num_n = (G.N + BN - 1) / BN;
   const int tiles_per_group = num_m * num_n;
   const int num_tiles = tiles_per_group * G.groups;
   const int num_kb = (G.K + Cfg::kBK - 1) / Cfg::kBK;
-  const int tile0 = MC ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
-  const int tstep = MC ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  const int tile0 = (int)blockIdx.x;
+  const int tstep = (int)gridDim.x;
 
   if (warp == 0 && lane == 0) {
     for (int p = 0; p < NP; ++p) { ptx::prefetch_tmap(&T.a[p]); ptx::prefetch_tmap(&T.b[p]); }
   }
   if (warp == 1 && lane == 0) {
-    for (int s = 0; s < NS; ++s) { ptx::mbar_init(&full[s], 1); ptx::mbar_init(&empty[s], MC ? 2 : 1); }
+    for (int s = 0; s < NS; ++s) { ptx::mbar_init(&full[s], 1); ptx::mbar_init(&empty[s], 1); }
     for (int a = 0; a < 2; ++a) { ptx::mbar_init(&tfull[a], 1); ptx::mbar_init(&tempty[a], TcThreads<MODE, EPI>::kEpiWarps); }
     ptx::fence_barrier_init();
   }
   if (warp == 2) ptx::tmem_alloc(tmem_ptr, Cfg::kTmemCols);
   ptx::tc_fence_before();
   __syncthreads();
-  if (MC) ptx::cluster_sync_all();          // the peer's barriers must exist before anything is multicast
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   // Programmatic dependent launch: everything above (barriers, TMEM, descriptor prefetch) touched no
@@ -344,21 +320,18 @@ tc_gemm_kernel(const __grid_constant__ TcMaps T, const __grid_constant__ TcGemmA
       int s = 0; uint32_t ph = 0;
       for (int tile = tile0; tile < num_tiles; tile += tstep) {
         const int grp = tile / tiles_per_group, tig = tile - grp * tiles_per_group;
-        const int m0 = ((tig / num_n) * (MC ? 2 : 1) + (int)crank) * kBM, n0 = (tig % num_n) * BN;
+        const int m0 = (tig / num_n) * kBM, n0 = (tig % num_n) * BN;
         if (n0 >= (grp == G.groups - 1 ? G.n_last : G.N)) continue;       // narrower last group
         const int arow = (int)(grp * G.a_grows) + m0, brow = (int)(grp * G.b_grows) + n0;
         for (int kb = 0; kb < num_kb; ++kb) {
-          ptx::mbar_wait(&empty[s], ph ^ 1);     // MC: both CTAs' MMAs have released this slot
+          ptx::mbar_wait(&empty[s], ph ^ 1);
           unsigned char* st = stages + s * Cfg::kStageBytes;
           ptx::mbar_expect_tx(&full[s], Cfg::kStageBytes);
           const int k0 = kb * Cfg::kBK;
 #pragma unroll
           for (int p = 0; p < NP; ++p) {
             ptx::tma_load_2d(&T.a[p], &full[s], st + p * Cfg::kABytes, k0, arow);
-            unsigned char* bdst = st + NP * Cfg::kABytes + p * Cfg::kBBytes;
-            if (MC) ptx::tma_load_2d_mc(&T.b[p], &full[s], bdst + crank * (Cfg::kBBytes / 2), k0,
-                                        brow + (int)crank * (BN / 2), (uint16_t)3);
-            else ptx::tma_load_2d(&T.b[p], &full[s], bdst, k0, brow);
+            ptx::tma_load_2d(&T.b[p], &full[s], st + NP * Cfg::kABytes + p * Cfg::kBBytes, k0, brow);
           }
           if (++s == NS) { s = 0; ph ^= 1; }
         }
@@ -408,8 +381,7 @@ tc_gemm_kernel(const __grid_constant__ TcMaps T, const __grid_constant__ TcGemmA
               ptx::mma_tf32(d_main, da[0] + ko, db[0] + ko, idesc, first);
             }
           }
-          if (MC) ptx::mma_commit_mc(&empty[s], (uint16_t)3);   // release the slot in BOTH CTAs
-          else ptx::mma_commit(&empty[s]);             // frees the ring slot when the MMAs retire
+          ptx::mma_commit(&empty[s]);                  // frees the ring slot when the MMAs retire
           if (kb == num_kb - 1) ptx::mma_commit(&tfull[acc]);
           if (++s == NS) { s = 0; ph ^= 1; }
         }
@@ -423,7 +395,7 @@ tc_gemm_kernel(const __grid_constant__ TcMaps T, const __grid_constant__ TcGemmA
     int acc = 0; uint32_t aph = 0;
     for (int tile = tile0; tile < num_tiles; tile += tstep) {
       const int grp = tile / tiles_per_group, tig = tile - grp * tiles_per_group;
-      const int m0 = ((tig / num_n) * (MC ? 2 : 1) + (int)crank) * kBM, n0 = (tig % num_n) * BN;
+      const int m0 = (tig / num_n) * kBM, n0 = (tig % num_n) * BN;
       const int Ng = grp == G.groups - 1 ? G.n_last : G.N;         // this group's output width
       if (n0 >= Ng) continue;
       const int gcol = (int)(grp * G.b_grows);                     // bias / scale / output-column offset
@@ -566,7 +538,6 @@ tc_gemm_kernel(const __grid_constant__ TcMaps T, const __grid_constant__ TcGemmA
   }
   ptx::tc_fence_before();
   __syncthreads();
-  if (MC) ptx::cluster_sync_all();          // no multicast / remote commit may target a CTA that has left
   if (warp == 2) ptx::tmem_dealloc(tmem_base, Cfg::kTmemCols);
 }
 
@@ -788,18 +759,6 @@ inline void tc_free_acts(TcActs* a) {
   a->rows = 0;
 }
 
-// PAYNE_GEMM_MULTICAST=1 enables the 2-CTA weight multicast for the lin6 GEMM (each CTA of a pair
-// loads half of the weight tile and TMA-multicasts it to both).  Measured on B200 (C2, B=4096) it
-// removes 25 % of the L2 reads and changes the time by < 1 %: the kernel was never short of operand
-// bandwidth -- ncu's source view put ~75 % of its instructions in the old row-loop epilogue, and the
-// TMA-store epilogue (not multicast) is what lifted the tensor pipe from 40 % to 73 %.  Kept, off by
-// default; bit-identical to the default path (tests/test_gpu_emulator_shapes.py runs it in a subprocess).
-inline bool tc_multicast_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("PAYNE_GEMM_MULTICAST"); v = (e && e[0] == '1') ? 1 : 0; }
-  return v != 0;
-}
-
 // PAYNE_GEMM_PDL=0 switches programmatic dependent launch of the layer chain off.
 inline bool tc_pdl_enabled() {
   static int v = -1;
@@ -813,16 +772,15 @@ struct TcGroups {
   long long a_grows = 0, out_gstride = 0;
 };
 
-template <int BN, int MODE, int EPI, int MC>
-inline int tc_launch_impl(const TcActs& A, int K, const TcWeights& W, const float* bias, void* out0, void* out1,
-                          void* out2, long long ldc, float bias_shift, int M, int sm_count, cudaStream_t st,
-                          TcMapCache* cache = nullptr, long long map_rows = 0, const TcGroups* grp = nullptr,
-                          int out_cols = 0, const float* rscale = nullptr) {
+template <int BN, int MODE, int EPI>
+inline int tc_launch(const TcActs& A, int K, const TcWeights& W, const float* bias, void* out0, void* out1,
+                     void* out2, long long ldc, float bias_shift, int M, int sm_count, cudaStream_t st,
+                     TcMapCache* cache = nullptr, long long map_rows = 0, const TcGroups* grp = nullptr,
+                     int out_cols = 0, const float* rscale = nullptr) {
   using Cfg = TcCfg<BN, MODE>;
   static_assert(Cfg::kStages >= 2, "ring too shallow");
-  constexpr int kVariant = BN * 1000 + MODE * 100 + EPI * 10 + MC;
+  constexpr int kVariant = BN * 100 + MODE * 10 + EPI;
   const bool grouped = grp && grp->groups > 1;
-  if (grouped && MC) return PAYNE_E_UNSUPPORTED;
   // grouped: the maps span every group's rows of the planes (a_grows rows each)
   const long long mrows = grouped ? grp->groups * grp->a_grows : ((cache && map_rows >= M) ? map_rows : M);
   TcMaps local;
@@ -836,12 +794,13 @@ inline int tc_launch_impl(const TcActs& A, int K, const TcWeights& W, const floa
     for (int p = 0; p < Cfg::kPlanes; ++p) {
       const void* wp = MODE == kModeX3 ? W.xplane[p] : W.plane[p];
       if (make_tmap(&T.a[p], A.plane[p], mrows, K, A.ld, kBM, Cfg::kElemBytes)) return PAYNE_E_CUDA;
-      if (make_tmap(&T.b[p], wp, W.N, K, W.Kp, MC ? BN / 2 : BN, Cfg::kElemBytes)) return PAYNE_E_CUDA;
+      if (make_tmap(&T.b[p], wp, W.N, K, W.Kp, BN, Cfg::kElemBytes)) return PAYNE_E_CUDA;
     }
     for (int p = Cfg::kPlanes; p < 3; ++p) { T.a[p] = T.a[0]; T.b[p] = T.b[0]; }
     if (EPI == 0) {
+      // out_cols: output width of a grouped launch (a launch of one group writes W.N columns)
       const long long orows = grouped ? ((cache && map_rows >= M) ? map_rows : M) : mrows;
-      if (int rc = make_tmap_out(&T.c, out0, orows, out_cols > 0 ? out_cols : W.N, ldc)) return rc;
+      if (int rc = make_tmap_out(&T.c, out0, orows, (grouped && out_cols > 0) ? out_cols : W.N, ldc)) return rc;
     } else T.c = T.a[0];
     if (cache) {
       for (int i = 0; i < 7; ++i) cache->ptr[i] = key[i];
@@ -854,7 +813,7 @@ inline int tc_launch_impl(const TcActs& A, int K, const TcWeights& W, const floa
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return PAYNE_E_CUDA;
   if (dev >= 64 || !((attr_set >> dev) & 1ull)) {
-    if (cudaFuncSetAttribute(tc_gemm_kernel<BN, MODE, EPI, MC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    if (cudaFuncSetAttribute(tc_gemm_kernel<BN, MODE, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              Cfg::kSmem) != cudaSuccess) return PAYNE_E_CUDA;
     if (dev < 64) attr_set |= 1ull << dev;
   }
@@ -864,48 +823,17 @@ inline int tc_launch_impl(const TcActs& A, int K, const TcWeights& W, const floa
     G.out_gstride = grp->out_gstride;
   }
   const int num_m = (M + kBM - 1) / kBM, num_n = (G.N + BN - 1) / BN;
-  if (MC) {
-    const int pair_tiles = ((num_m + 1) / 2) * num_n;
-    int grid = 2 * pair_tiles < (sm_count & ~1) ? 2 * pair_tiles : (sm_count & ~1);
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TcThreads<MODE, EPI>::value); cfg.dynamicSmemBytes = Cfg::kSmem; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    if (cudaLaunchKernelEx(&cfg, tc_gemm_kernel<BN, MODE, EPI, MC>, T, G) != cudaSuccess) return PAYNE_E_CUDA;
-  } else {
-    const int tiles = num_m * num_n * G.groups;
-    const int grid = tiles < sm_count ? tiles : sm_count;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TcThreads<MODE, EPI>::value); cfg.dynamicSmemBytes = Cfg::kSmem;
-    cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = tc_pdl_enabled() ? 1 : 0;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    if (cudaLaunchKernelEx(&cfg, tc_gemm_kernel<BN, MODE, EPI, MC>, T, G) != cudaSuccess) return PAYNE_E_CUDA;
-  }
+  const int tiles = num_m * num_n * G.groups;
+  const int grid = tiles < sm_count ? tiles : sm_count;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TcThreads<MODE, EPI>::value); cfg.dynamicSmemBytes = Cfg::kSmem;
+  cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = tc_pdl_enabled() ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
+  if (cudaLaunchKernelEx(&cfg, tc_gemm_kernel<BN, MODE, EPI>, T, G) != cudaSuccess) return PAYNE_E_CUDA;
   return cudaGetLastError() == cudaSuccess ? PAYNE_OK : PAYNE_E_CUDA;
-}
-
-template <int BN, int MODE, int EPI>
-inline int tc_launch(const TcActs& A, int K, const TcWeights& W, const float* bias, void* out0, void* out1,
-                     void* out2, long long ldc, float bias_shift, int M, int sm_count, cudaStream_t st,
-                     TcMapCache* cache = nullptr, long long map_rows = 0, const TcGroups* grp = nullptr,
-                     int out_cols = 0, const float* rscale = nullptr) {
-  if (rscale)      // scaled rows (leaky-ReLU nets): the plain single-CTA kernel
-    return tc_launch_impl<BN, MODE, EPI, 0>(A, K, W, bias, out0, out1, out2, ldc, bias_shift, M, sm_count, st, cache,
-                                            map_rows, grp, out_cols, rscale);
-  if (grp && grp->groups > 1)
-    return tc_launch_impl<BN, MODE, EPI, 0>(A, K, W, bias, out0, out1, out2, ldc, bias_shift, M, sm_count, st, cache,
-                                            map_rows, grp, out_cols);
-  // multicast pays when many row tiles share each weight tile (the wide last layer)
-  if (EPI == 0 && BN >= 128 && M > kBM && tc_multicast_enabled())
-    return tc_launch_impl<BN, MODE, EPI, 1>(A, K, W, bias, out0, out1, out2, ldc, bias_shift, M, sm_count, st, cache,
-                                            map_rows);
-  return tc_launch_impl<BN, MODE, EPI, 0>(A, K, W, bias, out0, out1, out2, ldc, bias_shift, M, sm_count, st, cache,
-                                          map_rows);
 }
 
 inline int tc_launch_hidden_stack(const TcWeights* tcw, float* const* bias, int layers, int H, TcActs* a0, TcActs* a1,

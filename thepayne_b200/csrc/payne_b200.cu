@@ -299,14 +299,6 @@ int build_tail(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs) {
     T.discard_rows = !(e && e[0] == '0');
   }
   T.inst_scale = kFwhmFit;
-  {
-    // Opt-in ("1"): measured on B200 at C2 (sigma 3.8-5.6 px, 49-71 taps) the stencil's inner loop alone
-    // takes as long as the whole FFT convolution it replaces (tools/bench/stencil_bench.cu: 73 FMA/clk/SM
-    // as shipped, 106 with the coefficient loads removed; direct and FFT convolution need about the same
-    // flops at these widths), so the FFT stays the default.
-    const char* e = getenv("PAYNE_GAUSS_STENCIL");
-    T.gauss_stencil = (e && e[0] == '1');
-  }
   // log-uniform check (informational; enables the analytic regrid fast path later)
   double maxdev = 0.0;
   for (int i = 0; i < n; ++i)
@@ -1402,7 +1394,6 @@ int64_t payne_ctx_query(PayneCtx* c, const char* key) {
   if (k == "max_batch") return c->slab;
   if (k == "sm_count") return c->sm_count;
   if (k == "tail_grid") return c->tail_grid;
-  if (k == "gauss_stencil") return PAYNE_WITH_STENCIL && c->tail.gauss_stencil && c->fast.win_floats >= payne::kStSideFloats;
   if (k == "rot_window_floats") return c->fast.win_floats;
   if (k == "tail_cluster") return c->use_fast && c->allow_fast && c->use_cluster && c->allow_cluster;
   if (k == "gemm_stack") return c->use_stack;
@@ -1446,13 +1437,11 @@ int payne_ctx_set(PayneCtx* c, const char* key, int64_t value) {
   if (k == "tail_cluster") { c->allow_cluster = value != 0; return PAYNE_OK; }
   if (k == "gemm_stack") { c->use_stack = value != 0; return PAYNE_OK; }
   if (k == "tail_grid_cap") { c->grid_cap = (int)std::max<int64_t>(0, value); return PAYNE_OK; }
-  if (k == "debug_skip") { c->tail.debug_skip = (int)value; return PAYNE_OK; }
-  // Inst_R column holds the sigma-resolution getspec takes (predictspec.py:255-263) instead of the FWHM
-  // resolution the likelihood samples (genmod.py:82-85)
-  if (k == "gauss_stencil") { c->tail.gauss_stencil = value != 0; return PAYNE_OK; }
   if (k == "discard_rows") { c->tail.discard_rows = value != 0; return PAYNE_OK; }
   if (k == "rows_may_nan") { c->tail.rows_may_nan = value != 0; return PAYNE_OK; }
-  if (k == "inst_r_is_sigma") { c->tail.inst_scale = value ? 1.0 : payne::kFwhmFit; return PAYNE_OK; }   // profiling aid, see tail.cuh
+  // Inst_R column holds the sigma-resolution getspec takes (predictspec.py:255-263) instead of the FWHM
+  // resolution the likelihood samples (genmod.py:82-85)
+  if (k == "inst_r_is_sigma") { c->tail.inst_scale = value ? 1.0 : payne::kFwhmFit; return PAYNE_OK; }
   return fail(PAYNE_E_INVALID, "unknown key " + k);
 }
 

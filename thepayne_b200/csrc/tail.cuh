@@ -75,12 +75,9 @@ struct TailParams {
   double* model_out;        // [B, ld_flux] or null: row p holds the first n_obs of p's star
   int* status;              // device flag: bit0 = a point needed a larger FFT than the carve-out
   int B;
-  int gauss_stencil;        // fast tail: instrumental broadening as a real-space stencil when the kernel is compact
   double inst_scale;        // Inst_R -> sigma-resolution: 2.355 (genmod.py:83, FWHM given) or 1 (getspec callers)
   int discard_rows;         // fast tail: drop a consumed row's lines from L2 without write-back (discard.global.L2)
   int rows_may_nan;         // rows can hold NaN although the labels are finite (continuum emulator attached)
-  int debug_skip;           // profiling aid (fast tail): bit0/1 skip stage 1/2 (regrid in + transforms),
-                            // bit3 the regrid back, bit4 the final pass; results are garbage
   // Multi-GPU all-gather of lnL fused into the tail (payne_lnlike_batch_gather; fast and cluster tails): the thread
   // that writes a point's lnL also stores it into every peer's gathered buffer through the NVLink peer mappings, and
   // the last CTA to leave the kernel raises this rank's flag on every rank behind a system-scope fence.  g_world = 0: off.
@@ -119,18 +116,16 @@ struct PointSetup {
   double vsini_scale;   // |vsini| * sb_scale
   double D;             // Doppler factor
   double u0, inv_du;    // resampled grid of stage 2 (observed frame)
-  double x0t, rho;      // rest-frame grid point of thread tid and ratio per kTailThreads steps
+  double rho;           // rest-frame grid ratio per kTailThreads steps
   double du, rM;
   double lnD, u0t;      // u0t = ln w[i0] in the rest frame
   double poly[PAYNE_MAX_POLY];
-  double sig_px2;       // instrumental kernel variance in pixels^2 of the stage-2 grid
   float taper_a;        // exp(-a k^2)
   float hdu;
   int do_rot, use_inst, bad, i0, i1, log2N2, clean;
 };
 
 // The point's star: observed pixels [off, off + n) of the concatenated arrays (0 pixels for an invalid star).
-// (Not in PointSetup: the fast tails' per-point record keeps the layout its kernels were tuned with.)
 struct ObsSlice {
   int off, n;
 };
@@ -333,7 +328,6 @@ static __device__ void tail_setup(const TailParams& P, const double* th, int p, 
   const double dv = kCkms * S.du;                  // smoothing.py:282
   const double nd = (double)N2 * dv;
   S.taper_a = (float)(2.0 * CUDART_PI * CUDART_PI * s2 / (nd * nd));
-  S.sig_px2 = s2 / (dv * dv);
 }
 
 }  // namespace payne

@@ -16,31 +16,6 @@
 #include "tail.cuh"
 #include "tail_general.cuh"
 
-// Resident CTAs per SM the register budget is sized for (transforms up to 16384 samples).  Measured at
-// C2: 3 (80 registers, a few spills) 0.76 ms; 2 (128 registers, no spills) 0.84 ms -- the convolution
-// core alone is 3 % faster with 2, but the latency-bound regrid / final phases lose a third of their warps.
-#ifndef PAYNE_TAIL_MINB
-#define PAYNE_TAIL_MINB 3
-#endif
-// The real-space stencil for the Gaussian stage (tail_stencil.cuh) is compiled in only on request
-// (-DPAYNE_WITH_STENCIL=1): measured on B200 it is no faster than the FFT convolution at C2's kernel widths,
-// and its 1.7 KB of static shared memory come out of the rotation-table window of every point.
-#ifndef PAYNE_WITH_STENCIL
-#define PAYNE_WITH_STENCIL 0
-#endif
-// A second, window-only instantiation of the rotation filter for points whose whole table range is staged (no per-lookup
-// choice, no table-end test) measured 1 % SLOWER at C2 both in round 2's first build (1.7 %) and with the shared passes
-// (0.6825 -> 0.689 ms, A/B on one box): off.
-// L2 prefetch (cp.async.bulk.prefetch.L2) of the row a CTA will work on next, issued when the point is claimed: measured
-// 0.6 % SLOWER at C2 (0.6823 -> 0.6864 ms, A/B on one box) -- with three CTAs per SM in different phases the row loads of the
-// fused first pass already overlap other CTAs' work, and the early fetch competes for L2 with rows still in use.  Off.
-#ifndef PAYNE_TAIL_PREFETCH
-#define PAYNE_TAIL_PREFETCH 0
-#endif
-#ifndef PAYNE_ROT_WINONLY
-#define PAYNE_ROT_WINONLY 0
-#endif
-
 namespace payne {
 
 struct FastGrid {
@@ -70,20 +45,11 @@ struct FastGrid {
 struct FastSetup {
   int s_incj, s_incr, s_den, s_num;   // stage 2: num = nM-1, den = N2-1, inc for pairs (2*256*num)
   float s_invden;
-  int st_R;                           // > 0: stage 2 is the real-space stencil of tail_stencil.cuh, half-width R
-  union {
-    struct {
-      int st_e4, st_n4;               // first coefficient step (in units of 4) and number of 4-step groups
-      double st_inv2s2;               // 1 / (2 sigma_px^2)
-    };
-    // cluster tail (contexts that have it never take the stencil, st_R = 0): first observed pixel at or beyond
-    // sample (r+1) N2/4 (the star's pixels sorted; jcut[0] = -1: not sorted, every CTA scans the star's pixels).
-    // Shares the stencil's bytes: the record sits in static shared memory and every 16 bytes of it come out of
-    // the rotation-table window.
-    int jcut[3];
-  };
+  // cluster tail: first observed pixel at or beyond sample (r+1) N2/4 (the star's pixels sorted; jcut[0] = -1: not
+  // sorted, every CTA scans the star's pixels)
+  int jcut[3];
   double q0, scale;                   // final: p = (obs_q - q0) * scale
-  ObsSlice obs;                       // the point's star (fills the record's padding: sizeof(FastPoint) stays 320)
+  ObsSlice obs;                       // the point's star
 };
 
 // Per-point setup, computed by tail_setup_kernel (one thread per point) ahead of the tail so that
@@ -341,10 +307,6 @@ __device__ __forceinline__ double final_pass(const TailParams& P, const FastGrid
   return acc;
 }
 
-}  // namespace payne
-#include "tail_stencil.cuh"
-namespace payne {
-
 // Drop the L2 lines lying wholly inside row[0, n) without write-back.  Not inlined on purpose: the tail kernel
 // sits at its 80-register cap, and these few instructions inlined at the end of the point loop changed the
 // allocation of the whole kernel (+1.5 % time).
@@ -359,17 +321,15 @@ static __device__ __noinline__ void discard_lines(const float* row, int n, int t
 // LOG2N1 == 16: split transform, half in shared memory (128 KB), half in the scratch line.
 // POLY: continuum polynomial and / or model output in the final pass (the host picks the instantiation).
 // STARS: a context of several stars (obs_lo / obs_hi).
+// (3 CTAs/SM, 80 registers with a few spills, measured at C2 0.76 ms against 0.84 ms with 2 CTAs/SM and no spills)
 template <int LOG2N1, bool POLY, bool STARS>
-__global__ void __launch_bounds__(kNT, LOG2N1 <= 14 ? PAYNE_TAIL_MINB : 1)
+__global__ void __launch_bounds__(kNT, LOG2N1 <= 14 ? 3 : 1)
 tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float2* z = reinterpret_cast<float2*>(smem_raw);
   float* zf = reinterpret_cast<float*>(smem_raw);
   __shared__ FastPoint SP;
   __shared__ double red[kNT / 32];
-#if PAYNE_WITH_STENCIL
-  __shared__ StencilShared SS;
-#endif
   PointSetup& S = SP.S;
   FastSetup& FS = SP.FS;
   const int tid = threadIdx.x;
@@ -398,14 +358,6 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
       reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(points + p) + tid);
     __syncthreads();
     pn = s_next;
-#if PAYNE_TAIL_PREFETCH
-    // the row of the point this CTA will work on next: from HBM into L2 now, so that its first pass finds it there
-    // (the slab is larger than L2: every row's first touch is a DRAM access otherwise)
-    if (tid == 0 && pn < P.B) {
-      const float* nrow = P.flux + (long long)pn * P.ldf;
-      asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(nrow), "r"((unsigned)((P.n * 4) & ~15)) : "memory");
-    }
-#endif
     if (S.bad) {
       if (P.model_out)
         for (int j = tid; j < obs_hi<STARS>(P, FS.obs) - obs_lo<STARS>(FS.obs); j += kNT) P.model_out[(long long)p * P.ld_flux + j] = nan;
@@ -426,32 +378,15 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
       float4* win4 = reinterpret_cast<float4*>(win);
       const int nwin = (int)fmin(fmin(xt_max + 2.0, (double)(F.win_floats >> 2)), (double)P.ntab);
       // (the window holds the first intervals of the one table: what an earlier point of this CTA staged stays valid)
-      if (PAYNE_WITH_STENCIL) win_have = 0;               // (the stencil stage reuses the window's space)
       for (int i = win_have + tid; i < nwin; i += kNT) win4[i] = __ldg(P.sbtab + i);
       win_have = max(win_have, nwin);
-      // (one filter instantiation with a per-lookup choice: see PAYNE_ROT_WINONLY)
       const RotHT<2> H{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, 1.0f / (float)(N1 >> 1), P.ntab, RotHT<2>::fix40(S.vsini_scale)};
       // pixels stage 2 will read: its mask [i0, i1] (one more on each side keeps the edge patch exact)
       const int blo = S.use_inst ? max(S.i0 - 1, 0) : 0, bhi = S.use_inst ? min(S.i1 + 1, n - 1) : n - 1;
       if constexpr (!kSplit) {
         // regrid fused into the first FFT pass (measured against the separate regrid: tail -5 %)
-        if (!(P.debug_skip & 1)) {
-#if PAYNE_ROT_WINONLY
-          // a point whose whole table range sits in the window (vsini <= ~5 km/s at C2) takes the filter
-          // instantiation without the per-lookup choice and the table-end test; only the filter stage is duplicated
-          ct_convolve_regrid_fwd<LOG2N1 - 1>(z, tw, F.twc, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
-          if (xt_max + 2.0 <= (double)nwin && H.s40 != ~0ull) {
-            const RotHT<1> H1{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, H.invM, P.ntab, H.s40};
-            ct_filter_pairs<LOG2N1 - 1>(z, tw, H1, tid);
-          } else {
-            ct_filter_pairs<LOG2N1 - 1>(z, tw, H, tid);
-          }
-          ct_convolve_inv<LOG2N1 - 1>(z, tw, F.twc, tid);
-#else
-          ct_convolve_regrid<LOG2N1 - 1>(z, tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
-#endif
-        }
-        if (!(P.debug_skip & 8)) regrid_back(row, zs, F, tid, n, N1, blo, bhi);
+        ct_convolve_regrid<LOG2N1 - 1>(z, tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
+        regrid_back(row, zs, F, tid, n, N1, blo, bhi);
       } else {
         stage_regrid(S, row, zp, tid, N1, F.f_num, F.f_den, 0, F.f_invden, F.c_native, F.f_incj, F.f_incr);
         __syncthreads();
@@ -469,12 +404,6 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
       GaussH H{S.taper_a, 2.0f / (float)N2};
       bool split2 = false;
       if constexpr (kSplit) split2 = (log2N2 == LOG2N1);
-#if PAYNE_WITH_STENCIL
-      if (!kSplit && FS.st_R > 0) {
-        // compact Gaussian: circular real-space stencil instead of the second transform pair
-        acc = stage2_stencil(P, F, S, FS, zf, win, SS, row, tid, p);
-      } else
-#endif
       if (split2) {
         if constexpr (kSplit) {
           stage_regrid(S, row, zp, tid, N2, FS.s_num, FS.s_den, i0, FS.s_invden, F.c_native, FS.s_incj, FS.s_incr);
@@ -493,14 +422,13 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
           fft_forward(z, log2N2 - 1, plan, twr, tid, kNT);
           filter_pairs(z, log2N2 - 1, plan, twr, H, tid, kNT);
           fft_inverse(z, log2N2 - 1, plan, twr, tid, kNT);
-        } else if (!(P.debug_skip & 2)) {
-          if (log2N2 == LA)
-            ct_convolve_regrid<LA - 1>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den, FS.s_invden, F.c_native, S.clean != 0);
-          else
-            ct_convolve_regrid<(LA >= 10 ? LA - 2 : 8)>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den,
-                                                         FS.s_invden, F.c_native, S.clean != 0);
+        } else if (log2N2 == LA) {
+          ct_convolve_regrid<LA - 1>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den, FS.s_invden, F.c_native, S.clean != 0);
+        } else {
+          ct_convolve_regrid<(LA >= 10 ? LA - 2 : 8)>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den,
+                                                       FS.s_invden, F.c_native, S.clean != 0);
         }
-        if (!(P.debug_skip & 16)) acc = final_pass<POLY, STARS>(P, F, S, FS, zs, tid, p, N2);
+        acc = final_pass<POLY, STARS>(P, F, S, FS, zs, tid, p, N2);
       }
     } else {
       // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289)
@@ -568,20 +496,6 @@ tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ 
     FS.s_invden = 1.0f / (float)(N2 - 1);
     FS.scale = (double)(N2 - 1) / (double)(nM - 1);
     FS.q0 = (double)S.i0 + S.lnD * F.inv_dlnw;
-    // stencil instead of the FFT when the kernel is compact and resolved (tail_stencil.cuh); the signal
-    // must fit the shared-memory transform buffer (no split transforms) and fill whole chunks
-    const double spx = sqrt(S.sig_px2);
-    const int R = (int)ceil(kStSigmas * spx);
-    // (the stencil's final pass walks the pixels of a single-star context: off with several stars)
-    if (PAYNE_WITH_STENCIL && P.gauss_stencil && P.n_stars == 1 && !P.rows_may_nan && spx >= kStMinSigmaPx && R <= kStMaxR && S.log2N2 >= 11 && S.log2N2 <= 15 &&
-        F.win_floats >= kStSideFloats) {
-      const int E = (R + 2) / 2;                       // offsets 2e-1, 2e, 2e+1 must cover [-R, R]
-      FS.st_R = R;
-      FS.st_e4 = -((E + 3) / 4);
-      FS.st_n4 = (E - 4 * FS.st_e4) / 4 + 1;
-      FS.st_inv2s2 = 0.5 / S.sig_px2;
-    }
-    if (F.cluster) FS.st_R = 0;
     if (F.cluster && P.stars[star_of(P.star, P.n_stars, p)].sorted) {
       // tail_cluster.cuh: CTA r of the cluster serves the observed pixels whose position falls into quarter r
       for (int r = 0; r < 3; ++r) {
