@@ -24,6 +24,8 @@
  *   payne_ctx_create_stars, payne_*_stars   one context for the observations of many stars that share the
  *                           emulators and the parameter layout (likelihood.__init__ per star; a survey fits
  *                           thousands of stars with one emulator): every point of a batch names its star.
+ *   payne_ctx_create_stars_opts  the same with each star's own fixed parameter values (fitstar.py:193-198 per star),
+ *                           photometric bands (likelihood.py:109-112 over the star's obs_phot) and LSF vector.
  *
  * Conventions: plain pointers and sizes only; every function returns 0 on success or a
  * negative PAYNE_E_* code and never throws; payne_last_error() gives the message of the
@@ -47,7 +49,7 @@
 extern "C" {
 #endif
 
-#define PAYNE_ABI_VERSION 6
+#define PAYNE_ABI_VERSION 7
 
 enum {
   PAYNE_OK = 0,
@@ -152,13 +154,37 @@ int payne_ctx_create(const PayneSpecNet* spec, const PaynePhotNet* phot, const P
                      const PayneLayout* layout, int device, PayneCtx** out);
 
 /* Observation set: obs is an array of n_stars PayneObs, HOST pointers, copied.  Every star must have the same nb
- * (= phot->nb when phot_bool).  Star k keeps its own n_obs, wavelength range, sort order and Chebyshev
+ * (= phot->nb when phot_bool; payne_ctx_create_stars_opts lifts this with band lists).  Star k keeps its own n_obs, wavelength range, sort order and Chebyshev
  * normalisation (polycalc on its own wave, fitutils.py:13-14).  The emulators, the parameter layout and every table
  * built from the emulator grid are shared.  A single-star context is the case n_stars = 1.
  * On a context of several stars, payne_ctx_set_lsf (the LSF vector is per observed pixel) and payne_gather_create
  * (the fused all-gather has no star argument) return PAYNE_E_UNSUPPORTED; payne_ctx_attach_continuum works. */
 int payne_ctx_create_stars(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs,
                            int32_t n_stars, const PayneLayout* layout, int device, PayneCtx** out);
+
+/* What may differ between the stars of an observation set besides the observation itself; HOST pointers, copied. */
+typedef struct {
+  const double*  fixed;  /* [PAYNE_NPAR] or NULL (= layout->fixed): this star's values of the parameters the layout
+                            does not sample (col < 0); NaN = absent, as in PayneLayout */
+  const int32_t* band;   /* [PayneObs.nb] or NULL: photometry-net band of each of this star's magnitudes, in PayneObs
+                            order, distinct, in [0, phot->nb); NULL = net order (then PayneObs.nb == phot->nb) */
+  const double*  lsf;    /* [PayneObs.n_obs] or NULL: dispersion (AA) at every observed pixel, as payne_ctx_set_lsf */
+} PayneStarOpts;
+
+/* payne_ctx_create_stars with per-star options: opts is an array of n_stars PayneStarOpts or NULL
+ * (payne_ctx_create_stars = this with opts NULL; a star whose fields are all NULL is a star of that call).
+ *   fixed: star k's row replaces the layout's fixed values everywhere they are read (emulator labels, Vrad, Vrot,
+ *          Inst_R, the photometry parameters).
+ *   band:  PayneObs.nb may differ between stars.  A star's SED chi2 is summed over its own bands in its PayneObs
+ *          order; payne_model_batch_stars writes row p's magnitudes in that order into columns [0, nb_k) of the
+ *          [B, phot->nb] output and leaves the other columns unwritten.  Out of range, duplicated or too many
+ *          entries: PAYNE_E_INVALID.
+ *   lsf:   given for every star or for none (a mix is PAYNE_E_UNSUPPORTED: the LSF tail and the scalar-R tails are
+ *          different kernels); every vector is checked as payne_ctx_set_lsf checks one, and while the vectors are set
+ *          Inst_R is ignored.  The vectors are fixed at creation: payne_ctx_set_lsf still refuses several stars. */
+int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs,
+                                const PayneStarOpts* opts, int32_t n_stars, const PayneLayout* layout, int device,
+                                PayneCtx** out);
 void payne_ctx_destroy(PayneCtx* ctx);
 
 /* theta_dev: [B, ld] fp64 row-major on the device.  lnl_dev: [B] fp64.

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PAYNE_LIB_PATH: development override (an instrumented build of the same sources)
 LIB_PATH = os.environ.get('PAYNE_LIB_PATH') or os.path.join(HERE, 'libpayne_b200.so')
 
-ABI_VERSION = 6          # PAYNE_ABI_VERSION of include/payne_b200.h the ctypes structs below mirror
+ABI_VERSION = 7          # PAYNE_ABI_VERSION of include/payne_b200.h the ctypes structs below mirror
 NPAR = 13
 MAX_POLY = 16
 PAR_INDEX = {
@@ -27,7 +27,7 @@ EXPORTS = ['payne_abi_version', 'payne_last_error', 'payne_ctx_create', 'payne_c
            'payne_ctx_attach_continuum', 'payne_ctx_set_lsf',
            'payne_gather_create', 'payne_gather_connect', 'payne_lnlike_batch_gather', 'payne_gather_flush',
            'payne_ctx_create_stars', 'payne_lnlike_batch_stars', 'payne_lnlike_batch_stars_host',
-           'payne_model_batch_stars']
+           'payne_model_batch_stars', 'payne_ctx_create_stars_opts']
 GATHER_HANDLE_BYTES = 128
 
 _f = C.POINTER(C.c_float)
@@ -50,6 +50,10 @@ class PaynePhotNet(C.Structure):
 class PayneObs(C.Structure):
     _fields_ = [('n_obs', C.c_int32), ('wave', _d), ('flux', _d), ('eflux', _d),
                 ('nb', C.c_int32), ('phot_mag', _d), ('phot_err', _d)]
+
+
+class PayneStarOpts(C.Structure):
+    _fields_ = [('fixed', _d), ('band', C.POINTER(C.c_int32)), ('lsf', _d)]
 
 
 class PayneLayout(C.Structure):
@@ -89,6 +93,10 @@ def load():
     lib.payne_ctx_create_stars.restype = C.c_int
     lib.payne_ctx_create_stars.argtypes = [C.POINTER(PayneSpecNet), C.POINTER(PaynePhotNet), C.POINTER(PayneObs),
                                            C.c_int32, C.POINTER(PayneLayout), C.c_int, C.POINTER(vp)]
+    lib.payne_ctx_create_stars_opts.restype = C.c_int
+    lib.payne_ctx_create_stars_opts.argtypes = [C.POINTER(PayneSpecNet), C.POINTER(PaynePhotNet), C.POINTER(PayneObs),
+                                                C.POINTER(PayneStarOpts), C.c_int32, C.POINTER(PayneLayout), C.c_int,
+                                                C.POINTER(vp)]
     lib.payne_lnlike_batch_stars.restype = C.c_int
     lib.payne_lnlike_batch_stars.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, vp]
     lib.payne_lnlike_batch_stars_host.restype = C.c_int

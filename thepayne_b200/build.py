@@ -15,7 +15,7 @@ OBJ = os.path.join(CSRC, '_build')
 OUT = os.path.join(HERE, 'libpayne_b200.so')
 HDR = os.path.join(os.path.dirname(HERE), 'include', 'payne_b200.h')
 
-_GEMM = ['mlp_tc.cuh', 'mlp_simt.cuh']
+_GEMM = ['mlp_tc.cuh', 'mlp_simt.cuh', 'obs_star.cuh']
 _FFT = ['fft.cuh', 'fft_ct.cuh', 'tail.cuh', 'obs_star.cuh']
 _FAST = _FFT + ['tail_fast.cuh', 'tail_general.cuh']
 # translation unit -> the headers whose change alters its object code

@@ -170,6 +170,7 @@ struct PayneCtx {
   long long n_obs_total = 0;
   std::vector<payne::ObsStar> stars;    // host copy of the records
   payne::ObsStar* stars_dev = nullptr;
+  double* star_fixed_dev = nullptr;     // [n_stars, PAYNE_NPAR] per-star fixed values (payne_ctx_create_stars_opts), or null
   // photometry
   bool has_phot = false;
   payne::PhotParams phot{};
@@ -638,12 +639,33 @@ int build_spec(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs, bool emu
   return PAYNE_OK;
 }
 
-int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs) {
+int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs, const PayneStarOpts* opts) {
   using namespace payne;
-  for (int k = 0; k < c->n_stars; ++k)
-    if (p->nb != obs[k].nb)
-      return fail(PAYNE_E_INVALID, "photometry net and observation of star " + std::to_string(k) + " disagree on nb");
   const int nb = p->nb, H = p->H;
+  // band list of every star: net band of each of its magnitudes; none given = the net's order
+  bool any_band = false;
+  for (int k = 0; k < c->n_stars; ++k) any_band |= opts && opts[k].band;
+  std::vector<int> band_slot(any_band ? (size_t)c->n_stars * nb : 0, -1);
+  for (int k = 0; k < c->n_stars; ++k) {
+    const int32_t* band = opts ? opts[k].band : nullptr;
+    if (!band) {
+      if (p->nb != obs[k].nb)
+        return fail(PAYNE_E_INVALID, "photometry net and observation of star " + std::to_string(k) + " disagree on nb");
+      for (int b = 0; b < nb && any_band; ++b) band_slot[(size_t)k * nb + b] = b;
+      continue;
+    }
+    if (obs[k].nb < 0 || obs[k].nb > nb)
+      return fail(PAYNE_E_INVALID, "star " + std::to_string(k) + ": " + std::to_string(obs[k].nb) +
+                  " magnitudes but the photometry net has " + std::to_string(nb) + " bands");
+    for (int i = 0; i < obs[k].nb; ++i) {
+      if (band[i] < 0 || band[i] >= nb)
+        return fail(PAYNE_E_INVALID, "star " + std::to_string(k) + ": band " + std::to_string(band[i]) + " outside [0, " +
+                    std::to_string(nb) + ")");
+      int& sl = band_slot[(size_t)k * nb + band[i]];
+      if (sl >= 0) return fail(PAYNE_E_INVALID, "star " + std::to_string(k) + ": band " + std::to_string(band[i]) + " given twice");
+      sl = i;
+    }
+  }
   PhotParams& P = c->phot;
   P.nb = nb; P.H = H;
   std::vector<float> w2t((size_t)nb * H * H);
@@ -661,13 +683,15 @@ int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs) {
   rc = upload_owned(c, &d6, p->b3, (size_t)nb); if (rc) return rc;
   P.w1 = d1; P.b1 = d2; P.w2t = d3; P.b2 = d4; P.w3 = d5; P.b3 = d6;
   for (int i = 0; i < 6; ++i) { P.xmin[i] = p->xmin[i]; P.xmax[i] = p->xmax[i]; }
-  // every star's magnitudes and errors back to back (star k at k * nb)
+  // every star's magnitudes and errors back to back, in its own order (without band lists star k is at k * nb)
   std::vector<double> mag, err;
   for (int k = 0; k < c->n_stars; ++k) {
-    if (nb > 0 && (!obs[k].phot_mag || !obs[k].phot_err)) return fail(PAYNE_E_INVALID, "null photometry array");
-    mag.insert(mag.end(), obs[k].phot_mag, obs[k].phot_mag + nb);
-    err.insert(err.end(), obs[k].phot_err, obs[k].phot_err + nb);
-    c->stars[k].phot_off = k * nb;
+    const int nbk = obs[k].nb;
+    if (nbk > 0 && (!obs[k].phot_mag || !obs[k].phot_err)) return fail(PAYNE_E_INVALID, "null photometry array");
+    c->stars[k].phot_off = (int)mag.size();
+    c->stars[k].nb = nbk;
+    mag.insert(mag.end(), obs[k].phot_mag, obs[k].phot_mag + nbk);
+    err.insert(err.end(), obs[k].phot_err, obs[k].phot_err + nbk);
   }
   double *h1, *h2, *h3;
   rc = upload_owned(c, &h1, p->hiav, (size_t)nb * 5); if (rc) return rc;
@@ -677,9 +701,59 @@ int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs) {
   for (int i = 0; i < PAYNE_NPAR; ++i) { P.col[i] = c->lay.col[i]; P.fixed[i] = c->lay.fixed[i]; }
   P.photscale = c->lay.photscale_bool;
   c->phot_smem = (size_t)2 * kPhotTile * H * sizeof(double);
+  if (any_band) {
+    int* ds = nullptr;
+    rc = upload_owned(c, &ds, band_slot.data(), band_slot.size()); if (rc) return rc;
+    P.band_slot = ds;
+    c->phot_smem += (size_t)kPhotTile * nb * sizeof(double);     // per-slot terms
+  }
   if (c->phot_smem > 200 * 1024) return fail(PAYNE_E_UNSUPPORTED, "photometry hidden width too large");
-  CU_TRY(cudaFuncSetAttribute(payne::phot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              (int)c->phot_smem));
+  CU_TRY(cudaFuncSetAttribute(any_band ? payne::phot_kernel<true> : payne::phot_kernel<false>,
+                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->phot_smem));
+  return PAYNE_OK;
+}
+
+// LSF tail (tail_lsf.cuh) for n_total observed pixels: occupancy probe, the vector and the per-CTA scratch.  Once
+// per context; the vector is then written by the caller.
+int lsf_alloc(PayneCtx* c, long long n_total) {
+  using namespace payne;
+  if (c->tail.log2N1 > 15) return fail(PAYNE_E_UNSUPPORTED, "LSF broadening is limited to emulator grids of 32768 pixels");
+  if (c->lsf.lsf) return PAYNE_OK;
+  LsfParams& L = c->lsf;
+  L.log2nx_max = std::min(15, c->tail.log2tw);
+  const size_t smem = (size_t)4 << std::max(L.log2nx_max, c->tail.log2N1);
+  int occ = 0;
+  if (!payne::probe_tail_lsf(smem, &occ) || occ < 1) return fail(PAYNE_E_UNSUPPORTED, "LSF tail kernel does not fit on an SM");
+  c->lsf_smem = smem; c->lsf_grid = occ * c->sm_count;
+  double* d = nullptr;
+  CU_TRY(cudaMalloc((void**)&d, (size_t)n_total * sizeof(double))); c->owned.push_back(d); L.lsf = d;
+  CU_TRY(cudaMalloc((void**)&d, (size_t)c->lsf_grid * c->D_out * sizeof(double))); c->owned.push_back(d); L.cdf = d;
+  CU_TRY(cudaMalloc((void**)&d, (size_t)c->lsf_grid * c->D_out * sizeof(double))); c->owned.push_back(d); L.aux = d;
+  CU_TRY(cudaMalloc((void**)&d, ((size_t)c->lsf_grid << L.log2nx_max) * sizeof(double))); c->owned.push_back(d); L.lam = d;
+  return PAYNE_OK;
+}
+
+// Per-star LSF vectors of payne_ctx_create_stars_opts: every star has one or none does; each is checked as
+// payne_ctx_set_lsf checks its vector and they go back to back like the observed pixels.
+int set_star_lsf(PayneCtx* c, const PayneObs* obs, const PayneStarOpts* opts) {
+  if (!opts) return PAYNE_OK;
+  int n_lsf = 0;
+  for (int k = 0; k < c->n_stars; ++k) n_lsf += opts[k].lsf != nullptr;
+  if (n_lsf == 0) return PAYNE_OK;
+  if (n_lsf != c->n_stars)
+    return fail(PAYNE_E_UNSUPPORTED, "an LSF vector for every star or for none (the LSF tail and the scalar-R tails are different kernels)");
+  if (!c->has_spec) return fail(PAYNE_E_INVALID, "context has no spectrum emulator");
+  std::vector<double> all;
+  all.reserve((size_t)c->n_obs_total);
+  for (int k = 0; k < c->n_stars; ++k)
+    for (int j = 0; j < obs[k].n_obs; ++j) {
+      if (!(opts[k].lsf[j] > 0.0)) return fail(PAYNE_E_INVALID, "LSF dispersions must be positive (star " + std::to_string(k) + ")");
+      all.push_back(opts[k].lsf[j]);
+    }
+  int rc = lsf_alloc(c, (long long)all.size());
+  if (rc) return rc;
+  CU_TRY(cudaMemcpy((void*)c->lsf.lsf, all.data(), all.size() * sizeof(double), cudaMemcpyHostToDevice));
+  c->lsf_on = true;
   return PAYNE_OK;
 }
 
@@ -871,7 +945,9 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         CU_TRY(cudaEventRecord(c->ev_join, c->side));
         c->launches++;
       }
-      rc = run_mlp(c, c->enc, th, ld, nb, c->flux, c->ldf, true, &is_depth, st);
+      EncodeParams E = c->enc;
+      E.star = star ? star + p0 : nullptr;
+      rc = run_mlp(c, E, th, ld, nb, c->flux, c->ldf, true, &is_depth, st);
       if (rc) return rc;
       if (c->cont) {
         // modspec *= np.interp(modwave, modcontwave, normalised F_lambda continuum) (predictspec.py:208-226)
@@ -881,7 +957,9 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         if (rc) return rc;
         int cdepth = 0;
         const long long l0 = cc->launches;
-        rc = run_mlp(cc, cc->enc, th, ld, nb, cc->flux, cc->ldf, true, &cdepth, st);
+        EncodeParams CE = cc->enc;
+        CE.star = E.star;
+        rc = run_mlp(cc, CE, th, ld, nb, cc->flux, cc->ldf, true, &cdepth, st);
         if (rc) return rc;
         if (!is_depth) return fail(PAYNE_E_UNSUPPORTED, "continuum multiply expects line-depth rows");
         ContParams C = c->contp;
@@ -897,7 +975,10 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
       P.mags_out = mags_out ? mags_out + p0 * P.nb : nullptr;
       P.star = star ? star + p0 : nullptr;
       P.status = c->status;
-      phot_kernel<<<(nb + kPhotTile - 1) / kPhotTile, kPhotThreads, c->phot_smem, st>>>(P);
+      if (P.band_slot)
+        phot_kernel<true><<<(nb + kPhotTile - 1) / kPhotTile, kPhotThreads, c->phot_smem, st>>>(P);
+      else
+        phot_kernel<false><<<(nb + kPhotTile - 1) / kPhotTile, kPhotThreads, c->phot_smem, st>>>(P);
       c->launches++;
     }
     if (c->timing) CU_TRY(cudaEventRecord(evs[2], st));
@@ -908,6 +989,7 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         TailParams TL = T;
         TL.col[PAYNE_P_INSTR] = -1;                                   // the vector replaces Inst_R
         TL.fixed[PAYNE_P_INSTR] = std::numeric_limits<double>::quiet_NaN();
+        TL.inst_scale = std::numeric_limits<double>::quiet_NaN();   // ... a star's own fixed Inst_R too (no scalar-R stage)
         if (payne::launch_tail_lsf(std::min(c->lsf_grid, nb), c->lsf_smem, st, TL, c->lsf)) return fail(PAYNE_E_CUDA, "tail launch");
       } else if (fast_tail && is_depth && c->use_cluster && c->allow_cluster) {
         payne::FastGrid FC = c->fast;
@@ -950,10 +1032,18 @@ int payne_ctx_create(const PayneSpecNet* spec, const PaynePhotNet* phot, const P
 
 int payne_ctx_create_stars(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs, int32_t n_stars,
                            const PayneLayout* layout, int device, PayneCtx** out) {
+  return payne_ctx_create_stars_opts(spec, phot, obs, nullptr, n_stars, layout, device, out);
+}
+
+int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs,
+                                const PayneStarOpts* opts, int32_t n_stars, const PayneLayout* layout, int device,
+                                PayneCtx** out) {
   if (!out || !layout || !obs) return fail(PAYNE_E_INVALID, "null argument");
   *out = nullptr;
   if (n_stars < 1) return fail(PAYNE_E_INVALID, "n_stars must be >= 1");
-  if (layout->phot_bool)
+  bool any_band = false, any_fixed = false;
+  for (int k = 0; opts && k < n_stars; ++k) { any_band |= opts[k].band != nullptr; any_fixed |= opts[k].fixed != nullptr; }
+  if (layout->phot_bool && !any_band)
     for (int k = 1; k < n_stars; ++k)
       if (obs[k].nb != obs[0].nb) return fail(PAYNE_E_INVALID, "every star must have the same nb (star " + std::to_string(k) + ")");
   if (layout->spec_bool && !spec) return fail(PAYNE_E_INVALID, "spec_bool set but no spectrum net");
@@ -984,11 +1074,20 @@ int payne_ctx_create_stars(const PayneSpecNet* spec, const PaynePhotNet* phot, c
   if (!rc && cudaMalloc((void**)&c->status, sizeof(int)) != cudaSuccess) rc = fail(PAYNE_E_NOMEM, "status");
   if (!rc) cudaMemset(c->status, 0, sizeof(int));
   if (!rc && c->has_spec) rc = build_spec(c, spec, obs);
-  if (!rc && c->has_phot) rc = build_phot(c, phot, obs);
+  if (!rc && c->has_phot) rc = build_phot(c, phot, obs, opts);
+  if (!rc) rc = set_star_lsf(c, obs, opts);
   if (!rc) rc = upload_owned(c, &c->stars_dev, c->stars.data(), c->stars.size());
+  if (!rc && any_fixed) {
+    // star k's row: its own values, or the layout's where it gives none
+    std::vector<double> fx((size_t)n_stars * PAYNE_NPAR);
+    for (int k = 0; k < n_stars; ++k)
+      std::memcpy(&fx[(size_t)k * PAYNE_NPAR], opts[k].fixed ? opts[k].fixed : layout->fixed, PAYNE_NPAR * sizeof(double));
+    rc = upload_owned(c, &c->star_fixed_dev, fx.data(), fx.size());
+  }
   if (!rc) {
     c->tail.stars = c->phot.stars = c->stars_dev;
-    c->tail.n_stars = c->phot.n_stars = n_stars;
+    c->tail.n_stars = c->phot.n_stars = c->enc.n_stars = n_stars;
+    c->tail.star_fixed = c->phot.star_fixed = c->enc.star_fixed = c->star_fixed_dev;
   }
   if (rc) { std::string keep = g_err; payne_ctx_destroy(c); g_err = keep; return rc; }
   *out = c;
@@ -1295,6 +1394,7 @@ int payne_ann_eval(PayneCtx* c, const double* x_dev, int64_t B, float* y_dev, in
   if (rc) return rc;
   payne::EncodeParams E = c->enc;
   for (int i = 0; i < E.D_in; ++i) E.col[i] = i;
+  E.star_fixed = nullptr;
   for (long long p0 = 0; p0 < B; p0 += c->slab) {
     const int nb = (int)std::min<long long>(c->slab, B - p0);
     int isd = 0;
@@ -1319,6 +1419,7 @@ int payne_ctx_attach_continuum(PayneCtx* c, const PayneSpecNet* cnet) {
   int rc = PAYNE_OK;
   if (cudaMalloc((void**)&cc->status, sizeof(int)) != cudaSuccess) rc = fail(PAYNE_E_NOMEM, "status");
   if (!rc) rc = build_spec(cc, cnet, nullptr, /*emulator_only=*/true);
+  cc->enc.star_fixed = c->enc.star_fixed; cc->enc.n_stars = c->enc.n_stars;   // labels: the same per-star values
   const int nc = cnet->D_out, n = c->D_out;
   cc->ldf = ((long long)nc + 3) / 4 * 4;
   std::vector<double> wc(cnet->wavelength, cnet->wavelength + nc), fac(nc);
@@ -1362,19 +1463,8 @@ int payne_ctx_set_lsf(PayneCtx* c, const double* lsf_host, int64_t n) {
   if (c->tail.log2N1 > 15) return fail(PAYNE_E_UNSUPPORTED, "LSF broadening is limited to emulator grids of 32768 pixels");
   for (int64_t j = 0; j < n; ++j)
     if (!(lsf_host[j] > 0.0)) return fail(PAYNE_E_INVALID, "LSF dispersions must be positive");
-  if (!c->lsf.lsf) {
-    LsfParams& L = c->lsf;
-    L.log2nx_max = std::min(15, c->tail.log2tw);
-    const size_t smem = (size_t)4 << std::max(L.log2nx_max, c->tail.log2N1);
-    int occ = 0;
-    if (!payne::probe_tail_lsf(smem, &occ) || occ < 1) return fail(PAYNE_E_UNSUPPORTED, "LSF tail kernel does not fit on an SM");
-    c->lsf_smem = smem; c->lsf_grid = occ * c->sm_count;
-    double* d = nullptr;
-    CU_TRY(cudaMalloc((void**)&d, (size_t)n * sizeof(double))); c->owned.push_back(d); L.lsf = d;
-    CU_TRY(cudaMalloc((void**)&d, (size_t)c->lsf_grid * c->D_out * sizeof(double))); c->owned.push_back(d); L.cdf = d;
-    CU_TRY(cudaMalloc((void**)&d, (size_t)c->lsf_grid * c->D_out * sizeof(double))); c->owned.push_back(d); L.aux = d;
-    CU_TRY(cudaMalloc((void**)&d, ((size_t)c->lsf_grid << L.log2nx_max) * sizeof(double))); c->owned.push_back(d); L.lam = d;
-  }
+  int rc = lsf_alloc(c, n);
+  if (rc) return rc;
   CU_TRY(cudaMemcpy((void*)c->lsf.lsf, lsf_host, (size_t)n * sizeof(double), cudaMemcpyHostToDevice));
   c->lsf_on = true;
   return PAYNE_OK;

@@ -93,6 +93,9 @@ struct TailParams {
   const ObsStar* stars;
   int n_stars;
   long long ld_flux;                 // model_out row stride
+  // Per-star fixed values (payne_ctx_create_stars_opts): [n_stars, PAYNE_NPAR], read where col < 0 in place of
+  // `fixed` / `label_fixed`; null when the context was created without them.
+  const double* star_fixed;
 };
 
 // lnL of point p: local result and, with the fused gather on, the copy in every peer's buffer
@@ -130,8 +133,9 @@ struct ObsSlice {
   int off, n;
 };
 
-__device__ __forceinline__ double get_par(const TailParams& P, const double* th, int which) {
-  return P.col[which] >= 0 ? th[P.col[which]] : P.fixed[which];
+// parameter `which` of point th of star k
+__device__ __forceinline__ double get_par(const TailParams& P, const double* th, int which, int k) {
+  return P.col[which] >= 0 ? th[P.col[which]] : fixed_of(P.star_fixed, P.fixed, k, which);
 }
 
 // float index of real sample k: 2*swz(k>>1) + (k&1) == k ^ (((k>>5)&7)<<2)
@@ -269,13 +273,15 @@ static __device__ void tail_setup(const TailParams& P, const double* th, int p, 
   }
   const ObsStar& st = P.stars[k];
   obs.off = st.off; obs.n = st.n_obs;
-  const double vrot = get_par(P, th, PAYNE_P_VROT);
-  const double vrad = get_par(P, th, PAYNE_P_VRAD);
-  const double instR = get_par(P, th, PAYNE_P_INSTR);
+  const double vrot = get_par(P, th, PAYNE_P_VROT, k);
+  const double vrad = get_par(P, th, PAYNE_P_VRAD, k);
+  const double instR = get_par(P, th, PAYNE_P_INSTR, k);
   S.bad = 0;
   S.clean = P.rows_may_nan ? 0 : 1;
   for (int i = 0; i < P.n_labels; ++i) {
-    const double v = P.label_col[i] >= 0 ? th[P.label_col[i]] : P.label_fixed[i];
+    const double v = P.label_col[i] >= 0 ? th[P.label_col[i]]
+                     : (P.star_fixed && label_param(i) >= 0 ? P.star_fixed[(long long)k * PAYNE_NPAR + label_param(i)]
+                                                            : P.label_fixed[i]);
     if (!isfinite(v)) S.clean = 0;
   }
   S.do_rot = (vrot != 0.0);                       // predictspec.py:231 (NaN != 0 is true)

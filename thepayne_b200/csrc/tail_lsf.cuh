@@ -22,7 +22,7 @@
 namespace payne {
 
 struct LsfParams {
-  const double* lsf;      // [n_obs] dispersion (AA) at the observed pixels
+  const double* lsf;      // dispersion (AA) at the observed pixels, the stars' vectors back to back like obs_w
   double* cdf;            // [grid, n]  scratch
   double* aux;            // [grid, n]  scratch: dw/sigma, then gradient(cdf)/(dw/sigma)
   double* lam;            // [grid, 2^log2nx_max] scratch
@@ -74,6 +74,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
   __shared__ int hist[256];
   __shared__ unsigned long long sh_prefix;
   __shared__ int sh_rank, sh_count, sh_i0, sh_i1;
+  __shared__ ObsSlice so;               // the point's star: observed pixels [off, off + n)
   const int tid = threadIdx.x;
   const Twiddles twr{P.tw, P.log2tw};
   const double nan = CUDART_NAN;
@@ -86,12 +87,12 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
     const double* th = P.theta + (long long)p * P.ld;
     float* row = P.flux + (long long)p * P.ldf;
     if (tid == 0) {
-      ObsSlice obs;                     // (star 0 throughout: the LSF vector is refused on several stars)
-      tail_setup(P, th, p, S, obs);            // Inst_R is absent in this mode: Doppler, rotation and polynomial only
+      tail_setup(P, th, p, S, so);             // Inst_R is absent in this mode: Doppler, rotation and polynomial only
       const double D = S.D;
-      const double lo = P.obs_min + 20.0 * 100.0 * -1.0, hi = P.obs_max + 20.0 * 100.0 * 1.0;   // smoothing.py:128, 643
       int i0 = n, i1 = -1;
       if (!S.bad) {
+        const ObsStar& st = P.stars[star_of(P.star, P.n_stars, p)];
+        const double lo = st.obs_min + 20.0 * 100.0 * -1.0, hi = st.obs_max + 20.0 * 100.0 * 1.0;   // smoothing.py:128, 643
         const double* w = P.w;
         auto ws = [w, D](int i) { return __ldg(w + i) * D; };
         if (ws(n - 1) > lo) i0 = ws(0) > lo ? 0 : last_le(ws, n, lo) + 1;        // first with w D > lo
@@ -104,9 +105,10 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
     }
     __syncthreads();
     const int i0 = sh_i0, i1 = sh_i1, nM = i1 - i0 + 1;
+    const int off = so.off, no = so.n;
     if (S.bad || nM < 17) {
       if (P.model_out)
-        for (int j = tid; j < P.n_obs; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
+        for (int j = tid; j < no; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
       if (tid == 0 && P.lnl) P.lnl[p] = nan;
       __syncthreads();
       continue;
@@ -145,13 +147,13 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
 
     // ---------------- dw / sigma on the masked, shifted emulator grid
     const double* w = P.w + i0;
-    const double* ow = P.obs_w;
-    const double* lsf = L.lsf;
+    const double* ow = P.obs_w + off;
+    const double* lsf = L.lsf + off;
     auto wave = [w, D](int i) { return __ldg(w + i) * D; };
     auto owf = [ow](int j) { return __ldg(ow + j); };
     auto lsff = [lsf](int j) { return __ldg(lsf + j); };
     for (int i = tid; i < nM; i += kTailThreads) {
-      const double disp = np_interp(wave(i), owf, lsff, P.n_obs);
+      const double disp = np_interp(wave(i), owf, lsff, no);
       const double dw = i == 0 ? wave(1) - wave(0)
                                : (i == nM - 1 ? wave(nM - 1) - wave(nM - 2) : (wave(i + 1) - wave(i - 1)) / 2.0);
       aux[i] = dw / disp;
@@ -194,7 +196,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
     if (log2nx < 5 || log2nx > L.log2nx_max) {
       if (tid == 0) { if (log2nx > L.log2nx_max) atomicOr(P.status, 1); if (P.lnl) P.lnl[p] = nan; }
       if (P.model_out)
-        for (int j = tid; j < P.n_obs; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
+        for (int j = tid; j < no; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
       __syncthreads();
       continue;
     }
@@ -230,10 +232,10 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
       auto lamf = [lamc](int k) { return lamc[k]; };
       const float* zc = zf;
       auto convf = [zc](int k) { return (double)zc[zidx(k)]; };
-      for (int j = tid; j < P.n_obs; j += kTailThreads) {
+      for (int j = off + tid; j < off + no; j += kTailThreads) {
         double m = 1.0 + np_interp(__ldg(P.obs_w + j), lamf, convf, nx);
         if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-        if (P.model_out) P.model_out[(long long)p * P.ld_flux + j] = m;
+        if (P.model_out) P.model_out[(long long)p * P.ld_flux + j - off] = m;
         const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
         acc += r * r;
       }

@@ -7,9 +7,14 @@ The parameter-vector convention is the reference's (Payne/fitting/likelihood.py:
 row of ``theta`` holds the free parameters in ``fitpars_i`` order, fixed ones come from
 ``fixedpars``, and spectral parameters that are neither are NaN.
 
-One context may hold the observations of many stars (``stars=[...]``): the emulators, the
-parameter layout and the fixed parameters are shared, and every row of a batch names its star.
+One context may hold the observations of many stars (``stars=[...]``): the emulators and the
+parameter layout are shared, and every row of a batch names its star.  Each star may bring its own
+fixed parameter values, its own subset of the photometric bands and its own LSF vector.
 A single-star engine is the case of one star.
+
+A fixed ``Inst_R`` that is a 1-D array is an LSF vector, the dispersion (AA) at every observed pixel,
+as in the reference (genmod.py:82-85 passes a non-float inst_R on to getspec's LSF branch,
+predictspec.py:265-286).
 """
 from __future__ import annotations
 
@@ -36,6 +41,21 @@ def _pf(a):
 
 def _pd(a):
     return a.ctypes.data_as(C.POINTER(C.c_double))
+
+
+def _split_fixed(fixedpars):
+    """fixedpars -> (PAYNE_NPAR fixed values with NaN where absent, LSF vector or None)."""
+    vals = np.full(_lib.NPAR, np.nan)
+    lsf = None
+    for name, k in PAR_INDEX.items():
+        if name not in fixedpars:
+            continue
+        v = fixedpars[name]
+        if name == 'Inst_R' and np.ndim(v) == 1:
+            lsf = _f64(v)
+        else:
+            vals[k] = float(v)
+    return vals, lsf
 
 
 def _specnet_struct(spec, keep):
@@ -78,7 +98,12 @@ class Engine:
                  precision='parity', device=None, stars=None):
         """``stars``: instead of ``obs_wave``, ``obs_flux``, ``obs_eflux`` and ``obs_phot``, a list of
         ``{'wave', 'flux', 'eflux', 'phot': {band: (mag, err)}}``, one per star; ``lnlike_batch`` and
-        ``model_batch`` then take the star index of every row."""
+        ``model_batch`` then take the star index of every row.  A star may also carry
+          ``'fixedpars'``: its fixed parameter values, in place of the shared ``fixedpars``;
+          ``'bands'``: the order of its magnitudes (its SED chi2 is summed in that order, likelihood.py:109-112).
+        Its ``'phot'`` keys may be any subset of the photometry net's bands; without ``'bands'`` they go in the
+        net's order.  A fixed ``Inst_R`` that is a 1-D array is the star's LSF vector (one dispersion per observed
+        pixel); every star has one or none does."""
         if stars is None:
             stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot}]
         elif any(v is not None for v in (obs_wave, obs_flux, obs_eflux, obs_phot)):
@@ -98,9 +123,10 @@ class Engine:
 
         lay = _lib.PayneLayout()
         lay.ndim = self.ndim
+        shared_vals, shared_lsf = _split_fixed(self.fixedpars)
         for name, k in PAR_INDEX.items():
             lay.col[k] = self.fitpars_i.index(name) if name in self.fitpars_i else -1
-            lay.fixed[k] = float(self.fixedpars[name]) if name in self.fixedpars else float('nan')
+            lay.fixed[k] = shared_vals[k]
         pcs = [i for i, p in enumerate(self.fitpars_i) if 'pc' in p]   # likelihood.py:56-57
         if modpoly_bool and len(pcs) > _lib.MAX_POLY:
             raise ValueError('at most %d continuum coefficients' % _lib.MAX_POLY)
@@ -119,6 +145,22 @@ class Engine:
             self.D_in, self.D_out = int(sp.D_in), int(sp.D_out)
         self.n_stars = len(stars)
         obs = (_lib.PayneObs * self.n_stars)()
+        opts = (_lib.PayneStarOpts * self.n_stars)()      # all fields NULL: the star has no option
+        self.star_fixedpars = [dict(st['fixedpars']) if st.get('fixedpars') is not None else self.fixedpars
+                               for st in stars]
+        for k, st in enumerate(stars):
+            vals, lsf = (shared_vals, shared_lsf) if st.get('fixedpars') is None else _split_fixed(st['fixedpars'])
+            if st.get('fixedpars') is not None:
+                keep.append(vals)
+                opts[k].fixed = _pd(vals)
+            if lsf is not None:
+                if not spec_bool:
+                    raise ValueError('an LSF vector (fixed Inst_R array) needs the spectrum emulator (star %d)' % k)
+                if len(lsf) != len(st['wave']):
+                    raise ValueError('star %d: the LSF vector needs one dispersion per observed pixel (%d, got %d)'
+                                     % (k, len(st['wave']), len(lsf)))
+                keep.append(lsf)
+                opts[k].lsf = _pd(lsf)
         self.n_obs_star = [0] * self.n_stars
         if spec_bool:
             for k, st in enumerate(stars):
@@ -131,6 +173,7 @@ class Engine:
         self.n_obs = max(self.n_obs_star)          # the largest star's
         ph = None
         self.bands = []
+        self.star_bands = [[] for _ in stars]
         if phot_bool:
             if phot is None or any(st.get('phot') is None for st in stars):
                 raise ValueError('phot_bool set but no photometry emulator / observation given')
@@ -145,16 +188,29 @@ class Engine:
             keep += [pxmin, pxmax, hiav]
             ph.xmin, ph.xmax, ph.hiav = _pd(pxmin), _pd(pxmax), _pd(hiav)
             for k, st in enumerate(stars):
-                mag = _f64([st['phot'][b][0] for b in self.bands])
-                err = _f64([st['phot'][b][1] for b in self.bands])
+                bands = list(st['bands']) if st.get('bands') is not None else \
+                    [b for b in self.bands if b in st['phot']]
+                unknown = [b for b in list(st['phot']) + bands if b not in self.bands]
+                if unknown:
+                    raise ValueError('star %d: bands %s are not in the photometry net' % (k, sorted(set(unknown))))
+                if sorted(bands) != sorted(st['phot']) or len(set(bands)) != len(bands):
+                    raise ValueError("star %d: 'bands' must list each of its 'phot' keys once" % k)
+                self.star_bands[k] = bands
+                mag = _f64([st['phot'][b][0] for b in bands])
+                err = _f64([st['phot'][b][1] for b in bands])
                 keep += [mag, err]
-                obs[k].nb, obs[k].phot_mag, obs[k].phot_err = len(self.bands), _pd(mag), _pd(err)
+                obs[k].nb, obs[k].phot_mag, obs[k].phot_err = len(bands), _pd(mag), _pd(err)
+                if bands != self.bands:
+                    idx = np.array([self.bands.index(b) for b in bands], dtype=np.int32)
+                    keep.append(idx)
+                    opts[k].band = idx.ctypes.data_as(C.POINTER(C.c_int32))
         self.nb = len(self.bands)
 
         ctx = C.c_void_p()
-        _lib.check(self.lib.payne_ctx_create_stars(C.byref(sp) if sp is not None else None,
-                                                    C.byref(ph) if ph is not None else None,
-                                                    obs, self.n_stars, C.byref(lay), self.device, C.byref(ctx)))
+        _lib.check(self.lib.payne_ctx_create_stars_opts(C.byref(sp) if sp is not None else None,
+                                                         C.byref(ph) if ph is not None else None,
+                                                         obs, opts, self.n_stars, C.byref(lay), self.device,
+                                                         C.byref(ctx)))
         self._ctx = ctx
         del keep
 
@@ -251,7 +307,7 @@ class Engine:
     def model_batch(self, theta, star=None, want_flux=True, want_mags=True):
         """Model spectra [B, n_obs], magnitudes [B, nb] and lnL [B] as CUDA float64 tensors.  With several
         stars, n_obs is the largest star's: row p holds the first ``n_obs_star[star[p]]`` pixels, the rest
-        stay NaN.  ``star`` as in ``lnlike_batch`` (numpy is copied to the device)."""
+        stay NaN; likewise row p of the magnitudes holds its star's ``star_bands[star[p]]``, the rest NaN.  ``star`` as in ``lnlike_batch`` (numpy is copied to the device)."""
         dev = torch.device('cuda', self.device)
         if not isinstance(theta, torch.Tensor):
             theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
@@ -262,7 +318,7 @@ class Engine:
         sv = self._star_dev(star.to(dev) if star is not None else None, B, dev)
         flux = torch.full((B, self.n_obs), float('nan'), dtype=torch.float64, device=dev) \
             if (want_flux and self.n_obs) else None
-        mags = torch.empty((B, self.nb), dtype=torch.float64, device=dev) if (want_mags and self.nb) else None
+        mags = torch.full((B, self.nb), float('nan'), dtype=torch.float64, device=dev) if (want_mags and self.nb) else None
         lnl = torch.empty(B, dtype=torch.float64, device=dev)
         st = torch.cuda.current_stream(dev).cuda_stream
         _lib.check(self.lib.payne_model_batch_stars(

@@ -29,9 +29,17 @@ class GenMod(object):
             self.filterarray = self.fppsed.filternames
 
     def genspec(self, pars, outwave=None, verbose=False, modpoly=False, carbon_bool=False):
-        """genmod.py:58-108: pars = [Teff, logg, FeH, aFe, Vrad, Vrot, Vmic, Inst_R, pc_0...]."""
+        """genmod.py:58-108: pars = [Teff, logg, FeH, aFe, Vrad, Vrot, Vmic, Inst_R, pc_0...].  An Inst_R that is a
+        1-D array is the LSF vector on ``outwave`` (genmod.py:82-85 -> predictspec.py:265-286)."""
         if carbon_bool:
             raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
+        pars = list(pars)
+        lsf = None
+        if np.ndim(pars[7]) == 1:
+            if outwave is None:
+                raise ValueError('an LSF vector Inst_R gives the dispersion at the pixels of outwave: give outwave')
+            lsf = np.ascontiguousarray(pars[7], dtype=np.float64)
+            pars[7] = np.nan                               # the vector replaces the scalar-R stage
         pars = [float(p) for p in pars]
         polycoef = pars[8:] if modpoly else []
         if outwave is None:
@@ -43,7 +51,7 @@ class GenMod(object):
                 from .fitutils import polycalc
                 flux = flux * polycalc(polycoef, wave)
             return wave, flux
-        eng = self.PP.anns.engine_for(outwave, npoly=len(polycoef))
+        eng = self.PP.anns.engine_for(outwave, npoly=len(polycoef), lsf=lsf)
         row = np.array([pars[:8] + list(polycoef)], dtype=np.float64)
         flux, _, _ = eng.model_batch(row, want_mags=False)
         return outwave, flux[0].cpu().numpy()

@@ -4,6 +4,10 @@
 The caller (dynesty through ``fitstar.lnprobfn``, fitstar.py:647-659) reads ``parsdict`` after
 ``lnlikefn``; after a batched call it holds the LAST row, which is what the reference's logging
 expects (fitstar.py:342-348).
+
+A fixed ``Inst_R`` that is a 1-D array is the LSF vector of the observation (one dispersion per observed
+pixel), as in the reference: lnlikefn passes it on to genspec, which hands a non-float ``inst_R`` to getspec's
+LSF branch (genmod.py:82-85, predictspec.py:265-286).
 """
 from __future__ import annotations
 
@@ -63,10 +67,16 @@ class likelihood(object):
     def lnlike(self, specpars=None, photpars=None):
         """Explicit ``specpars`` / ``photpars`` lists as built by lnlikefn (likelihood.py:84-117)."""
         names, vals = [], []
+        lsf = None
         if self.spec_bool:
-            sp = [float(v) for v in specpars]
-            names += _SPEC + ['pc_%d' % k for k in range(len(sp) - 8)]
-            vals += sp
+            sp = list(specpars)
+            if np.ndim(sp[7]) == 1:                     # an LSF vector in place of Inst_R (genmod.py:82-85)
+                lsf = np.ascontiguousarray(sp[7], dtype=np.float64)
+                names += [n for n in _SPEC if n != 'Inst_R'] + ['pc_%d' % k for k in range(len(sp) - 8)]
+                vals += [float(v) for v in sp[:7] + sp[8:]]
+            else:
+                names += _SPEC + ['pc_%d' % k for k in range(len(sp) - 8)]
+                vals += [float(v) for v in sp]
         if self.phot_bool:
             pp = list(photpars)
             pn = ['log(A)', 'Av'] if self.photscale_bool else ['log(R)', 'Dist', 'Av']
@@ -75,7 +85,7 @@ class likelihood(object):
                     continue
                 names.append(n)
                 vals.append(float(v))
-        key = tuple(names)
+        key = (tuple(names), None if lsf is None else lsf.tobytes())
         if self._explicit is None or self._explicit[0] != key:
             if self._explicit is not None:
                 self._explicit[1].close()
@@ -84,6 +94,7 @@ class likelihood(object):
                          phot=self.GM.fppsed.net if self.phot_bool else None,
                          obs_wave=fa.get('obs_wave_fit'), obs_flux=fa.get('obs_flux_fit'),
                          obs_eflux=fa.get('obs_eflux_fit'), obs_phot=fa.get('obs_phot'), fitpars_i=names,
+                         fixedpars=None if lsf is None else {'Inst_R': lsf},
                          runbools=[self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
                          precision=self.precision)
             self._explicit = (key, eng)

@@ -1,8 +1,10 @@
 """Fitting many stars at once: one engine for all their observations, and their samplers in lock-step.
 
-A survey fits thousands of stars with the same emulator.  Between two stars only the observation changes
-(wavelengths, fluxes, errors, magnitudes); the emulator weights, the parameter layout and every table built
-from the emulator grid stay the same.  A single star's sampler hands over a few hundred points per call, which
+A survey fits thousands of stars with the same emulator.  Between two stars the observation changes
+(wavelengths, fluxes, errors, which magnitudes and in what order), and so may the values of the fixed parameters
+(an instrumental resolution or LSF vector, a catalogue distance or extinction, an asteroseismic log(g)); the
+emulator weights, the free parameters, the names of the fixed ones and every table built from the emulator grid
+stay the same.  A single star's sampler hands over a few hundred points per call, which
 leaves the GPU latency-bound; the points of many stars together make one full-size batch.
 
 ``StarSetLikelihood`` builds one ``Engine`` holding every star's observation.  ``star(k)`` is a view with the
@@ -37,10 +39,14 @@ def _same(a, b):
 
 
 class StarSetLikelihood(object):
-    """The likelihoods of several stars that share emulators, free parameters, fixed parameters and bands.
+    """The likelihoods of several stars that share emulators, free parameters and the names of the fixed ones.
 
     ``fitargs_list``: one ``fitargs`` per star (as ``FitPayne.run`` builds them).  ``fitpars`` / ``runbools``:
-    one value for every star, or a list with one per star (they must then agree)."""
+    one value for every star, or a list with one per star (they must then agree).  Each star keeps its own fixed
+    values (a vector ``Inst_R`` is its LSF) and its own photometric bands: the photometry net covers the union of
+    the stars' bands in order of first appearance, and each star's SED chi2 is summed in its ``obs_phot`` order,
+    as a separate ``likelihood`` of that star sums it.  The fixed parameters' names must agree: they are the
+    columns of every star's output file."""
 
     def __init__(self, fitargs_list, fitpars, runbools, precision='parity', device=None):
         fitargs_list = list(fitargs_list)
@@ -63,10 +69,8 @@ class StarSetLikelihood(object):
                     raise ValueError('star %d: %s differs from star 0' % (k, key))
             if fa.get('NNtype', 'LinNet') != fa0.get('NNtype', 'LinNet'):
                 raise ValueError('star %d: NNtype differs from star 0' % k)
-            if dict(fa.get('fixedpars', {})) != dict(fa0.get('fixedpars', {})):
-                raise ValueError('star %d: fixedpars differ from star 0' % k)
-            if rb0[1] and set(fa['obs_phot'].keys()) != set(fa0['obs_phot'].keys()):
-                raise ValueError('star %d: photometric bands differ from star 0' % k)
+            if set(fa.get('fixedpars', {})) != set(fa0.get('fixedpars', {})):
+                raise ValueError('star %d: fixedpars names differ from star 0' % k)
         self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool = rb0
         if self.carbon_bool:
             raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
@@ -77,12 +81,16 @@ class StarSetLikelihood(object):
         self.GM = GenMod(precision=precision)            # the emulators, as likelihood.__init__ loads them
         if self.spec_bool:
             self.GM._initspecnn(nnpath=fa0['specANNpath'], NNtype=fa0.get('NNtype', 'LinNet'), carbon_bool=False)
+        self.bands = []
         if self.phot_bool:
-            self.GM._initphotnn(fa0['obs_phot'].keys(), nnpath=fa0['photANNpath'])
+            for fa in fitargs_list:
+                self.bands += [b for b in fa['obs_phot'].keys() if b not in self.bands]
+            self.GM._initphotnn(self.bands, nnpath=fa0['photANNpath'])
         self.fitpars_i = free0
         self.ndim = len(free0)
         stars = [{'wave': fa.get('obs_wave_fit'), 'flux': fa.get('obs_flux_fit'), 'eflux': fa.get('obs_eflux_fit'),
-                  'phot': fa.get('obs_phot')} for fa in fitargs_list]
+                  'phot': fa.get('obs_phot'), 'bands': list(fa['obs_phot'].keys()) if self.phot_bool else None,
+                  'fixedpars': dict(fa.get('fixedpars', {}))} for fa in fitargs_list]
         self.engine = Engine(spec=self.GM.PP.anns.model if self.spec_bool else None,
                              phot=self.GM.fppsed.net if self.phot_bool else None, stars=stars,
                              fitpars_i=self.fitpars_i, fixedpars=self.fixedpars,
@@ -110,12 +118,13 @@ def _is_per_star(fitpars, S):
 
 class StarView(object):
     """One star of a ``StarSetLikelihood``: ``lnlikefn``, ``lnlike_batch(theta)``, ``parsdict``, ``fitpars_i``,
-    ``ndim``, ``fixedpars`` as in ``likelihood.likelihood``."""
+    ``ndim``, ``fixedpars`` (the star's own) as in ``likelihood.likelihood``."""
 
     def __init__(self, owner, k):
         self.owner, self.k = owner, int(k)
-        self.fitpars_i, self.ndim, self.fixedpars = owner.fitpars_i, owner.ndim, owner.fixedpars
+        self.fitpars_i, self.ndim = owner.fitpars_i, owner.ndim
         self.fitargs = owner.fitargs_list[self.k]
+        self.fixedpars = self.fitargs.get('fixedpars', {})
         self.parsdict = {}
 
     def _set_parsdict(self, pars):

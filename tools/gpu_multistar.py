@@ -12,7 +12,11 @@ Device time: CUDA events around the case, median over --reps repetitions.  Host-
 the case and a device synchronise (what a sampler waiting for its lnL sees), median.  Inputs are drawn once per
 (K, b); every case is warmed up before it is timed.  The GPU name and power limit are read in the same run.
 
-usage: python tools/gpu_multistar.py [--out DIR] [--ks 1,4,16,64] [--bs 64,128,256,512] [--reps 30]
+--lsf: every star brings its own LSF vector (a fixed Inst_R array, payne_ctx_create_stars_opts), the single-star
+contexts too; every row then also records the LSF tail's device time per point (payne_ctx_last_ms(..., 1) of one
+multi-star call over its points).
+
+usage: python tools/gpu_multistar.py [--out DIR] [--ks 1,4,16,64] [--bs 64,128,256,512] [--reps 30] [--lsf]
 Prints one line per (K, b) and the GPU record; with --out DIR it also writes every row to DIR/multistar.json.
 """
 import argparse
@@ -92,6 +96,7 @@ def main():
     ap.add_argument('--ks', default='1,4,16,64')
     ap.add_argument('--bs', default='64,128,256,512')
     ap.add_argument('--reps', type=int, default=30)
+    ap.add_argument('--lsf', action='store_true', help='per-star LSF vectors (the LSF tail)')
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit('gpu_multistar.py measures on the GPU: no CUDA device')
@@ -102,7 +107,12 @@ def main():
     kw = dict(spec=spec, fitpars_i=FIT, fixedpars={}, runbools=[True, False, False, False, False], precision='parity')
     Kmax = max(ks)
     all_stars = make_stars(spec, Kmax)
-    singles = [Engine(obs_wave=s['wave'], obs_flux=s['flux'], obs_eflux=s['eflux'], **kw) for s in all_stars]
+    if args.lsf:
+        for k, s in enumerate(all_stars):
+            g = s['wave']
+            s['fixedpars'] = {'Inst_R': 0.04 + 0.002 * (k % 5) + 0.01 * (g - g[0]) / (g[-1] - g[0])}
+    singles = [Engine(obs_wave=s['wave'], obs_flux=s['flux'], obs_eflux=s['eflux'],
+                      **dict(kw, fixedpars=s.get('fixedpars', {}))) for s in all_stars]
     rows = []
     for K in ks:
         multi = Engine(stars=all_stars[:K], **kw)
@@ -126,6 +136,12 @@ def main():
             res['speedup_dev'] = res['singles_dev_ms'] / res['multi_dev_ms']
             res['multi_over_ceiling_dev'] = res['multi_dev_ms'] / res['ceiling_dev_ms']
             res['multi_Mevals_s'] = K * b / res['multi_host_ms'] / 1e3
+            if args.lsf:
+                multi.set('timing', 1)
+                multi.lnlike_batch(th, star)
+                res['lsf_tail_us_per_point'] = 1e3 * multi.last_ms('tail') / (K * b)
+                multi.set('timing', 0)
+                print('K=%3d b=%4d  LSF tail %.1f us per point' % (K, b, res['lsf_tail_us_per_point']), flush=True)
             rows.append(res)
             print('K=%3d b=%4d  multi %.3f ms dev / %.3f ms host | %d singles %.3f / %.3f | ceiling %.3f / %.3f | '
                   'x%.2f host  x%.2f dev  multi/ceiling %.3f  %s' % (
@@ -136,7 +152,8 @@ def main():
         multi.close()
     for e in singles:
         e.close()
-    doc = {'gpu': gpu_info(), 'workload': 'C2 emulator LinNet 4-256-256-256-14172, per-star n_obs 3000-7000, parity',
+    doc = {'gpu': gpu_info(), 'workload': 'C2 emulator LinNet 4-256-256-256-14172, per-star n_obs 3000-7000, parity' +
+           (', per-star LSF vectors' if args.lsf else ''),
            'reps': args.reps, 'rows': rows}
     if args.out:
         os.makedirs(args.out, exist_ok=True)
