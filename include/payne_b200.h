@@ -25,7 +25,8 @@
  *                           emulators and the parameter layout (likelihood.__init__ per star; a survey fits
  *                           thousands of stars with one emulator): every point of a batch names its star.
  *   payne_ctx_create_stars_opts  the same with each star's own fixed parameter values (fitstar.py:193-198 per star),
- *                           photometric bands (likelihood.py:109-112 over the star's obs_phot) and LSF vector.
+ *                           photometric bands (likelihood.py:109-112 over the star's obs_phot), LSF vector and
+ *                           parameter layout (fitstar.py:50-65, 202-207 per star).
  *
  * Conventions: plain pointers and sizes only; every function returns 0 on success or a
  * negative PAYNE_E_* code and never throws; payne_last_error() gives the message of the
@@ -49,7 +50,7 @@
 extern "C" {
 #endif
 
-#define PAYNE_ABI_VERSION 7
+#define PAYNE_ABI_VERSION 8
 
 enum {
   PAYNE_OK = 0,
@@ -169,6 +170,7 @@ typedef struct {
   const int32_t* band;   /* [PayneObs.nb] or NULL: photometry-net band of each of this star's magnitudes, in PayneObs
                             order, distinct, in [0, phot->nb); NULL = net order (then PayneObs.nb == phot->nb) */
   const double*  lsf;    /* [PayneObs.n_obs] or NULL: dispersion (AA) at every observed pixel, as payne_ctx_set_lsf */
+  const PayneLayout* layout;  /* or NULL (= the context layout): this star's own parameter layout (ABI 8) */
 } PayneStarOpts;
 
 /* payne_ctx_create_stars with per-star options: opts is an array of n_stars PayneStarOpts or NULL
@@ -181,13 +183,26 @@ typedef struct {
  *          entries: PAYNE_E_INVALID.
  *   lsf:   given for every star or for none (a mix is PAYNE_E_UNSUPPORTED: the LSF tail and the scalar-R tails are
  *          different kernels); every vector is checked as payne_ctx_set_lsf checks one, and while the vectors are set
- *          Inst_R is ignored.  The vectors are fixed at creation: payne_ctx_set_lsf still refuses several stars. */
+ *          Inst_R is ignored.  The vectors are fixed at creation: payne_ctx_set_lsf still refuses several stars.
+ *   layout: the star's own ndim, col[], fixed[], n_poly, poly_col[], photscale_bool and phot_bool: its free parameters,
+ *          their order in its theta row, its continuum order and its photometry may differ from the other stars'.
+ *          fixed[] is the star's fixed values (giving `fixed` too is PAYNE_E_INVALID).  phot_bool 0: the star has no
+ *          magnitudes (PayneObs.nb must be 0) and its SED chi2 is 0.  PAYNE_E_INVALID: a col or poly_col outside
+ *          [0, ndim) or used twice (col -1 = not sampled), n_poly above PAYNE_MAX_POLY, spec_bool or precision other
+ *          than the context layout's, nothing to fit, photometry in a context whose layout has phot_bool 0.
+ *          PAYNE_E_UNSUPPORTED: stars with and without a continuum polynomial (modpoly_bool with n_poly >= 1) in one
+ *          set -- the polynomial and the plain final pass round differently, so such a star would not get the bits of
+ *          its single-star context; n_poly >= 1 may differ.  Every star's polynomial is evaluated to the set's largest
+ *          order, its own coefficients followed by zeros (exact at finite abscissae): PAYNE_E_UNSUPPORTED as well for a
+ *          star below that order whose Chebyshev abscissae are not finite (n_obs = 1 or all its wavelengths equal).  A star without a layout has the context layout.  In the
+ *          batch entries ld must be at least the largest ndim (context layout's and the stars'); row p reads columns
+ *          [0, ndim) of its star only. */
 int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* phot, const PayneObs* obs,
                                 const PayneStarOpts* opts, int32_t n_stars, const PayneLayout* layout, int device,
                                 PayneCtx** out);
 void payne_ctx_destroy(PayneCtx* ctx);
 
-/* theta_dev: [B, ld] fp64 row-major on the device.  lnl_dev: [B] fp64.
+/* theta_dev: [B, ld] fp64 row-major on the device, ld >= ndim (with per-star layouts: the largest).  lnl_dev: [B] fp64.
  * star_dev: [B] int32 on the device, the star of every row of theta; NULL = star 0 for every row, which a context of
  * several stars refuses (PAYNE_E_INVALID).  A row whose star lies outside [0, n_stars) cannot be checked without a
  * synchronise: it gets lnL NaN, no model row and sets status bit 2; the other rows are not affected.

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PAYNE_LIB_PATH: development override (an instrumented build of the same sources)
 LIB_PATH = os.environ.get('PAYNE_LIB_PATH') or os.path.join(HERE, 'libpayne_b200.so')
 
-ABI_VERSION = 7          # PAYNE_ABI_VERSION of include/payne_b200.h the ctypes structs below mirror
+ABI_VERSION = 8          # PAYNE_ABI_VERSION of include/payne_b200.h the ctypes structs below mirror
 NPAR = 13
 MAX_POLY = 16
 PAR_INDEX = {
@@ -52,15 +52,15 @@ class PayneObs(C.Structure):
                 ('nb', C.c_int32), ('phot_mag', _d), ('phot_err', _d)]
 
 
-class PayneStarOpts(C.Structure):
-    _fields_ = [('fixed', _d), ('band', C.POINTER(C.c_int32)), ('lsf', _d)]
-
-
 class PayneLayout(C.Structure):
     _fields_ = [('ndim', C.c_int32), ('col', C.c_int32 * NPAR), ('fixed', C.c_double * NPAR),
                 ('n_poly', C.c_int32), ('poly_col', C.c_int32 * MAX_POLY),
                 ('spec_bool', C.c_int32), ('phot_bool', C.c_int32), ('modpoly_bool', C.c_int32),
                 ('photscale_bool', C.c_int32), ('precision', C.c_int32)]
+
+
+class PayneStarOpts(C.Structure):
+    _fields_ = [('fixed', _d), ('band', C.POINTER(C.c_int32)), ('lsf', _d), ('layout', C.POINTER(PayneLayout))]
 
 
 class PayneError(RuntimeError):

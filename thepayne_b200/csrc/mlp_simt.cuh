@@ -31,18 +31,19 @@ struct EncodeParams {
   double offset;
   int cast32;        // labels through fp32 first (predictspec.py:70); 0 for the fp64 YST1 path
   int act;           // kActSigmoid / kActLeaky for the first layer
-  // per-star fixed values (payne_ctx_create_stars_opts): label i with col[i] < 0 of point p reads
-  // star_fixed[star[p] * PAYNE_NPAR + label_param(i)] instead of fixed[i]; null without them
+  // per-star fixed values and layouts (payne_ctx_create_stars_opts), null without them: label i of point p is
+  // parameter label_param(i) of star star[p] (param_of)
   const double* star_fixed;
   const int* star;   // [B] star of every row of this slab (null: star 0)
   int n_stars;
+  const StarLayout* star_lay;
 };
 
-// label i of row p where the layout does not sample it
-__device__ __forceinline__ double fixed_label(const EncodeParams& E, int p, int i) {
-  if (!E.star_fixed || label_param(i) < 0) return E.fixed[i];
-  const int k = star_of(E.star, E.n_stars, p);
-  return k < 0 ? E.fixed[i] : E.star_fixed[(long long)k * PAYNE_NPAR + label_param(i)];
+// raw value of label i of row p
+__device__ __forceinline__ double label_of(const EncodeParams& E, const double* x, long long ld, int p, int i) {
+  const int which = label_param(i);
+  const int k = (which >= 0 && (E.star_fixed || E.star_lay)) ? star_of(E.star, E.n_stars, p) : -1;
+  return param_of(E.star_lay, E.col[i], E.fixed[i], E.star_fixed, x + (long long)p * ld, k, which);
 }
 
 // h1[p, h] = sigmoid(W1[h, :] . enc(x_p) + b1[h]); optionally also the tf32 hi/lo split planes.
@@ -56,7 +57,7 @@ encode_layer1_kernel(const __grid_constant__ EncodeParams E, const double* __res
   const int p = (int)(idx / H1), h = (int)(idx % H1);
   float acc = 0.f;
   for (int i = 0; i < E.D_in; ++i) {
-    const double raw = E.col[i] >= 0 ? x[(long long)p * ld + E.col[i]] : fixed_label(E, p, i);
+    const double raw = label_of(E, x, ld, p, i);
     const double x = E.cast32 ? (double)(float)raw : raw;            // predictspec.py:70
     const float enc = (float)((x - E.xmin[i]) / (E.xmax[i] - E.xmin[i]) - E.offset);
     acc = fmaf(enc, __ldg(W1 + h * E.D_in + i), acc);

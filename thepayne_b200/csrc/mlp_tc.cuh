@@ -619,7 +619,7 @@ encode_layer1_x3_kernel(const __grid_constant__ EncodeParams E, const double* __
   if (p >= B) return;
   float mine = 0.f;
   if (lane < E.D_in) {
-    const double raw = E.col[lane] >= 0 ? x[(long long)p * ld + E.col[lane]] : fixed_label(E, p, lane);
+    const double raw = label_of(E, x, ld, p, lane);
     const double xv = E.cast32 ? (double)(float)raw : raw;          // predictspec.py:70
     mine = (float)((xv - E.xmin[lane]) / (E.xmax[lane] - E.xmin[lane]) - E.offset);
   }

@@ -21,11 +21,34 @@ __host__ __device__ constexpr int label_param(int i) {
        : i == 4 ? PAYNE_P_VMIC : -1;
 }
 
-// Value of a parameter the layout does not sample (col < 0): star k's own value when the context was created with
-// per-star fixed values (star_fixed [n_stars, PAYNE_NPAR]), the layout's otherwise.  k < 0 (no such star): the
-// layout's; every consumer turns such a point into NaN anyway.
-__device__ __forceinline__ double fixed_of(const double* star_fixed, const double* fixed, int k, int which) {
-  return (star_fixed && k >= 0) ? star_fixed[(long long)k * PAYNE_NPAR + which] : fixed[which];
+// Per-star parameter layout (PayneStarOpts.layout): where star k's parameters sit in its own theta row.  The records
+// [n_stars] are uploaded only when some star of the set gives a layout (a star without one gets the context layout's
+// record); without them the pointer is null and every consumer reads its own copy of the context layout.
+struct StarLayout {
+  int col[PAYNE_NPAR];            // column in theta, -1: not sampled (star_fixed)
+  int n_poly;                     // pc_k coefficients (0 without a continuum polynomial)
+  int poly_col[PAYNE_MAX_POLY];
+  int photscale;                  // photscale_bool
+};
+
+// Parameter `which` of theta row th of star k: the column of star k's layout when the context has per-star layouts,
+// ctx_col (the consumer's copy of the context layout) otherwise.  Where that column is -1: star k's own value when the
+// context has per-star fixed values (star_fixed [n_stars, PAYNE_NPAR]), ctx_fixed otherwise.  k < 0 (no such star --
+// every consumer turns such a point into NaN anyway -- or a label beyond PAYNE_P_*): the context's column and value.
+__device__ __forceinline__ double param_of(const StarLayout* star_lay, int ctx_col, double ctx_fixed,
+                                           const double* star_fixed, const double* th, int k, int which) {
+  const int c = (star_lay && k >= 0) ? star_lay[k].col[which] : ctx_col;
+  if (c >= 0) return th[c];
+  return (star_fixed && k >= 0) ? star_fixed[(long long)k * PAYNE_NPAR + which] : ctx_fixed;
+}
+
+// Continuum coefficients of theta row th of star k into poly[]; returns their number.
+__device__ __forceinline__ int poly_of(const StarLayout* star_lay, int ctx_n_poly, const int* ctx_poly_col,
+                                       const double* th, int k, double* poly) {
+  const bool own = star_lay && k >= 0;
+  const int n = own ? star_lay[k].n_poly : ctx_n_poly;
+  for (int i = 0; i < n; ++i) poly[i] = th[own ? star_lay[k].poly_col[i] : ctx_poly_col[i]];
+  return n;
 }
 
 // star index of batch point p (null array: star 0), or -1 when outside [0, n_stars)

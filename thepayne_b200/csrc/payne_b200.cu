@@ -171,6 +171,8 @@ struct PayneCtx {
   std::vector<payne::ObsStar> stars;    // host copy of the records
   payne::ObsStar* stars_dev = nullptr;
   double* star_fixed_dev = nullptr;     // [n_stars, PAYNE_NPAR] per-star fixed values (payne_ctx_create_stars_opts), or null
+  payne::StarLayout* star_lay_dev = nullptr;   // [n_stars] per-star layouts (PayneStarOpts.layout), or null
+  int ndim_max = 0;                     // the largest ndim of the context layout and the stars' layouts
   // photometry
   bool has_phot = false;
   payne::PhotParams phot{};
@@ -643,10 +645,13 @@ int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs, const Pa
   using namespace payne;
   const int nb = p->nb, H = p->H;
   // band list of every star: net band of each of its magnitudes; none given = the net's order
+  // a star whose own layout has no photometry (phot_bool 0, PayneObs.nb 0) has no slots
+  auto no_phot = [&](int k) { return opts && opts[k].layout && !opts[k].layout->phot_bool; };
   bool any_band = false;
-  for (int k = 0; k < c->n_stars; ++k) any_band |= opts && opts[k].band;
+  for (int k = 0; k < c->n_stars; ++k) any_band |= opts && (opts[k].band || no_phot(k));
   std::vector<int> band_slot(any_band ? (size_t)c->n_stars * nb : 0, -1);
   for (int k = 0; k < c->n_stars; ++k) {
+    if (no_phot(k)) continue;
     const int32_t* band = opts ? opts[k].band : nullptr;
     if (!band) {
       if (p->nb != obs[k].nb)
@@ -894,7 +899,7 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
               long long ld_flux, double* mags_out, double* lnl, cudaStream_t st) {
   using namespace payne;
   if (B <= 0) return PAYNE_OK;
-  if (ld < c->lay.ndim) return fail(PAYNE_E_INVALID, "ld < ndim");
+  if (ld < c->ndim_max) return fail(PAYNE_E_INVALID, "ld < ndim (the largest star's with per-star layouts)");
   if (flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
   int rc = ensure_workspace(c, B);
   if (rc) return rc;
@@ -989,7 +994,8 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         TailParams TL = T;
         TL.col[PAYNE_P_INSTR] = -1;                                   // the vector replaces Inst_R
         TL.fixed[PAYNE_P_INSTR] = std::numeric_limits<double>::quiet_NaN();
-        TL.inst_scale = std::numeric_limits<double>::quiet_NaN();   // ... a star's own fixed Inst_R too (no scalar-R stage)
+        // ... a star's own fixed Inst_R and a per-star layout's Inst_R column too: Rs = NaN, no scalar-R stage
+        TL.inst_scale = std::numeric_limits<double>::quiet_NaN();
         if (payne::launch_tail_lsf(std::min(c->lsf_grid, nb), c->lsf_smem, st, TL, c->lsf)) return fail(PAYNE_E_CUDA, "tail launch");
       } else if (fast_tail && is_depth && c->use_cluster && c->allow_cluster) {
         payne::FastGrid FC = c->fast;
@@ -1018,6 +1024,78 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
   return mark_done(c, st);
 }
 
+// Per-star layouts (PayneStarOpts.layout): every rule that does not depend on the device.  A star without a layout
+// has the context layout.
+int check_star_layouts(const PayneLayout* ctx, const PayneObs* obs, const PayneStarOpts* opts, int n_stars) {
+  auto lay_of = [&](int k) { return (opts && opts[k].layout) ? opts[k].layout : ctx; };
+  auto has_poly = [](const PayneLayout* L) { return L->modpoly_bool && L->n_poly > 0; };
+  for (int k = 0; opts && k < n_stars; ++k) {
+    const PayneLayout* L = opts[k].layout;
+    if (!L) continue;
+    const std::string who = "star " + std::to_string(k) + ": ";
+    if (opts[k].fixed) return fail(PAYNE_E_INVALID, who + "give its fixed values in its layout or in PayneStarOpts.fixed, not both");
+    if (L->ndim < 0) return fail(PAYNE_E_INVALID, who + "ndim < 0");
+    if (L->n_poly < 0 || L->n_poly > PAYNE_MAX_POLY) return fail(PAYNE_E_INVALID, who + "n_poly out of range");
+    if (L->spec_bool != ctx->spec_bool) return fail(PAYNE_E_INVALID, who + "spec_bool differs from the context's");
+    if (L->precision != ctx->precision) return fail(PAYNE_E_INVALID, who + "precision differs from the context's");
+    if (!L->spec_bool && !L->phot_bool) return fail(PAYNE_E_INVALID, who + "nothing to fit");
+    if (L->phot_bool && !ctx->phot_bool) return fail(PAYNE_E_INVALID, who + "photometry in a context without a photometry net");
+    if (!L->phot_bool && obs[k].nb != 0) return fail(PAYNE_E_INVALID, who + "phot_bool 0 but PayneObs.nb != 0");
+    // every sampled column in [0, ndim), none used twice
+    std::vector<char> used((size_t)L->ndim, 0);
+    auto take = [&](int col, const std::string& what) -> int {
+      if (col < 0 || col >= L->ndim) return fail(PAYNE_E_INVALID, who + what + " column " + std::to_string(col) + " outside [0, ndim)");
+      if (used[col]) return fail(PAYNE_E_INVALID, who + "column " + std::to_string(col) + " used twice");
+      used[col] = 1;
+      return PAYNE_OK;
+    };
+    for (int i = 0; i < PAYNE_NPAR; ++i)
+      if (L->col[i] != -1) { int rc = take(L->col[i], "parameter " + std::to_string(i)); if (rc) return rc; }
+    for (int i = 0; L->modpoly_bool && i < L->n_poly; ++i) { int rc = take(L->poly_col[i], "pc_" + std::to_string(i)); if (rc) return rc; }
+  }
+  // The polynomial and the plain final pass round differently ((1 + d) / sigma - o / sigma against d / sigma -
+  // (o - 1) / sigma): a star without a polynomial in a polynomial launch would not give its single-star result.
+  for (int k = 1; k < n_stars; ++k)
+    if (has_poly(lay_of(k)) != has_poly(lay_of(0)))
+      return fail(PAYNE_E_UNSUPPORTED, "stars with and without a continuum polynomial (modpoly_bool, n_poly >= 1) in one set (star " +
+                  std::to_string(k) + ")");
+  return PAYNE_OK;
+}
+
+// Device records of the per-star layouts, wired into the consumers.  A star with fewer continuum coefficients than the
+// set's largest order gets zeros after its own (tail_setup); that keeps its bits only at finite Chebyshev abscissae, so
+// such a star whose abscissae are not all finite (n_obs = 1 or all wavelengths equal: 0/0 in polycalc) is refused.
+int upload_star_layouts(PayneCtx* c, const PayneLayout* ctx, const PayneStarOpts* opts, const PayneObs* obs) {
+  using namespace payne;
+  const int S = c->n_stars;
+  std::vector<StarLayout> rec(S);
+  int n_poly_max = 0;
+  for (int k = 0; k < S; ++k) {
+    const PayneLayout* L = opts[k].layout ? opts[k].layout : ctx;
+    StarLayout& r = rec[k];
+    for (int i = 0; i < PAYNE_NPAR; ++i) r.col[i] = L->col[i];
+    r.n_poly = L->modpoly_bool ? L->n_poly : 0;
+    for (int i = 0; i < PAYNE_MAX_POLY; ++i) r.poly_col[i] = L->poly_col[i];
+    r.photscale = L->photscale_bool;
+    n_poly_max = std::max(n_poly_max, r.n_poly);
+    c->ndim_max = std::max(c->ndim_max, (int)L->ndim);
+  }
+  for (int k = 0; k < S && c->has_spec; ++k) {
+    if (rec[k].n_poly == n_poly_max) continue;
+    const double* w = obs[k].wave;
+    const double omin = *std::min_element(w, w + obs[k].n_obs), omax = *std::max_element(w, w + obs[k].n_obs);
+    for (int j = 0; j < obs[k].n_obs; ++j)
+      if (!std::isfinite(2.0 * ((w[j] - omin) / (omax - omin)) - 1.0))     // append_star_obs's abscissa
+        return fail(PAYNE_E_UNSUPPORTED, "star " + std::to_string(k) + ": its continuum order is below the set's largest "
+                    "and its Chebyshev abscissae are not finite (n_obs = 1 or all wavelengths equal)");
+  }
+  int rc = upload_owned(c, &c->star_lay_dev, rec.data(), rec.size());
+  if (rc) return rc;
+  c->tail.n_poly = n_poly_max;       // the final passes evaluate this many coefficients (tail_setup pads with zeros)
+  c->tail.star_lay = c->phot.star_lay = c->enc.star_lay = c->star_lay_dev;
+  return PAYNE_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1041,8 +1119,11 @@ int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* ph
   if (!out || !layout || !obs) return fail(PAYNE_E_INVALID, "null argument");
   *out = nullptr;
   if (n_stars < 1) return fail(PAYNE_E_INVALID, "n_stars must be >= 1");
-  bool any_band = false, any_fixed = false;
-  for (int k = 0; opts && k < n_stars; ++k) { any_band |= opts[k].band != nullptr; any_fixed |= opts[k].fixed != nullptr; }
+  bool any_band = false, any_fixed = false, any_layout = false;
+  for (int k = 0; opts && k < n_stars; ++k) {
+    any_band |= opts[k].band != nullptr || opts[k].layout != nullptr;    // a layout may drop the star's photometry
+    any_fixed |= opts[k].fixed != nullptr; any_layout |= opts[k].layout != nullptr;
+  }
   if (layout->phot_bool && !any_band)
     for (int k = 1; k < n_stars; ++k)
       if (obs[k].nb != obs[0].nb) return fail(PAYNE_E_INVALID, "every star must have the same nb (star " + std::to_string(k) + ")");
@@ -1050,6 +1131,7 @@ int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* ph
   if (layout->phot_bool && !phot) return fail(PAYNE_E_INVALID, "phot_bool set but no photometry net");
   if (!layout->spec_bool && !layout->phot_bool) return fail(PAYNE_E_INVALID, "nothing to fit");
   if (layout->n_poly < 0 || layout->n_poly > PAYNE_MAX_POLY) return fail(PAYNE_E_INVALID, "n_poly out of range");
+  if (any_layout) { int rc = check_star_layouts(layout, obs, opts, n_stars); if (rc) return rc; }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(PAYNE_E_CUDA, "no CUDA device: this library has no CPU fallback");
@@ -1062,7 +1144,7 @@ int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* ph
   { const char* e = getenv("PAYNE_GEMM_STACK"); c->use_stack = !(e && e[0] == '0'); }
   c->device = device; c->sm_count = prop.multiProcessorCount; c->lay = *layout;
   c->has_spec = layout->spec_bool != 0; c->has_phot = layout->phot_bool != 0;
-  c->n_stars = n_stars;
+  c->n_stars = n_stars; c->ndim_max = layout->ndim;
   c->stars.assign(n_stars, payne::ObsStar{});
   int rc = PAYNE_OK;
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) rc = fail(PAYNE_E_CUDA, "stream");
@@ -1077,18 +1159,20 @@ int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* ph
   if (!rc && c->has_phot) rc = build_phot(c, phot, obs, opts);
   if (!rc) rc = set_star_lsf(c, obs, opts);
   if (!rc) rc = upload_owned(c, &c->stars_dev, c->stars.data(), c->stars.size());
-  if (!rc && any_fixed) {
-    // star k's row: its own values, or the layout's where it gives none
+  if (!rc && (any_fixed || any_layout)) {
+    // star k's row: its own values (PayneStarOpts.fixed or its layout's), or the context layout's where it gives none
     std::vector<double> fx((size_t)n_stars * PAYNE_NPAR);
     for (int k = 0; k < n_stars; ++k)
-      std::memcpy(&fx[(size_t)k * PAYNE_NPAR], opts[k].fixed ? opts[k].fixed : layout->fixed, PAYNE_NPAR * sizeof(double));
+      std::memcpy(&fx[(size_t)k * PAYNE_NPAR], opts[k].fixed ? opts[k].fixed : opts[k].layout ? opts[k].layout->fixed : layout->fixed,
+                  PAYNE_NPAR * sizeof(double));
     rc = upload_owned(c, &c->star_fixed_dev, fx.data(), fx.size());
   }
   if (!rc) {
     c->tail.stars = c->phot.stars = c->stars_dev;
     c->tail.n_stars = c->phot.n_stars = c->enc.n_stars = n_stars;
-    c->tail.star_fixed = c->phot.star_fixed = c->enc.star_fixed = c->star_fixed_dev;
   }
+  if (!rc && any_layout) rc = upload_star_layouts(c, layout, opts, obs);
+  if (!rc) c->tail.star_fixed = c->phot.star_fixed = c->enc.star_fixed = c->star_fixed_dev;
   if (rc) { std::string keep = g_err; payne_ctx_destroy(c); g_err = keep; return rc; }
   *out = c;
   return PAYNE_OK;
@@ -1394,7 +1478,7 @@ int payne_ann_eval(PayneCtx* c, const double* x_dev, int64_t B, float* y_dev, in
   if (rc) return rc;
   payne::EncodeParams E = c->enc;
   for (int i = 0; i < E.D_in; ++i) E.col[i] = i;
-  E.star_fixed = nullptr;
+  E.star_fixed = nullptr; E.star_lay = nullptr;
   for (long long p0 = 0; p0 < B; p0 += c->slab) {
     const int nb = (int)std::min<long long>(c->slab, B - p0);
     int isd = 0;
@@ -1420,6 +1504,7 @@ int payne_ctx_attach_continuum(PayneCtx* c, const PayneSpecNet* cnet) {
   if (cudaMalloc((void**)&cc->status, sizeof(int)) != cudaSuccess) rc = fail(PAYNE_E_NOMEM, "status");
   if (!rc) rc = build_spec(cc, cnet, nullptr, /*emulator_only=*/true);
   cc->enc.star_fixed = c->enc.star_fixed; cc->enc.n_stars = c->enc.n_stars;   // labels: the same per-star values
+  cc->enc.star_lay = c->enc.star_lay;                                          // ... and columns
   const int nc = cnet->D_out, n = c->D_out;
   cc->ldf = ((long long)nc + 3) / 4 * 4;
   std::vector<double> wc(cnet->wavelength, cnet->wavelength + nc), fac(nc);

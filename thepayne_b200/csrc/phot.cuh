@@ -46,10 +46,12 @@ struct PhotParams {
   // With it, a point's terms are stored per slot and summed in slot order at the end, so that its chi2 has the order
   // a single-star context of that star's bands gives; mags_out row p gets its magnitudes in slots [0, nb_k).
   const int* band_slot;
+  const StarLayout* star_lay;   // [n_stars] per-star layouts (columns, photscale), null without them; a star without
+                                // photometry has no slots (band_slot row all -1)
 };
 
 __device__ __forceinline__ double phot_par(const PhotParams& P, const double* th, int which, int k) {
-  return P.col[which] >= 0 ? th[P.col[which]] : fixed_of(P.star_fixed, P.fixed, k, which);
+  return param_of(P.star_lay, P.col[which], P.fixed[which], P.star_fixed, th, k, which);
 }
 __device__ __forceinline__ double sigmoid_d(double a) { return 1.0 / (1.0 + exp(-a)); }
 
@@ -91,7 +93,7 @@ phot_kernel(const __grid_constant__ PhotParams P) {
       for (int i = 0; i < 6; ++i) zin[tid][i] = (x[i] - P.xmin[i]) / (P.xmax[i] - P.xmin[i]);
       aux[tid][0] = logt; aux[tid][1] = av; aux[tid][2] = hi ? 1.0 : 0.0;
       double base;
-      if (P.photscale) {
+      if ((P.star_lay && k >= 0) ? P.star_lay[k].photscale : P.photscale) {
         base = 5.0 * phot_par(P, th, PAYNE_P_LOGA, k) - 10.0 * (logt - log10_tsun) - 0.26;   // predictsed.py:96
       } else {
         const double logl = 2.0 * phot_par(P, th, PAYNE_P_LOGR, k) + 4.0 * (logt - log10_tsun);   // genmod.py:128

@@ -96,6 +96,7 @@ struct TailParams {
   // Per-star fixed values (payne_ctx_create_stars_opts): [n_stars, PAYNE_NPAR], read where col < 0 in place of
   // `fixed` / `label_fixed`; null when the context was created without them.
   const double* star_fixed;
+  const StarLayout* star_lay;        // [n_stars] per-star layouts (obs_star.cuh), null without them
 };
 
 // lnL of point p: local result and, with the fused gather on, the copy in every peer's buffer
@@ -135,7 +136,7 @@ struct ObsSlice {
 
 // parameter `which` of point th of star k
 __device__ __forceinline__ double get_par(const TailParams& P, const double* th, int which, int k) {
-  return P.col[which] >= 0 ? th[P.col[which]] : fixed_of(P.star_fixed, P.fixed, k, which);
+  return param_of(P.star_lay, P.col[which], P.fixed[which], P.star_fixed, th, k, which);
 }
 
 // float index of real sample k: 2*swz(k>>1) + (k&1) == k ^ (((k>>5)&7)<<2)
@@ -279,9 +280,8 @@ static __device__ void tail_setup(const TailParams& P, const double* th, int p, 
   S.bad = 0;
   S.clean = P.rows_may_nan ? 0 : 1;
   for (int i = 0; i < P.n_labels; ++i) {
-    const double v = P.label_col[i] >= 0 ? th[P.label_col[i]]
-                     : (P.star_fixed && label_param(i) >= 0 ? P.star_fixed[(long long)k * PAYNE_NPAR + label_param(i)]
-                                                            : P.label_fixed[i]);
+    const int which = label_param(i);
+    const double v = param_of(P.star_lay, P.label_col[i], P.label_fixed[i], P.star_fixed, th, which >= 0 ? k : -1, which);
     if (!isfinite(v)) S.clean = 0;
   }
   S.do_rot = (vrot != 0.0);                       // predictspec.py:231 (NaN != 0 is true)
@@ -290,7 +290,10 @@ static __device__ void tail_setup(const TailParams& P, const double* th, int p, 
   S.D = (vrad != 0.0) ? 1.0 + (vrad / kSpeedOfLight) : 1.0;   // predictspec.py:245-249
   if (!(S.D > 0.0)) S.bad = 1;
   S.lnD = log(S.D);
-  for (int k = 0; k < P.n_poly; ++k) S.poly[k] = th[P.poly_col[k]];
+  // A star with fewer coefficients than the launch's n_poly (per-star layouts: the largest) gets zeros after its own.
+  // Clenshaw's recurrence passes through trailing zero coefficients exactly at a finite abscissa ((a, 0) -> (c, a)),
+  // so the final passes keep one constant-bank n_poly and every star gets the bits of its own continuum order.
+  for (int i = poly_of(P.star_lay, P.n_poly, P.poly_col, th, k, S.poly); i < P.n_poly; ++i) S.poly[i] = 0.0;
   const double Rs = P.inst_scale * instR;         // genmod.py:83 (inst_scale = 2.355) or predictspec.py:255-263 (1)
   S.use_inst = (Rs > 0.0);                        // predictspec.py:257 (false for NaN)
   S.log2N2 = 0; S.i0 = 0; S.i1 = P.n - 1;

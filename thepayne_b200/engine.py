@@ -7,10 +7,10 @@ The parameter-vector convention is the reference's (Payne/fitting/likelihood.py:
 row of ``theta`` holds the free parameters in ``fitpars_i`` order, fixed ones come from
 ``fixedpars``, and spectral parameters that are neither are NaN.
 
-One context may hold the observations of many stars (``stars=[...]``): the emulators and the
-parameter layout are shared, and every row of a batch names its star.  Each star may bring its own
-fixed parameter values, its own subset of the photometric bands and its own LSF vector.
-A single-star engine is the case of one star.
+One context may hold the observations of many stars (``stars=[...]``): the emulators are shared, and
+every row of a batch names its star.  Each star may bring its own fixed parameter values, its own subset
+of the photometric bands, its own LSF vector and its own parameter layout (free parameters and their
+order, continuum order, photometry).  A single-star engine is the case of one star.
 
 A fixed ``Inst_R`` that is a 1-D array is an LSF vector, the dispersion (AA) at every observed pixel,
 as in the reference (genmod.py:82-85 passes a non-float inst_R on to getspec's LSF branch,
@@ -58,6 +58,26 @@ def _split_fixed(fixedpars):
     return vals, lsf
 
 
+def _layout(fitpars_i, fixed_vals, runbools, precision):
+    """PayneLayout (include/payne_b200.h) of one parameter layout (likelihood.py:42-72)."""
+    spec_bool, phot_bool, modpoly_bool, photscale_bool = [bool(b) for b in runbools[:4]]
+    lay = _lib.PayneLayout()
+    lay.ndim = len(fitpars_i)
+    for name, k in PAR_INDEX.items():
+        lay.col[k] = fitpars_i.index(name) if name in fitpars_i else -1
+        lay.fixed[k] = fixed_vals[k]
+    pcs = [i for i, p in enumerate(fitpars_i) if 'pc' in p]   # likelihood.py:56-57
+    if modpoly_bool and len(pcs) > _lib.MAX_POLY:
+        raise ValueError('at most %d continuum coefficients' % _lib.MAX_POLY)
+    lay.n_poly = len(pcs) if modpoly_bool else 0
+    for i, c in enumerate(pcs[:_lib.MAX_POLY]):
+        lay.poly_col[i] = c
+    lay.spec_bool, lay.phot_bool = int(spec_bool), int(phot_bool)
+    lay.modpoly_bool, lay.photscale_bool = int(modpoly_bool), int(photscale_bool)
+    lay.precision = PREC[precision] if isinstance(precision, str) else int(precision)
+    return lay
+
+
 def _specnet_struct(spec, keep):
     """PayneSpecNet (include/payne_b200.h) for a ``synth.SpecNet``-like container; the numpy buffers the
     struct points into are appended to ``keep``."""
@@ -100,10 +120,14 @@ class Engine:
         ``{'wave', 'flux', 'eflux', 'phot': {band: (mag, err)}}``, one per star; ``lnlike_batch`` and
         ``model_batch`` then take the star index of every row.  A star may also carry
           ``'fixedpars'``: its fixed parameter values, in place of the shared ``fixedpars``;
-          ``'bands'``: the order of its magnitudes (its SED chi2 is summed in that order, likelihood.py:109-112).
+          ``'bands'``: the order of its magnitudes (its SED chi2 is summed in that order, likelihood.py:109-112);
+          ``'fitpars_i'`` / ``'runbools'``: its own free parameters in its theta order (``pc_k`` among them) and
+          run booleans, in place of the shared ones.
         Its ``'phot'`` keys may be any subset of the photometry net's bands; without ``'bands'`` they go in the
-        net's order.  A fixed ``Inst_R`` that is a 1-D array is the star's LSF vector (one dispersion per observed
-        pixel); every star has one or none does."""
+        net's order.  In a photometry engine a star without ``'phot'`` is a star without photometry.  A fixed
+        ``Inst_R`` that is a 1-D array is the star's LSF vector (one dispersion per observed pixel); every star
+        has one or none does.  ``ndim`` is the largest star's: a row of ``theta`` holds its star's
+        ``star_fitpars_i[k]`` in its first ``star_ndim[k]`` columns, and the columns after those are ignored."""
         if stars is None:
             stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot}]
         elif any(v is not None for v in (obs_wave, obs_flux, obs_eflux, obs_phot)):
@@ -116,26 +140,30 @@ class Engine:
             raise _lib.PayneError('no CUDA device: thepayne_b200 has no CPU fallback')
         self.device = torch.cuda.current_device() if device is None else int(device)
         self.fitpars_i = list(fitpars_i)
-        self.ndim = len(self.fitpars_i)
         self.fixedpars = dict(fixedpars or {})
-        spec_bool, phot_bool, modpoly_bool, photscale_bool = [bool(b) for b in runbools[:4]]
         keep = []   # numpy buffers referenced by the structs until create returns
-
-        lay = _lib.PayneLayout()
-        lay.ndim = self.ndim
+        # every star's layout: its own free parameters and run booleans or the shared ones; a star of a photometry
+        # engine without 'phot' has none
+        self.star_fitpars_i = [list(st['fitpars_i']) if st.get('fitpars_i') is not None else self.fitpars_i
+                               for st in stars]
+        star_rb = [[bool(b) for b in (st['runbools'] if st.get('runbools') is not None else runbools)[:4]]
+                   for st in stars]
+        for rb, st in zip(star_rb, stars):
+            rb[1] = rb[1] and st.get('phot') is not None
+        self.star_ndim = [len(f) for f in self.star_fitpars_i]
+        self.ndim = max(self.star_ndim)
+        own_layouts = any(st.get('fitpars_i') is not None or st.get('runbools') is not None for st in stars) or \
+            any(rb != star_rb[0] for rb in star_rb)
+        spec_bool, phot_bool, modpoly_bool, photscale_bool = [bool(b) for b in runbools[:4]]
+        if own_layouts:
+            # the context layout is star 0's; its phot_bool says whether the engine has a photometry net
+            spec_bool, modpoly_bool, photscale_bool = star_rb[0][0], star_rb[0][2], star_rb[0][3]
+            phot_bool = any(rb[1] for rb in star_rb)
+        elif phot_bool and any(st.get('phot') is None for st in stars):
+            raise ValueError('phot_bool set but no photometry emulator / observation given')
         shared_vals, shared_lsf = _split_fixed(self.fixedpars)
-        for name, k in PAR_INDEX.items():
-            lay.col[k] = self.fitpars_i.index(name) if name in self.fitpars_i else -1
-            lay.fixed[k] = shared_vals[k]
-        pcs = [i for i, p in enumerate(self.fitpars_i) if 'pc' in p]   # likelihood.py:56-57
-        if modpoly_bool and len(pcs) > _lib.MAX_POLY:
-            raise ValueError('at most %d continuum coefficients' % _lib.MAX_POLY)
-        lay.n_poly = len(pcs) if modpoly_bool else 0
-        for i, c in enumerate(pcs[:_lib.MAX_POLY]):
-            lay.poly_col[i] = c
-        lay.spec_bool, lay.phot_bool = int(spec_bool), int(phot_bool)
-        lay.modpoly_bool, lay.photscale_bool = int(modpoly_bool), int(photscale_bool)
-        lay.precision = PREC[precision] if isinstance(precision, str) else int(precision)
+        lay = _layout(self.star_fitpars_i[0] if own_layouts else self.fitpars_i, shared_vals,
+                      [spec_bool, phot_bool, modpoly_bool, photscale_bool], precision)
 
         sp = None
         if spec_bool:
@@ -150,7 +178,11 @@ class Engine:
                                for st in stars]
         for k, st in enumerate(stars):
             vals, lsf = (shared_vals, shared_lsf) if st.get('fixedpars') is None else _split_fixed(st['fixedpars'])
-            if st.get('fixedpars') is not None:
+            if own_layouts:
+                sl = _layout(self.star_fitpars_i[k], vals, star_rb[k], precision)
+                keep.append(sl)
+                opts[k].layout = C.pointer(sl)
+            elif st.get('fixedpars') is not None:
                 keep.append(vals)
                 opts[k].fixed = _pd(vals)
             if lsf is not None:
@@ -175,7 +207,7 @@ class Engine:
         self.bands = []
         self.star_bands = [[] for _ in stars]
         if phot_bool:
-            if phot is None or any(st.get('phot') is None for st in stars):
+            if phot is None:
                 raise ValueError('phot_bool set but no photometry emulator / observation given')
             self.bands = list(phot.bands)
             ph = _lib.PaynePhotNet()
@@ -188,6 +220,8 @@ class Engine:
             keep += [pxmin, pxmax, hiav]
             ph.xmin, ph.xmax, ph.hiav = _pd(pxmin), _pd(pxmax), _pd(hiav)
             for k, st in enumerate(stars):
+                if not star_rb[k][1]:
+                    continue                                # a star without photometry: nb = 0
                 bands = list(st['bands']) if st.get('bands') is not None else \
                     [b for b in self.bands if b in st['phot']]
                 unknown = [b for b in list(st['phot']) + bands if b not in self.bands]
@@ -257,7 +291,7 @@ class Engine:
         return float(self.lib.payne_ctx_last_ms(self._ctx, {'mlp': 0, 'tail': 1, 'phot': 2}[which]))
 
     # ------------------------------------------------------------------ compute
-    def _theta_dev(self, theta):
+    def _theta_dev(self, theta):   # [B, ndim]: row p's star reads its first star_ndim columns
         if not (theta.is_cuda and theta.dtype == torch.float64 and theta.dim() == 2):
             raise ValueError('theta must be a 2-D float64 CUDA tensor')
         if theta.shape[1] != self.ndim:

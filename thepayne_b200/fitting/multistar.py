@@ -2,8 +2,9 @@
 
 A survey fits thousands of stars with the same emulator.  Between two stars the observation changes
 (wavelengths, fluxes, errors, which magnitudes and in what order), and so may the values of the fixed parameters
-(an instrumental resolution or LSF vector, a catalogue distance or extinction, an asteroseismic log(g)); the
-emulator weights, the free parameters, the names of the fixed ones and every table built from the emulator grid
+(an instrumental resolution or LSF vector, a catalogue distance or extinction, an asteroseismic log(g)) and, given
+one ``fitpars`` per star, the parameter layout itself (which parameters are free, the continuum order, photometry
+or not, ``log(A)`` or ``log(R)`` + ``Dist``); the emulator weights and every table built from the emulator grid
 stay the same.  A single star's sampler hands over a few hundred points per call, which
 leaves the GPU latency-bound; the points of many stars together make one full-size batch.
 
@@ -39,41 +40,57 @@ def _same(a, b):
 
 
 class StarSetLikelihood(object):
-    """The likelihoods of several stars that share emulators, free parameters and the names of the fixed ones.
+    """The likelihoods of several stars that share emulators.
 
     ``fitargs_list``: one ``fitargs`` per star (as ``FitPayne.run`` builds them).  ``fitpars`` / ``runbools``:
-    one value for every star, or a list with one per star (they must then agree).  Each star keeps its own fixed
-    values (a vector ``Inst_R`` is its LSF) and its own photometric bands: the photometry net covers the union of
-    the stars' bands in order of first appearance, and each star's SED chi2 is summed in its ``obs_phot`` order,
-    as a separate ``likelihood`` of that star sums it.  The fixed parameters' names must agree: they are the
-    columns of every star's output file."""
+    one value for every star, or a list with one per star.  Each star keeps its own fixed values (a vector
+    ``Inst_R`` is its LSF) and its own photometric bands: the photometry net covers the union of the bands of the
+    stars that have photometry, in order of first appearance, and each star's SED chi2 is summed in its
+    ``obs_phot`` order, as a separate ``likelihood`` of that star sums it.
+
+    With one shared ``fitpars`` the stars share one layout, and the names of the fixed parameters must agree
+    (they are the columns of every star's output file).  With one ``fitpars`` per star each star has its own
+    layout: its free parameters, photometry, photscale, continuum order and fixed parameter names may differ;
+    the emulator paths, ``NNtype``, ``spec_bool`` and ``modpoly_bool`` must agree."""
 
     def __init__(self, fitargs_list, fitpars, runbools, precision='parity', device=None):
         fitargs_list = list(fitargs_list)
         if not fitargs_list:
             raise ValueError('no stars')
         S = len(fitargs_list)
-        fp_list = list(fitpars) if _is_per_star(fitpars, S) else [fitpars] * S
+        per_star = _is_per_star(fitpars, S)
+        fp_list = list(fitpars) if per_star else [fitpars] * S
         rb_list = list(runbools) if isinstance(runbools[0], (list, tuple)) else [runbools] * S
         if len(rb_list) != S:
             raise ValueError('runbools: one list for all stars or one per star')
-        fa0, free0, rb0 = fitargs_list[0], free_parameters(fp_list[0]), [bool(b) for b in rb_list[0][:5]]
+        rb_list = [[bool(b) for b in rb[:5]] for rb in rb_list]
+        free_list = [free_parameters(fp) for fp in fp_list]
+        fa0, free0, rb0 = fitargs_list[0], free_list[0], rb_list[0]
+        if any(rb[4] for rb in rb_list):
+            raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
+        phot_stars = [k for k in range(S) if rb_list[k][1]]
         for k in range(1, S):
             fa = fitargs_list[k]
-            if [bool(b) for b in rb_list[k][:5]] != rb0:
-                raise ValueError('star %d: runbools differ from star 0' % k)
-            if free_parameters(fp_list[k]) != free0:
-                raise ValueError('star %d: free parameters differ from star 0' % k)
-            for key in ('specANNpath', 'photANNpath'):
-                if not _same(fa.get(key), fa0.get(key)):
-                    raise ValueError('star %d: %s differs from star 0' % (k, key))
+            if per_star:
+                for i, name in ((0, 'spec_bool'), (2, 'modpoly_bool')):
+                    if rb_list[k][i] != rb0[i]:
+                        raise ValueError('star %d: %s differs from star 0' % (k, name))
+            else:
+                if rb_list[k] != rb0:
+                    raise ValueError('star %d: runbools differ from star 0' % k)
+                if free_list[k] != free0:
+                    raise ValueError('star %d: free parameters differ from star 0' % k)
+            if not _same(fa.get('specANNpath'), fa0.get('specANNpath')):
+                raise ValueError('star %d: specANNpath differs from star 0' % k)
             if fa.get('NNtype', 'LinNet') != fa0.get('NNtype', 'LinNet'):
                 raise ValueError('star %d: NNtype differs from star 0' % k)
-            if set(fa.get('fixedpars', {})) != set(fa0.get('fixedpars', {})):
+            if not per_star and set(fa.get('fixedpars', {})) != set(fa0.get('fixedpars', {})):
                 raise ValueError('star %d: fixedpars names differ from star 0' % k)
-        self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool = rb0
-        if self.carbon_bool:
-            raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
+        for k in phot_stars[1:]:
+            if not _same(fitargs_list[k].get('photANNpath'), fitargs_list[phot_stars[0]].get('photANNpath')):
+                raise ValueError('star %d: photANNpath differs from star %d' % (k, phot_stars[0]))
+        self.spec_bool, _, self.modpoly_bool, self.photscale_bool, self.carbon_bool = rb0
+        self.phot_bool = bool(phot_stars)
         self.n_stars = S
         self.fitargs_list = fitargs_list
         self.fixedpars = fa0['fixedpars']
@@ -83,19 +100,24 @@ class StarSetLikelihood(object):
             self.GM._initspecnn(nnpath=fa0['specANNpath'], NNtype=fa0.get('NNtype', 'LinNet'), carbon_bool=False)
         self.bands = []
         if self.phot_bool:
-            for fa in fitargs_list:
-                self.bands += [b for b in fa['obs_phot'].keys() if b not in self.bands]
-            self.GM._initphotnn(self.bands, nnpath=fa0['photANNpath'])
-        self.fitpars_i = free0
-        self.ndim = len(free0)
+            for k in phot_stars:
+                self.bands += [b for b in fitargs_list[k]['obs_phot'].keys() if b not in self.bands]
+            self.GM._initphotnn(self.bands, nnpath=fitargs_list[phot_stars[0]]['photANNpath'])
         stars = [{'wave': fa.get('obs_wave_fit'), 'flux': fa.get('obs_flux_fit'), 'eflux': fa.get('obs_eflux_fit'),
-                  'phot': fa.get('obs_phot'), 'bands': list(fa['obs_phot'].keys()) if self.phot_bool else None,
-                  'fixedpars': dict(fa.get('fixedpars', {}))} for fa in fitargs_list]
+                  'phot': fa.get('obs_phot') if rb[1] else None,
+                  'bands': list(fa['obs_phot'].keys()) if rb[1] else None,
+                  'fixedpars': dict(fa.get('fixedpars', {}))} for fa, rb in zip(fitargs_list, rb_list)]
+        if any(free != free0 for free in free_list) or any(rb != rb0 for rb in rb_list):
+            for st, free, rb in zip(stars, free_list, rb_list):     # each star's own layout
+                st['fitpars_i'], st['runbools'] = free, rb
         self.engine = Engine(spec=self.GM.PP.anns.model if self.spec_bool else None,
                              phot=self.GM.fppsed.net if self.phot_bool else None, stars=stars,
-                             fitpars_i=self.fitpars_i, fixedpars=self.fixedpars,
+                             fitpars_i=free0, fixedpars=self.fixedpars,
                              runbools=[self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
                              precision=precision, device=device)
+        self.fitpars_i = free0
+        self.star_fitpars_i, self.star_ndim = self.engine.star_fitpars_i, self.engine.star_ndim
+        self.ndim = self.engine.ndim                      # the largest star's: the width of a batch row
         self.ncalls = 0                                   # lnlike_batch calls made on the engine
 
     def lnlike_batch(self, theta, star):
@@ -118,14 +140,28 @@ def _is_per_star(fitpars, S):
 
 class StarView(object):
     """One star of a ``StarSetLikelihood``: ``lnlikefn``, ``lnlike_batch(theta)``, ``parsdict``, ``fitpars_i``,
-    ``ndim``, ``fixedpars`` (the star's own) as in ``likelihood.likelihood``."""
+    ``ndim``, ``fixedpars`` (the star's own) as in ``likelihood.likelihood``.  Its rows [B, ndim] are padded to the
+    engine's width before they are posted."""
 
     def __init__(self, owner, k):
         self.owner, self.k = owner, int(k)
-        self.fitpars_i, self.ndim = owner.fitpars_i, owner.ndim
+        own = getattr(owner, 'star_fitpars_i', None)        # an owner without it has one layout for all stars
+        self.fitpars_i = own[self.k] if own is not None else owner.fitpars_i
+        self.ndim = len(self.fitpars_i)
         self.fitargs = owner.fitargs_list[self.k]
         self.fixedpars = self.fitargs.get('fixedpars', {})
         self.parsdict = {}
+
+    def _pad(self, theta):
+        # columns beyond the star's ndim are never read (NaN keeps a wrong read visible)
+        w = self.owner.ndim - self.ndim
+        if w == 0:
+            return theta
+        if hasattr(theta, 'is_cuda'):
+            import torch
+            return torch.nn.functional.pad(theta, (0, w), value=float('nan'))
+        theta = np.asarray(theta, dtype=np.float64)
+        return np.concatenate([theta, np.full((len(theta), w), np.nan)], axis=1)
 
     def _set_parsdict(self, pars):
         self.parsdict = {pp: vv for pp, vv in zip(self.fitpars_i, pars)}
@@ -133,6 +169,7 @@ class StarView(object):
             self.parsdict[kk] = self.fixedpars[kk]
 
     def _lnlike(self, theta):
+        theta = self._pad(theta)
         if hasattr(theta, 'is_cuda') and theta.is_cuda:
             import torch
             star = torch.full((theta.shape[0],), self.k, dtype=torch.int32, device=theta.device)
@@ -227,7 +264,7 @@ class _BatchedStarView(StarView):
         self.batcher = batcher
 
     def lnlike_batch(self, theta):
-        out = self.batcher.call(self.k, theta)
+        out = self.batcher.call(self.k, self._pad(theta))
         last = theta[-1]
         self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
         return out

@@ -16,7 +16,16 @@ the case and a device synchronise (what a sampler waiting for its lnL sees), med
 contexts too; every row then also records the LSF tail's device time per point (payne_ctx_last_ms(..., 1) of one
 multi-star call over its points).
 
-usage: python tools/gpu_multistar.py [--out DIR] [--ks 1,4,16,64] [--bs 64,128,256,512] [--reps 30] [--lsf]
+--layouts: every star has its own parameter layout (PayneStarOpts.layout), on the C2 emulator plus the C3 photometry
+net (7 bands, H = 128): continuum polynomials of 2 to 6 coefficients (star k: 2 + k % 5), photometry for every third
+star (alternately log(A) and log(R) + Dist), Vrad fixed on stars k % 4 == 1 and Vrot on k % 4 == 2; every single-star
+context has its star's own layout and theta rows its own columns.  A second set is the same with star 0's polynomial
+raised to 16 coefficients (every star's polynomial is evaluated to the set's largest order).  Besides the three cases,
+each row records the per-kernel device time (payne_ctx_last_ms: emulator, tail, photometry; median over --reps calls)
+of the mixed call and of calls of the same size on one context whose stars all have one layout (every spectral
+parameter free, no photometry, 2, 6 and 16 coefficients).
+
+usage: python tools/gpu_multistar.py [--out DIR] [--ks 1,4,16,64] [--bs 64,128,256,512] [--reps 30] [--lsf | --layouts]
 Prints one line per (K, b) and the GPU record; with --out DIR it also writes every row to DIR/multistar.json.
 """
 import argparse
@@ -72,6 +81,101 @@ def draw(B, seed):
     return lo + (hi - lo) * rng.random((B, len(FIT)))
 
 
+def draw_fit(fit, B, rng):
+    box = dict(synth._BOX, **{p: ((0.75, 1.25) if p == 'pc_0' else (-0.05, 0.05)) for p in fit if p.startswith('pc_')})
+    lo = np.array([box[p][0] for p in fit])
+    hi = np.array([box[p][1] for p in fit])
+    return lo + (hi - lo) * rng.random((B, len(fit)))
+
+
+def star_layout(k, npoly):
+    """--layouts: star k's free parameters, run booleans and fixed values"""
+    fit = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]'] + [p for i, p in ((1, 'Vrad'), (2, 'Vrot')) if k % 4 != i] + ['Inst_R']
+    fixed = {'Vrad': 5.0} if k % 4 == 1 else {'Vrot': 3.0} if k % 4 == 2 else {}
+    phot = k % 3 == 0
+    scaled = phot and (k // 3) % 2 == 0
+    if phot:
+        fit += ['log(A)', 'Av'] if scaled else ['log(R)', 'Dist', 'Av']
+    fit += ['pc_%d' % i for i in range(npoly)]
+    return fit, [True, phot, True, scaled], fixed
+
+
+def kernel_ms(eng, th, star, reps):
+    """median per-kernel device time (emulator, tail, photometry) of one call"""
+    eng.set('timing', 1)
+    rows = []
+    for _ in range(reps):
+        eng.lnlike_batch(th, star)
+        torch.cuda.synchronize()
+        rows.append([max(0.0, eng.last_ms(w)) for w in ('mlp', 'tail', 'phot')])
+    eng.set('timing', 0)
+    return [float(v) for v in np.median(np.array(rows), axis=0)]
+
+
+def run_layouts(args, spec, ks, bs):
+    phot = synth.make_photnet(synth.PROCYON_BANDS, H=128)                   # C3 (synth.config_c3)
+    kmax = max(ks)
+    base = make_stars(spec, kmax)
+    obs_phot = {b: (6.0 + 0.1 * i, 0.03) for i, b in enumerate(synth.PROCYON_BANDS)}
+    rows = []
+    for label, high in (('mixed n_poly 2-6', False), ('mixed n_poly 2-6, star 0 at 16', True)):
+        stars = []
+        for k, s in enumerate(base):
+            fit, rb, fixed = star_layout(k, 16 if (high and k == 0) else 2 + k % 5)
+            stars.append(dict(s, fitpars_i=fit, runbools=rb, fixedpars=fixed, phot=obs_phot if rb[1] else None))
+        singles = [Engine(obs_wave=s['wave'], obs_flux=s['flux'], obs_eflux=s['eflux'], obs_phot=s['phot'],
+                          spec=spec, phot=phot if s['runbools'][1] else None, fitpars_i=s['fitpars_i'],
+                          fixedpars=s['fixedpars'], runbools=s['runbools'] + [False], precision='parity')
+                   for s in stars]
+        for K in ks:
+            multi = Engine(stars=stars[:K], spec=spec, phot=phot, runbools=[True, True, True, False, False],
+                           precision='parity')
+            for b in bs:
+                rng = np.random.default_rng(K * 1000 + b)
+                parts_np = [draw_fit(stars[k]['fitpars_i'], b, rng) for k in range(K)]
+                th_np = np.full((K * b, multi.ndim), np.nan)
+                for k in range(K):
+                    th_np[k * b:(k + 1) * b, :parts_np[k].shape[1]] = parts_np[k]
+                th = torch.from_numpy(th_np).cuda()
+                parts = [torch.from_numpy(p).cuda() for p in parts_np]
+                star = torch.repeat_interleave(torch.arange(K, dtype=torch.int32), b).cuda()
+                th0 = torch.from_numpy(draw_fit(stars[0]['fitpars_i'], K * b, rng)).cuda()
+                res = {'set': label, 'K': K, 'b': b, 'points': K * b}
+                res['multi_dev_ms'], res['multi_host_ms'], res['multi_dev_min_ms'] = time_case(
+                    lambda: multi.lnlike_batch(th, star), args.reps)
+                res['singles_dev_ms'], res['singles_host_ms'], res['singles_dev_min_ms'] = time_case(
+                    lambda: [singles[k].lnlike_batch(parts[k]) for k in range(K)], args.reps)
+                res['ceiling_dev_ms'], res['ceiling_host_ms'], res['ceiling_dev_min_ms'] = time_case(
+                    lambda: singles[0].lnlike_batch(th0), args.reps)
+                got = multi.lnlike_batch(th, star)
+                ref = torch.cat([singles[k].lnlike_batch(parts[k]) for k in range(K)])
+                torch.cuda.synchronize()
+                res['bit_identical'] = bool(torch.equal(torch.nan_to_num(got, nan=1.5), torch.nan_to_num(ref, nan=1.5)))
+                res['kernel_ms_mixed'] = kernel_ms(multi, th, star, args.reps)
+                for npoly in (2, 6, 16):                       # one layout for every star, same size
+                    fit = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot', 'Inst_R'] + ['pc_%d' % i for i in range(npoly)]
+                    uni = Engine(stars=[{x: s[x] for x in ('wave', 'flux', 'eflux')} for s in stars[:K]], spec=spec, fitpars_i=fit,
+                                 runbools=[True, False, True, False, False], precision='parity')
+                    thu = torch.from_numpy(draw_fit(fit, K * b, rng)).cuda()
+                    res['kernel_ms_uniform_%d' % npoly] = kernel_ms(uni, thu, star, args.reps)
+                    uni.close()
+                rows.append(res)
+                km = res['kernel_ms_mixed']
+                print('%s K=%3d b=%4d  multi %.3f ms dev / %.3f host | %d singles %.3f / %.3f | ceiling %.3f / %.3f | '
+                      'x%.2f host  %s | kernels mlp/tail/phot ms: mixed %.3f/%.3f/%.3f  uniform 2: %.3f/%.3f  '
+                      '6: %.3f/%.3f  16: %.3f/%.3f' % (
+                          label, K, b, res['multi_dev_ms'], res['multi_host_ms'], K, res['singles_dev_ms'],
+                          res['singles_host_ms'], res['ceiling_dev_ms'], res['ceiling_host_ms'],
+                          res['singles_host_ms'] / res['multi_host_ms'],
+                          'bit-identical' if res['bit_identical'] else 'DIFFERENT', km[0], km[1], km[2],
+                          *res['kernel_ms_uniform_2'][:2], *res['kernel_ms_uniform_6'][:2],
+                          *res['kernel_ms_uniform_16'][:2]), flush=True)
+            multi.close()
+        for e in singles:
+            e.close()
+    return rows
+
+
 def time_case(fn, reps, warm=3):
     for _ in range(warm):
         fn()
@@ -97,6 +201,7 @@ def main():
     ap.add_argument('--bs', default='64,128,256,512')
     ap.add_argument('--reps', type=int, default=30)
     ap.add_argument('--lsf', action='store_true', help='per-star LSF vectors (the LSF tail)')
+    ap.add_argument('--layouts', action='store_true', help='per-star parameter layouts, C2 + C3 photometry net')
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit('gpu_multistar.py measures on the GPU: no CUDA device')
@@ -104,6 +209,16 @@ def main():
     bs = [int(v) for v in args.bs.split(',')]
     wave, rsig = synth.ann_wavegrid(5130.0, 5340.0, 50000.0)              # C2 (synth.config_c2)
     spec = synth.make_specnet(4, 256, wave, rsig, seed=0)
+    if args.layouts:
+        rows = run_layouts(args, spec, ks, bs)
+        doc = {'gpu': gpu_info(), 'workload': 'C2 emulator + C3 photometry net, per-star layouts, parity',
+               'reps': args.reps, 'rows': rows}
+        if args.out:
+            os.makedirs(args.out, exist_ok=True)
+            with open(os.path.join(args.out, 'multistar_layouts.json'), 'w') as f:
+                json.dump(doc, f, indent=1)
+        print(json.dumps(doc['gpu']))
+        return
     kw = dict(spec=spec, fitpars_i=FIT, fixedpars={}, runbools=[True, False, False, False, False], precision='parity')
     Kmax = max(ks)
     all_stars = make_stars(spec, Kmax)
