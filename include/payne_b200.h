@@ -228,6 +228,36 @@ int payne_model_batch(PayneCtx* ctx, const double* theta_dev, int64_t B, int64_t
 int payne_model_batch_stars(PayneCtx* ctx, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
                             double* flux_dev, int64_t ld_flux, double* mags_dev, double* lnl_dev, void* stream);
 
+/* Targets: stars observed in several spectra (echelle orders, spectrograph arms, epochs).  A target is a run of
+ * consecutive stars of the observation set, its members, that describe one physical star: target t holds the stars
+ * [first[t], first[t+1]).  first[n_targets + 1] (HOST, copied) must start at 0, increase strictly and end at n_stars;
+ * NULL removes the targets.  A point of the _targets entries names a target, and is evaluated as
+ *   the emulator row (and the continuum emulator) once, from the first member's labels;
+ *   rotational broadening once;
+ *   for every member m in order: Doppler shift, mask, instrumental broadening, resampling on m's pixels, m's continuum
+ *     polynomial, chi2_m -- each chi2_m has the bits of -2 lnL of a single-star context of star m without photometry;
+ *   the SED chi2 once, from the first member's magnitudes;
+ *   lnL = -0.5 * ((((chi2_0 + chi2_1) + ...) + chi2_{K-1}) + chi2_sed).
+ * Members may differ in Vrad, Inst_R (column or fixed value), pixels and continuum order.  At set time
+ * PAYNE_E_INVALID: members that resolve Teff, log(g), [Fe/H], [a/Fe], Vmic or Vrot to different columns or fixed
+ * values; magnitudes on a member other than the first.  PAYNE_E_UNSUPPORTED: a context without the fast tail (emulator
+ * grid not uniform in ln wavelength), with LSF vectors or with the fused gather.  The entries without _targets keep
+ * naming stars.  A target outside [0, n_targets): PAYNE_E_INVALID from the _host entry before anything is launched; on
+ * the device lnL NaN, no model row or chi2, status bit 2.  A member that is bad by itself (e.g. Inst_R above the
+ * emulator's resolution) makes lnL NaN; the other members' model rows and chi2 keep their values.  ld >= the largest
+ * ndim.  Per-(point, member) records bound a slab to min(max_batch, 65536 / the largest member count) points. */
+int payne_ctx_set_targets(PayneCtx* ctx, const int32_t* first, int32_t n_targets);
+int payne_lnlike_batch_targets(PayneCtx* ctx, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
+                               double* lnl_dev, void* stream);
+int payne_lnlike_batch_targets_host(PayneCtx* ctx, const double* theta_host, const int32_t* target_host, int64_t B,
+                                    int64_t ld, double* lnl_host);
+/* flux_dev [B, ld_flux]: row p holds the members' model spectra back to back in member order (ld_flux >= the largest
+ * target's pixel count); chi2_dev [B, ld_chi2]: chi2_dev[p, m] = chi2_m (ld_chi2 >= the largest member count); mags_dev
+ * [B, nb]: the first member's magnitudes.  Any output may be NULL. */
+int payne_model_batch_targets(PayneCtx* ctx, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
+                              double* flux_dev, int64_t ld_flux, double* chi2_dev, int64_t ld_chi2, double* mags_dev,
+                              double* lnl_dev, void* stream);
+
 /* Continuum emulator (HOST pointers, copied): any PayneSpecNet the spectrum emulator could be; its
  * `wavelength` is the continuum's own grid.  From then on every model spectrum is multiplied, right after
  * the emulator and before any broadening, by np.interp(modwave, contwave, c / nanmedian(c), left=nan,
@@ -270,11 +300,11 @@ int payne_lnlike_batch_gather(PayneCtx* ctx, const double* theta_dev, int64_t B,
 int payne_gather_flush(PayneCtx* ctx, void* stream, double** gathered_last);
 
 /* Introspection for benches/tests: key is one of "n_ann","n_obs" (the largest star's),"n_stars","n_obs_total"
- * (observed pixels of all stars),"nfft1","launches",
+ * (observed pixels of all stars),"n_targets","nfft1","launches",
  * "grid_loguniform","fast_tail","max_batch","sm_count","tail_grid","precision","continuum","lsf","legacy_tc"
  * (a leaky-ReLU stack whose output layer runs on the tensor cores),"status"
  * (bit0: a point needed a larger transform than the shared-memory carve-out; bit1: a peer of the gather never arrived;
- * bit2: a point named a star outside [0, n_stars)).
+ * bit2: a point named a star outside [0, n_stars), or a target outside [0, n_targets)).
  * Returns the value or -1. */
 int64_t payne_ctx_query(PayneCtx* ctx, const char* key);
 /* Runtime switches: "precision" (PAYNE_PREC_*), "max_batch" (workspace slab, points), "timing" (0/1,

@@ -27,7 +27,9 @@ EXPORTS = ['payne_abi_version', 'payne_last_error', 'payne_ctx_create', 'payne_c
            'payne_ctx_attach_continuum', 'payne_ctx_set_lsf',
            'payne_gather_create', 'payne_gather_connect', 'payne_lnlike_batch_gather', 'payne_gather_flush',
            'payne_ctx_create_stars', 'payne_lnlike_batch_stars', 'payne_lnlike_batch_stars_host',
-           'payne_model_batch_stars', 'payne_ctx_create_stars_opts']
+           'payne_model_batch_stars', 'payne_ctx_create_stars_opts',
+           'payne_ctx_set_targets', 'payne_lnlike_batch_targets', 'payne_lnlike_batch_targets_host',
+           'payne_model_batch_targets']
 GATHER_HANDLE_BYTES = 128
 
 _f = C.POINTER(C.c_float)
@@ -103,6 +105,14 @@ def load():
     lib.payne_lnlike_batch_stars_host.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp]
     lib.payne_model_batch_stars.restype = C.c_int
     lib.payne_model_batch_stars.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, vp, vp]
+    lib.payne_ctx_set_targets.restype = C.c_int
+    lib.payne_ctx_set_targets.argtypes = [vp, vp, C.c_int32]
+    lib.payne_lnlike_batch_targets.restype = C.c_int
+    lib.payne_lnlike_batch_targets.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, vp]
+    lib.payne_lnlike_batch_targets_host.restype = C.c_int
+    lib.payne_lnlike_batch_targets_host.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp]
+    lib.payne_model_batch_targets.restype = C.c_int
+    lib.payne_model_batch_targets.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, C.c_int64, vp, vp, vp]
     lib.payne_ctx_destroy.restype = None
     lib.payne_ctx_destroy.argtypes = [vp]
     lib.payne_lnlike_batch.restype = C.c_int

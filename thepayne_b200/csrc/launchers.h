@@ -52,6 +52,15 @@ bool probe_tail_fast_poly(int l2, size_t smem_bytes, int* ctas_per_sm);
 int launch_tail_fast_plain(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
 int launch_tail_fast_poly(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
 int launch_tail_setup(int nb, cudaStream_t st, const TailParams& T, const FastGrid& F);
+// targets (payne_ctx_set_targets): the TGT instantiations of tail_fast_kernel and the per-(point, member) setup
+bool probe_tail_fast_targets(int l2, size_t smem_bytes, int* ctas_per_sm);
+bool probe_tail_fast_targets_plain(int l2, size_t smem_bytes, int* ctas_per_sm);
+bool probe_tail_fast_targets_poly(int l2, size_t smem_bytes, int* ctas_per_sm);
+int launch_tail_fast_targets(int l2, bool poly, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T,
+                             const FastGrid& F);
+int launch_tail_fast_targets_plain(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
+int launch_tail_fast_targets_poly(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
+int launch_tail_setup_targets(long long items, cudaStream_t st, const TailParams& T, const FastGrid& F);
 
 // ---- tail_cluster_tu.cu: the same tail with one transform spread over a cluster of four CTAs (tail_cluster.cuh;
 // emulator grids above 16384 pixels).  max_clusters = co-resident clusters on the device.

@@ -8,6 +8,7 @@
 #include <cstring>
 #include <limits>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <cuda_runtime.h>
@@ -173,6 +174,15 @@ struct PayneCtx {
   double* star_fixed_dev = nullptr;     // [n_stars, PAYNE_NPAR] per-star fixed values (payne_ctx_create_stars_opts), or null
   payne::StarLayout* star_lay_dev = nullptr;   // [n_stars] per-star layouts (PayneStarOpts.layout), or null
   int ndim_max = 0;                     // the largest ndim of the context layout and the stars' layouts
+  std::vector<double> star_fixed_h;     // host copies of star_fixed_dev / star_lay_dev (empty without them)
+  std::vector<payne::StarLayout> star_lay_h;
+  // targets (payne_ctx_set_targets): runs of consecutive stars that describe one physical star
+  int n_targets = 0, tgt_kmax = 0, tgt_grid = 0;
+  long long tgt_nobs_max = 0;           // the largest sum of the members' n_obs (model row of a target)
+  int* tfirst_dev = nullptr;            // [n_targets + 1]
+  payne::FastPoint* tgt_points = nullptr;   // [tgt_rows * tgt_kmax] per-(point, member) records
+  int* tgt_star = nullptr;              // [tgt_rows] first member's star of every point of a slab
+  long long tgt_rows = 0, tgt_rec_alloc = 0;
   // photometry
   bool has_phot = false;
   payne::PhotParams phot{};
@@ -894,20 +904,57 @@ int need_star_array(const PayneCtx* c, const int32_t* star, const char* entry) {
   return PAYNE_OK;
 }
 
-// star: [B] star index of every point (null: star 0); flux_out rows are ld_flux apart
+// target: [B] target of every point (payne_ctx_set_targets); the points then name targets and `star` is unused
+__global__ void target_star_kernel(const int* target, const int* tfirst, int n_targets, int* star, int n) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n) return;
+  const int t = target[p];
+  star[p] = (t >= 0 && t < n_targets) ? tfirst[t] : -1;
+}
+
+// Per-(point, member) records of the target tail: at most this many, so the slab of a call with targets is
+// min(max_batch, kTargetRecords / the largest member count) points (20 MB of records).
+constexpr long long kTargetRecords = 65536;
+
+int ensure_target_workspace(PayneCtx* c, long long rows) {
+  if (rows <= c->tgt_rows && rows * c->tgt_kmax <= c->tgt_rec_alloc) return PAYNE_OK;
+  CU_TRY(cudaDeviceSynchronize());                       // earlier calls may still read the records
+  if (c->tgt_points) cudaFree(c->tgt_points);
+  if (c->tgt_star) cudaFree(c->tgt_star);
+  c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
+  const long long rec = rows * c->tgt_kmax;
+  CU_TRY(cudaMalloc((void**)&c->tgt_points, (size_t)rec * sizeof(payne::FastPoint)));
+  CU_TRY(cudaMemset(c->tgt_points, 0, (size_t)rec * sizeof(payne::FastPoint)));
+  CU_TRY(cudaMalloc((void**)&c->tgt_star, (size_t)rows * sizeof(int)));
+  CU_TRY(cudaDeviceSynchronize());
+  c->tgt_rows = rows; c->tgt_rec_alloc = rec;
+  return PAYNE_OK;
+}
+
+// star: [B] star index of every point (null: star 0); flux_out rows are ld_flux apart.  target: see above; chi2_out
+// [B, ld_chi2] the chi2 of every member (targets only)
 int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, long long ld, double* flux_out,
-              long long ld_flux, double* mags_out, double* lnl, cudaStream_t st) {
+              long long ld_flux, double* mags_out, double* lnl, cudaStream_t st, const int* target = nullptr,
+              double* chi2_out = nullptr, long long ld_chi2 = 0) {
   using namespace payne;
   if (B <= 0) return PAYNE_OK;
   if (ld < c->ndim_max) return fail(PAYNE_E_INVALID, "ld < ndim (the largest star's with per-star layouts)");
-  if (flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
+  if (!target && flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
+  const long long slab = target ? std::min(c->slab, std::max(1LL, kTargetRecords / c->tgt_kmax)) : c->slab;
   int rc = ensure_workspace(c, B);
   if (rc) return rc;
+  if (target) { rc = ensure_target_workspace(c, std::min(B, slab)); if (rc) return rc; }
   rc = order_after_previous(c, st);
   if (rc) return rc;
   if (c->timing) { c->ms_acc[0] = c->ms_acc[1] = c->ms_acc[2] = 0; c->ms_valid = false; c->pending.clear(); }
-  for (long long p0 = 0; p0 < B; p0 += c->slab) {
-    const int nb = (int)std::min(c->slab, B - p0);
+  for (long long p0 = 0; p0 < B; p0 += slab) {
+    const int nb = (int)std::min(slab, B - p0);
+    if (target) {
+      // the emulators and the photometry see every point as its target's first member
+      target_star_kernel<<<(nb + 255) / 256, 256, 0, st>>>(target + p0, c->tfirst_dev, c->n_targets, c->tgt_star, nb);
+      c->launches++;
+    }
+    const int* star_s = target ? c->tgt_star : star ? star + p0 : nullptr;   // this slab's star of every point
     const double* th = theta + p0 * ld;
     std::array<cudaEvent_t, 4> evs{};
     if (c->timing) {
@@ -924,8 +971,12 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
       T.lnl = lnl ? lnl + p0 : nullptr;
       T.model_out = flux_out ? flux_out + p0 * ld_flux : nullptr;
       T.ld_flux = ld_flux;
-      T.star = star ? star + p0 : nullptr;
+      T.star = star_s;
       T.status = c->status;
+      if (target) {
+        T.target = target + p0; T.tfirst = c->tfirst_dev; T.n_targets = c->n_targets; T.kmax = c->tgt_kmax;
+        T.chi2_out = chi2_out ? chi2_out + p0 * ld_chi2 : nullptr; T.ld_chi2 = ld_chi2;
+      }
       if (gather_here) {
         // all-gather fused into the tail (tail.cuh store_lnl / gather_exit): this slab's slice of every peer's buffer
         T.g_world = c->g_world; T.g_rank = c->g_rank; T.g_done = c->g_done;
@@ -939,10 +990,18 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         // per-point setup depends only on theta: fork it beside the emulator GEMMs, join before the tail
         CU_TRY(cudaEventRecord(c->ev_fork, st));
         CU_TRY(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-        c->fast.work_start = (c->use_cluster && c->allow_cluster) ? (int)std::min<long long>(c->cluster_n, nb)
+        c->fast.work_start = target ? std::min(c->tgt_grid, nb)
+                           : (c->use_cluster && c->allow_cluster) ? (int)std::min<long long>(c->cluster_n, nb)
                                                                   : std::min(c->tail_grid_fast, nb);
         if (c->grid_cap > 0) c->fast.work_start = std::min(c->fast.work_start, c->grid_cap);
-        if (payne::launch_tail_setup(nb, c->side, T, c->fast)) return fail(PAYNE_E_CUDA, "tail_setup launch");
+        if (target) {
+          FastGrid FT = c->fast;
+          FT.points = c->tgt_points; FT.cluster = 0;
+          if (payne::launch_tail_setup_targets((long long)nb * c->tgt_kmax, c->side, T, FT))
+            return fail(PAYNE_E_CUDA, "tail_setup launch");
+        } else if (payne::launch_tail_setup(nb, c->side, T, c->fast)) {
+          return fail(PAYNE_E_CUDA, "tail_setup launch");
+        }
         if (gather_here && p0 == 0 && c->g_wait_for)
           // the buffer the tail is about to write on the peers is free once every rank's previous step has landed here;
           // waited for on the side stream, beside the emulator GEMMs
@@ -951,7 +1010,7 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         c->launches++;
       }
       EncodeParams E = c->enc;
-      E.star = star ? star + p0 : nullptr;
+      E.star = star_s;
       rc = run_mlp(c, E, th, ld, nb, c->flux, c->ldf, true, &is_depth, st);
       if (rc) return rc;
       if (c->cont) {
@@ -978,7 +1037,7 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
       PhotParams P = c->phot;
       P.theta = th; P.ld = ld; P.B = nb; P.chi2_sed = c->chi2_sed;
       P.mags_out = mags_out ? mags_out + p0 * P.nb : nullptr;
-      P.star = star ? star + p0 : nullptr;
+      P.star = star_s;
       P.status = c->status;
       if (P.band_slot)
         phot_kernel<true><<<(nb + kPhotTile - 1) / kPhotTile, kPhotThreads, c->phot_smem, st>>>(P);
@@ -997,6 +1056,14 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         // ... a star's own fixed Inst_R and a per-star layout's Inst_R column too: Rs = NaN, no scalar-R stage
         TL.inst_scale = std::numeric_limits<double>::quiet_NaN();
         if (payne::launch_tail_lsf(std::min(c->lsf_grid, nb), c->lsf_smem, st, TL, c->lsf)) return fail(PAYNE_E_CUDA, "tail launch");
+      } else if (target) {
+        // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no target form)
+        if (!(fast_tail && is_depth)) return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail on line-depth rows");
+        FastGrid FT = c->fast;
+        FT.points = c->tgt_points; FT.cluster = 0;
+        const bool poly = T.n_poly != 0 || T.model_out != nullptr;
+        if (payne::launch_tail_fast_targets(T.log2N1, poly, c->fast.work_start, c->fast_smem, st, T, FT))
+          return fail(PAYNE_E_CUDA, "tail launch");
       } else if (fast_tail && is_depth && c->use_cluster && c->allow_cluster) {
         payne::FastGrid FC = c->fast;
         FC.win_floats = c->cluster_win_floats;
@@ -1091,14 +1158,173 @@ int upload_star_layouts(PayneCtx* c, const PayneLayout* ctx, const PayneStarOpts
   }
   int rc = upload_owned(c, &c->star_lay_dev, rec.data(), rec.size());
   if (rc) return rc;
+  c->star_lay_h = rec;
   c->tail.n_poly = n_poly_max;       // the final passes evaluate this many coefficients (tail_setup pads with zeros)
   c->tail.star_lay = c->phot.star_lay = c->enc.star_lay = c->star_lay_dev;
   return PAYNE_OK;
 }
 
+// The target entries: targets set, and the context still runs the tail they need.
+int need_targets(const PayneCtx* c) {
+  if (c->n_targets == 0) return fail(PAYNE_E_INVALID, "no targets: payne_ctx_set_targets first");
+  if (!(c->use_fast && c->allow_fast) || c->lsf_on || c->g_world > 0)
+    return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail without LSF vectors or the fused gather");
+  return PAYNE_OK;
+}
+
+// The host-buffer entries: idx_host is every point's star, or its target (targets = true), or null (star 0).
+int lnlike_host(PayneCtx* c, const double* theta_host, const int32_t* star_host, int64_t B, int64_t ld, double* lnl_host,
+                bool targets) {
+  int rc;
+  const int n_idx = targets ? c->n_targets : c->n_stars;
+  if (star_host)
+    for (int64_t i = 0; i < B; ++i)
+      if (star_host[i] < 0 || star_host[i] >= n_idx)
+        return fail(PAYNE_E_INVALID, std::string(targets ? "target" : "star") + " index " + std::to_string(star_host[i]) +
+                    " of point " + std::to_string(i) + " outside [0, " + std::to_string(n_idx) + ")");
+  DeviceGuard dg(c->device);
+  if (star_host && B > c->star_cap) {
+    if (c->star_pin) cudaFreeHost(c->star_pin);
+    if (c->star_stage) cudaFree(c->star_stage);
+    c->star_pin = c->star_stage = nullptr; c->star_cap = 0;
+    CU_TRY(cudaMallocHost((void**)&c->star_pin, (size_t)B * sizeof(int)));
+    CU_TRY(cudaMalloc((void**)&c->star_stage, (size_t)B * sizeof(int)));
+    c->star_cap = B;
+  }
+  if (B > c->stage_cap || ld != c->stage_ld) {
+    if (c->theta_pin) cudaFreeHost(c->theta_pin);
+    if (c->lnl_pin) cudaFreeHost(c->lnl_pin);
+    if (c->theta_stage) cudaFree(c->theta_stage);
+    if (c->lnl_stage) cudaFree(c->lnl_stage);
+    c->theta_pin = c->lnl_pin = c->theta_stage = c->lnl_stage = nullptr; c->lnl_map = nullptr; c->stage_cap = 0;
+    CU_TRY(cudaMallocHost((void**)&c->theta_pin, (size_t)B * ld * sizeof(double)));
+    CU_TRY(cudaMallocHost((void**)&c->lnl_pin, (size_t)B * sizeof(double)));
+    CU_TRY(cudaMalloc((void**)&c->theta_stage, (size_t)B * ld * sizeof(double)));
+    CU_TRY(cudaMalloc((void**)&c->lnl_stage, (size_t)B * sizeof(double)));
+    c->stage_cap = B; c->stage_ld = ld;
+    // 8 bytes per point: the last kernel writes them into the pinned buffer itself (mapped under unified
+    // addressing) instead of a device buffer + a D2H copy behind it (one enqueue and one copy latency per call)
+    void* dp = nullptr;
+    const char* zenv = getenv("PAYNE_ZERO_COPY_LNL");
+    c->lnl_map = (!(zenv && zenv[0] == '0') && cudaHostGetDevicePointer(&dp, c->lnl_pin, 0) == cudaSuccess) ? (double*)dp : nullptr;
+    cudaGetLastError();
+  }
+  std::memcpy(c->theta_pin, theta_host, (size_t)B * ld * sizeof(double));
+  CU_TRY(cudaMemcpyAsync(c->theta_stage, c->theta_pin, (size_t)B * ld * sizeof(double),
+                         cudaMemcpyHostToDevice, c->stream));
+  if (star_host) {
+    std::memcpy(c->star_pin, star_host, (size_t)B * sizeof(int));
+    CU_TRY(cudaMemcpyAsync(c->star_stage, c->star_pin, (size_t)B * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+  }
+  const int* idx = star_host ? c->star_stage : nullptr;
+  rc = run_batch(c, c->theta_stage, targets ? nullptr : idx, B, ld, nullptr, 0, nullptr,
+                 c->lnl_map ? c->lnl_map : c->lnl_stage, c->stream, targets ? idx : nullptr);
+  if (rc) return rc;
+  if (!c->lnl_map)
+    CU_TRY(cudaMemcpyAsync(c->lnl_pin, c->lnl_stage, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost,
+                           c->stream));
+  CU_TRY(cudaStreamSynchronize(c->stream));
+  std::memcpy(lnl_host, c->lnl_pin, (size_t)B * sizeof(double));
+  return PAYNE_OK;
+}
+
+
+// The value of parameter `which` that star k resolves to: its column, or (column -1) its fixed value.
+std::pair<int, double> resolve_param(const PayneCtx* c, int k, int which) {
+  const int col = c->star_lay_h.empty() ? c->lay.col[which] : c->star_lay_h[k].col[which];
+  if (col >= 0) return {col, 0.0};
+  return {-1, c->star_fixed_h.empty() ? c->lay.fixed[which] : c->star_fixed_h[(size_t)k * PAYNE_NPAR + which]};
+}
+
 }  // namespace
 
 extern "C" {
+
+int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  if (!first) {
+    CU_TRY(cudaDeviceSynchronize());                     // earlier calls may still read the table
+    if (c->tfirst_dev) cudaFree(c->tfirst_dev);
+    if (c->tgt_points) cudaFree(c->tgt_points);
+    if (c->tgt_star) cudaFree(c->tgt_star);
+    c->tfirst_dev = nullptr; c->n_targets = 0; c->tgt_kmax = 0; c->tgt_nobs_max = 0;
+    c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
+    return PAYNE_OK;
+  }
+  if (!c->has_spec) return fail(PAYNE_E_UNSUPPORTED, "targets need the spectrum emulator");
+  if (!c->use_fast) return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail (an emulator grid uniform in ln wavelength)");
+  if (c->lsf_on) return fail(PAYNE_E_UNSUPPORTED, "targets with LSF vectors are not supported");
+  if (c->g_world > 0) return fail(PAYNE_E_UNSUPPORTED, "targets on a context with the fused gather are not supported");
+  if (n_targets < 1) return fail(PAYNE_E_INVALID, "n_targets must be >= 1");
+  if (first[0] != 0 || first[n_targets] != c->n_stars)
+    return fail(PAYNE_E_INVALID, "first[0] must be 0 and first[n_targets] n_stars (" + std::to_string(c->n_stars) + ")");
+  int kmax = 0;
+  long long nobs_max = 0;
+  for (int t = 0; t < n_targets; ++t) {
+    if (first[t + 1] <= first[t]) return fail(PAYNE_E_INVALID, "first[] must increase strictly (target " + std::to_string(t) + ")");
+    kmax = std::max(kmax, first[t + 1] - first[t]);
+    long long no = 0;
+    for (int k = first[t]; k < first[t + 1]; ++k) no += c->stars[k].n_obs;
+    nobs_max = std::max(nobs_max, no);
+    static const char* names[6] = {"Teff", "log(g)", "[Fe/H]", "[a/Fe]", "Vmic", "Vrot"};
+    static const int which[6] = {PAYNE_P_TEFF, PAYNE_P_LOGG, PAYNE_P_FEH, PAYNE_P_AFE, PAYNE_P_VMIC, PAYNE_P_VROT};
+    for (int k = first[t] + 1; k < first[t + 1]; ++k) {
+      const std::string who = "target " + std::to_string(t) + ", member " + std::to_string(k - first[t]) + ": ";
+      for (int i = 0; i < 6; ++i) {
+        // the emulator row and stage 1 are computed once per point, from these values of the first member
+        const auto a = resolve_param(c, first[t], which[i]), b = resolve_param(c, k, which[i]);
+        if (a.first != b.first || (a.first < 0 && std::memcmp(&a.second, &b.second, sizeof(double)) != 0))
+          return fail(PAYNE_E_INVALID, who + std::string(names[i]) + " differs from the first member's (column or fixed value)");
+      }
+      if (c->has_phot && c->stars[k].nb > 0)
+        return fail(PAYNE_E_INVALID, who + "photometry on a member other than the first");
+    }
+  }
+  int occ = 0;
+  if (!payne::probe_tail_fast_targets(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
+    return fail(PAYNE_E_UNSUPPORTED, "target tail kernel does not fit on an SM");
+  CU_TRY(cudaDeviceSynchronize());
+  if (c->tfirst_dev) cudaFree(c->tfirst_dev);
+  c->tfirst_dev = nullptr; c->n_targets = 0;
+  int rc = upload(&c->tfirst_dev, first, (size_t)n_targets + 1);
+  if (rc) return rc;
+  if (c->tgt_kmax != kmax) {                             // the record stride changes: reallocate at the next call
+    if (c->tgt_points) cudaFree(c->tgt_points);
+    if (c->tgt_star) cudaFree(c->tgt_star);
+    c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
+  }
+  c->n_targets = n_targets; c->tgt_kmax = kmax; c->tgt_nobs_max = nobs_max;
+  // the split kernel's scratch lines exist for tail_grid_fast CTAs
+  c->tgt_grid = std::min(occ * c->sm_count, c->tail_grid_fast);
+  return PAYNE_OK;
+}
+
+int payne_lnlike_batch_targets(PayneCtx* c, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
+                               double* lnl_dev, void* stream) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B == 0) return PAYNE_OK;
+  if (!theta_dev || !target_dev || !lnl_dev) return fail(PAYNE_E_INVALID, "null argument");
+  int rc = need_targets(c);
+  if (rc) return rc;
+  DeviceGuard dg(c->device);
+  return run_batch(c, theta_dev, nullptr, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, target_dev);
+}
+
+int payne_model_batch_targets(PayneCtx* c, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
+                              double* flux_dev, int64_t ld_flux, double* chi2_dev, int64_t ld_chi2, double* mags_dev,
+                              double* lnl_dev, void* stream) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B == 0) return PAYNE_OK;
+  if (!theta_dev || !target_dev) return fail(PAYNE_E_INVALID, "null argument");
+  int rc = need_targets(c);
+  if (rc) return rc;
+  if (flux_dev && ld_flux < c->tgt_nobs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest target's pixels (all members)");
+  if (chi2_dev && ld_chi2 < c->tgt_kmax) return fail(PAYNE_E_INVALID, "ld_chi2 < the largest member count");
+  DeviceGuard dg(c->device);
+  return run_batch(c, theta_dev, nullptr, B, ld, flux_dev, ld_flux, mags_dev, lnl_dev, (cudaStream_t)stream, target_dev,
+                   chi2_dev, ld_chi2);
+}
 
 int payne_abi_version(void) { return PAYNE_ABI_VERSION; }
 const char* payne_last_error(void) { return g_err.c_str(); }
@@ -1166,6 +1392,7 @@ int payne_ctx_create_stars_opts(const PayneSpecNet* spec, const PaynePhotNet* ph
       std::memcpy(&fx[(size_t)k * PAYNE_NPAR], opts[k].fixed ? opts[k].fixed : opts[k].layout ? opts[k].layout->fixed : layout->fixed,
                   PAYNE_NPAR * sizeof(double));
     rc = upload_owned(c, &c->star_fixed_dev, fx.data(), fx.size());
+    c->star_fixed_h = fx;
   }
   if (!rc) {
     c->tail.stars = c->phot.stars = c->stars_dev;
@@ -1189,6 +1416,7 @@ void payne_ctx_destroy(PayneCtx* c) {
   c->fast.points = nullptr; drop(c->status);
   payne::tc_free_acts_x(&c->actA); payne::tc_free_acts_x(&c->actB);
   drop(c->theta_stage); drop(c->lnl_stage); drop(c->star_stage);
+  drop(c->tfirst_dev); drop(c->tgt_points); drop(c->tgt_star);
   if (c->star_pin) cudaFreeHost(c->star_pin);
   for (int r = 0; r < 16; ++r)
     if (c->g_opened[r]) { cudaIpcCloseMemHandle(c->g_peer_buf[r]); cudaIpcCloseMemHandle(c->g_peer_flag[r]); }
@@ -1248,54 +1476,17 @@ int payne_lnlike_batch_stars_host(PayneCtx* c, const double* theta_host, const i
   if (B <= 0) return PAYNE_OK;
   int rc = need_star_array(c, star_host, "payne_lnlike_batch_stars_host");
   if (rc) return rc;
-  if (star_host)
-    for (int64_t i = 0; i < B; ++i)
-      if (star_host[i] < 0 || star_host[i] >= c->n_stars)
-        return fail(PAYNE_E_INVALID, "star index " + std::to_string(star_host[i]) + " of point " + std::to_string(i) +
-                    " outside [0, " + std::to_string(c->n_stars) + ")");
-  DeviceGuard dg(c->device);
-  if (star_host && B > c->star_cap) {
-    if (c->star_pin) cudaFreeHost(c->star_pin);
-    if (c->star_stage) cudaFree(c->star_stage);
-    c->star_pin = c->star_stage = nullptr; c->star_cap = 0;
-    CU_TRY(cudaMallocHost((void**)&c->star_pin, (size_t)B * sizeof(int)));
-    CU_TRY(cudaMalloc((void**)&c->star_stage, (size_t)B * sizeof(int)));
-    c->star_cap = B;
-  }
-  if (B > c->stage_cap || ld != c->stage_ld) {
-    if (c->theta_pin) cudaFreeHost(c->theta_pin);
-    if (c->lnl_pin) cudaFreeHost(c->lnl_pin);
-    if (c->theta_stage) cudaFree(c->theta_stage);
-    if (c->lnl_stage) cudaFree(c->lnl_stage);
-    c->theta_pin = c->lnl_pin = c->theta_stage = c->lnl_stage = nullptr; c->lnl_map = nullptr; c->stage_cap = 0;
-    CU_TRY(cudaMallocHost((void**)&c->theta_pin, (size_t)B * ld * sizeof(double)));
-    CU_TRY(cudaMallocHost((void**)&c->lnl_pin, (size_t)B * sizeof(double)));
-    CU_TRY(cudaMalloc((void**)&c->theta_stage, (size_t)B * ld * sizeof(double)));
-    CU_TRY(cudaMalloc((void**)&c->lnl_stage, (size_t)B * sizeof(double)));
-    c->stage_cap = B; c->stage_ld = ld;
-    // 8 bytes per point: the last kernel writes them into the pinned buffer itself (mapped under unified
-    // addressing) instead of a device buffer + a D2H copy behind it (one enqueue and one copy latency per call)
-    void* dp = nullptr;
-    const char* zenv = getenv("PAYNE_ZERO_COPY_LNL");
-    c->lnl_map = (!(zenv && zenv[0] == '0') && cudaHostGetDevicePointer(&dp, c->lnl_pin, 0) == cudaSuccess) ? (double*)dp : nullptr;
-    cudaGetLastError();
-  }
-  std::memcpy(c->theta_pin, theta_host, (size_t)B * ld * sizeof(double));
-  CU_TRY(cudaMemcpyAsync(c->theta_stage, c->theta_pin, (size_t)B * ld * sizeof(double),
-                         cudaMemcpyHostToDevice, c->stream));
-  if (star_host) {
-    std::memcpy(c->star_pin, star_host, (size_t)B * sizeof(int));
-    CU_TRY(cudaMemcpyAsync(c->star_stage, c->star_pin, (size_t)B * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-  }
-  rc = run_batch(c, c->theta_stage, star_host ? c->star_stage : nullptr, B, ld, nullptr, 0, nullptr,
-                 c->lnl_map ? c->lnl_map : c->lnl_stage, c->stream);
+  return lnlike_host(c, theta_host, star_host, B, ld, lnl_host, false);
+}
+
+int payne_lnlike_batch_targets_host(PayneCtx* c, const double* theta_host, const int32_t* target_host, int64_t B,
+                                    int64_t ld, double* lnl_host) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B <= 0) return PAYNE_OK;
+  if (!theta_host || !target_host || !lnl_host) return fail(PAYNE_E_INVALID, "null argument");
+  int rc = need_targets(c);
   if (rc) return rc;
-  if (!c->lnl_map)
-    CU_TRY(cudaMemcpyAsync(c->lnl_pin, c->lnl_stage, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost,
-                           c->stream));
-  CU_TRY(cudaStreamSynchronize(c->stream));
-  std::memcpy(lnl_host, c->lnl_pin, (size_t)B * sizeof(double));
-  return PAYNE_OK;
+  return lnlike_host(c, theta_host, target_host, B, ld, lnl_host, true);
 }
 
 }  // extern "C"
@@ -1561,6 +1752,7 @@ int64_t payne_ctx_query(PayneCtx* c, const char* key) {
   if (k == "n_ann") return c->D_out;
   if (k == "n_obs") return c->n_obs_max;
   if (k == "n_stars") return c->n_stars;
+  if (k == "n_targets") return c->n_targets;
   if (k == "n_obs_total") return c->n_obs_total;
   if (k == "nfft1") return c->has_spec ? (1LL << c->tail.log2N1) : 0;
   if (k == "launches") return c->launches;

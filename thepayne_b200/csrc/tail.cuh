@@ -97,6 +97,14 @@ struct TailParams {
   // `fixed` / `label_fixed`; null when the context was created without them.
   const double* star_fixed;
   const StarLayout* star_lay;        // [n_stars] per-star layouts (obs_star.cuh), null without them
+  // Targets (payne_ctx_set_targets; fast tail only): point p names target[p], whose members are the stars
+  // [tfirst[t], tfirst[t + 1]); member m's per-point record is FastPoint p * kmax + m.  A target outside
+  // [0, n_targets) gets lnL NaN, no model row and status bit 2.  Null target: the points name stars.
+  const int* target;
+  const int* tfirst;                 // [n_targets + 1]
+  int n_targets, kmax;               // kmax: the largest member count
+  double* chi2_out;                  // [B, ld_chi2] chi2 of every member, or null
+  long long ld_chi2;
 };
 
 // lnL of point p: local result and, with the fused gather on, the copy in every peer's buffer
@@ -264,8 +272,9 @@ __device__ __forceinline__ float depth_of(float v, bool is_depth, bool fill_nan)
   return is_depth ? v : v - 1.f;
 }
 
-static __device__ void tail_setup(const TailParams& P, const double* th, int p, PointSetup& S, ObsSlice& obs) {
-  const int k = star_of(P.star, P.n_stars, p);
+// Point setup of theta row th against star k (k < 0: no such star).
+static __device__ __forceinline__ void tail_setup_star(const TailParams& P, const double* th, int k, PointSetup& S,
+                                                       ObsSlice& obs) {
   if (k < 0) {                                    // no observation to compare with: NaN, nothing written
     S.bad = 1; S.use_inst = 0; S.do_rot = 0;
     obs.off = 0; obs.n = 0;
@@ -337,6 +346,10 @@ static __device__ void tail_setup(const TailParams& P, const double* th, int p, 
   const double dv = kCkms * S.du;                  // smoothing.py:282
   const double nd = (double)N2 * dv;
   S.taper_a = (float)(2.0 * CUDART_PI * CUDART_PI * s2 / (nd * nd));
+}
+
+static __device__ void tail_setup(const TailParams& P, const double* th, int p, PointSetup& S, ObsSlice& obs) {
+  tail_setup_star(P, th, star_of(P.star, P.n_stars, p), S, obs);
 }
 
 }  // namespace payne

@@ -203,15 +203,16 @@ __device__ __forceinline__ int obs_hi(const TailParams& P, const ObsSlice& o) { 
 // (positions -> samples -> depth; then the per-pixel constants -> Clenshaw on four abscissae at once ->
 // residuals).  It lives in its own instantiation of the kernel (POLY = true): the plain path sits at its 80-register
 // cap and any code beside it changes its allocation (measured: +0.5 % with this loop behind a call).
+// moff: column of the point's first pixel in its model row (a target's member m: the pixels of members 0 .. m-1).
 template <bool STARS, class ZV>
 __device__ __forceinline__ double final_pass_poly(const TailParams& P, const FastGrid& F, const PointSetup& S,
-                                                  const FastSetup& FS, const ZV& zv, int tid, int p, int N2) {
+                                                  const FastSetup& FS, const ZV& zv, int tid, int p, int N2, int moff = 0) {
   const double nan = CUDART_NAN;
   const double pmax = (double)(N2 - 1);
   const float hdu = S.hdu;
   const double q0 = FS.q0, scale = FS.scale;
   const int off = obs_lo<STARS>(FS.obs), jend = obs_hi<STARS>(P, FS.obs);   // the point's star: pixels [off, jend)
-  double* mrow = P.model_out ? P.model_out + (long long)p * P.ld_flux : nullptr;
+  double* mrow = P.model_out ? P.model_out + (long long)p * P.ld_flux + moff : nullptr;
   double acc = 0.0;
   constexpr int U = 4;
 #pragma unroll 1
@@ -261,7 +262,7 @@ __device__ __forceinline__ double final_pass_poly(const TailParams& P, const Fas
 // observed pixels, continuum, residuals; returns this thread's partial chi2
 template <bool POLY, bool STARS, class ZV>
 __device__ __forceinline__ double final_pass(const TailParams& P, const FastGrid& F, const PointSetup& S,
-                                             const FastSetup& FS, const ZV& zv, int tid, int p, int N2) {
+                                             const FastSetup& FS, const ZV& zv, int tid, int p, int N2, int moff = 0) {
   const double nan = CUDART_NAN;
   const double pmax = (double)(N2 - 1);
   const float hdu = S.hdu;
@@ -302,7 +303,7 @@ __device__ __forceinline__ double final_pass(const TailParams& P, const FastGrid
       }
     }
   } else {
-    acc = final_pass_poly<STARS>(P, F, S, FS, zv, tid, p, N2);
+    acc = final_pass_poly<STARS>(P, F, S, FS, zv, tid, p, N2, moff);
   }
   return acc;
 }
@@ -317,12 +318,84 @@ static __device__ __noinline__ void discard_lines(const float* row, int n, int t
     asm volatile("discard.global.L2 [%0], 128;" ::"l"(a));
 }
 
+// Stage 2 and the final pass of one point against its star (S, FS) on the row that stage 1 left; returns this
+// thread's partial chi2.  z / zs / zp / gline: the kernel's transform buffer and its views.
+template <int LOG2N1, bool POLY, bool STARS>
+__device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid& F, const PointSetup& S,
+                                             const FastSetup& FS, float2* z, const ZSmem& zs, const ZSplit& zp,
+                                             float* gline, const TwTab& tw, const float* row, int tid, int p, int moff) {
+  constexpr bool kSplit = LOG2N1 >= 16;
+  constexpr int LOG2MH = kSplit ? LOG2N1 - 2 : 8;
+  const double nan = CUDART_NAN;
+  const bool is_depth = true;   // this kernel is only launched on line-depth rows (f - 1)
+  double acc = 0.0;
+  if (S.use_inst) {
+    // ---------------- stage 2: mask, regrid, Gaussian broadening
+    const int log2N2 = S.log2N2, N2 = 1 << log2N2;
+    const int i0 = S.i0;
+    GaussH H{S.taper_a, 2.0f / (float)N2};
+    bool split2 = false;
+    if constexpr (kSplit) split2 = (log2N2 == LOG2N1);
+    if (split2) {
+      if constexpr (kSplit) {
+        stage_regrid(S, row, zp, tid, N2, FS.s_num, FS.s_den, i0, FS.s_invden, F.c_native, FS.s_incj, FS.s_incr);
+        __syncthreads();
+        ct_convolve_split<LOG2MH>(z, reinterpret_cast<float2*>(gline), tw, F.twc, H, tid);
+        acc = final_pass<POLY, STARS>(P, F, S, FS, zp, tid, p, N2, moff);
+      }
+    } else {
+      constexpr int LA = LOG2N1 > 15 ? 15 : LOG2N1;       // largest all-in-smem transform
+      if (!(log2N2 == LA || (LA >= 10 && log2N2 == LA - 1))) {
+        // small masks: separate regrid, runtime-planned transform
+        stage_regrid(S, row, zs, tid, N2, FS.s_num, FS.s_den, i0, FS.s_invden, F.c_native, FS.s_incj, FS.s_incr);
+        __syncthreads();
+        const Twiddles twr{tw.tab, tw.log2n};
+        FftPlan plan; plan.make(log2N2 - 1);
+        fft_forward(z, log2N2 - 1, plan, twr, tid, kNT);
+        filter_pairs(z, log2N2 - 1, plan, twr, H, tid, kNT);
+        fft_inverse(z, log2N2 - 1, plan, twr, tid, kNT);
+      } else if (log2N2 == LA) {
+        ct_convolve_regrid<LA - 1>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den, FS.s_invden, F.c_native, S.clean != 0);
+      } else {
+        ct_convolve_regrid<(LA >= 10 ? LA - 2 : 8)>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den,
+                                                     FS.s_invden, F.c_native, S.clean != 0);
+      }
+      acc = final_pass<POLY, STARS>(P, F, S, FS, zs, tid, p, N2, moff);
+    }
+  } else {
+    // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289)
+    const int n = P.n;
+    const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
+    const int off = obs_lo<STARS>(FS.obs), jend = obs_hi<STARS>(P, FS.obs);
+    for (int j = off + tid; j < jend; j += kNT) {
+      const double x = __ldg(P.obs_w + j);
+      double m;
+      if (!(x >= wlo && x <= whi)) m = nan;
+      else {
+        const int g = (int)((__ldg(P.obs_lnw + j) - S.lnD - P.lnw0) * P.inv_dlnw);
+        const int jj = locate(P.w, S.D, x, g, 0, n - 2);
+        const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
+        const double a = (double)depth_of(row[jj], is_depth, false);
+        const double b = (double)depth_of(row[jj + 1], is_depth, false);
+        m = 1.0 + ((b - a) / (wb - wa) * (x - wa) + a);
+      }
+      if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
+      if (P.model_out) P.model_out[(long long)p * P.ld_flux + moff + (j - off)] = m;
+      const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
+      acc += r * r;
+    }
+  }
+  return acc;
+}
+
 // LOG2N1 <= 15: the whole transform sits in shared memory (3 CTAs/SM up to 2^14).
 // LOG2N1 == 16: split transform, half in shared memory (128 KB), half in the scratch line.
 // POLY: continuum polynomial and / or model output in the final pass (the host picks the instantiation).
 // STARS: a context of several stars (obs_lo / obs_hi).
+// TGT: every point names a target (TailParams::target; STARS is then true): stage 1 runs once on the row, then stage 2
+// and the final pass once per member against that member's record, and lnL is the members' chi2 summed in member order.
 // (3 CTAs/SM, 80 registers with a few spills, measured at C2 0.76 ms against 0.84 ms with 2 CTAs/SM and no spills)
-template <int LOG2N1, bool POLY, bool STARS>
+template <int LOG2N1, bool POLY, bool STARS, bool TGT = false>
 __global__ void __launch_bounds__(kNT, LOG2N1 <= 14 ? 3 : 1)
 tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -354,21 +427,50 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
     // the next point is claimed now (its latency hides under this point) and read after the barrier below; thread 0
     // writes s_next again only behind this iteration's last barrier
     if (tid == 0) s_next = F.work_counter ? atomicAdd(F.work_counter, 1) : p + (int)gridDim.x;
+    const FastPoint* rec = points + p;
+    int K = 1;                                            // members (targets; 0: no such target)
+    if constexpr (TGT) {
+      const int t = __ldg(P.target + p);
+      K = (t >= 0 && t < P.n_targets) ? __ldg(P.tfirst + t + 1) - __ldg(P.tfirst + t) : 0;
+      rec = points + (long long)p * P.kmax;
+      if (tid >= 32 && tid < 64) {
+        // warp 1: the pixels that the members' stage 2 and final passes read, the union of their windows (in red[1],
+        // dead like red[0] until the first member's reduction)
+        int lo = P.n, hi = -1;
+        for (int m = tid - 32; m < K; m += 32) {
+          const PointSetup& Sm = rec[m].S;
+          if (Sm.bad) continue;
+          lo = min(lo, Sm.use_inst ? max(Sm.i0 - 1, 0) : 0);
+          hi = max(hi, Sm.use_inst ? min(Sm.i1 + 1, P.n - 1) : P.n - 1);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+          hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+        }
+        if (tid == 32) *reinterpret_cast<int2*>(&red[1]) = make_int2(lo, hi);
+      }
+    }
     if (tid < (int)(sizeof(FastPoint) / 16))
-      reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(points + p) + tid);
+      reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(rec) + tid);
     __syncthreads();
     pn = s_next;
-    if (S.bad) {
+    int2 tu = make_int2(0, -1);
+    if constexpr (TGT) {
+      tu = *reinterpret_cast<const int2*>(&red[1]);
+      __syncthreads();                                    // red[1] is read everywhere before a member's reduction
+    }
+    if (TGT ? K == 0 : S.bad) {
       if (P.model_out)
         for (int j = tid; j < obs_hi<STARS>(P, FS.obs) - obs_lo<STARS>(FS.obs); j += kNT) P.model_out[(long long)p * P.ld_flux + j] = nan;
       if (tid == 0 && P.lnl) store_lnl(P, p, nan);
       __syncthreads();
       continue;
     }
-    const bool is_depth = true;   // this kernel is only launched on line-depth rows (f - 1)
-
     // ---------------- stage 1: rotational broadening on the full emulator grid
-    if (S.do_rot) {
+    // (a target: the labels and Vrot of every member are the first member's -- payne_ctx_set_targets -- so its
+    // do_rot, vsini_scale and clean hold for the row; skipped when every member is bad)
+    if (TGT ? (S.do_rot && tu.x <= tu.y) : S.do_rot) {
       const int n = P.n;
       // the table entries this point can touch: [0, vsini_scale * N1/2 + 3]; staged in shared
       // memory when they fit (the barrier after the regrid below publishes them)
@@ -382,7 +484,8 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
       win_have = max(win_have, nwin);
       const RotHT<2> H{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, 1.0f / (float)(N1 >> 1), P.ntab, RotHT<2>::fix40(S.vsini_scale)};
       // pixels stage 2 will read: its mask [i0, i1] (one more on each side keeps the edge patch exact)
-      const int blo = S.use_inst ? max(S.i0 - 1, 0) : 0, bhi = S.use_inst ? min(S.i1 + 1, n - 1) : n - 1;
+      const int blo = TGT ? tu.x : S.use_inst ? max(S.i0 - 1, 0) : 0;
+      const int bhi = TGT ? tu.y : S.use_inst ? min(S.i1 + 1, n - 1) : n - 1;
       if constexpr (!kSplit) {
         // regrid fused into the first FFT pass (measured against the separate regrid: tail -5 %)
         ct_convolve_regrid<LOG2N1 - 1>(z, tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
@@ -396,73 +499,54 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
       __syncthreads();
     }
 
-    double acc = 0.0;
-    if (S.use_inst) {
-      // ---------------- stage 2: mask, regrid, Gaussian broadening
-      const int log2N2 = S.log2N2, N2 = 1 << log2N2;
-      const int i0 = S.i0;
-      GaussH H{S.taper_a, 2.0f / (float)N2};
-      bool split2 = false;
-      if constexpr (kSplit) split2 = (log2N2 == LOG2N1);
-      if (split2) {
-        if constexpr (kSplit) {
-          stage_regrid(S, row, zp, tid, N2, FS.s_num, FS.s_den, i0, FS.s_invden, F.c_native, FS.s_incj, FS.s_incr);
-          __syncthreads();
-          ct_convolve_split<LOG2MH>(z, reinterpret_cast<float2*>(gline), tw, F.twc, H, tid);
-          acc = final_pass<POLY, STARS>(P, F, S, FS, zp, tid, p, N2);
-        }
-      } else {
-        constexpr int LA = LOG2N1 > 15 ? 15 : LOG2N1;       // largest all-in-smem transform
-        if (!(log2N2 == LA || (LA >= 10 && log2N2 == LA - 1))) {
-          // small masks: separate regrid, runtime-planned transform
-          stage_regrid(S, row, zs, tid, N2, FS.s_num, FS.s_den, i0, FS.s_invden, F.c_native, FS.s_incj, FS.s_incr);
-          __syncthreads();
-          const Twiddles twr{tw.tab, tw.log2n};
-          FftPlan plan; plan.make(log2N2 - 1);
-          fft_forward(z, log2N2 - 1, plan, twr, tid, kNT);
-          filter_pairs(z, log2N2 - 1, plan, twr, H, tid, kNT);
-          fft_inverse(z, log2N2 - 1, plan, twr, tid, kNT);
-        } else if (log2N2 == LA) {
-          ct_convolve_regrid<LA - 1>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den, FS.s_invden, F.c_native, S.clean != 0);
-        } else {
-          ct_convolve_regrid<(LA >= 10 ? LA - 2 : 8)>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den,
-                                                       FS.s_invden, F.c_native, S.clean != 0);
-        }
-        acc = final_pass<POLY, STARS>(P, F, S, FS, zs, tid, p, N2);
+    if constexpr (!TGT) {
+      double acc = point_chi2<LOG2N1, POLY, STARS>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, 0);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+      if ((tid & 31) == 0) red[tid >> 5] = acc;
+      __syncthreads();
+      if (tid == 0 && P.lnl) {
+        double c2 = 0.0;
+#pragma unroll
+        for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
+        if (P.chi2_sed) c2 += P.chi2_sed[p];
+        store_lnl(P, p, -0.5 * c2);
       }
     } else {
-      // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289)
-      const int n = P.n;
-      const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
-      const int off = obs_lo<STARS>(FS.obs), jend = obs_hi<STARS>(P, FS.obs);
-      for (int j = off + tid; j < jend; j += kNT) {
-        const double x = __ldg(P.obs_w + j);
-        double m;
-        if (!(x >= wlo && x <= whi)) m = nan;
-        else {
-          const int g = (int)((__ldg(P.obs_lnw + j) - S.lnD - P.lnw0) * P.inv_dlnw);
-          const int jj = locate(P.w, S.D, x, g, 0, n - 2);
-          const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
-          const double a = (double)depth_of(row[jj], is_depth, false);
-          const double b = (double)depth_of(row[jj + 1], is_depth, false);
-          m = 1.0 + ((b - a) / (wb - wa) * (x - wa) + a);
+      // every member against its own record: the row is read-only from here on.  Member m's model pixels follow
+      // those of members 0 .. m-1 (the members' observations lie back to back in the set's arrays).
+      const int off0 = FS.obs.off;
+      double tot = 0.0;                                   // thread 0: chi2 of members 0 .. m, summed in that order
+      for (int m = 0; m < K; ++m) {
+        if (m > 0) {
+          __syncthreads();                                // member m-1's record, transform buffer and red[] are free
+          if (tid < (int)(sizeof(FastPoint) / 16))
+            reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(rec + m) + tid);
+          __syncthreads();
         }
-        if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-        if (P.model_out) P.model_out[(long long)p * P.ld_flux + (j - off)] = m;
-        const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
-        acc += r * r;
+        const bool bad = S.bad != 0;
+        const int moff = FS.obs.off - off0;
+        double acc = 0.0;
+        if (!bad) acc = point_chi2<LOG2N1, POLY, true>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, moff);
+        else if (P.model_out)
+          for (int j = tid; j < FS.obs.n; j += kNT) P.model_out[(long long)p * P.ld_flux + moff + j] = nan;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+        if ((tid & 31) == 0) red[tid >> 5] = acc;
+        __syncthreads();
+        if (tid == 0) {
+          double c2 = 0.0;
+#pragma unroll
+          for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
+          if (bad) c2 = nan;
+          if (P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2 + m] = c2;
+          tot = m == 0 ? c2 : tot + c2;
+        }
       }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if ((tid & 31) == 0) red[tid >> 5] = acc;
-    __syncthreads();
-    if (tid == 0 && P.lnl) {
-      double c2 = 0.0;
-#pragma unroll
-      for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
-      if (P.chi2_sed) c2 += P.chi2_sed[p];
-      store_lnl(P, p, -0.5 * c2);
+      if (tid == 0 && P.lnl) {
+        if (P.chi2_sed) tot += P.chi2_sed[p];
+        store_lnl(P, p, -0.5 * tot);
+      }
     }
     // The row is scratch and fully consumed: L2 is told to drop its lines instead of writing them back
     // (discard.global.L2).  Without this every row crosses HBM three times (the emulator's write is evicted --
@@ -473,6 +557,18 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
     __syncthreads();
   }
   if (tid == 0) gather_exit(P, gridDim.x);
+}
+
+// stage-2 and final regrid ratios of a point with an instrumental stage
+__device__ __forceinline__ void stage2_setup(const FastGrid& F, const PointSetup& S, FastSetup& FS) {
+  const int nM = S.i1 - S.i0 + 1, N2 = 1 << S.log2N2;
+  FS.s_num = nM - 1; FS.s_den = N2 - 1;
+  const long long inc = 2LL * kNT * (nM - 1);
+  FS.s_incj = (int)(inc / (N2 - 1));
+  FS.s_incr = (int)(inc - (long long)FS.s_incj * (N2 - 1));
+  FS.s_invden = 1.0f / (float)(N2 - 1);
+  FS.scale = (double)(N2 - 1) / (double)(nM - 1);
+  FS.q0 = (double)S.i0 + S.lnD * F.inv_dlnw;
 }
 
 // One thread per point: mask limits, transform sizes, Doppler factor, taper constant, and the
@@ -488,14 +584,7 @@ tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ 
   FastSetup FS{};
   tail_setup(P, P.theta + (long long)p * P.ld, p, S, FS.obs);
   if (!S.bad && S.use_inst) {
-    const int nM = S.i1 - S.i0 + 1, N2 = 1 << S.log2N2;
-    FS.s_num = nM - 1; FS.s_den = N2 - 1;
-    const long long inc = 2LL * kNT * (nM - 1);
-    FS.s_incj = (int)(inc / (N2 - 1));
-    FS.s_incr = (int)(inc - (long long)FS.s_incj * (N2 - 1));
-    FS.s_invden = 1.0f / (float)(N2 - 1);
-    FS.scale = (double)(N2 - 1) / (double)(nM - 1);
-    FS.q0 = (double)S.i0 + S.lnD * F.inv_dlnw;
+    stage2_setup(F, S, FS);
     if (F.cluster && P.stars[star_of(P.star, P.n_stars, p)].sorted) {
       // tail_cluster.cuh: CTA r of the cluster serves the observed pixels whose position falls into quarter r
       for (int r = 0; r < 3; ++r) {
@@ -511,6 +600,33 @@ tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ 
       FS.jcut[0] = -1;
     }
   }
+  out->S = S;
+  out->FS = FS;
+}
+
+// Targets: one thread per (point, member) item, item i = p * kmax + m (the items of members a target does not have
+// are not written).  A point whose target lies outside [0, n_targets) gets a bad record at item p * kmax.
+template <int kUnused = 0>
+__global__ void __launch_bounds__(64)
+tail_setup_targets_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long long)P.B * P.kmax) return;
+  if (i == 0 && F.work_counter) *F.work_counter = F.work_start;
+  const int p = (int)(i / P.kmax), m = (int)(i - (long long)p * P.kmax);
+  const int t = P.target[p];
+  int k = -1;
+  if (t >= 0 && t < P.n_targets) {
+    const int f = P.tfirst[t];
+    if (m >= P.tfirst[t + 1] - f) return;
+    k = f + m;
+  } else if (m > 0) {
+    return;
+  }
+  PointSetup S{};
+  FastSetup FS{};
+  tail_setup_star(P, P.theta + (long long)p * P.ld, k, S, FS.obs);
+  if (!S.bad && S.use_inst) stage2_setup(F, S, FS);
+  FastPoint* out = reinterpret_cast<FastPoint*>(F.points) + i;
   out->S = S;
   out->FS = FS;
 }

@@ -12,6 +12,11 @@ every row of a batch names its star.  Each star may bring its own fixed paramete
 of the photometric bands, its own LSF vector and its own parameter layout (free parameters and their
 order, continuum order, photometry).  A single-star engine is the case of one star.
 
+Consecutive stars of a set may form a *target* (``targets=[...]``): one physical star observed in several spectra
+(echelle orders, spectrograph arms, epochs) that share its labels.  A row of a target batch is evaluated with one
+emulator row and one rotation stage, then once per spectrum (member): Doppler shift, instrumental stage, resampling,
+continuum and chi2.
+
 A fixed ``Inst_R`` that is a 1-D array is an LSF vector, the dispersion (AA) at every observed pixel,
 as in the reference (genmod.py:82-85 passes a non-float inst_R on to getspec's LSF branch,
 predictspec.py:265-286).
@@ -115,7 +120,7 @@ def _specnet_struct(spec, keep):
 class Engine:
     def __init__(self, spec=None, phot=None, obs_wave=None, obs_flux=None, obs_eflux=None,
                  obs_phot=None, fitpars_i=(), fixedpars=None, runbools=(True, False, False, False, False),
-                 precision='parity', device=None, stars=None):
+                 precision='parity', device=None, stars=None, targets=None):
         """``stars``: instead of ``obs_wave``, ``obs_flux``, ``obs_eflux`` and ``obs_phot``, a list of
         ``{'wave', 'flux', 'eflux', 'phot': {band: (mag, err)}}``, one per star; ``lnlike_batch`` and
         ``model_batch`` then take the star index of every row.  A star may also carry
@@ -127,7 +132,10 @@ class Engine:
         net's order.  In a photometry engine a star without ``'phot'`` is a star without photometry.  A fixed
         ``Inst_R`` that is a 1-D array is the star's LSF vector (one dispersion per observed pixel); every star
         has one or none does.  ``ndim`` is the largest star's: a row of ``theta`` holds its star's
-        ``star_fitpars_i[k]`` in its first ``star_ndim[k]`` columns, and the columns after those are ignored."""
+        ``star_fitpars_i[k]`` in its first ``star_ndim[k]`` columns, and the columns after those are ignored.
+
+        ``targets``: member counts [n_0, n_1, ...] summing to the number of stars; target t is the next n_t stars
+        (see ``set_targets``)."""
         if stars is None:
             stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot}]
         elif any(v is not None for v in (obs_wave, obs_flux, obs_eflux, obs_phot)):
@@ -247,6 +255,9 @@ class Engine:
                                                          C.byref(ctx)))
         self._ctx = ctx
         del keep
+        self.n_targets = 0
+        if targets is not None:
+            self.set_targets(targets)
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -286,6 +297,80 @@ class Engine:
         if v.ndim != 1 or len(v) != self.n_obs:
             raise ValueError('the LSF vector needs one dispersion per observed pixel (%d)' % self.n_obs)
         _lib.check(self.lib.payne_ctx_set_lsf(self._ctx, v.ctypes.data, len(v)))
+
+    def set_targets(self, counts):
+        """Group the stars into targets: target t is the next ``counts[t]`` stars, its members, which share the
+        emulator labels and ``Vrot`` (same columns or fixed values) and may differ in ``Vrad``, ``Inst_R``, pixels and
+        continuum order; only the first member may have photometry.  None removes the targets."""
+        if counts is None:
+            _lib.check(self.lib.payne_ctx_set_targets(self._ctx, None, 0))
+            self.n_targets = 0
+            return
+        counts = [int(n) for n in counts]
+        if not counts or min(counts) < 1 or sum(counts) != self.n_stars:
+            raise ValueError('targets: member counts >= 1 that sum to the number of stars (%d)' % self.n_stars)
+        first = np.ascontiguousarray(np.concatenate([[0], np.cumsum(counts)]), dtype=np.int32)
+        _lib.check(self.lib.payne_ctx_set_targets(self._ctx, first.ctypes.data, len(counts)))
+        self.n_targets = len(counts)
+        self.target_first = first
+        self.target_members = [list(range(first[t], first[t + 1])) for t in range(len(counts))]
+        # a target's model row: its members' pixels back to back
+        self.target_n_obs = [sum(self.n_obs_star[k] for k in m) for m in self.target_members]
+        self.target_kmax = max(counts)
+
+    def lnlike_batch_targets(self, theta, target):
+        """lnL of every row against its target: ``target`` [B], as ``star`` in ``lnlike_batch`` (int32 CUDA tensor
+        with a CUDA theta: stream-ordered, an index outside [0, n_targets) gives NaN and status bit 2; else numpy
+        through the host entry, which refuses such an index)."""
+        if not self.n_targets:
+            raise ValueError('no targets: set_targets first')
+        if isinstance(theta, torch.Tensor) and theta.is_cuda:
+            th = self._theta_dev(theta)
+            tv = self._star_dev(target, th.shape[0], th.device)
+            out = torch.empty(th.shape[0], dtype=torch.float64, device=th.device)
+            st = torch.cuda.current_stream(th.device).cuda_stream
+            _lib.check(self.lib.payne_lnlike_batch_targets(self._ctx, th.data_ptr(), tv.data_ptr(), th.shape[0],
+                                                           th.shape[1], out.data_ptr(), st))
+            return out
+        th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
+        if th.ndim != 2 or th.shape[1] != self.ndim:
+            raise ValueError('theta must be [B, %d]' % self.ndim)
+        if isinstance(target, torch.Tensor):
+            target = target.cpu().numpy()
+        tv = np.ascontiguousarray(np.asarray(target).astype(np.int32, casting='same_kind'))
+        if tv.shape != (th.shape[0],):
+            raise ValueError('target must be [%d]' % th.shape[0])
+        out = np.empty(th.shape[0], dtype=np.float64)
+        _lib.check(self.lib.payne_lnlike_batch_targets_host(self._ctx, th.ctypes.data, tv.ctypes.data, th.shape[0],
+                                                            th.shape[1], out.ctypes.data))
+        return out
+
+    def model_batch_targets(self, theta, target, want_flux=True, want_chi2=True, want_mags=True):
+        """Model spectra [B, max target_n_obs] (row p: its members' spectra back to back in member order, the rest
+        NaN), chi2 [B, target_kmax] (chi2[p, m] of member m, the rest NaN), the first member's magnitudes [B, nb] and
+        lnL [B], as CUDA float64 tensors."""
+        if not self.n_targets:
+            raise ValueError('no targets: set_targets first')
+        dev = torch.device('cuda', self.device)
+        if not isinstance(theta, torch.Tensor):
+            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
+        th = self._theta_dev(theta.to(dev))
+        B = th.shape[0]
+        if not isinstance(target, torch.Tensor):
+            target = torch.from_numpy(np.ascontiguousarray(np.asarray(target).astype(np.int32, casting='same_kind')))
+        tv = self._star_dev(target.to(dev), B, dev)
+        nf = max(self.target_n_obs)
+        flux = torch.full((B, nf), float('nan'), dtype=torch.float64, device=dev) if want_flux else None
+        chi2 = torch.full((B, self.target_kmax), float('nan'), dtype=torch.float64, device=dev) if want_chi2 else None
+        mags = torch.full((B, self.nb), float('nan'), dtype=torch.float64, device=dev) if (want_mags and self.nb) else None
+        lnl = torch.empty(B, dtype=torch.float64, device=dev)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(self.lib.payne_model_batch_targets(
+            self._ctx, th.data_ptr(), tv.data_ptr(), B, th.shape[1],
+            flux.data_ptr() if flux is not None else None, nf,
+            chi2.data_ptr() if chi2 is not None else None, self.target_kmax,
+            mags.data_ptr() if mags is not None else None, lnl.data_ptr(), st))
+        return flux, chi2, mags, lnl
 
     def last_ms(self, which):
         return float(self.lib.payne_ctx_last_ms(self._ctx, {'mlp': 0, 'tail': 1, 'phot': 2}[which]))

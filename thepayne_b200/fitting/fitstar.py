@@ -16,7 +16,11 @@ What differs, on purpose:
     demo/runPayne.py:112), ``samplerbounds`` is a single ellipsoid, ``samplertype`` 'Static';
   * the parameters written for a dead point are that point's own (the reference writes
     ``likeobj.parsdict``, i.e. whatever vector the likelihood saw last, fitstar.py:347);
-  * ``inputdict['precision']`` / ``['device']`` select the CUDA precision mode and device.
+  * ``inputdict['precision']`` / ``['device']`` select the CUDA precision mode and device;
+  * ``inputdict['spec']`` may be a list of spectrum dictionaries (echelle orders, spectrograph arms), each with the
+    keys of the single one.  The labels, ``Vrad`` and ``Vrot`` are shared; spectrum s has its own ``Inst_R_<s>`` and
+    continuum coefficients ``pc_<s>_<k>``, whose priors come from ``priordict['Inst_R_<s>']`` and
+    ``priordict['blaze_coeff_<s>']`` (``multispec.MultiSpecLikelihood``).
 """
 from __future__ import annotations
 
@@ -61,7 +65,9 @@ class FitPayne(object):
         self.fitpars = list(_ALLPARS)
         self.fitpars_bool = {pp: False for pp in self.fitpars}
 
-        if 'spec' in inputdict:                                            # fitstar.py:70-154
+        if isinstance(inputdict.get('spec'), (list, tuple)):
+            self._setup_spectra(inputdict)
+        elif 'spec' in inputdict:                                          # fitstar.py:70-154
             sp = inputdict['spec']
             self.spec_bool = True
             fa['obs_wave'], fa['obs_flux'], fa['obs_eflux'] = sp['obs_wave'], sp['obs_flux'], sp['obs_eflux']
@@ -120,6 +126,52 @@ class FitPayne(object):
                 'priordict': self.priordict,
                 'runbools': [self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool]}
 
+    def _setup_spectra(self, inputdict):
+        """A list-valued ``spec``: every spectrum's observation as the single one's (wave_minmax, convertair), the
+        shared spectral parameters once, ``Inst_R_<s>`` and ``pc_<s>_<k>`` per spectrum."""
+        specs = list(inputdict['spec'])
+        if not specs:
+            raise ValueError("inputdict['spec'] is an empty list")
+        if any('Vrad' in sp for sp in specs) or any(k.startswith('Vrad_') for k in self.priordict):
+            raise NotImplementedError('a Vrad per spectrum: FitPayne fits one Vrad shared by every spectrum')
+        fa = self.fitargs
+        self.spec_bool = True
+        fa['specANNpath'] = inputdict.get('specANNpath', None)
+        fa['NNtype'] = inputdict.get('NNtype', 'LinNet')
+        fa['spectra'] = []
+        for sp in specs:
+            w = np.asarray(sp['obs_wave'], dtype=np.float64)
+            sel = slice(None)
+            if 'wave_minmax' in sp:
+                sel = (w >= sp['wave_minmax'][0]) & (w <= sp['wave_minmax'][1])
+            one = {'obs_%s_fit' % k: np.asarray(sp['obs_' + k], dtype=np.float64)[sel] for k in ['wave', 'flux', 'eflux']}
+            if sp.get('convertair', True):
+                one['obs_wave_fit'] = airtovacuum(one['obs_wave_fit'])
+            fa['spectra'].append(one)
+        on = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot'] + (['Vmic'] if fa['NNtype'] == 'YST2' else [])
+        for pp in on:
+            self.fitpars_bool[pp] = True
+        self.fitpars.remove('Inst_R')
+        self.fitpars_bool.pop('Inst_R')
+        for s in range(len(specs)):
+            self.fitpars.append('Inst_R_%d' % s)
+            self.fitpars_bool['Inst_R_%d' % s] = True
+        if len({bool(sp.get('modpoly', False)) for sp in specs}) > 1:
+            raise ValueError('every spectrum has a continuum polynomial (modpoly) or none does')
+        self.modpoly_bool = bool(specs[0].get('modpoly', False))
+        for s, sp in enumerate(specs):
+            if not self.modpoly_bool:
+                break
+            key = 'blaze_coeff_%d' % s
+            if key not in self.priordict:                                  # as fitstar.py:110-147 per spectrum
+                if 'polyorder' in sp:
+                    self.priordict[key] = [[0.0, sp.get('polysigma', 1.0)] for _ in range(sp['polyorder'] + 1)]
+                else:
+                    self.priordict[key] = [[0.0, 1.0] for _ in range(3)]
+            for k in range(len(self.priordict[key])):
+                self.fitpars.append('pc_%d_%d' % (s, k))
+                self.fitpars_bool['pc_%d_%d' % (s, k)] = True
+
     def __call__(self, indicts):
         return self.run_dynesty(indicts)
 
@@ -127,9 +179,11 @@ class FitPayne(object):
         """Name kept from the reference (fitstar.py:236-258); the sampler is the batched one."""
         fitargs, fitpars, runbools = indicts['fitargs'], indicts['fitpars'], indicts['runbools']
         self._prepare(indicts)
-        self.likeobj = self.likelihood(fitargs, fitpars, runbools, verbose=False,
-                                       precision=getattr(self, 'precision', 'parity'),
-                                       device=getattr(self, 'device', None))
+        like = self.likelihood
+        if 'spectra' in fitargs:
+            from .multispec import MultiSpecLikelihood as like
+        self.likeobj = like(fitargs, fitpars, runbools, verbose=False, precision=getattr(self, 'precision', 'parity'),
+                            device=getattr(self, 'device', None))
         self._check_sampler(indicts)
         return self._runsampler(indicts['sampler'])
 

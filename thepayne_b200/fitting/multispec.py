@@ -1,0 +1,100 @@
+"""``MultiSpecLikelihood``: one star observed in several spectra (echelle orders, spectrograph arms), the
+``likelihood`` interface (``lnlikefn``, ``lnlike_batch``, ``parsdict``, ``fitpars_i``, ``ndim``, ``fixedpars``).
+
+The spectra are the members of one target of an observation set (``Engine(stars=[...], targets=[S])``): the labels,
+``Vrad`` and ``Vrot`` are shared, spectrum s has its own resolving power ``Inst_R_<s>`` and continuum coefficients
+``pc_<s>_<k>``, and the photometry belongs to the first spectrum.  A sampler row holds every free parameter once; each
+spectrum's layout reads its own columns under the reference's names (``Inst_R_<s>`` as ``Inst_R``, ``pc_<s>_<k>`` as
+``pc_k``), so lnL = -0.5 (chi2_0 + ... + chi2_{S-1} + chi2_sed) with each chi2_s what a single-spectrum ``likelihood``
+of spectrum s gives.  ``fitargs['spectra']`` is the list of ``{'obs_wave_fit', 'obs_flux_fit', 'obs_eflux_fit'}``
+(``FitPayne`` builds it from a list-valued ``inputdict['spec']``).
+"""
+from __future__ import annotations
+
+import re
+
+import numpy as np
+import torch
+
+from ..engine import Engine
+from .genmod import GenMod
+from .likelihood import free_parameters
+
+_PHOT = ['log(R)', 'Dist', 'log(A)', 'Av', 'Rv']
+
+
+def spectrum_name(name, s):
+    """The reference name under which spectrum s reads sampler parameter ``name``; None: not spectrum s's."""
+    m = re.fullmatch(r'Inst_R_(\d+)', name)
+    if m:
+        return 'Inst_R' if int(m.group(1)) == s else None
+    m = re.fullmatch(r'pc_(\d+)_(\d+)', name)
+    if m:
+        return 'pc_%s' % m.group(2) if int(m.group(1)) == s else None
+    return name
+
+
+class MultiSpecLikelihood(object):
+    def __init__(self, fitargs, fitpars, runbools, **kwargs):
+        self.fitargs = fitargs
+        self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool = runbools[:5]
+        if not self.spec_bool:
+            raise ValueError('MultiSpecLikelihood needs spectra')
+        if self.carbon_bool:
+            raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
+        self.fixedpars = fitargs['fixedpars']
+        self.precision = kwargs.get('precision', 'parity')
+        self.GM = GenMod(precision=self.precision)
+        self.GM._initspecnn(nnpath=fitargs['specANNpath'], NNtype=fitargs.get('NNtype', 'LinNet'))
+        if self.phot_bool:
+            self.GM._initphotnn(fitargs['obs_phot'].keys(), nnpath=fitargs['photANNpath'])
+        self.fitpars_i = free_parameters(fitpars)
+        self.ndim = len(self.fitpars_i)
+        self.parsdict = {}
+        spectra = fitargs['spectra']
+        stars = []
+        for s, sp in enumerate(spectra):
+            fit = [spectrum_name(p, s) for p in self.fitpars_i]
+            if s > 0:                                        # the photometry is the first spectrum's
+                fit = [None if p in _PHOT else p for p in fit]
+            fit = [p if p is not None else 'pad' for p in fit]
+            fixed = {}
+            for kk, v in self.fixedpars.items():
+                name = spectrum_name(kk, s)
+                if name is not None and not (s > 0 and name in _PHOT):
+                    fixed[name] = v
+            poly = any(p.startswith('pc_') for p in fit)
+            st = {'wave': sp['obs_wave_fit'], 'flux': sp['obs_flux_fit'], 'eflux': sp['obs_eflux_fit'],
+                  'fitpars_i': fit, 'fixedpars': fixed,
+                  'runbools': [True, bool(self.phot_bool) and s == 0, poly, bool(self.photscale_bool)]}
+            if self.phot_bool and s == 0:
+                st['phot'] = fitargs['obs_phot']
+            stars.append(st)
+        if len({s['runbools'][2] for s in stars}) > 1:
+            raise ValueError('every spectrum has a continuum polynomial (modpoly) or none does')
+        self.engine = Engine(spec=self.GM.PP.anns.model, phot=self.GM.fppsed.net if self.phot_bool else None,
+                             stars=stars, targets=[len(stars)],
+                             runbools=[True, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
+                             precision=self.precision, device=kwargs.get('device'))
+
+    def _set_parsdict(self, pars):
+        self.parsdict = {pp: vv for pp, vv in zip(self.fitpars_i, pars)}
+        for kk in self.fixedpars.keys():
+            self.parsdict[kk] = self.fixedpars[kk]
+
+    def lnlikefn(self, pars):
+        """One parameter vector -> float."""
+        self._set_parsdict(pars)
+        th = np.asarray(pars, dtype=np.float64).reshape(1, self.ndim)
+        return float(self.engine.lnlike_batch_targets(th, np.zeros(1, np.int32))[0])
+
+    def lnlike_batch(self, theta):
+        """theta [B, ndim] (CUDA float64 tensor, or numpy) -> lnL [B] of the same kind."""
+        if isinstance(theta, torch.Tensor) and theta.is_cuda:
+            target = torch.zeros(theta.shape[0], dtype=torch.int32, device=theta.device)
+        else:
+            target = np.zeros(len(theta), np.int32)
+        out = self.engine.lnlike_batch_targets(theta, target)
+        last = theta[-1]
+        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
+        return out

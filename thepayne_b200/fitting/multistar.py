@@ -283,6 +283,8 @@ class FitPayneMany(object):
         verbose = kwargs.get('verbose', True)
         fits, indicts = [], []
         for d in inputdicts:
+            if isinstance(d.get('spec'), (list, tuple)):
+                raise NotImplementedError('FitPayneMany with several spectra per star (a list-valued spec)')
             f = FitPayne()
             ind = f._setup(inputdict=d, verbose=verbose)
             f._prepare(ind)

@@ -10,14 +10,20 @@ pv_tgaussian / pv_exp / pv_texp, reference defaults otherwise, ``pc_0`` in [0.75
 proposal queue (scipy's ppf functions are vectorised), so the sampler side keeps up with
 ``likelihood.lnlike_batch``.  The brutus-derived IMF / Galactic / Vrot / Vtot priors
 (``advancedpriors.py``, astropy-based) are outside the accelerated path and raise.
+
+Several spectra (``FitPayne`` with a list-valued ``spec``): ``Inst_R_<s>`` takes the priors and default range of
+``Inst_R``, and ``pc_<s>_<k>`` those of ``pc_k`` with ``blaze_coeff_<s>`` in place of ``blaze_coeff``.
 """
 from __future__ import annotations
+
+import re
 
 import numpy as np
 from scipy.stats import expon, norm, truncexpon, truncnorm
 
 _SPEC = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot', 'Inst_R', 'CarbonScale']
 _ISO = ['log(A)', 'log(R)', 'Av', 'Rv', 'Dist']
+_SPECTRUM = re.compile(r'(Inst_R|pc)_(\d+)(?:_(\d+))?$')     # Inst_R_<s>, pc_<s>_<k>
 _PV = {'pv_uniform': 'uniform', 'pv_gaussian': 'gaussian', 'pv_tgaussian': 'tgaussian', 'pv_exp': 'exp',
        'pv_texp': 'texp'}
 
@@ -31,9 +37,12 @@ class prior(object):
         self.priordict = {k: {} for k in ['uniform', 'gaussian', 'tgaussian', 'exp', 'texp']}
         self.additionalpriors = {}
         self.polycoefarr = None
+        self.spectrum_polycoef = {}                            # s -> blaze_coeff_<s>
         for kk in inpriordict.keys():
             if kk == 'blaze_coeff':
                 self.polycoefarr = inpriordict['blaze_coeff']
+            elif kk.startswith('blaze_coeff_'):
+                self.spectrum_polycoef[int(kk[len('blaze_coeff_'):])] = inpriordict[kk]
             elif kk in ('IMF', 'GAL', 'VROT', 'VTOT', 'AngDia'):
                 raise NotImplementedError('%s prior (advancedpriors.py) is outside the accelerated path' % kk)
             else:
@@ -74,10 +83,21 @@ class prior(object):
             lo, hi, sc = pd['texp'][name]
             x = truncexpon.ppf(u, (hi - lo) / sc, loc=lo, scale=sc)
             return np.where(x == np.inf, hi, x) if np.ndim(x) else (hi if x == np.inf else x)
-        lo, hi = self.defaultpars[name]
+        lo, hi = self.defaultpars['Inst_R' if _SPECTRUM.match(name) else name]
         return (hi - lo) * u + lo
 
     def _column(self, name, u):
+        m = _SPECTRUM.match(name)
+        if m and self.spec_bool:                               # Inst_R_<s>, pc_<s>_<k>
+            if m.group(1) == 'Inst_R' and m.group(3) is None:
+                return self._transform(name, u, iso=False)
+            if m.group(1) == 'pc' and m.group(3) is not None:
+                k = int(m.group(3))
+                if k == 0:
+                    return (1.25 - 0.75) * u + 0.75
+                c = self.spectrum_polycoef[int(m.group(2))][k]
+                pcmax, pcmin = c[0] + 5.0 * c[1], c[0] - 5.0 * c[1]
+                return (pcmax - pcmin) * u + pcmin
         if 'pc' in name:
             if not self.spec_bool:
                 raise KeyError(name)
@@ -109,7 +129,7 @@ class prior(object):
             return out
         groups = []
         if self.spec_bool:
-            groups.append(_SPEC)
+            groups.append(_SPEC + [p for p in self.fitpars_i if p.startswith('Inst_R_')])
         if self.phot_bool:
             g = [] if self.spec_bool else ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]']
             g += [p for p in ['log(R)', 'Dist', 'log(A)', 'Av'] if p in self.fitpars_i]
