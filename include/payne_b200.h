@@ -238,14 +238,19 @@ int payne_model_batch_stars(PayneCtx* ctx, const double* theta_dev, const int32_
  *     polynomial, chi2_m -- each chi2_m has the bits of -2 lnL of a single-star context of star m without photometry;
  *   the SED chi2 once, from the first member's magnitudes;
  *   lnL = -0.5 * ((((chi2_0 + chi2_1) + ...) + chi2_{K-1}) + chi2_sed).
- * Members may differ in Vrad, Inst_R (column or fixed value), pixels and continuum order.  At set time
- * PAYNE_E_INVALID: members that resolve Teff, log(g), [Fe/H], [a/Fe], Vmic or Vrot to different columns or fixed
- * values; magnitudes on a member other than the first.  PAYNE_E_UNSUPPORTED: a context without the fast tail (emulator
- * grid not uniform in ln wavelength), with LSF vectors or with the fused gather.  The entries without _targets keep
- * naming stars.  A target outside [0, n_targets): PAYNE_E_INVALID from the _host entry before anything is launched; on
- * the device lnL NaN, no model row or chi2, status bit 2.  A member that is bad by itself (e.g. Inst_R above the
- * emulator's resolution) makes lnL NaN; the other members' model rows and chi2 keep their values.  ld >= the largest
- * ndim.  Per-(point, member) records bound a slab to min(max_batch, 65536 / the largest member count) points. */
+ * Members may differ in Vrad, Inst_R (column or fixed value) or LSF vector, pixels and continuum order.  With LSF vectors
+ * (PayneStarOpts.lsf) the instrumental stage of every member is its own vector's; the emulator grid need not be uniform
+ * in ln wavelength then.  At set time PAYNE_E_INVALID: members that resolve Teff, log(g), [Fe/H], [a/Fe], Vmic or Vrot
+ * to different columns or fixed values; magnitudes on a member other than the first; with LSF vectors, a member whose
+ * Inst_R is a theta column (nothing reads it beside the vector).  PAYNE_E_UNSUPPORTED: without LSF vectors, a context
+ * without the fast tail (emulator grid not uniform in ln wavelength); a context with the fused gather.  A one-star
+ * context may switch its LSF vector on or off afterwards (payne_ctx_set_lsf); the _targets entries then check these
+ * rules again.  The entries without _targets keep naming stars.  A target outside [0, n_targets): PAYNE_E_INVALID from
+ * the _host entry before anything is launched; on the device lnL NaN, no model row or chi2, status bit 2.  A member that
+ * is bad by itself (e.g. Inst_R above the emulator's resolution, a mask of fewer than 17 emulator pixels, or an LSF
+ * transform above 32768 samples: status bit 0) makes lnL NaN; the other members' model rows and chi2 keep their values.
+ * ld >= the largest ndim.  Without LSF vectors, per-(point, member) records bound a slab to
+ * min(max_batch, 65536 / the largest member count) points. */
 int payne_ctx_set_targets(PayneCtx* ctx, const int32_t* first, int32_t n_targets);
 int payne_lnlike_batch_targets(PayneCtx* ctx, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
                                double* lnl_dev, void* stream);
@@ -269,7 +274,8 @@ int payne_ctx_attach_continuum(PayneCtx* ctx, const PayneSpecNet* cont);
  * instrumental stage is smooth_lsf_fft (smoothing.py:482-586) instead of the scalar-R Gaussian and the
  * Inst_R parameter is ignored; observed pixels outside the emulator's coverage take the edge value (the
  * reference's np.interp clamps there) instead of NaN.  NULL switches back.  Emulator grids up to 32768
- * pixels; a point whose cdf grid would need more than 32768 samples returns NaN and sets status bit 0. */
+ * pixels; a point whose cdf grid would need more than 32768 samples returns NaN and sets status bit 0.
+ * Targets (payne_ctx_set_targets) run with LSF vectors too, see there. */
 int payne_ctx_set_lsf(PayneCtx* ctx, const double* lsf_host, int64_t n);
 
 /* Emulator forward pass only.  x_dev: [B, D_in] fp64 labels; y_dev: [B, ldy] fp32, ldy>=D_out.

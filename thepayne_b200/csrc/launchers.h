@@ -72,6 +72,10 @@ bool probe_tail_general(int l2, size_t smem_bytes, int* ctas_per_sm);
 int launch_tail_general(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const TwConst& tc);
 bool probe_tail_lsf(size_t smem_bytes, int* ctas_per_sm);
 int launch_tail_lsf(int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const LsfParams& L);
+// targets on a context with LSF vectors (payne_ctx_set_targets): the TGT instantiation of tail_lsf_kernel, same grid and
+// dynamic shared memory as the star form (lsf_alloc)
+bool probe_tail_lsf_targets(size_t smem_bytes, int* ctas_per_sm);
+int launch_tail_lsf_targets(int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const LsfParams& L);
 int launch_continuum(int grid, cudaStream_t st, const ContParams& C);
 // unit-test convolution: y = irfft(rfft(x) * H) of 2^log2N real samples (device buffers; H[0..N/2] without the
 // 1/M; tw = the N/2-entry twiddle table of the tails), one CTA on the default stream

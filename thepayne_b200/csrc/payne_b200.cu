@@ -177,10 +177,12 @@ struct PayneCtx {
   std::vector<double> star_fixed_h;     // host copies of star_fixed_dev / star_lay_dev (empty without them)
   std::vector<payne::StarLayout> star_lay_h;
   // targets (payne_ctx_set_targets): runs of consecutive stars that describe one physical star
-  int n_targets = 0, tgt_kmax = 0, tgt_grid = 0;
+  int n_targets = 0, tgt_kmax = 0, tgt_grid = 0;   // tgt_grid: CTAs of the fast target kernel, 0 until it is probed
+  bool tgt_lsf_probed = false;          // the LSF target kernel's shared-memory opt-in is set
+  std::string tgt_instr_col;            // the first member with an Inst_R column (refused beside LSF vectors), or empty
   long long tgt_nobs_max = 0;           // the largest sum of the members' n_obs (model row of a target)
   int* tfirst_dev = nullptr;            // [n_targets + 1]
-  payne::FastPoint* tgt_points = nullptr;   // [tgt_rows * tgt_kmax] per-(point, member) records
+  payne::FastPoint* tgt_points = nullptr;   // [tgt_rows * tgt_kmax] per-(point, member) records (fast tail only)
   int* tgt_star = nullptr;              // [tgt_rows] first member's star of every point of a slab
   long long tgt_rows = 0, tgt_rec_alloc = 0;
   // photometry
@@ -912,19 +914,22 @@ __global__ void target_star_kernel(const int* target, const int* tfirst, int n_t
   star[p] = (t >= 0 && t < n_targets) ? tfirst[t] : -1;
 }
 
-// Per-(point, member) records of the target tail: at most this many, so the slab of a call with targets is
-// min(max_batch, kTargetRecords / the largest member count) points (20 MB of records).
+// Per-(point, member) records of the fast target tail: at most this many, so the slab of a fast-tail call with targets
+// is min(max_batch, kTargetRecords / the largest member count) points (20 MB of records).  The LSF target tail sets its
+// members up inside the kernel and has no records.
 constexpr long long kTargetRecords = 65536;
 
-int ensure_target_workspace(PayneCtx* c, long long rows) {
-  if (rows <= c->tgt_rows && rows * c->tgt_kmax <= c->tgt_rec_alloc) return PAYNE_OK;
+int ensure_target_workspace(PayneCtx* c, long long rows, bool records) {
+  const long long rec = records ? rows * c->tgt_kmax : 0;
+  if (rows <= c->tgt_rows && rec <= c->tgt_rec_alloc) return PAYNE_OK;
   CU_TRY(cudaDeviceSynchronize());                       // earlier calls may still read the records
   if (c->tgt_points) cudaFree(c->tgt_points);
   if (c->tgt_star) cudaFree(c->tgt_star);
   c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
-  const long long rec = rows * c->tgt_kmax;
-  CU_TRY(cudaMalloc((void**)&c->tgt_points, (size_t)rec * sizeof(payne::FastPoint)));
-  CU_TRY(cudaMemset(c->tgt_points, 0, (size_t)rec * sizeof(payne::FastPoint)));
+  if (rec) {
+    CU_TRY(cudaMalloc((void**)&c->tgt_points, (size_t)rec * sizeof(payne::FastPoint)));
+    CU_TRY(cudaMemset(c->tgt_points, 0, (size_t)rec * sizeof(payne::FastPoint)));
+  }
   CU_TRY(cudaMalloc((void**)&c->tgt_star, (size_t)rows * sizeof(int)));
   CU_TRY(cudaDeviceSynchronize());
   c->tgt_rows = rows; c->tgt_rec_alloc = rec;
@@ -940,10 +945,11 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
   if (B <= 0) return PAYNE_OK;
   if (ld < c->ndim_max) return fail(PAYNE_E_INVALID, "ld < ndim (the largest star's with per-star layouts)");
   if (!target && flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
-  const long long slab = target ? std::min(c->slab, std::max(1LL, kTargetRecords / c->tgt_kmax)) : c->slab;
+  const bool records = target && !c->lsf_on;             // the fast target tail's per-(point, member) records
+  const long long slab = records ? std::min(c->slab, std::max(1LL, kTargetRecords / c->tgt_kmax)) : c->slab;
   int rc = ensure_workspace(c, B);
   if (rc) return rc;
-  if (target) { rc = ensure_target_workspace(c, std::min(B, slab)); if (rc) return rc; }
+  if (target) { rc = ensure_target_workspace(c, std::min(B, slab), records); if (rc) return rc; }
   rc = order_after_previous(c, st);
   if (rc) return rc;
   if (c->timing) { c->ms_acc[0] = c->ms_acc[1] = c->ms_acc[2] = 0; c->ms_valid = false; c->pending.clear(); }
@@ -1055,7 +1061,10 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         TL.fixed[PAYNE_P_INSTR] = std::numeric_limits<double>::quiet_NaN();
         // ... a star's own fixed Inst_R and a per-star layout's Inst_R column too: Rs = NaN, no scalar-R stage
         TL.inst_scale = std::numeric_limits<double>::quiet_NaN();
-        if (payne::launch_tail_lsf(std::min(c->lsf_grid, nb), c->lsf_smem, st, TL, c->lsf)) return fail(PAYNE_E_CUDA, "tail launch");
+        const int grid = std::min(c->lsf_grid, nb);
+        if (target ? payne::launch_tail_lsf_targets(grid, c->lsf_smem, st, TL, c->lsf)
+                   : payne::launch_tail_lsf(grid, c->lsf_smem, st, TL, c->lsf))
+          return fail(PAYNE_E_CUDA, "tail launch");
       } else if (target) {
         // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no target form)
         if (!(fast_tail && is_depth)) return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail on line-depth rows");
@@ -1164,12 +1173,34 @@ int upload_star_layouts(PayneCtx* c, const PayneLayout* ctx, const PayneStarOpts
   return PAYNE_OK;
 }
 
-// The target entries: targets set, and the context still runs the tail they need.
-int need_targets(const PayneCtx* c) {
-  if (c->n_targets == 0) return fail(PAYNE_E_INVALID, "no targets: payne_ctx_set_targets first");
-  if (!(c->use_fast && c->allow_fast) || c->lsf_on || c->g_world > 0)
-    return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail without LSF vectors or the fused gather");
+// The target kernel of the tail the context runs now, probed once: the LSF target tail (its shared-memory opt-in, and
+// as many resident CTAs as the star form's grid), or the fast one (its grid).
+int probe_targets(PayneCtx* c) {
+  int occ = 0;
+  if (c->lsf_on) {
+    if (c->tgt_lsf_probed) return PAYNE_OK;
+    if (!payne::probe_tail_lsf_targets(c->lsf_smem, &occ) || occ * c->sm_count < c->lsf_grid)
+      return fail(PAYNE_E_UNSUPPORTED, "LSF target tail kernel does not fit on an SM");
+    c->tgt_lsf_probed = true;
+    return PAYNE_OK;
+  }
+  if (c->tgt_grid > 0) return PAYNE_OK;
+  if (!payne::probe_tail_fast_targets(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
+    return fail(PAYNE_E_UNSUPPORTED, "target tail kernel does not fit on an SM");
+  // the split kernel's scratch lines exist for tail_grid_fast CTAs
+  c->tgt_grid = std::min(occ * c->sm_count, c->tail_grid_fast);
   return PAYNE_OK;
+}
+
+// The target entries: targets set, and the context still runs a tail they can use (a one-star context may have
+// switched its LSF vector on or off since payne_ctx_set_targets).
+int need_targets(PayneCtx* c) {
+  if (c->n_targets == 0) return fail(PAYNE_E_INVALID, "no targets: payne_ctx_set_targets first");
+  if (c->g_world > 0) return fail(PAYNE_E_UNSUPPORTED, "targets on a context with the fused gather are not supported");
+  if (c->lsf_on && !c->tgt_instr_col.empty()) return fail(PAYNE_E_INVALID, c->tgt_instr_col);
+  if (!c->lsf_on && !(c->use_fast && c->allow_fast))
+    return fail(PAYNE_E_UNSUPPORTED, "targets without LSF vectors need the fast tail");
+  return probe_targets(c);
 }
 
 // The host-buffer entries: idx_host is every point's star, or its target (targets = true), or null (star 0).
@@ -1250,17 +1281,20 @@ int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) 
     if (c->tgt_star) cudaFree(c->tgt_star);
     c->tfirst_dev = nullptr; c->n_targets = 0; c->tgt_kmax = 0; c->tgt_nobs_max = 0;
     c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
+    c->tgt_instr_col.clear();
     return PAYNE_OK;
   }
   if (!c->has_spec) return fail(PAYNE_E_UNSUPPORTED, "targets need the spectrum emulator");
-  if (!c->use_fast) return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail (an emulator grid uniform in ln wavelength)");
-  if (c->lsf_on) return fail(PAYNE_E_UNSUPPORTED, "targets with LSF vectors are not supported");
+  // the LSF tail runs on every grid it accepts; the scalar-R target tail is the fast one
+  if (!c->lsf_on && !c->use_fast)
+    return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail (an emulator grid uniform in ln wavelength)");
   if (c->g_world > 0) return fail(PAYNE_E_UNSUPPORTED, "targets on a context with the fused gather are not supported");
   if (n_targets < 1) return fail(PAYNE_E_INVALID, "n_targets must be >= 1");
   if (first[0] != 0 || first[n_targets] != c->n_stars)
     return fail(PAYNE_E_INVALID, "first[0] must be 0 and first[n_targets] n_stars (" + std::to_string(c->n_stars) + ")");
   int kmax = 0;
   long long nobs_max = 0;
+  std::string instr_col;
   for (int t = 0; t < n_targets; ++t) {
     if (first[t + 1] <= first[t]) return fail(PAYNE_E_INVALID, "first[] must increase strictly (target " + std::to_string(t) + ")");
     kmax = std::max(kmax, first[t + 1] - first[t]);
@@ -1280,23 +1314,29 @@ int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) 
       if (c->has_phot && c->stars[k].nb > 0)
         return fail(PAYNE_E_INVALID, who + "photometry on a member other than the first");
     }
+    // Under an LSF vector no kernel reads Inst_R: a member's Inst_R column would be a sampled dimension without effect.
+    for (int k = first[t]; k < first[t + 1] && instr_col.empty(); ++k) {
+      const int col = resolve_param(c, k, PAYNE_P_INSTR).first;
+      if (col >= 0)
+        instr_col = "target " + std::to_string(t) + ", member " + std::to_string(k - first[t]) + ": Inst_R in theta column " +
+                    std::to_string(col) + " beside its LSF vector (the vector replaces Inst_R: give Inst_R no column)";
+    }
   }
-  int occ = 0;
-  if (!payne::probe_tail_fast_targets(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
-    return fail(PAYNE_E_UNSUPPORTED, "target tail kernel does not fit on an SM");
+  if (c->lsf_on && !instr_col.empty()) return fail(PAYNE_E_INVALID, instr_col);
+  c->tgt_grid = 0; c->tgt_lsf_probed = false;           // probed again for this context's current tail
+  int rc = probe_targets(c);
+  if (rc) return rc;
   CU_TRY(cudaDeviceSynchronize());
   if (c->tfirst_dev) cudaFree(c->tfirst_dev);
   c->tfirst_dev = nullptr; c->n_targets = 0;
-  int rc = upload(&c->tfirst_dev, first, (size_t)n_targets + 1);
+  rc = upload(&c->tfirst_dev, first, (size_t)n_targets + 1);
   if (rc) return rc;
   if (c->tgt_kmax != kmax) {                             // the record stride changes: reallocate at the next call
     if (c->tgt_points) cudaFree(c->tgt_points);
     if (c->tgt_star) cudaFree(c->tgt_star);
     c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
   }
-  c->n_targets = n_targets; c->tgt_kmax = kmax; c->tgt_nobs_max = nobs_max;
-  // the split kernel's scratch lines exist for tail_grid_fast CTAs
-  c->tgt_grid = std::min(occ * c->sm_count, c->tail_grid_fast);
+  c->n_targets = n_targets; c->tgt_kmax = kmax; c->tgt_nobs_max = nobs_max; c->tgt_instr_col = instr_col;
   return PAYNE_OK;
 }
 
@@ -1305,9 +1345,9 @@ int payne_lnlike_batch_targets(PayneCtx* c, const double* theta_dev, const int32
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   if (B == 0) return PAYNE_OK;
   if (!theta_dev || !target_dev || !lnl_dev) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
   int rc = need_targets(c);
   if (rc) return rc;
-  DeviceGuard dg(c->device);
   return run_batch(c, theta_dev, nullptr, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, target_dev);
 }
 
@@ -1317,11 +1357,11 @@ int payne_model_batch_targets(PayneCtx* c, const double* theta_dev, const int32_
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   if (B == 0) return PAYNE_OK;
   if (!theta_dev || !target_dev) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
   int rc = need_targets(c);
   if (rc) return rc;
   if (flux_dev && ld_flux < c->tgt_nobs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest target's pixels (all members)");
   if (chi2_dev && ld_chi2 < c->tgt_kmax) return fail(PAYNE_E_INVALID, "ld_chi2 < the largest member count");
-  DeviceGuard dg(c->device);
   return run_batch(c, theta_dev, nullptr, B, ld, flux_dev, ld_flux, mags_dev, lnl_dev, (cudaStream_t)stream, target_dev,
                    chi2_dev, ld_chi2);
 }
@@ -1484,6 +1524,7 @@ int payne_lnlike_batch_targets_host(PayneCtx* c, const double* theta_host, const
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   if (B <= 0) return PAYNE_OK;
   if (!theta_host || !target_host || !lnl_host) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);                             // (need_targets may probe a target kernel)
   int rc = need_targets(c);
   if (rc) return rc;
   return lnlike_host(c, theta_host, target_host, B, ld, lnl_host, true);

@@ -33,17 +33,26 @@ int launch_tail_general(int l2, int grid, size_t smem, cudaStream_t st, const Ta
   return cudaGetLastError() == cudaSuccess ? PAYNE_OK : PAYNE_E_CUDA;
 }
 
-bool probe_tail_lsf(size_t bytes, int* occ) {
-  if (cudaFuncSetAttribute(tail_lsf_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, tail_lsf_kernel<0>, kTailThreads, bytes) != cudaSuccess) {
+template <bool TGT>
+static bool probe_lsf(size_t bytes, int* occ) {
+  if (cudaFuncSetAttribute(tail_lsf_kernel<TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, tail_lsf_kernel<TGT>, kTailThreads, bytes) != cudaSuccess) {
     cudaGetLastError();
     return false;
   }
   return true;
 }
 
+bool probe_tail_lsf(size_t bytes, int* occ) { return probe_lsf<false>(bytes, occ); }
+bool probe_tail_lsf_targets(size_t bytes, int* occ) { return probe_lsf<true>(bytes, occ); }
+
 int launch_tail_lsf(int grid, size_t smem, cudaStream_t st, const TailParams& T, const LsfParams& L) {
-  tail_lsf_kernel<0><<<grid, kTailThreads, smem, st>>>(T, L);
+  tail_lsf_kernel<false><<<grid, kTailThreads, smem, st>>>(T, L);
+  return cudaGetLastError() == cudaSuccess ? PAYNE_OK : PAYNE_E_CUDA;
+}
+
+int launch_tail_lsf_targets(int grid, size_t smem, cudaStream_t st, const TailParams& T, const LsfParams& L) {
+  tail_lsf_kernel<true><<<grid, kTailThreads, smem, st>>>(T, L);
   return cudaGetLastError() == cudaSuccess ? PAYNE_OK : PAYNE_E_CUDA;
 }
 

@@ -14,8 +14,8 @@ order, continuum order, photometry).  A single-star engine is the case of one st
 
 Consecutive stars of a set may form a *target* (``targets=[...]``): one physical star observed in several spectra
 (echelle orders, spectrograph arms, epochs) that share its labels.  A row of a target batch is evaluated with one
-emulator row and one rotation stage, then once per spectrum (member): Doppler shift, instrumental stage, resampling,
-continuum and chi2.
+emulator row and one rotation stage, then once per spectrum (member): Doppler shift, instrumental stage (scalar R or
+the member's LSF vector), resampling, continuum and chi2.
 
 A fixed ``Inst_R`` that is a 1-D array is an LSF vector, the dispersion (AA) at every observed pixel,
 as in the reference (genmod.py:82-85 passes a non-float inst_R on to getspec's LSF branch,
@@ -135,7 +135,8 @@ class Engine:
         ``star_fitpars_i[k]`` in its first ``star_ndim[k]`` columns, and the columns after those are ignored.
 
         ``targets``: member counts [n_0, n_1, ...] summing to the number of stars; target t is the next n_t stars
-        (see ``set_targets``)."""
+        (see ``set_targets``).  Targets work with LSF vectors too: every star then carries its fixed ``Inst_R`` vector
+        and none has an ``Inst_R`` column."""
         if stars is None:
             stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot}]
         elif any(v is not None for v in (obs_wave, obs_flux, obs_eflux, obs_phot)):
@@ -301,7 +302,9 @@ class Engine:
     def set_targets(self, counts):
         """Group the stars into targets: target t is the next ``counts[t]`` stars, its members, which share the
         emulator labels and ``Vrot`` (same columns or fixed values) and may differ in ``Vrad``, ``Inst_R``, pixels and
-        continuum order; only the first member may have photometry.  None removes the targets."""
+        continuum order; only the first member may have photometry.  With LSF vectors each member is broadened by its
+        own vector, on any emulator grid the LSF tail takes, and a member with an ``Inst_R`` column is refused (nothing
+        would read it).  Without them the emulator grid must be uniform in ln wavelength.  None removes the targets."""
         if counts is None:
             _lib.check(self.lib.payne_ctx_set_targets(self._ctx, None, 0))
             self.n_targets = 0

@@ -20,7 +20,9 @@ What differs, on purpose:
   * ``inputdict['spec']`` may be a list of spectrum dictionaries (echelle orders, spectrograph arms), each with the
     keys of the single one.  The labels, ``Vrad`` and ``Vrot`` are shared; spectrum s has its own ``Inst_R_<s>`` and
     continuum coefficients ``pc_<s>_<k>``, whose priors come from ``priordict['Inst_R_<s>']`` and
-    ``priordict['blaze_coeff_<s>']`` (``multispec.MultiSpecLikelihood``).
+    ``priordict['blaze_coeff_<s>']`` (``multispec.MultiSpecLikelihood``).  ``priordict['Inst_R_<s>'] = {'fixed': lsf}``
+    with a 1-D ``lsf`` (one dispersion per fitted pixel of spectrum s, for every s) fits with LSF vectors; the output
+    file then has no column for them.
 """
 from __future__ import annotations
 
@@ -236,7 +238,10 @@ class FitPayne(object):
         sampler = BatchedNestedSampler(lnprob.batch, self.priorobj.priortrans_batch, self.ndim, nlive=npoints,
                                        walks=numwalks, queue_size=samplerdict.get('queue_size', None),
                                        reflective=reflective, seed=samplerdict.get('seed', None))
-        parnames = list(self.likeobj.fitpars_i) + list(self.likeobj.fixedpars.keys())
+        # several spectra: an LSF vector (one value per pixel, the same in every row) gets no column
+        multi = 'spectra' in self.fitargs
+        parnames = list(self.likeobj.fitpars_i) + [kk for kk, vv in self.likeobj.fixedpars.items()
+                                                    if not (multi and np.ndim(vv) > 0)]
         self._initoutput(parnames)
         ncall, nit = 0, 0
         for it, res in enumerate(sampler.sample(dlogz=delta_logz_final, maxiter=maxiter, maxcall=maxcall)):

@@ -8,6 +8,9 @@ spectrum's layout reads its own columns under the reference's names (``Inst_R_<s
 ``pc_k``), so lnL = -0.5 (chi2_0 + ... + chi2_{S-1} + chi2_sed) with each chi2_s what a single-spectrum ``likelihood``
 of spectrum s gives.  ``fitargs['spectra']`` is the list of ``{'obs_wave_fit', 'obs_flux_fit', 'obs_eflux_fit'}``
 (``FitPayne`` builds it from a list-valued ``inputdict['spec']``).
+
+A fixed ``Inst_R_<s>`` that is a 1-D array is spectrum s's LSF vector, one dispersion (AA) per fitted pixel of that
+spectrum, as a fixed ``Inst_R`` array is in the single-spectrum ``likelihood``.  Every spectrum has one or none does.
 """
 from __future__ import annotations
 
@@ -43,6 +46,12 @@ class MultiSpecLikelihood(object):
         if self.carbon_bool:
             raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
         self.fixedpars = fitargs['fixedpars']
+        spectra = fitargs['spectra']
+        lsf = [np.ndim(self.fixedpars.get('Inst_R_%d' % s, 0.0)) == 1 for s in range(len(spectra))]
+        if any(lsf) and not all(lsf):
+            raise ValueError('spectra %s have an LSF vector (a fixed Inst_R_<s> array) and spectra %s do not: every '
+                             'spectrum has one or none does' % ([s for s, v in enumerate(lsf) if v],
+                                                                [s for s, v in enumerate(lsf) if not v]))
         self.precision = kwargs.get('precision', 'parity')
         self.GM = GenMod(precision=self.precision)
         self.GM._initspecnn(nnpath=fitargs['specANNpath'], NNtype=fitargs.get('NNtype', 'LinNet'))
@@ -51,7 +60,6 @@ class MultiSpecLikelihood(object):
         self.fitpars_i = free_parameters(fitpars)
         self.ndim = len(self.fitpars_i)
         self.parsdict = {}
-        spectra = fitargs['spectra']
         stars = []
         for s, sp in enumerate(spectra):
             fit = [spectrum_name(p, s) for p in self.fitpars_i]

@@ -15,7 +15,12 @@ included -- and around the tail), median over --reps calls.  Per call: CUDA even
 cases must give the same lnL bits (checked on every (K, B)).  Inputs are drawn once per (K, B) and every case is
 warmed up before it is timed.  The GPU name and power limit are read in the same run.
 
-usage: python tools/gpu_targets.py [--out DIR] [--ks 1,2,4,8] [--bs 512,4096] [--reps 30]
+--lsf: every member has its own LSF vector (a fixed Inst_R array, the shape of test_gpu_star_opts._lsf) and its own
+Vrad column in place of the Inst_R column; the labels and Vrot are shared.  Each member's LSF mask reaches 2000 AA past
+its pixels, so its LSF stage spans about the whole emulator grid whatever its slice: targets save the K-1 emulator
+rows and rotation stages per point, not LSF work.
+
+usage: python tools/gpu_targets.py [--out DIR] [--ks 1,2,4,8] [--bs 512,4096] [--reps 30] [--lsf]
 """
 import argparse
 import json
@@ -34,9 +39,14 @@ from thepayne_b200.engine import Engine  # noqa: E402
 from gpu_multistar import gpu_info  # noqa: E402
 
 SHARED = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot']
+SHARED_LSF = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrot']
 
 
-def members(spec, K, seed=1):
+def lsf_vector(wave, k):
+    return 0.035 + 0.004 * k + 0.01 * (wave - wave.min()) / (wave.max() - wave.min()) + 0.003 * np.sin(wave / 2.0)
+
+
+def members(spec, K, lsf=False, seed=1):
     w = spec.wavelength
     a, b = w[0], w[-1]
     lo, hi = a + 0.04 * (b - a), b - 0.04 * (b - a)
@@ -46,17 +56,23 @@ def members(spec, K, seed=1):
     out = []
     for m in range(K):
         g = np.linspace(edges[m], edges[m + 1], n)
-        fit = SHARED + ['pad'] * m + ['Inst_R']           # member m's Inst_R in column 6 + m
-        out.append({'wave': g, 'flux': 1.0 + 0.02 * rng.standard_normal(n), 'eflux': np.full(n, 0.02),
-                    'fitpars_i': fit, 'runbools': [True, False, False, False]})
+        st = {'wave': g, 'flux': 1.0 + 0.02 * rng.standard_normal(n), 'eflux': np.full(n, 0.02),
+              'runbools': [True, False, False, False]}
+        if lsf:                                           # member m's Vrad in column 5 + m
+            st['fitpars_i'] = SHARED_LSF + ['pad'] * m + ['Vrad']
+            st['fixedpars'] = {'Inst_R': lsf_vector(g, m)}
+        else:                                             # member m's Inst_R in column 6 + m
+            st['fitpars_i'] = SHARED + ['pad'] * m + ['Inst_R']
+        out.append(st)
     return out
 
 
-def draw(K, B, seed):
+def draw(K, B, seed, lsf=False):
     rng = np.random.default_rng(seed)
     box = synth._BOX
-    th = np.empty((B, len(SHARED) + K))
-    for i, p in enumerate(SHARED + ['Inst_R'] * K):
+    cols = SHARED_LSF + ['Vrad'] * K if lsf else SHARED + ['Inst_R'] * K
+    th = np.empty((B, len(cols)))
+    for i, p in enumerate(cols):
         th[:, i] = box[p][0] + (box[p][1] - box[p][0]) * rng.random(B)
     return th
 
@@ -88,6 +104,7 @@ def main():
     ap.add_argument('--ks', default='1,2,4,8')
     ap.add_argument('--bs', default='512,4096')
     ap.add_argument('--reps', type=int, default=30)
+    ap.add_argument('--lsf', action='store_true', help='members with their own LSF vectors and Vrad columns')
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit('gpu_targets.py needs a CUDA device')
@@ -97,11 +114,11 @@ def main():
     print('gpu:', json.dumps(info))
     rows = []
     for K in [int(v) for v in args.ks.split(',')]:
-        mem = members(spec, K)
+        mem = members(spec, K, args.lsf)
         eng = Engine(spec=spec, stars=mem, targets=[K], precision='parity')
         for B in [int(v) for v in args.bs.split(',')]:
             eng.set('max_batch', max(8192, K * B))           # one slab for either case
-            th = torch.from_numpy(draw(K, B, K * 100 + B)).cuda()
+            th = torch.from_numpy(draw(K, B, K * 100 + B, args.lsf)).cuda()
             tgt = torch.zeros(B, dtype=torch.int32, device='cuda')
             th_dup = th.repeat_interleave(K, dim=0).contiguous()   # row p*K + m: point p, member m
             star = torch.arange(K, dtype=torch.int32, device='cuda').repeat(B).contiguous()
@@ -116,7 +133,7 @@ def main():
             for m in range(1, K):
                 tot = tot + c2[:, m]
             same = bool(np.array_equal(-0.5 * tot, out['t'].cpu().numpy(), equal_nan=True))
-            row = {'K': K, 'B': B, 'identical_lnl': same,
+            row = {'K': K, 'B': B, 'lsf': args.lsf, 'identical_lnl': same,
                    'targets_ms': timed(f_t, args.reps), 'duplicated_ms': timed(f_d, args.reps),
                    'targets_kernels_ms': kernels(eng, f_t, args.reps),
                    'duplicated_kernels_ms': kernels(eng, f_d, args.reps)}
@@ -129,7 +146,7 @@ def main():
         eng.close()
     if args.out:
         os.makedirs(args.out, exist_ok=True)
-        with open(os.path.join(args.out, 'targets.json'), 'w') as f:
+        with open(os.path.join(args.out, 'targets_lsf.json' if args.lsf else 'targets.json'), 'w') as f:
             json.dump({'gpu': info, 'rows': rows}, f, indent=1)
     if not all(r['identical_lnl'] for r in rows):
         sys.exit('lnL of the two cases differ')
