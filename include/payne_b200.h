@@ -263,6 +263,44 @@ int payne_model_batch_targets(PayneCtx* ctx, const double* theta_dev, const int3
                               double* flux_dev, int64_t ld_flux, double* chi2_dev, int64_t ld_chi2, double* mags_dev,
                               double* lnl_dev, void* stream);
 
+/* Double-lined binaries: one observed spectrum modelled as the flux-weighted sum of two stars.  Component 1 (the
+ * primary) has the parameters of the layout, as everywhere else.  Component 2 (the secondary) resolves each of Teff,
+ * log(g), [Fe/H], [a/Fe], Vmic, Vrad and Vrot to col[P] (a theta column) if col[P] >= 0, else to fixed[P] if that is
+ * not NaN, else to the primary's value.  Inst_R and the continuum polynomial are shared.  Rratio = R_sec / R_pri is
+ * theta column rratio_col, or rratio_fixed when rratio_col < 0.  Per observed pixel j (wavelength lambda_j):
+ *   a_c[j]  component c's model before the continuum (1 + line depth after rotation, Doppler shift, instrumental
+ *           stage or plain interpolation, resampling; NaN where the single-star model is NaN);
+ *   k_j     = Rratio^2 * expm1(c2 / (lambda_j Teff_1)) / expm1(c2 / (lambda_j Teff_2)), c2 = 1.438776877e8 AA K
+ *           (both stars radiate as blackbodies of radius R);
+ *   m_j     = (a_1[j] + k_j a_2[j]) / (1 + k_j), times the continuum polynomial when the layout has one;
+ * chi2 and lnL as for one star.  With Rratio = 0 and a finite a_2, m and lnL have the bits of the primary alone
+ * through payne_model_batch_stars.  A component that is bad by itself makes lnL and the model NaN. */
+typedef struct {
+  int32_t col[PAYNE_NPAR];   /* secondary's theta column, -1: not sampled */
+  double  fixed[PAYNE_NPAR]; /* secondary's fixed value where col < 0; NaN: the primary's value */
+  int32_t rratio_col;        /* Rratio's theta column, -1: rratio_fixed */
+  double  rratio_fixed;
+} PayneBinary;
+
+/* Sets the binary description (HOST pointer, copied); NULL removes it.  PAYNE_E_INVALID: a column or non-NaN fixed
+ * value on a parameter other than the seven above, a column outside [0, ndim), Rratio neither sampled nor fixed to a
+ * finite value.  PAYNE_E_UNSUPPORTED, here and again in every _binary entry: photometry (phot_bool), LSF vectors, an
+ * attached continuum emulator, targets, per-star layouts (PayneStarOpts.layout), the fused gather, and contexts without
+ * the fast tail (emulator grid not uniform in ln wavelength).  Per-star fixed values apply to the shared parameters.
+ * The entries without _binary are unchanged by it.  Every point runs both components' emulator rows in one pass of the
+ * emulator, so a slab holds max_batch / 2 points. */
+int payne_ctx_set_binary(PayneCtx* ctx, const PayneBinary* binary);
+/* star_dev: [B] int32 or NULL (star 0), as in the _stars entries (a star outside [0, n_stars): lnL NaN, status bit 2;
+ * the _host entry returns PAYNE_E_INVALID before launching). */
+int payne_lnlike_batch_binary(PayneCtx* ctx, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                              double* lnl_dev, void* stream);
+int payne_lnlike_batch_binary_host(PayneCtx* ctx, const double* theta_host, const int32_t* star_host, int64_t B,
+                                   int64_t ld, double* lnl_host);
+/* flux_dev [B, ld_flux]: m; comp_dev [B, 2, ld_flux]: a_1 and a_2 (ld_flux >= the largest n_obs); lnl_dev [B].  Any
+ * output may be NULL; row p gets the first n_obs of its star, the rest is not written. */
+int payne_model_batch_binary(PayneCtx* ctx, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                             double* flux_dev, int64_t ld_flux, double* comp_dev, double* lnl_dev, void* stream);
+
 /* Continuum emulator (HOST pointers, copied): any PayneSpecNet the spectrum emulator could be; its
  * `wavelength` is the continuum's own grid.  From then on every model spectrum is multiplied, right after
  * the emulator and before any broadening, by np.interp(modwave, contwave, c / nanmedian(c), left=nan,
@@ -306,7 +344,7 @@ int payne_lnlike_batch_gather(PayneCtx* ctx, const double* theta_dev, int64_t B,
 int payne_gather_flush(PayneCtx* ctx, void* stream, double** gathered_last);
 
 /* Introspection for benches/tests: key is one of "n_ann","n_obs" (the largest star's),"n_stars","n_obs_total"
- * (observed pixels of all stars),"n_targets","nfft1","launches",
+ * (observed pixels of all stars),"n_targets","binary" (1 while a PayneBinary is set),"nfft1","launches",
  * "grid_loguniform","fast_tail","max_batch","sm_count","tail_grid","precision","continuum","lsf","legacy_tc"
  * (a leaky-ReLU stack whose output layer runs on the tensor cores),"status"
  * (bit0: a point needed a larger transform than the shared-memory carve-out; bit1: a peer of the gather never arrived;

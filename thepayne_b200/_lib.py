@@ -29,7 +29,9 @@ EXPORTS = ['payne_abi_version', 'payne_last_error', 'payne_ctx_create', 'payne_c
            'payne_ctx_create_stars', 'payne_lnlike_batch_stars', 'payne_lnlike_batch_stars_host',
            'payne_model_batch_stars', 'payne_ctx_create_stars_opts',
            'payne_ctx_set_targets', 'payne_lnlike_batch_targets', 'payne_lnlike_batch_targets_host',
-           'payne_model_batch_targets']
+           'payne_model_batch_targets',
+           'payne_ctx_set_binary', 'payne_lnlike_batch_binary', 'payne_lnlike_batch_binary_host',
+           'payne_model_batch_binary']
 GATHER_HANDLE_BYTES = 128
 
 _f = C.POINTER(C.c_float)
@@ -63,6 +65,11 @@ class PayneLayout(C.Structure):
 
 class PayneStarOpts(C.Structure):
     _fields_ = [('fixed', _d), ('band', C.POINTER(C.c_int32)), ('lsf', _d), ('layout', C.POINTER(PayneLayout))]
+
+
+class PayneBinary(C.Structure):
+    _fields_ = [('col', C.c_int32 * NPAR), ('fixed', C.c_double * NPAR), ('rratio_col', C.c_int32),
+                ('rratio_fixed', C.c_double)]
 
 
 class PayneError(RuntimeError):
@@ -113,6 +120,14 @@ def load():
     lib.payne_lnlike_batch_targets_host.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp]
     lib.payne_model_batch_targets.restype = C.c_int
     lib.payne_model_batch_targets.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, C.c_int64, vp, vp, vp]
+    lib.payne_ctx_set_binary.restype = C.c_int
+    lib.payne_ctx_set_binary.argtypes = [vp, C.POINTER(PayneBinary)]
+    lib.payne_lnlike_batch_binary.restype = C.c_int
+    lib.payne_lnlike_batch_binary.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, vp]
+    lib.payne_lnlike_batch_binary_host.restype = C.c_int
+    lib.payne_lnlike_batch_binary_host.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp]
+    lib.payne_model_batch_binary.restype = C.c_int
+    lib.payne_model_batch_binary.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, vp, vp]
     lib.payne_ctx_destroy.restype = None
     lib.payne_ctx_destroy.argtypes = [vp]
     lib.payne_lnlike_batch.restype = C.c_int

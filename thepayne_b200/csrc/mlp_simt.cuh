@@ -37,13 +37,20 @@ struct EncodeParams {
   const int* star;   // [B] star of every row of this slab (null: star 0)
   int n_stars;
   const StarLayout* star_lay;
+  // binaries (payne_ctx_set_binary): rows [half, 2 half) are the secondaries of points [0, half), whose theta rows
+  // and stars are those of the primaries; null without a binary
+  const PayneBinary* binary;
+  int half;
 };
 
 // raw value of label i of row p
 __device__ __forceinline__ double label_of(const EncodeParams& E, const double* x, long long ld, int p, int i) {
   const int which = label_param(i);
+  const bool sec = E.binary && p >= E.half;
+  if (sec) p -= E.half;
   const int k = (which >= 0 && (E.star_fixed || E.star_lay)) ? star_of(E.star, E.n_stars, p) : -1;
-  return param_of(E.star_lay, E.col[i], E.fixed[i], E.star_fixed, x + (long long)p * ld, k, which);
+  const double v = param_of(E.star_lay, E.col[i], E.fixed[i], E.star_fixed, x + (long long)p * ld, k, which);
+  return sec ? secondary_of(E.binary, x + (long long)p * ld, which, v) : v;
 }
 
 // h1[p, h] = sigmoid(W1[h, :] . enc(x_p) + b1[h]); optionally also the tf32 hi/lo split planes.

@@ -42,6 +42,16 @@ __device__ __forceinline__ double param_of(const StarLayout* star_lay, int ctx_c
   return (star_fixed && k >= 0) ? star_fixed[(long long)k * PAYNE_NPAR + which] : ctx_fixed;
 }
 
+// Parameter `which` of a binary's secondary (payne_ctx_set_binary) in theta row th: its own column, else its own fixed
+// value when that is not NaN, else `prim`, the primary's value (param_of).  bin null (no binary): prim.
+__device__ __forceinline__ double secondary_of(const PayneBinary* bin, const double* th, int which, double prim) {
+  if (!bin || which < 0) return prim;
+  const int c = bin->col[which];
+  if (c >= 0) return th[c];
+  const double f = bin->fixed[which];
+  return f == f ? f : prim;
+}
+
 // Continuum coefficients of theta row th of star k into poly[]; returns their number.
 __device__ __forceinline__ int poly_of(const StarLayout* star_lay, int ctx_n_poly, const int* ctx_poly_col,
                                        const double* th, int k, double* poly) {

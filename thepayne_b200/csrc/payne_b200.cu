@@ -185,6 +185,13 @@ struct PayneCtx {
   payne::FastPoint* tgt_points = nullptr;   // [tgt_rows * tgt_kmax] per-(point, member) records (fast tail only)
   int* tgt_star = nullptr;              // [tgt_rows] first member's star of every point of a slab
   long long tgt_rows = 0, tgt_rec_alloc = 0;
+  // binaries (payne_ctx_set_binary): the secondary's description, the binary tail's grid and its workspace
+  bool has_binary = false;
+  PayneBinary* binary_dev = nullptr;
+  int bin_grid = 0;
+  double* bin_scratch = nullptr;        // [bin_grid, n_obs_max] a_1 of every CTA's current point
+  double* bin_par = nullptr;            // [bin_rows, 3] Teff_1, Teff_2, Rratio of the points of a slab
+  long long bin_rows = 0;
   // photometry
   bool has_phot = false;
   payne::PhotParams phot{};
@@ -936,20 +943,34 @@ int ensure_target_workspace(PayneCtx* c, long long rows, bool records) {
   return PAYNE_OK;
 }
 
+// Binaries: Teff_1, Teff_2 and Rratio of the points of a slab of `rows` points
+int ensure_binary_workspace(PayneCtx* c, long long rows) {
+  if (rows <= c->bin_rows) return PAYNE_OK;
+  CU_TRY(cudaDeviceSynchronize());                       // earlier calls may still read them
+  if (c->bin_par) cudaFree(c->bin_par);
+  c->bin_par = nullptr; c->bin_rows = 0;
+  CU_TRY(cudaMalloc((void**)&c->bin_par, (size_t)rows * 3 * sizeof(double)));
+  c->bin_rows = rows;
+  return PAYNE_OK;
+}
+
 // star: [B] star index of every point (null: star 0); flux_out rows are ld_flux apart.  target: see above; chi2_out
-// [B, ld_chi2] the chi2 of every member (targets only)
+// [B, ld_chi2] the chi2 of every member (targets only).  binary: every point is a binary (payne_ctx_set_binary), the
+// emulator runs 2 nb rows per slab of nb points; comp_out [B, 2, ld_flux] its components' spectra.
 int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, long long ld, double* flux_out,
               long long ld_flux, double* mags_out, double* lnl, cudaStream_t st, const int* target = nullptr,
-              double* chi2_out = nullptr, long long ld_chi2 = 0) {
+              double* chi2_out = nullptr, long long ld_chi2 = 0, bool binary = false, double* comp_out = nullptr) {
   using namespace payne;
   if (B <= 0) return PAYNE_OK;
   if (ld < c->ndim_max) return fail(PAYNE_E_INVALID, "ld < ndim (the largest star's with per-star layouts)");
   if (!target && flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
   const bool records = target && !c->lsf_on;             // the fast target tail's per-(point, member) records
-  const long long slab = records ? std::min(c->slab, std::max(1LL, kTargetRecords / c->tgt_kmax)) : c->slab;
-  int rc = ensure_workspace(c, B);
+  const long long slab = records ? std::min(c->slab, std::max(1LL, kTargetRecords / c->tgt_kmax))
+                       : binary ? std::max(1LL, c->slab / 2) : c->slab;
+  int rc = ensure_workspace(c, binary ? 2 * B : B);
   if (rc) return rc;
   if (target) { rc = ensure_target_workspace(c, std::min(B, slab), records); if (rc) return rc; }
+  if (binary) { rc = ensure_binary_workspace(c, std::min(B, slab)); if (rc) return rc; }
   rc = order_after_previous(c, st);
   if (rc) return rc;
   if (c->timing) { c->ms_acc[0] = c->ms_acc[1] = c->ms_acc[2] = 0; c->ms_valid = false; c->pending.clear(); }
@@ -983,6 +1004,10 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         T.target = target + p0; T.tfirst = c->tfirst_dev; T.n_targets = c->n_targets; T.kmax = c->tgt_kmax;
         T.chi2_out = chi2_out ? chi2_out + p0 * ld_chi2 : nullptr; T.ld_chi2 = ld_chi2;
       }
+      if (binary) {
+        T.binary = c->binary_dev; T.bin_par = c->bin_par; T.bin_scratch = c->bin_scratch; T.bin_ld = c->n_obs_max;
+        T.comp_out = comp_out ? comp_out + p0 * 2 * ld_flux : nullptr;
+      }
       if (gather_here) {
         // all-gather fused into the tail (tail.cuh store_lnl / gather_exit): this slab's slice of every peer's buffer
         T.g_world = c->g_world; T.g_rank = c->g_rank; T.g_done = c->g_done;
@@ -996,7 +1021,7 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         // per-point setup depends only on theta: fork it beside the emulator GEMMs, join before the tail
         CU_TRY(cudaEventRecord(c->ev_fork, st));
         CU_TRY(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-        c->fast.work_start = target ? std::min(c->tgt_grid, nb)
+        c->fast.work_start = target ? std::min(c->tgt_grid, nb) : binary ? std::min(c->bin_grid, nb)
                            : (c->use_cluster && c->allow_cluster) ? (int)std::min<long long>(c->cluster_n, nb)
                                                                   : std::min(c->tail_grid_fast, nb);
         if (c->grid_cap > 0) c->fast.work_start = std::min(c->fast.work_start, c->grid_cap);
@@ -1005,6 +1030,10 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
           FT.points = c->tgt_points; FT.cluster = 0;
           if (payne::launch_tail_setup_targets((long long)nb * c->tgt_kmax, c->side, T, FT))
             return fail(PAYNE_E_CUDA, "tail_setup launch");
+        } else if (binary) {
+          FastGrid FB = c->fast;
+          FB.cluster = 0;
+          if (payne::launch_tail_setup_binary(nb, c->side, T, FB)) return fail(PAYNE_E_CUDA, "tail_setup launch");
         } else if (payne::launch_tail_setup(nb, c->side, T, c->fast)) {
           return fail(PAYNE_E_CUDA, "tail_setup launch");
         }
@@ -1017,7 +1046,8 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
       }
       EncodeParams E = c->enc;
       E.star = star_s;
-      rc = run_mlp(c, E, th, ld, nb, c->flux, c->ldf, true, &is_depth, st);
+      if (binary) { E.binary = c->binary_dev; E.half = nb; }   // rows [nb, 2 nb): the secondaries
+      rc = run_mlp(c, E, th, ld, binary ? 2 * nb : nb, c->flux, c->ldf, true, &is_depth, st);
       if (rc) return rc;
       if (c->cont) {
         // modspec *= np.interp(modwave, modcontwave, normalised F_lambda continuum) (predictspec.py:208-226)
@@ -1064,6 +1094,13 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         const int grid = std::min(c->lsf_grid, nb);
         if (target ? payne::launch_tail_lsf_targets(grid, c->lsf_smem, st, TL, c->lsf)
                    : payne::launch_tail_lsf(grid, c->lsf_smem, st, TL, c->lsf))
+          return fail(PAYNE_E_CUDA, "tail launch");
+      } else if (binary) {
+        // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no binary form)
+        if (!(fast_tail && is_depth)) return fail(PAYNE_E_UNSUPPORTED, "binaries need the fast tail on line-depth rows");
+        FastGrid FB = c->fast;
+        FB.cluster = 0;
+        if (payne::launch_tail_fast_binary(T.log2N1, c->fast.work_start, c->fast_smem, st, T, FB))
           return fail(PAYNE_E_CUDA, "tail launch");
       } else if (target) {
         // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no target form)
@@ -1205,7 +1242,7 @@ int need_targets(PayneCtx* c) {
 
 // The host-buffer entries: idx_host is every point's star, or its target (targets = true), or null (star 0).
 int lnlike_host(PayneCtx* c, const double* theta_host, const int32_t* star_host, int64_t B, int64_t ld, double* lnl_host,
-                bool targets) {
+                bool targets, bool binary = false) {
   int rc;
   const int n_idx = targets ? c->n_targets : c->n_stars;
   if (star_host)
@@ -1249,7 +1286,7 @@ int lnlike_host(PayneCtx* c, const double* theta_host, const int32_t* star_host,
   }
   const int* idx = star_host ? c->star_stage : nullptr;
   rc = run_batch(c, c->theta_stage, targets ? nullptr : idx, B, ld, nullptr, 0, nullptr,
-                 c->lnl_map ? c->lnl_map : c->lnl_stage, c->stream, targets ? idx : nullptr);
+                 c->lnl_map ? c->lnl_map : c->lnl_stage, c->stream, targets ? idx : nullptr, nullptr, 0, binary);
   if (rc) return rc;
   if (!c->lnl_map)
     CU_TRY(cudaMemcpyAsync(c->lnl_pin, c->lnl_stage, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost,
@@ -1267,9 +1304,108 @@ std::pair<int, double> resolve_param(const PayneCtx* c, int k, int which) {
   return {-1, c->star_fixed_h.empty() ? c->lay.fixed[which] : c->star_fixed_h[(size_t)k * PAYNE_NPAR + which]};
 }
 
+// What the binary tail cannot take (payne_ctx_set_binary and every _binary entry: the context may have changed since).
+int binary_unsupported(PayneCtx* c) {
+  const char* why = !c->has_spec ? "the spectrum emulator is missing"
+                  : c->has_phot ? "photometry (phot_bool) is not supported"
+                  : c->lsf_on ? "LSF vectors are not supported"
+                  : c->cont ? "an attached continuum emulator is not supported"
+                  : c->n_targets ? "targets are not supported"
+                  : c->star_lay_dev ? "per-star layouts (PayneStarOpts.layout) are not supported"
+                  : c->g_world > 0 ? "the fused gather is not supported"
+                  : !(c->use_fast && c->allow_fast) ? "binaries need the fast tail (an emulator grid uniform in ln wavelength)"
+                  : nullptr;
+  return why ? fail(PAYNE_E_UNSUPPORTED, std::string("binary: ") + why) : PAYNE_OK;
+}
+
+int need_binary(PayneCtx* c) {
+  if (!c->has_binary) return fail(PAYNE_E_INVALID, "no binary: payne_ctx_set_binary first");
+  return binary_unsupported(c);
+}
+
 }  // namespace
 
 extern "C" {
+
+int payne_ctx_set_binary(PayneCtx* c, const PayneBinary* b) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  auto drop = [&]() -> int {
+    CU_TRY(cudaDeviceSynchronize());                     // earlier calls may still read them
+    if (c->binary_dev) cudaFree(c->binary_dev);
+    if (c->bin_scratch) cudaFree(c->bin_scratch);
+    c->binary_dev = nullptr; c->bin_scratch = nullptr; c->has_binary = false;
+    return PAYNE_OK;
+  };
+  if (!b) return drop();
+  int rc = binary_unsupported(c);
+  if (rc) return rc;
+  static const char* names[PAYNE_NPAR] = {"Teff", "log(g)", "[Fe/H]", "[a/Fe]", "Vrad", "Vrot", "Vmic", "Inst_R",
+                                          "log(R)", "Dist", "log(A)", "Av", "Rv"};
+  const int ndim = c->lay.ndim;
+  for (int i = 0; i < PAYNE_NPAR; ++i) {
+    const bool own = i == PAYNE_P_TEFF || i == PAYNE_P_LOGG || i == PAYNE_P_FEH || i == PAYNE_P_AFE || i == PAYNE_P_VMIC ||
+                     i == PAYNE_P_VRAD || i == PAYNE_P_VROT;
+    if (!own && (b->col[i] >= 0 || !std::isnan(b->fixed[i])))
+      return fail(PAYNE_E_INVALID, std::string("binary: ") + names[i] + " is shared by both components (the secondary "
+                  "may have its own Teff, log(g), [Fe/H], [a/Fe], Vmic, Vrad and Vrot only)");
+    if (b->col[i] >= ndim)
+      return fail(PAYNE_E_INVALID, std::string("binary: ") + names[i] + " column " + std::to_string(b->col[i]) +
+                  " outside [0, ndim = " + std::to_string(ndim) + ")");
+  }
+  if (b->rratio_col >= ndim)
+    return fail(PAYNE_E_INVALID, "binary: Rratio column " + std::to_string(b->rratio_col) + " outside [0, ndim = " +
+                std::to_string(ndim) + ")");
+  if (b->rratio_col < 0 && !std::isfinite(b->rratio_fixed))
+    return fail(PAYNE_E_INVALID, "binary: Rratio needs a theta column or a finite fixed value");
+  int occ = 0;
+  if (!payne::probe_tail_fast_binary(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
+    return fail(PAYNE_E_UNSUPPORTED, "binary tail kernel does not fit on an SM");
+  rc = drop();
+  if (rc) return rc;
+  c->bin_grid = std::min(occ * c->sm_count, c->tail_grid_fast);   // the split kernel's scratch lines exist for these
+  rc = upload(&c->binary_dev, b, 1);
+  if (rc) return rc;
+  CU_TRY(cudaMalloc((void**)&c->bin_scratch, (size_t)c->bin_grid * c->n_obs_max * sizeof(double)));
+  c->has_binary = true;
+  return PAYNE_OK;
+}
+
+int payne_lnlike_batch_binary(PayneCtx* c, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                              double* lnl_dev, void* stream) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B == 0) return PAYNE_OK;
+  if (!theta_dev || !lnl_dev) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  int rc = need_binary(c);
+  if (rc) return rc;
+  return run_batch(c, theta_dev, star_dev, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, nullptr, nullptr, 0,
+                   true);
+}
+
+int payne_lnlike_batch_binary_host(PayneCtx* c, const double* theta_host, const int32_t* star_host, int64_t B, int64_t ld,
+                                   double* lnl_host) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B <= 0) return PAYNE_OK;
+  if (!theta_host || !lnl_host) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  int rc = need_binary(c);
+  if (rc) return rc;
+  return lnlike_host(c, theta_host, star_host, B, ld, lnl_host, false, true);
+}
+
+int payne_model_batch_binary(PayneCtx* c, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                             double* flux_dev, int64_t ld_flux, double* comp_dev, double* lnl_dev, void* stream) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B == 0) return PAYNE_OK;
+  if (!theta_dev) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  int rc = need_binary(c);
+  if (rc) return rc;
+  if ((flux_dev || comp_dev) && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
+  return run_batch(c, theta_dev, star_dev, B, ld, flux_dev, ld_flux, nullptr, lnl_dev, (cudaStream_t)stream, nullptr,
+                   nullptr, 0, true, comp_dev);
+}
 
 int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) {
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
@@ -1457,6 +1593,7 @@ void payne_ctx_destroy(PayneCtx* c) {
   payne::tc_free_acts_x(&c->actA); payne::tc_free_acts_x(&c->actB);
   drop(c->theta_stage); drop(c->lnl_stage); drop(c->star_stage);
   drop(c->tfirst_dev); drop(c->tgt_points); drop(c->tgt_star);
+  drop(c->binary_dev); drop(c->bin_scratch); drop(c->bin_par);
   if (c->star_pin) cudaFreeHost(c->star_pin);
   for (int r = 0; r < 16; ++r)
     if (c->g_opened[r]) { cudaIpcCloseMemHandle(c->g_peer_buf[r]); cudaIpcCloseMemHandle(c->g_peer_flag[r]); }
@@ -1794,6 +1931,7 @@ int64_t payne_ctx_query(PayneCtx* c, const char* key) {
   if (k == "n_obs") return c->n_obs_max;
   if (k == "n_stars") return c->n_stars;
   if (k == "n_targets") return c->n_targets;
+  if (k == "binary") return c->has_binary ? 1 : 0;
   if (k == "n_obs_total") return c->n_obs_total;
   if (k == "nfft1") return c->has_spec ? (1LL << c->tail.log2N1) : 0;
   if (k == "launches") return c->launches;

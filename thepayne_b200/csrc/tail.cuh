@@ -105,6 +105,13 @@ struct TailParams {
   int n_targets, kmax;               // kmax: the largest member count
   double* chi2_out;                  // [B, ld_chi2] chi2 of every member, or null
   long long ld_chi2;
+  // Binaries (payne_ctx_set_binary; fast tail only): point p's component c has emulator row c * B + p and FastPoint
+  // record c * B + p.  Null binary: no binary.
+  const PayneBinary* binary;         // device copy
+  double* bin_par;                   // [B, 3] Teff_1, Teff_2, Rratio of every point (tail_setup_binary_kernel)
+  double* bin_scratch;               // [grid, bin_ld] a_1 of the CTA's current point
+  long long bin_ld;
+  double* comp_out;                  // [B, 2, ld_flux] a_1 and a_2, or null
 };
 
 // lnL of point p: local result and, with the fused gather on, the copy in every peer's buffer
@@ -272,9 +279,10 @@ __device__ __forceinline__ float depth_of(float v, bool is_depth, bool fill_nan)
   return is_depth ? v : v - 1.f;
 }
 
-// Point setup of theta row th against star k (k < 0: no such star).
+// Point setup of theta row th against star k (k < 0: no such star).  sec: the binary whose secondary this record
+// describes (its labels, Vrad and Vrot; secondary_of), null for the primary or a single star.
 static __device__ __forceinline__ void tail_setup_star(const TailParams& P, const double* th, int k, PointSetup& S,
-                                                       ObsSlice& obs) {
+                                                       ObsSlice& obs, const PayneBinary* sec = nullptr) {
   if (k < 0) {                                    // no observation to compare with: NaN, nothing written
     S.bad = 1; S.use_inst = 0; S.do_rot = 0;
     obs.off = 0; obs.n = 0;
@@ -283,14 +291,15 @@ static __device__ __forceinline__ void tail_setup_star(const TailParams& P, cons
   }
   const ObsStar& st = P.stars[k];
   obs.off = st.off; obs.n = st.n_obs;
-  const double vrot = get_par(P, th, PAYNE_P_VROT, k);
-  const double vrad = get_par(P, th, PAYNE_P_VRAD, k);
+  const double vrot = secondary_of(sec, th, PAYNE_P_VROT, get_par(P, th, PAYNE_P_VROT, k));
+  const double vrad = secondary_of(sec, th, PAYNE_P_VRAD, get_par(P, th, PAYNE_P_VRAD, k));
   const double instR = get_par(P, th, PAYNE_P_INSTR, k);
   S.bad = 0;
   S.clean = P.rows_may_nan ? 0 : 1;
   for (int i = 0; i < P.n_labels; ++i) {
     const int which = label_param(i);
-    const double v = param_of(P.star_lay, P.label_col[i], P.label_fixed[i], P.star_fixed, th, which >= 0 ? k : -1, which);
+    const double v = secondary_of(sec, th, which,
+                                  param_of(P.star_lay, P.label_col[i], P.label_fixed[i], P.star_fixed, th, which >= 0 ? k : -1, which));
     if (!isfinite(v)) S.clean = 0;
   }
   S.do_rot = (vrot != 0.0);                       // predictspec.py:231 (NaN != 0 is true)

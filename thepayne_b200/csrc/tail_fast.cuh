@@ -259,6 +259,138 @@ __device__ __forceinline__ double final_pass_poly(const TailParams& P, const Fas
   return acc;
 }
 
+// Binaries (payne_ctx_set_binary): the point's pixels with final_pass_poly's thread mapping and order.  BM = 1 (component
+// 1): a_1 = 1 + d (NaN outside the grid) into the CTA's scratch and comp row 0.  BM = 2 (component 2): a_2, a_1 read
+// back from the scratch (by the thread that wrote it), m = (a_1 + k a_2) / (1 + k) with the blackbody flux ratio k, the
+// continuum, chi2; a_2 into comp row 1 and m into the model row.  At k = 0 and a finite a_2, m is a_1 and the chi2 has
+// the bits of final_pass_poly.
+constexpr double kC2 = 1.438776877e8;   // second radiation constant hc / k_B, AA K
+
+__device__ __forceinline__ double flux_ratio(double lam, double t1, double t2, double rr2) {
+  return rr2 * expm1(kC2 / (lam * t1)) / expm1(kC2 / (lam * t2));
+}
+
+template <int BM, class ZV>
+__device__ __forceinline__ double final_pass_bin(const TailParams& P, const FastGrid& F, const PointSetup& S,
+                                                 const FastSetup& FS, const ZV& zv, int tid, int p, int N2) {
+  const double nan = CUDART_NAN;
+  const double pmax = (double)(N2 - 1);
+  const float hdu = S.hdu;
+  const double q0 = FS.q0, scale = FS.scale;
+  const int off = FS.obs.off, jend = FS.obs.off + FS.obs.n;
+  double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  double* crow = P.comp_out ? P.comp_out + ((long long)p * 2 + (BM - 1)) * P.ld_flux : nullptr;
+  double* mrow = (BM == 2 && P.model_out) ? P.model_out + (long long)p * P.ld_flux : nullptr;
+  const double t1 = __ldg(P.bin_par + 3LL * p), t2 = __ldg(P.bin_par + 3LL * p + 1), rr = __ldg(P.bin_par + 3LL * p + 2);
+  const double rr2 = rr * rr;
+  double acc = 0.0;
+  constexpr int U = 4;
+#pragma unroll 1
+  for (int j0 = off + tid; j0 < jend; j0 += U * kNT) {
+    float d[U];
+    unsigned okm = 0;
+    {
+      double q[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) q[u] = (j0 + u * kNT < jend) ? __ldcg(F.obs_q + j0 + u * kNT) : -1.0;
+      float g0[U], g1[U], dl[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const double pp = (q[u] - q0) * scale;
+        const bool ok = (pp >= 0.0 && pp <= pmax);         // smoothing.py:289 left/right = nan
+        const int k = ok ? min((int)pp, N2 - 2) : 0;
+        okm |= (unsigned)ok << u;
+        dl[u] = (float)(pp - (double)k);
+        g0[u] = zv.ld(k); g1[u] = zv.ld(k + 1);
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) d[u] = fmaf(interp_w(dl[u], hdu), g1[u] - g0[u], g0[u]);
+    }
+    if constexpr (BM == 1) {
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int j = j0 + u * kNT;
+        if (j < jend) {
+          const double a = ((okm >> u) & 1u) ? 1.0 + (double)d[u] : nan;
+          scr[j - off] = a;
+          if (crow) crow[j - off] = a;
+        }
+      }
+    } else {
+      double is[U], ot[U], x[U], cv[U], a1[U], lam[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int j = j0 + u * kNT;
+        const bool in = j < jend;
+        is[u] = in ? __ldcg(P.obs_inv_s + j) : 0.0;
+        ot[u] = in ? __ldcg(P.obs_ot + j) : 0.0;
+        x[u] = (in && P.n_poly) ? __ldcg(P.obs_x + j) : 0.0;
+        a1[u] = in ? scr[j - off] : 0.0;
+        lam[u] = in ? __ldcg(P.obs_w + j) : 1.0;
+      }
+      if (P.n_poly) chebval_dev4(x, S.poly, P.n_poly, cv);
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int j = j0 + u * kNT;
+        const double a2 = ((okm >> u) & 1u) ? 1.0 + (double)d[u] : nan;
+        const double k = flux_ratio(lam[u], t1, t2, rr2);
+        double m = (a1[u] + k * a2) / (1.0 + k);
+        if (P.n_poly) m *= cv[u];
+        if (j < jend) {
+          if (crow) crow[j - off] = a2;
+          if (mrow) mrow[j - off] = m;
+          const double r = fma(m, is[u], -ot[u]);
+          acc = fma(r, r, acc);
+        }
+      }
+    }
+  }
+  return acc;
+}
+
+// The same without an instrumental stage (plain np.interp, predictspec.py:288-289), with the thread mapping and order of
+// point_chi2's plain branch.
+template <int BM>
+__device__ __forceinline__ double plain_pass_bin(const TailParams& P, const PointSetup& S, const FastSetup& FS,
+                                                 const float* row, int tid, int p) {
+  const double nan = CUDART_NAN;
+  const int n = P.n;
+  const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
+  const int off = FS.obs.off, jend = FS.obs.off + FS.obs.n;
+  double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  double* crow = P.comp_out ? P.comp_out + ((long long)p * 2 + (BM - 1)) * P.ld_flux : nullptr;
+  double* mrow = (BM == 2 && P.model_out) ? P.model_out + (long long)p * P.ld_flux : nullptr;
+  const double t1 = __ldg(P.bin_par + 3LL * p), t2 = __ldg(P.bin_par + 3LL * p + 1), rr = __ldg(P.bin_par + 3LL * p + 2);
+  const double rr2 = rr * rr;
+  double acc = 0.0;
+  for (int j = off + tid; j < jend; j += kNT) {
+    const double x = __ldg(P.obs_w + j);
+    double a;
+    if (!(x >= wlo && x <= whi)) a = nan;
+    else {
+      const int g = (int)((__ldg(P.obs_lnw + j) - S.lnD - P.lnw0) * P.inv_dlnw);
+      const int jj = locate(P.w, S.D, x, g, 0, n - 2);
+      const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
+      const double va = (double)depth_of(row[jj], true, false);
+      const double vb = (double)depth_of(row[jj + 1], true, false);
+      a = 1.0 + ((vb - va) / (wb - wa) * (x - wa) + va);
+    }
+    if constexpr (BM == 1) {
+      scr[j - off] = a;
+      if (crow) crow[j - off] = a;
+    } else {
+      const double k = flux_ratio(x, t1, t2, rr2);
+      double m = (scr[j - off] + k * a) / (1.0 + k);
+      if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
+      if (crow) crow[j - off] = a;
+      if (mrow) mrow[j - off] = m;
+      const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
+      acc += r * r;
+    }
+  }
+  return acc;
+}
+
 // observed pixels, continuum, residuals; returns this thread's partial chi2
 template <bool POLY, bool STARS, class ZV>
 __device__ __forceinline__ double final_pass(const TailParams& P, const FastGrid& F, const PointSetup& S,
@@ -320,7 +452,8 @@ static __device__ __noinline__ void discard_lines(const float* row, int n, int t
 
 // Stage 2 and the final pass of one point against its star (S, FS) on the row that stage 1 left; returns this
 // thread's partial chi2.  z / zs / zp / gline: the kernel's transform buffer and its views.
-template <int LOG2N1, bool POLY, bool STARS>
+// BM: 0 a point of one star; 1 / 2 component 1 / 2 of a binary (final_pass_bin, plain_pass_bin).
+template <int LOG2N1, bool POLY, bool STARS, int BM = 0>
 __device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid& F, const PointSetup& S,
                                              const FastSetup& FS, float2* z, const ZSmem& zs, const ZSplit& zp,
                                              float* gline, const TwTab& tw, const float* row, int tid, int p, int moff) {
@@ -341,7 +474,8 @@ __device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid
         stage_regrid(S, row, zp, tid, N2, FS.s_num, FS.s_den, i0, FS.s_invden, F.c_native, FS.s_incj, FS.s_incr);
         __syncthreads();
         ct_convolve_split<LOG2MH>(z, reinterpret_cast<float2*>(gline), tw, F.twc, H, tid);
-        acc = final_pass<POLY, STARS>(P, F, S, FS, zp, tid, p, N2, moff);
+        if constexpr (BM == 0) acc = final_pass<POLY, STARS>(P, F, S, FS, zp, tid, p, N2, moff);
+        else acc = final_pass_bin<BM>(P, F, S, FS, zp, tid, p, N2);
       }
     } else {
       constexpr int LA = LOG2N1 > 15 ? 15 : LOG2N1;       // largest all-in-smem transform
@@ -360,8 +494,11 @@ __device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid
         ct_convolve_regrid<(LA >= 10 ? LA - 2 : 8)>(z, tw, F.twc, H, tid, row + i0, FS.s_num, FS.s_den,
                                                      FS.s_invden, F.c_native, S.clean != 0);
       }
-      acc = final_pass<POLY, STARS>(P, F, S, FS, zs, tid, p, N2, moff);
+      if constexpr (BM == 0) acc = final_pass<POLY, STARS>(P, F, S, FS, zs, tid, p, N2, moff);
+      else acc = final_pass_bin<BM>(P, F, S, FS, zs, tid, p, N2);
     }
+  } else if constexpr (BM != 0) {
+    acc = plain_pass_bin<BM>(P, S, FS, row, tid, p);
   } else {
     // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289)
     const int n = P.n;
@@ -388,14 +525,52 @@ __device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid
   return acc;
 }
 
+// Stage 1 of tail_fast_kernel (rotational broadening on the full emulator grid) for a binary's component: writes back
+// the row's pixels [blo, bhi] and ends with a barrier.  win / win_have: the CTA's shared-memory window of the rotation
+// table.  (The kernel's other instantiations keep their own copy: moving theirs into this function cost the 4096- and
+// 8192-sample plain kernels 92 bytes of spills.)
+template <int LOG2N1>
+__device__ __forceinline__ void rot_stage(const TailParams& P, const FastGrid& F, const PointSetup& S, float2* z,
+                                          const ZSmem& zs, const ZSplit& zp, float* gline, const TwTab& tw, float* win,
+                                          int& win_have, float* row, int tid, int blo, int bhi) {
+  constexpr int N1 = 1 << LOG2N1;
+  constexpr bool kSplit = LOG2N1 >= 16;
+  constexpr int LOG2MH = kSplit ? LOG2N1 - 2 : 8;          // complex points per half (split only)
+  const int n = P.n;
+  // the table entries this point can touch: [0, vsini_scale * N1/2 + 3]; staged in shared
+  // memory when they fit (the barrier after the regrid below publishes them)
+  const double xt_max = S.vsini_scale * (double)(N1 >> 1);
+  // (a point whose range is longer keeps its first win_floats/4 intervals there and reads the rest
+  // from the global table)
+  float4* win4 = reinterpret_cast<float4*>(win);
+  const int nwin = (int)fmin(fmin(xt_max + 2.0, (double)(F.win_floats >> 2)), (double)P.ntab);
+  // (the window holds the first intervals of the one table: what an earlier point of this CTA staged stays valid)
+  for (int i = win_have + tid; i < nwin; i += kNT) win4[i] = __ldg(P.sbtab + i);
+  win_have = max(win_have, nwin);
+  const RotHT<2> H{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, 1.0f / (float)(N1 >> 1), P.ntab, RotHT<2>::fix40(S.vsini_scale)};
+  if constexpr (!kSplit) {
+    // regrid fused into the first FFT pass (measured against the separate regrid: tail -5 %)
+    ct_convolve_regrid<LOG2N1 - 1>(z, tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
+    regrid_back(row, zs, F, tid, n, N1, blo, bhi);
+  } else {
+    stage_regrid(S, row, zp, tid, N1, F.f_num, F.f_den, 0, F.f_invden, F.c_native, F.f_incj, F.f_incr);
+    __syncthreads();
+    ct_convolve_split<LOG2MH>(z, reinterpret_cast<float2*>(gline), tw, F.twc, H, tid);
+    regrid_back(row, zp, F, tid, n, N1, blo, bhi);
+  }
+  __syncthreads();
+}
+
 // LOG2N1 <= 15: the whole transform sits in shared memory (3 CTAs/SM up to 2^14).
 // LOG2N1 == 16: split transform, half in shared memory (128 KB), half in the scratch line.
 // POLY: continuum polynomial and / or model output in the final pass (the host picks the instantiation).
 // STARS: a context of several stars (obs_lo / obs_hi).
 // TGT: every point names a target (TailParams::target; STARS is then true): stage 1 runs once on the row, then stage 2
 // and the final pass once per member against that member's record, and lnL is the members' chi2 summed in member order.
+// BIN: every point is a binary (TailParams::binary; POLY and STARS are then true): component 1's record and row, stage 1,
+// stage 2 and a final pass that keeps a_1; then component 2's, whose final pass combines the two (final_pass_bin).
 // (3 CTAs/SM, 80 registers with a few spills, measured at C2 0.76 ms against 0.84 ms with 2 CTAs/SM and no spills)
-template <int LOG2N1, bool POLY, bool STARS, bool TGT = false>
+template <int LOG2N1, bool POLY, bool STARS, bool TGT = false, bool BIN = false>
 __global__ void __launch_bounds__(kNT, LOG2N1 <= 14 ? 3 : 1)
 tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -459,6 +634,53 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
     if constexpr (TGT) {
       tu = *reinterpret_cast<const int2*>(&red[1]);
       __syncthreads();                                    // red[1] is read everywhere before a member's reduction
+    }
+    if constexpr (BIN) {
+      // component c: record c * B + p, row c * B + p
+      double acc = 0.0;
+      bool bad = false;
+      for (int c = 0; c < 2; ++c) {
+        float* rowc = row + (long long)c * P.B * P.ldf;
+        if (c == 1) {
+          __syncthreads();                                // component 1's record and transform buffer are free
+          if (tid < (int)(sizeof(FastPoint) / 16))
+            reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(points + P.B + p) + tid);
+          __syncthreads();
+        }
+        if (S.bad) {                                      // NaN a_c: the model and lnL of the point are NaN
+          bad = true;
+          double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+          for (int j = tid; j < FS.obs.n; j += kNT) {
+            if (c == 0) scr[j] = nan;
+            if (P.comp_out) P.comp_out[((long long)p * 2 + c) * P.ld_flux + j] = nan;
+            if (c == 1 && P.model_out) P.model_out[(long long)p * P.ld_flux + j] = nan;
+          }
+          continue;
+        }
+        if (S.do_rot) {
+          const int blo = S.use_inst ? max(S.i0 - 1, 0) : 0;
+          const int bhi = S.use_inst ? min(S.i1 + 1, P.n - 1) : P.n - 1;
+          rot_stage<LOG2N1>(P, F, S, z, zs, zp, gline, tw, win, win_have, rowc, tid, blo, bhi);
+        }
+        if (c == 0) point_chi2<LOG2N1, true, true, 1>(P, F, S, FS, z, zs, zp, gline, tw, rowc, tid, p, 0);
+        else acc = point_chi2<LOG2N1, true, true, 2>(P, F, S, FS, z, zs, zp, gline, tw, rowc, tid, p, 0);
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+      if ((tid & 31) == 0) red[tid >> 5] = acc;
+      __syncthreads();
+      if (tid == 0 && P.lnl) {
+        double c2 = 0.0;
+#pragma unroll
+        for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
+        store_lnl(P, p, bad ? nan : -0.5 * c2);
+      }
+      if (P.discard_rows) {
+        discard_lines(row, P.n, tid);
+        discard_lines(row + (long long)P.B * P.ldf, P.n, tid);
+      }
+      __syncthreads();
+      continue;
     }
     if (TGT ? K == 0 : S.bad) {
       if (P.model_out)
@@ -629,6 +851,33 @@ tail_setup_targets_kernel(const __grid_constant__ TailParams P, const __grid_con
   FastPoint* out = reinterpret_cast<FastPoint*>(F.points) + i;
   out->S = S;
   out->FS = FS;
+}
+
+// Binaries: one thread per (point, component) item, item i = c * B + p: component c's record i (the secondary's
+// labels, Vrad and Vrot through P.binary) and, from component 1's thread, the point's Teff_1, Teff_2 and Rratio.
+template <int kUnused = 0>
+__global__ void __launch_bounds__(64)
+tail_setup_binary_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= 2LL * P.B) return;
+  if (i == 0 && F.work_counter) *F.work_counter = F.work_start;
+  const int c = (int)(i / P.B), p = (int)(i - (long long)c * P.B);
+  const double* th = P.theta + (long long)p * P.ld;
+  const int k = star_of(P.star, P.n_stars, p);
+  PointSetup S{};
+  FastSetup FS{};
+  tail_setup_star(P, th, k, S, FS.obs, c ? P.binary : nullptr);
+  if (!S.bad && S.use_inst) stage2_setup(F, S, FS);
+  FastPoint* out = reinterpret_cast<FastPoint*>(F.points) + i;
+  out->S = S;
+  out->FS = FS;
+  if (c == 0) {
+    const double t1 = get_par(P, th, PAYNE_P_TEFF, k);
+    const PayneBinary& b = *P.binary;
+    P.bin_par[3LL * p] = t1;
+    P.bin_par[3LL * p + 1] = secondary_of(&b, th, PAYNE_P_TEFF, t1);
+    P.bin_par[3LL * p + 2] = b.rratio_col >= 0 ? th[b.rratio_col] : b.rratio_fixed;
+  }
 }
 
 }  // namespace payne

@@ -17,6 +17,8 @@ Consecutive stars of a set may form a *target* (``targets=[...]``): one physical
 emulator row and one rotation stage, then once per spectrum (member): Doppler shift, instrumental stage (scalar R or
 the member's LSF vector), resampling, continuum and chi2.
 
+``binary=True`` models every spectrum as a double-lined binary: the flux-weighted sum of two stars (``set_binary``).
+
 A fixed ``Inst_R`` that is a 1-D array is an LSF vector, the dispersion (AA) at every observed pixel,
 as in the reference (genmod.py:82-85 passes a non-float inst_R on to getspec's LSF branch,
 predictspec.py:265-286).
@@ -46,6 +48,29 @@ def _pf(a):
 
 def _pd(a):
     return a.ctypes.data_as(C.POINTER(C.c_double))
+
+
+# the secondary's own parameters of a binary (``Engine(binary=True)``) and the primary's parameter each one replaces
+# (names ending in ``_<digit>`` already mean "spectrum s" in the multi-spectrum fit)
+BINARY_PARS = {'Teff_sec': 'Teff', 'log(g)_sec': 'log(g)', '[Fe/H]_sec': '[Fe/H]', '[a/Fe]_sec': '[a/Fe]',
+               'Vmic_sec': 'Vmic', 'Vrad_sec': 'Vrad', 'Vrot_sec': 'Vrot'}
+
+
+def _binary(fitpars_i, fixedpars):
+    """PayneBinary (include/payne_b200.h): each secondary parameter and ``Rratio`` from its column in ``fitpars_i`` or
+    its value in ``fixedpars``; a secondary parameter in neither is the primary's."""
+    b = _lib.PayneBinary()
+    for k in range(_lib.NPAR):
+        b.col[k], b.fixed[k] = -1, np.nan
+    for name, base in BINARY_PARS.items():
+        k = PAR_INDEX[base]
+        if name in fitpars_i:
+            b.col[k] = fitpars_i.index(name)
+        elif name in fixedpars:
+            b.fixed[k] = float(fixedpars[name])
+    b.rratio_col = fitpars_i.index('Rratio') if 'Rratio' in fitpars_i else -1
+    b.rratio_fixed = float(fixedpars.get('Rratio', np.nan)) if b.rratio_col < 0 else np.nan
+    return b
 
 
 def _split_fixed(fixedpars):
@@ -120,7 +145,7 @@ def _specnet_struct(spec, keep):
 class Engine:
     def __init__(self, spec=None, phot=None, obs_wave=None, obs_flux=None, obs_eflux=None,
                  obs_phot=None, fitpars_i=(), fixedpars=None, runbools=(True, False, False, False, False),
-                 precision='parity', device=None, stars=None, targets=None):
+                 precision='parity', device=None, stars=None, targets=None, binary=False):
         """``stars``: instead of ``obs_wave``, ``obs_flux``, ``obs_eflux`` and ``obs_phot``, a list of
         ``{'wave', 'flux', 'eflux', 'phot': {band: (mag, err)}}``, one per star; ``lnlike_batch`` and
         ``model_batch`` then take the star index of every row.  A star may also carry
@@ -136,7 +161,11 @@ class Engine:
 
         ``targets``: member counts [n_0, n_1, ...] summing to the number of stars; target t is the next n_t stars
         (see ``set_targets``).  Targets work with LSF vectors too: every star then carries its fixed ``Inst_R`` vector
-        and none has an ``Inst_R`` column."""
+        and none has an ``Inst_R`` column.
+
+        ``binary``: every spectrum is a double-lined binary, read from ``fitpars_i`` / ``fixedpars`` under the names
+        ``Teff_sec``, ``log(g)_sec``, ``[Fe/H]_sec``, ``[a/Fe]_sec``, ``Vmic_sec``, ``Vrad_sec``, ``Vrot_sec`` and
+        ``Rratio`` (see ``set_binary``)."""
         if stars is None:
             stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot}]
         elif any(v is not None for v in (obs_wave, obs_flux, obs_eflux, obs_phot)):
@@ -259,6 +288,9 @@ class Engine:
         self.n_targets = 0
         if targets is not None:
             self.set_targets(targets)
+        self.binary = False
+        if binary:
+            self.set_binary()
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -320,6 +352,69 @@ class Engine:
         # a target's model row: its members' pixels back to back
         self.target_n_obs = [sum(self.n_obs_star[k] for k in m) for m in self.target_members]
         self.target_kmax = max(counts)
+
+    def set_binary(self, on=True, fitpars_i=None, fixedpars=None):
+        """Model every spectrum as a double-lined binary: (a_1 + k a_2) / (1 + k) times the continuum, a_c the
+        spectrum of component c before the continuum and k = Rratio^2 B(lambda, Teff_1) / B(lambda, Teff_2) the
+        blackbody flux ratio (include/payne_b200.h, PayneBinary).  The secondary's parameters and ``Rratio`` come from
+        ``fitpars_i`` / ``fixedpars`` (default: the engine's) under the names of ``BINARY_PARS`` and ``Rratio``; a
+        secondary parameter in neither is the primary's.  ``Inst_R`` and the continuum are shared.  ``on=False``
+        removes it.  Photometry, LSF vectors, targets, per-star layouts and grids without the fast tail are refused."""
+        if not on:
+            _lib.check(self.lib.payne_ctx_set_binary(self._ctx, None))
+            self.binary = False
+            return
+        b = _binary(list(self.fitpars_i if fitpars_i is None else fitpars_i),
+                    dict(self.fixedpars if fixedpars is None else fixedpars))
+        _lib.check(self.lib.payne_ctx_set_binary(self._ctx, C.byref(b)))
+        self.binary = True
+
+    def lnlike_batch_binary(self, theta, star=None):
+        """lnL of every row as a binary, ``theta`` and ``star`` as in ``lnlike_batch`` (None: star 0)."""
+        if isinstance(theta, torch.Tensor) and theta.is_cuda:
+            th = self._theta_dev(theta)
+            sv = self._star_dev(star, th.shape[0], th.device)
+            out = torch.empty(th.shape[0], dtype=torch.float64, device=th.device)
+            st = torch.cuda.current_stream(th.device).cuda_stream
+            _lib.check(self.lib.payne_lnlike_batch_binary(self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None,
+                                                          th.shape[0], th.shape[1], out.data_ptr(), st))
+            return out
+        th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
+        if th.ndim != 2 or th.shape[1] != self.ndim:
+            raise ValueError('theta must be [B, %d]' % self.ndim)
+        sv = None
+        if star is not None:
+            if isinstance(star, torch.Tensor):
+                star = star.cpu().numpy()
+            sv = np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind'))
+            if sv.shape != (th.shape[0],):
+                raise ValueError('star must be [%d]' % th.shape[0])
+        out = np.empty(th.shape[0], dtype=np.float64)
+        _lib.check(self.lib.payne_lnlike_batch_binary_host(self._ctx, th.ctypes.data,
+                                                           sv.ctypes.data if sv is not None else None,
+                                                           th.shape[0], th.shape[1], out.ctypes.data))
+        return out
+
+    def model_batch_binary(self, theta, star=None, want_flux=True, want_comp=True):
+        """Model spectra [B, n_obs], the components' spectra before the continuum [B, 2, n_obs] and lnL [B] of every
+        row as a binary, as CUDA float64 tensors (the pixels beyond a row's star stay NaN)."""
+        dev = torch.device('cuda', self.device)
+        if not isinstance(theta, torch.Tensor):
+            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
+        th = self._theta_dev(theta.to(dev))
+        B = th.shape[0]
+        if star is not None and not isinstance(star, torch.Tensor):
+            star = torch.from_numpy(np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind')))
+        sv = self._star_dev(star.to(dev) if star is not None else None, B, dev)
+        flux = torch.full((B, self.n_obs), float('nan'), dtype=torch.float64, device=dev) if want_flux else None
+        comp = torch.full((B, 2, self.n_obs), float('nan'), dtype=torch.float64, device=dev) if want_comp else None
+        lnl = torch.empty(B, dtype=torch.float64, device=dev)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(self.lib.payne_model_batch_binary(
+            self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None, B, th.shape[1],
+            flux.data_ptr() if flux is not None else None, self.n_obs,
+            comp.data_ptr() if comp is not None else None, lnl.data_ptr(), st))
+        return flux, comp, lnl
 
     def lnlike_batch_targets(self, theta, target):
         """lnL of every row against its target: ``target`` [B], as ``star`` in ``lnlike_batch`` (int32 CUDA tensor

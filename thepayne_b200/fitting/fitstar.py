@@ -22,7 +22,11 @@ What differs, on purpose:
     continuum coefficients ``pc_<s>_<k>``, whose priors come from ``priordict['Inst_R_<s>']`` and
     ``priordict['blaze_coeff_<s>']`` (``multispec.MultiSpecLikelihood``).  ``priordict['Inst_R_<s>'] = {'fixed': lsf}``
     with a 1-D ``lsf`` (one dispersion per fitted pixel of spectrum s, for every s) fits with LSF vectors; the output
-    file then has no column for them.
+    file then has no column for them;
+  * ``inputdict['binary'] = True`` with a single ``spec`` fits a double-lined binary (``binary.BinaryLikelihood``): the
+    secondary's ``Teff_sec``, ``log(g)_sec``, ``Vrad_sec`` and ``Vrot_sec`` and the radius ratio ``Rratio`` follow the
+    reference parameters (before ``pc_k``); ``[Fe/H]_sec``, ``[a/Fe]_sec`` and ``Vmic_sec`` get a column only when
+    ``priordict`` names them, and are the primary's otherwise.  ``{'fixed': v}`` fixes any of them.
 """
 from __future__ import annotations
 
@@ -37,6 +41,9 @@ from .nested import BatchedNestedSampler
 
 _ALLPARS = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot', 'Vmic', 'Inst_R', 'log(R)', 'Dist', 'log(A)',
             'Av', 'Rv', 'CarbonScale']
+# a binary's own parameters in sampler order; those outside _BINARY_ON only when priordict names them
+_BINARY = ['Teff_sec', 'log(g)_sec', '[Fe/H]_sec', '[a/Fe]_sec', 'Vrad_sec', 'Vrot_sec', 'Vmic_sec', 'Rratio']
+_BINARY_ON = ['Teff_sec', 'log(g)_sec', 'Vrad_sec', 'Vrot_sec', 'Rratio']
 
 
 class FitPayne(object):
@@ -67,6 +74,11 @@ class FitPayne(object):
         self.fitpars = list(_ALLPARS)
         self.fitpars_bool = {pp: False for pp in self.fitpars}
 
+        self.binary_bool = bool(inputdict.get('binary', False))
+        if self.binary_bool and isinstance(inputdict.get('spec'), (list, tuple)):
+            raise NotImplementedError('binary with several spectra (a list-valued spec)')
+        if self.binary_bool and 'phot' in inputdict:
+            raise NotImplementedError('binary with photometry: the SED of two stars is not modelled')
         if isinstance(inputdict.get('spec'), (list, tuple)):
             self._setup_spectra(inputdict)
         elif 'spec' in inputdict:                                          # fitstar.py:70-154
@@ -118,6 +130,16 @@ class FitPayne(object):
                 self.fitpars_bool['Dist'] = True
             if inputdict.get('Rvfree', False):
                 raise NotImplementedError('Rvfree: the likelihood never forwards Rv (likelihood.py:103-106)')
+
+        if self.binary_bool:
+            if not self.spec_bool:
+                raise ValueError("binary needs inputdict['spec']")
+            names = [pp for pp in _BINARY if pp in _BINARY_ON or pp in self.priordict]
+            at = next((i for i, pp in enumerate(self.fitpars) if pp.startswith('pc_')), len(self.fitpars))
+            self.fitpars[at:at] = names
+            for pp in names:
+                self.fitpars_bool[pp] = True
+            fa['binary'] = True
 
         fa['fixedpars'] = {}                                               # fitstar.py:193-198
         for kk in self.priordict.keys():
@@ -184,6 +206,8 @@ class FitPayne(object):
         like = self.likelihood
         if 'spectra' in fitargs:
             from .multispec import MultiSpecLikelihood as like
+        elif fitargs.get('binary', False):
+            from .binary import BinaryLikelihood as like
         self.likeobj = like(fitargs, fitpars, runbools, verbose=False, precision=getattr(self, 'precision', 'parity'),
                             device=getattr(self, 'device', None))
         self._check_sampler(indicts)

@@ -285,6 +285,8 @@ class FitPayneMany(object):
         for d in inputdicts:
             if isinstance(d.get('spec'), (list, tuple)):
                 raise NotImplementedError('FitPayneMany with several spectra per star (a list-valued spec)')
+            if d.get('binary', False):
+                raise NotImplementedError('FitPayneMany with binaries: fit each binary with FitPayne')
             f = FitPayne()
             ind = f._setup(inputdict=d, verbose=verbose)
             f._prepare(ind)

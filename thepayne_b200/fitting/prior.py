@@ -13,6 +13,9 @@ proposal queue (scipy's ppf functions are vectorised), so the sampler side keeps
 
 Several spectra (``FitPayne`` with a list-valued ``spec``): ``Inst_R_<s>`` takes the priors and default range of
 ``Inst_R``, and ``pc_<s>_<k>`` those of ``pc_k`` with ``blaze_coeff_<s>`` in place of ``blaze_coeff``.
+
+Binaries (``FitPayne`` with ``'binary': True``): ``<name>_sec`` takes the default range of ``<name>`` (``Vmic_sec``: none,
+like ``Vmic``), and ``Rratio`` defaults to uniform [0, 1].
 """
 from __future__ import annotations
 
@@ -22,6 +25,7 @@ import numpy as np
 from scipy.stats import expon, norm, truncexpon, truncnorm
 
 _SPEC = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot', 'Inst_R', 'CarbonScale']
+_BINARY = [p + '_sec' for p in _SPEC[:6]] + ['Vmic_sec', 'Rratio']
 _ISO = ['log(A)', 'log(R)', 'Av', 'Rv', 'Dist']
 _SPECTRUM = re.compile(r'(Inst_R|pc)_(\d+)(?:_(\d+))?$')     # Inst_R_<s>, pc_<s>_<k>
 _PV = {'pv_uniform': 'uniform', 'pv_gaussian': 'gaussian', 'pv_tgaussian': 'tgaussian', 'pv_exp': 'exp',
@@ -58,7 +62,8 @@ class prior(object):
             'Teff': [3000.0, 17000.0], 'log(g)': [-1.0, 5.5], '[Fe/H]': [-4.0, 0.5], '[a/Fe]': [-0.2, 0.6],
             'Vrad': [-700.0, 700.0], 'Vrot': [0, 300.0], 'Inst_R': [10000.0, 60000.0], 'log(A)': [-3.0, 7.0],
             'log(R)': [-2.0, 3.0], 'Dist': [0.0, 100000.0], 'Av': [0.0, 5.0], 'Rv': [2.0, 5.0],
-            'CarbonScale': [0.0, 2.0]}
+            'CarbonScale': [0.0, 2.0], 'Rratio': [0.0, 1.0]}
+        self.defaultpars.update({p + '_sec': self.defaultpars[p] for p in _SPEC[:6]})
 
     # ------------------------------------------------------------------ unit cube -> parameters
     def _transform(self, name, u, iso):
@@ -107,7 +112,7 @@ class prior(object):
             pcmax = self.polycoefarr[k][0] + 5.0 * self.polycoefarr[k][1]
             pcmin = self.polycoefarr[k][0] - 5.0 * self.polycoefarr[k][1]
             return (pcmax - pcmin) * u + pcmin
-        if self.spec_bool and name in _SPEC:
+        if self.spec_bool and (name in _SPEC or name in _BINARY):
             return self._transform(name, u, iso=False)
         if self.phot_bool and (name in _ISO or (not self.spec_bool and name in _SPEC[:4])):
             return self._transform(name, u, iso=name in _ISO)
@@ -129,7 +134,7 @@ class prior(object):
             return out
         groups = []
         if self.spec_bool:
-            groups.append(_SPEC + [p for p in self.fitpars_i if p.startswith('Inst_R_')])
+            groups.append(_SPEC + _BINARY + [p for p in self.fitpars_i if p.startswith('Inst_R_')])
         if self.phot_bool:
             g = [] if self.spec_bool else ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]']
             g += [p for p in ['log(R)', 'Dist', 'log(A)', 'Av'] if p in self.fitpars_i]
