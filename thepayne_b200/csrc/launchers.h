@@ -11,6 +11,12 @@
 
 namespace payne {
 
+// cudaFuncAttributeMaxDynamicSharedMemorySize of `func` on the current device, raised to at least `bytes` and never
+// lowered (tail_general_tu.cu).  The attribute belongs to the function on the device, not to a context: contexts that
+// share one instantiation at different sizes (LSF, photometry and general tails) must not cap each other's launches.
+// A high-water mark per (function, device) behind a mutex; only a successful call raises it.
+cudaError_t raise_max_dyn_smem(const void* func, size_t bytes);
+
 // ---- gemm_tu.cu: lin2..lin6 on tcgen05 (mlp_tc.cuh)
 int tc_prepare_weights_x(TcWeights* w, const float* W_host, int N, int K, std::vector<void*>* owned);
 int tc_alloc_acts_x(TcActs* a, long long rows, long long ld);

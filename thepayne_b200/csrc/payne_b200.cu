@@ -732,8 +732,8 @@ int build_phot(PayneCtx* c, const PaynePhotNet* p, const PayneObs* obs, const Pa
     c->phot_smem += (size_t)kPhotTile * nb * sizeof(double);     // per-slot terms
   }
   if (c->phot_smem > 200 * 1024) return fail(PAYNE_E_UNSUPPORTED, "photometry hidden width too large");
-  CU_TRY(cudaFuncSetAttribute(any_band ? payne::phot_kernel<true> : payne::phot_kernel<false>,
-                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->phot_smem));
+  CU_TRY(payne::raise_max_dyn_smem(any_band ? (const void*)payne::phot_kernel<true> : (const void*)payne::phot_kernel<false>,
+                                    c->phot_smem));
   return PAYNE_OK;
 }
 

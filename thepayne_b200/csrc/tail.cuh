@@ -157,6 +157,21 @@ __device__ __forceinline__ double get_par(const TailParams& P, const double* th,
 // float index of real sample k: 2*swz(k>>1) + (k&1) == k ^ (((k>>5)&7)<<2)
 __device__ __forceinline__ int zidx(int k) { return k ^ (((k >> 5) & 7) << 2); }
 
+// np.interp between (wa, a) and (wb, b), wa <= x <= wb, as numpy's compiled_interp has it: an exact hit returns its
+// value (also beside a NaN neighbour, e.g. where a continuum emulator's NaN ends meet the grid), else
+// slope * (x - wa) + a, with its fallbacks for NaN / inf neighbours
+__device__ __forceinline__ double np_interp_pair(double x, double wa, double wb, double a, double b) {
+  if (x == wa) return a;
+  if (x == wb) return b;
+  const double slope = (b - a) / (wb - wa);
+  double r = slope * (x - wa) + a;
+  if (r != r) {
+    r = slope * (x - wb) + b;
+    if (r != r && a == b) r = a;
+  }
+  return r;
+}
+
 // largest j in [lo, hi] with w[j]*D <= x, assuming w[lo]*D <= x; starts from a guess.
 __device__ __forceinline__ int locate(const double* __restrict__ w, double D, double x, int guess,
                                       int lo, int hi) {

@@ -373,7 +373,7 @@ __device__ __forceinline__ double plain_pass_bin(const TailParams& P, const Poin
       const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
       const double va = (double)depth_of(row[jj], true, false);
       const double vb = (double)depth_of(row[jj + 1], true, false);
-      a = 1.0 + ((vb - va) / (wb - wa) * (x - wa) + va);
+      a = 1.0 + np_interp_pair(x, wa, wb, va, vb);
     }
     if constexpr (BM == 1) {
       scr[j - off] = a;
@@ -514,7 +514,7 @@ __device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid
         const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
         const double a = (double)depth_of(row[jj], is_depth, false);
         const double b = (double)depth_of(row[jj + 1], is_depth, false);
-        m = 1.0 + ((b - a) / (wb - wa) * (x - wa) + a);
+        m = 1.0 + np_interp_pair(x, wa, wb, a, b);
       }
       if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
       if (P.model_out) P.model_out[(long long)p * P.ld_flux + moff + (j - off)] = m;

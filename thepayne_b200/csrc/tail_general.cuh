@@ -131,7 +131,7 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
           const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
           const double a = (double)depth_of(row[jj], is_depth, false);
           const double b = (double)depth_of(row[jj + 1], is_depth, false);
-          m = 1.0 + ((b - a) / (wb - wa) * (x - wa) + a);
+          m = 1.0 + np_interp_pair(x, wa, wb, a, b);
         }
         if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
         if (P.model_out) P.model_out[(long long)p * P.ld_flux + (j - off)] = m;

@@ -1,9 +1,28 @@
 // Translation unit of the general-grid fused tail (tail_general.cuh), the LSF-vector tail (tail_lsf.cuh) and
-// the continuum-emulator multiply (continuum.cuh) and the unit-test hook of the runtime-planned FFT (fft.cuh);
+// the continuum-emulator multiply (continuum.cuh), the unit-test hook of the runtime-planned FFT (fft.cuh) and the
+// dynamic shared-memory opt-in helper raise_max_dyn_smem;
 // see launchers.h.
+#include <map>
+#include <mutex>
+#include <utility>
+
 #include "launchers.h"
 
 namespace payne {
+
+cudaError_t raise_max_dyn_smem(const void* func, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> mark;
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& m = mark[std::make_pair(func, dev)];
+  if (bytes <= m) return cudaSuccess;
+  e = cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess) m = bytes;
+  return e;
+}
 
 #define PAYNE_GEN_SIZES(X) X(10) X(11) X(12) X(13) X(14) X(15)
 
@@ -12,7 +31,7 @@ bool probe_tail_general(int l2, size_t bytes, int* occ) {
   switch (l2 < 10 ? 10 : l2) {
 #define X(L)                                                                                                      \
     case L:                                                                                                       \
-      e1 = cudaFuncSetAttribute(tail_general_kernel<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); \
+      e1 = raise_max_dyn_smem((const void*)tail_general_kernel<L>, bytes);                                        \
       e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, tail_general_kernel<L>, kTailThreads, bytes);       \
       break;
     PAYNE_GEN_SIZES(X)
@@ -35,7 +54,7 @@ int launch_tail_general(int l2, int grid, size_t smem, cudaStream_t st, const Ta
 
 template <bool TGT>
 static bool probe_lsf(size_t bytes, int* occ) {
-  if (cudaFuncSetAttribute(tail_lsf_kernel<TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess ||
+  if (raise_max_dyn_smem((const void*)tail_lsf_kernel<TGT>, bytes) != cudaSuccess ||
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, tail_lsf_kernel<TGT>, kTailThreads, bytes) != cudaSuccess) {
     cudaGetLastError();
     return false;

@@ -14,7 +14,8 @@
 //   outspec = np.interp(outwave, lam, spec_conv)          (edges clamp, no NaN)           :584
 // One CTA per point; the cumulative sum is a block scan, the median an exact radix selection
 // (continuum.cuh), the three np.interp are bisections with numpy's slope formula, and the convolution is
-// the runtime-planned in-shared-memory FFT of fft.cuh on the line depth.  Wavelength arithmetic is fp64.
+// the runtime-planned in-shared-memory FFT of fft.cuh on the line depth (nx = 2 .. 16, below its smallest plan: a
+// direct circular convolution, lsf_small_conv; nx = 1 is NaN).  Wavelength arithmetic is fp64.
 #pragma once
 #include "continuum.cuh"
 #include "tail.cuh"
@@ -60,6 +61,29 @@ __device__ __forceinline__ double np_interp(double x, const XF& xp, const FF& fp
     if (r != r && f0 == f1) r = f0;
   }
   return r;
+}
+
+// irfft(rfft(x) * exp(-2 pi^2 xps^2 k^2)) of the nx < 32 samples zf[zidx(0 .. nx)], below the smallest plan of the
+// runtime FFT: the same transfer function as a direct circular convolution in fp64 with its impulse response
+// h[m] = (T_0 + 2 sum_{0<k<nx/2} T_k cos(2 pi k m / nx) + T_{nx/2} cos(pi m)) / nx (the Nyquist term real, as irfft
+// takes it).  h goes to hbuf[0, nx); all threads call it, and the result is in zf when it returns.
+__device__ __forceinline__ void lsf_small_conv(float* zf, int nx, double xps, double* hbuf, int tid) {
+  const double a = 2.0 * CUDART_PI * CUDART_PI * xps * xps;
+  if (tid < nx) {
+    double h = 0.0;
+    for (int k = 0; k <= nx / 2; ++k) {
+      const double t = exp(-a * (double)k * (double)k);
+      h += ((k == 0 || 2 * k == nx) ? 1.0 : 2.0) * t * cospi((double)((2 * k * tid) % (2 * nx)) / (double)nx);
+    }
+    hbuf[tid] = h / (double)nx;
+  }
+  __syncthreads();
+  double y = 0.0;
+  if (tid < nx)
+    for (int j = 0; j < nx; ++j) y += (double)zf[zidx(j)] * hbuf[(tid - j) & (nx - 1)];
+  __syncthreads();
+  if (tid < nx) zf[zidx(tid)] = (float)y;
+  __syncthreads();
 }
 
 // Emulator pixels [i0, i1] inside the LSF mask of star st at Doppler factor D (thread 0; i1 < i0: none).
@@ -218,7 +242,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
       const double xps = nanmedian_dev([auxc](int j) { return auxc[j]; }, nM, hist, &sh_prefix, &sh_rank, &sh_count);
       const double Nf = 2.0 / xps;                                    // pix_per_sigma = 2
       const int log2nx = (Nf == Nf && Nf > 0.0 && Nf < 1e9) ? (int)ceil(log2(Nf)) : -1;
-      if (log2nx < 5 || log2nx > L.log2nx_max) {
+      if (log2nx < 1 || log2nx > L.log2nx_max) {               // nx = 1: the reference's irfft raises (DESIGN §5)
         if (tid == 0) { if (log2nx > L.log2nx_max) atomicOr(P.status, 1); if (P.lnl) P.lnl[p] = nan; }
         if (P.model_out)
           for (int j = tid; j < no; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
@@ -241,7 +265,9 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
         }
       }
       __syncthreads();
-      {
+      if (log2nx < 5) {
+        lsf_small_conv(zf, nx, xps, part, tid);
+      } else {
         const int log2M = log2nx - 1;
         const float a = (float)(2.0 * CUDART_PI * CUDART_PI * xps * xps);   // ss = rfftfreq(nx, 1/nx) = k
         GaussH H{a, 1.0f / (float)(1 << log2M)};
@@ -361,7 +387,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
       const double xps = nanmedian_dev([auxc](int j) { return auxc[j]; }, nM, hist, &sh_prefix, &sh_rank, &sh_count);
       const double Nf = 2.0 / xps;                                    // pix_per_sigma = 2
       const int log2nx = (Nf == Nf && Nf > 0.0 && Nf < 1e9) ? (int)ceil(log2(Nf)) : -1;
-      if (log2nx < 5 || log2nx > L.log2nx_max) {
+      if (log2nx < 1 || log2nx > L.log2nx_max) {               // nx = 1: the reference's irfft raises (DESIGN §5)
         if (tid == 0 && log2nx > L.log2nx_max) atomicOr(P.status, 1);
         if (mrow)
           for (int j = tid; j < no; j += kTailThreads) mrow[j] = nan;
@@ -383,7 +409,9 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
         }
       }
       __syncthreads();
-      {
+      if (log2nx < 5) {
+        lsf_small_conv(zf, nx, xps, part, tid);
+      } else {
         const int log2M = log2nx - 1;
         const float a = (float)(2.0 * CUDART_PI * CUDART_PI * xps * xps);   // ss = rfftfreq(nx, 1/nx) = k
         GaussH H{a, 1.0f / (float)(1 << log2M)};
