@@ -301,6 +301,47 @@ int payne_lnlike_batch_binary_host(PayneCtx* ctx, const double* theta_host, cons
 int payne_model_batch_binary(PayneCtx* ctx, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
                              double* flux_dev, int64_t ld_flux, double* comp_dev, double* lnl_dev, void* stream);
 
+/* Continuum marginalisation: the Chebyshev continuum of a star's model, m_j = a_j * sum_k c_k T_k(x_j), is linear in
+ * its K coefficients, so chi2 is an exact quadratic in c and the coefficients can be integrated out per point instead
+ * of being sampled (K fewer dimensions for the sampler per spectrum).  Per star with the setting, over its pixels j:
+ *   a_j     the model before the continuum (1 + depth after rotation, Doppler shift, instrumental stage or plain
+ *           interpolation, resampling; NaN where the sampled model is NaN); x_j its Chebyshev abscissa;
+ *   b_jk    = a_j T_k(x_j) / sigma_j,  y_j = flux_j / sigma_j;
+ *   G       = sum_j b_j b_j^T = L L^T (Cholesky),  h = sum_j b_j y_j,  c-hat = G^-1 h, all in fp64;
+ *   Q       = chi2 at c-hat, with the bits of -2 lnL of a context that samples pc_0 .. pc_{K-1} (no photometry) at
+ *           theta with c-hat appended;
+ *   M       = -sum_k ln L_kk + sum_k (ln(2 pi) / 2 - ln(hi_k - lo_k));
+ *   lnL     = -0.5 (Q + chi2_sed) + M, the log of the integral of exp(-chi2(c) / 2) prod_k dc_k / (hi_k - lo_k) over R^K
+ *           (equal to the box integral when the box holds the coefficients' conditional posterior; not truncated).
+ * A target (payne_ctx_set_targets) of n members: lnL = -0.5 ((((Q_0 + Q_1) + ...) + Q_{n-1}) + chi2_sed) +
+ * ((M_0 + M_1) + ...) + M_{n-1}.  Any NaN a_j makes lnL NaN.  A finite G with a pivot at or below 1e-10 of its
+ * diagonal entry (fewer usable pixels than K, all a_j zero) makes lnL, c-hat, Q and the model NaN and sets status bit 3.
+ * While the setting is on, every likelihood and model entry (plain, _stars, _targets, their _host twins) returns this
+ * lnL and the model at c-hat. */
+typedef struct {
+  int32_t n_coef;                /* K in [1, PAYNE_MAX_POLY]; 0: the star has no setting */
+  double lo[PAYNE_MAX_POLY];     /* the coefficients' box: its widths enter M */
+  double hi[PAYNE_MAX_POLY];
+} PayneContMarg;
+
+/* per_star [n_stars] (HOST, copied); NULL removes the setting.  PAYNE_E_INVALID: a star with the setting whose layout
+ * also samples pc_k (modpoly_bool with n_poly > 0), n_coef outside [0, PAYNE_MAX_POLY] or 0 for every star, a
+ * non-finite box or lo >= hi.  PAYNE_E_UNSUPPORTED: some stars with the setting and others without, LSF vectors, a
+ * binary, an attached continuum emulator, a grid without the fast tail, the fused gather.  Every entry checks these
+ * rules again (the context may change in between).  Transforms of 65536 samples run on the single-CTA kernel. */
+int payne_ctx_set_cont_marg(PayneCtx* ctx, const PayneContMarg* per_star);
+/* Per point p (all outputs device pointers, any may be NULL): coef_dev[p, :K] c-hat, chol_dev[p, :K(K+1)/2] L as packed
+ * lower triangle (row by row: L00, L10, L11, L20, ...), chi2_dev[p] Q, lnl_dev[p] lnL.  ld_coef >= the largest K,
+ * ld_chol >= the largest K(K+1)/2.  star_dev as in the _stars entries. */
+int payne_cont_batch_stars(PayneCtx* ctx, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                           double* coef_dev, int64_t ld_coef, double* chol_dev, int64_t ld_chol,
+                           double* chi2_dev, double* lnl_dev, void* stream);
+/* The same for targets: the members' c-hat and L lie back to back in member order (ld_coef >= the largest sum of the
+ * members' K, ld_chol likewise), chi2_dev[p, m] = Q_m (ld_chi2 >= the largest member count). */
+int payne_cont_batch_targets(PayneCtx* ctx, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
+                             double* coef_dev, int64_t ld_coef, double* chol_dev, int64_t ld_chol,
+                             double* chi2_dev, int64_t ld_chi2, double* lnl_dev, void* stream);
+
 /* Continuum emulator (HOST pointers, copied): any PayneSpecNet the spectrum emulator could be; its
  * `wavelength` is the continuum's own grid.  From then on every model spectrum is multiplied, right after
  * the emulator and before any broadening, by np.interp(modwave, contwave, c / nanmedian(c), left=nan,
@@ -348,7 +389,8 @@ int payne_gather_flush(PayneCtx* ctx, void* stream, double** gathered_last);
  * "grid_loguniform","fast_tail","max_batch","sm_count","tail_grid","precision","continuum","lsf","legacy_tc"
  * (a leaky-ReLU stack whose output layer runs on the tensor cores),"status"
  * (bit0: a point needed a larger transform than the shared-memory carve-out; bit1: a peer of the gather never arrived;
- * bit2: a point named a star outside [0, n_stars), or a target outside [0, n_targets)).
+ * bit2: a point named a star outside [0, n_stars), or a target outside [0, n_targets); bit3: continuum marginalisation
+ * met a finite Gram matrix with a pivot at or below 1e-10 of its diagonal entry), "cont_marg" (1 while payne_ctx_set_cont_marg is on).
  * Returns the value or -1. */
 int64_t payne_ctx_query(PayneCtx* ctx, const char* key);
 /* Runtime switches: "precision" (PAYNE_PREC_*), "max_batch" (workspace slab, points), "timing" (0/1,

@@ -31,7 +31,8 @@ EXPORTS = ['payne_abi_version', 'payne_last_error', 'payne_ctx_create', 'payne_c
            'payne_ctx_set_targets', 'payne_lnlike_batch_targets', 'payne_lnlike_batch_targets_host',
            'payne_model_batch_targets',
            'payne_ctx_set_binary', 'payne_lnlike_batch_binary', 'payne_lnlike_batch_binary_host',
-           'payne_model_batch_binary']
+           'payne_model_batch_binary',
+           'payne_ctx_set_cont_marg', 'payne_cont_batch_stars', 'payne_cont_batch_targets']
 GATHER_HANDLE_BYTES = 128
 
 _f = C.POINTER(C.c_float)
@@ -70,6 +71,10 @@ class PayneStarOpts(C.Structure):
 class PayneBinary(C.Structure):
     _fields_ = [('col', C.c_int32 * NPAR), ('fixed', C.c_double * NPAR), ('rratio_col', C.c_int32),
                 ('rratio_fixed', C.c_double)]
+
+
+class PayneContMarg(C.Structure):
+    _fields_ = [('n_coef', C.c_int32), ('lo', C.c_double * MAX_POLY), ('hi', C.c_double * MAX_POLY)]
 
 
 class PayneError(RuntimeError):
@@ -128,6 +133,13 @@ def load():
     lib.payne_lnlike_batch_binary_host.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp]
     lib.payne_model_batch_binary.restype = C.c_int
     lib.payne_model_batch_binary.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, vp, vp]
+    lib.payne_ctx_set_cont_marg.restype = C.c_int
+    lib.payne_ctx_set_cont_marg.argtypes = [vp, C.POINTER(PayneContMarg)]
+    lib.payne_cont_batch_stars.restype = C.c_int
+    lib.payne_cont_batch_stars.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, C.c_int64, vp, vp, vp]
+    lib.payne_cont_batch_targets.restype = C.c_int
+    lib.payne_cont_batch_targets.argtypes = [vp, vp, vp, C.c_int64, C.c_int64, vp, C.c_int64, vp, C.c_int64, vp,
+                                             C.c_int64, vp, vp]
     lib.payne_ctx_destroy.restype = None
     lib.payne_ctx_destroy.argtypes = [vp]
     lib.payne_lnlike_batch.restype = C.c_int

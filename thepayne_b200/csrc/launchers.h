@@ -72,6 +72,11 @@ int launch_tail_setup_targets(long long items, cudaStream_t st, const TailParams
 bool probe_tail_fast_binary(int l2, size_t smem_bytes, int* ctas_per_sm);
 int launch_tail_fast_binary(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
 int launch_tail_setup_binary(int nb, cudaStream_t st, const TailParams& T, const FastGrid& F);
+// continuum marginalisation (payne_ctx_set_cont_marg): the MARG instantiations of tail_fast_kernel (tail_fast_poly_tu.cu),
+// for points naming stars and (targets = true) targets; their setup is launch_tail_setup / launch_tail_setup_targets
+bool probe_tail_fast_marg(int l2, size_t smem_bytes, int* ctas_per_sm);
+int launch_tail_fast_marg(int l2, bool targets, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T,
+                          const FastGrid& F);
 
 // ---- tail_cluster_tu.cu: the same tail with one transform spread over a cluster of four CTAs (tail_cluster.cuh;
 // emulator grids above 16384 pixels).  max_clusters = co-resident clusters on the device.

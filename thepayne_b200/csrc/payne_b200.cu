@@ -182,6 +182,7 @@ struct PayneCtx {
   std::string tgt_instr_col;            // the first member with an Inst_R column (refused beside LSF vectors), or empty
   long long tgt_nobs_max = 0;           // the largest sum of the members' n_obs (model row of a target)
   int* tfirst_dev = nullptr;            // [n_targets + 1]
+  std::vector<int> tfirst_h;            // its host copy
   payne::FastPoint* tgt_points = nullptr;   // [tgt_rows * tgt_kmax] per-(point, member) records (fast tail only)
   int* tgt_star = nullptr;              // [tgt_rows] first member's star of every point of a slab
   long long tgt_rows = 0, tgt_rec_alloc = 0;
@@ -192,6 +193,13 @@ struct PayneCtx {
   double* bin_scratch = nullptr;        // [bin_grid, n_obs_max] a_1 of every CTA's current point
   double* bin_par = nullptr;            // [bin_rows, 3] Teff_1, Teff_2, Rratio of the points of a slab
   long long bin_rows = 0;
+  // continuum marginalisation (payne_ctx_set_cont_marg): every star's K and C, the MARG kernels' grid and their scratch
+  bool has_marg = false;
+  std::vector<int> marg_k_h;            // [n_stars] K of every star
+  int* marg_k_dev = nullptr;
+  double* marg_c_dev = nullptr;         // [n_stars] sum_k (ln(2 pi) / 2 - ln w_k)
+  int marg_grid = 0;
+  double* marg_scratch = nullptr;       // [marg_grid, n_obs_max] a_j of every CTA's current point
   // photometry
   bool has_phot = false;
   payne::PhotParams phot{};
@@ -957,11 +965,18 @@ int ensure_binary_workspace(PayneCtx* c, long long rows) {
 // star: [B] star index of every point (null: star 0); flux_out rows are ld_flux apart.  target: see above; chi2_out
 // [B, ld_chi2] the chi2 of every member (targets only).  binary: every point is a binary (payne_ctx_set_binary), the
 // emulator runs 2 nb rows per slab of nb points; comp_out [B, 2, ld_flux] its components' spectra.
+int marg_unsupported(PayneCtx* c);
+
+// coef_out / chol_out (continuum marginalisation, payne_ctx_set_cont_marg): [B, ld_coef] c-hat and [B, ld_chol] the
+// packed Cholesky factor of every point; chi2_out is then every point's Q (ld_chi2 = 1 for points naming stars).
 int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, long long ld, double* flux_out,
               long long ld_flux, double* mags_out, double* lnl, cudaStream_t st, const int* target = nullptr,
-              double* chi2_out = nullptr, long long ld_chi2 = 0, bool binary = false, double* comp_out = nullptr) {
+              double* chi2_out = nullptr, long long ld_chi2 = 0, bool binary = false, double* comp_out = nullptr,
+              double* coef_out = nullptr, long long ld_coef = 0, double* chol_out = nullptr, long long ld_chol = 0) {
   using namespace payne;
   if (B <= 0) return PAYNE_OK;
+  const bool marg = c->has_marg;
+  if (marg) { int rc = marg_unsupported(c); if (rc) return rc; }
   if (ld < c->ndim_max) return fail(PAYNE_E_INVALID, "ld < ndim (the largest star's with per-star layouts)");
   if (!target && flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
   const bool records = target && !c->lsf_on;             // the fast target tail's per-(point, member) records
@@ -1008,6 +1023,12 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         T.binary = c->binary_dev; T.bin_par = c->bin_par; T.bin_scratch = c->bin_scratch; T.bin_ld = c->n_obs_max;
         T.comp_out = comp_out ? comp_out + p0 * 2 * ld_flux : nullptr;
       }
+      if (marg) {
+        T.marg_k = c->marg_k_dev; T.marg_c = c->marg_c_dev; T.bin_scratch = c->marg_scratch; T.bin_ld = c->n_obs_max;
+        T.chi2_out = chi2_out ? chi2_out + p0 * ld_chi2 : nullptr; T.ld_chi2 = ld_chi2;
+        T.coef_out = coef_out ? coef_out + p0 * ld_coef : nullptr; T.ld_coef = ld_coef;
+        T.chol_out = chol_out ? chol_out + p0 * ld_chol : nullptr; T.ld_chol = ld_chol;
+      }
       if (gather_here) {
         // all-gather fused into the tail (tail.cuh store_lnl / gather_exit): this slab's slice of every peer's buffer
         T.g_world = c->g_world; T.g_rank = c->g_rank; T.g_done = c->g_done;
@@ -1021,7 +1042,8 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         // per-point setup depends only on theta: fork it beside the emulator GEMMs, join before the tail
         CU_TRY(cudaEventRecord(c->ev_fork, st));
         CU_TRY(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-        c->fast.work_start = target ? std::min(c->tgt_grid, nb) : binary ? std::min(c->bin_grid, nb)
+        c->fast.work_start = marg ? std::min(c->marg_grid, nb) : target ? std::min(c->tgt_grid, nb)
+                           : binary ? std::min(c->bin_grid, nb)
                            : (c->use_cluster && c->allow_cluster) ? (int)std::min<long long>(c->cluster_n, nb)
                                                                   : std::min(c->tail_grid_fast, nb);
         if (c->grid_cap > 0) c->fast.work_start = std::min(c->fast.work_start, c->grid_cap);
@@ -1034,6 +1056,10 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
           FastGrid FB = c->fast;
           FB.cluster = 0;
           if (payne::launch_tail_setup_binary(nb, c->side, T, FB)) return fail(PAYNE_E_CUDA, "tail_setup launch");
+        } else if (marg) {
+          FastGrid FM = c->fast;
+          FM.cluster = 0;
+          if (payne::launch_tail_setup(nb, c->side, T, FM)) return fail(PAYNE_E_CUDA, "tail_setup launch");
         } else if (payne::launch_tail_setup(nb, c->side, T, c->fast)) {
           return fail(PAYNE_E_CUDA, "tail_setup launch");
         }
@@ -1094,6 +1120,15 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         const int grid = std::min(c->lsf_grid, nb);
         if (target ? payne::launch_tail_lsf_targets(grid, c->lsf_smem, st, TL, c->lsf)
                    : payne::launch_tail_lsf(grid, c->lsf_smem, st, TL, c->lsf))
+          return fail(PAYNE_E_CUDA, "tail launch");
+      } else if (marg) {
+        // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no such form)
+        if (!(fast_tail && is_depth))
+          return fail(PAYNE_E_UNSUPPORTED, "continuum marginalisation needs the fast tail on line-depth rows");
+        FastGrid FM = c->fast;
+        FM.cluster = 0;
+        if (target) FM.points = c->tgt_points;
+        if (payne::launch_tail_fast_marg(T.log2N1, target != nullptr, c->fast.work_start, c->fast_smem, st, T, FM))
           return fail(PAYNE_E_CUDA, "tail launch");
       } else if (binary) {
         // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no binary form)
@@ -1313,6 +1348,7 @@ int binary_unsupported(PayneCtx* c) {
                   : c->n_targets ? "targets are not supported"
                   : c->star_lay_dev ? "per-star layouts (PayneStarOpts.layout) are not supported"
                   : c->g_world > 0 ? "the fused gather is not supported"
+                  : c->has_marg ? "continuum marginalisation is not supported"
                   : !(c->use_fast && c->allow_fast) ? "binaries need the fast tail (an emulator grid uniform in ln wavelength)"
                   : nullptr;
   return why ? fail(PAYNE_E_UNSUPPORTED, std::string("binary: ") + why) : PAYNE_OK;
@@ -1321,6 +1357,34 @@ int binary_unsupported(PayneCtx* c) {
 int need_binary(PayneCtx* c) {
   if (!c->has_binary) return fail(PAYNE_E_INVALID, "no binary: payne_ctx_set_binary first");
   return binary_unsupported(c);
+}
+
+// What continuum marginalisation cannot take (payne_ctx_set_cont_marg and every entry while it is on).
+int marg_unsupported(PayneCtx* c) {
+  const char* why = !c->has_spec ? "the spectrum emulator is missing"
+                  : c->lsf_on ? "LSF vectors are not supported"
+                  : c->has_binary ? "binaries are not supported"
+                  : c->cont ? "an attached continuum emulator is not supported"
+                  : c->g_world > 0 ? "the fused gather is not supported"
+                  : !(c->use_fast && c->allow_fast) ? "it needs the fast tail (an emulator grid uniform in ln wavelength)"
+                  : nullptr;
+  return why ? fail(PAYNE_E_UNSUPPORTED, std::string("continuum marginalisation: ") + why) : PAYNE_OK;
+}
+
+// The _cont entries: the setting is on and the output strides hold the largest star (or target).
+int need_marg(PayneCtx* c, bool targets, int64_t ld_coef, int64_t ld_chol) {
+  if (!c->has_marg) return fail(PAYNE_E_INVALID, "no continuum marginalisation: payne_ctx_set_cont_marg first");
+  long long kc = 0, kl = 0;
+  const int n = targets ? c->n_targets : c->n_stars;
+  for (int t = 0; t < n; ++t) {
+    long long a = 0, b = 0;
+    const int k0 = targets ? c->tfirst_h[t] : t, k1 = targets ? c->tfirst_h[t + 1] : t + 1;
+    for (int k = k0; k < k1; ++k) { a += c->marg_k_h[k]; b += (long long)c->marg_k_h[k] * (c->marg_k_h[k] + 1) / 2; }
+    kc = std::max(kc, a); kl = std::max(kl, b);
+  }
+  if (ld_coef < kc) return fail(PAYNE_E_INVALID, "ld_coef < " + std::to_string(kc) + " (the largest K" + (targets ? ", summed over a target's members)" : ")"));
+  if (ld_chol < kl) return fail(PAYNE_E_INVALID, "ld_chol < " + std::to_string(kl) + " (the largest K (K + 1) / 2" + (targets ? ", summed over a target's members)" : ")"));
+  return PAYNE_OK;
 }
 
 }  // namespace
@@ -1407,6 +1471,91 @@ int payne_model_batch_binary(PayneCtx* c, const double* theta_dev, const int32_t
                    nullptr, 0, true, comp_dev);
 }
 
+int payne_ctx_set_cont_marg(PayneCtx* c, const PayneContMarg* per_star) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  auto drop = [&]() -> int {
+    CU_TRY(cudaDeviceSynchronize());                     // earlier calls may still read them
+    if (c->marg_k_dev) cudaFree(c->marg_k_dev);
+    if (c->marg_c_dev) cudaFree(c->marg_c_dev);
+    if (c->marg_scratch) cudaFree(c->marg_scratch);
+    c->marg_k_dev = nullptr; c->marg_c_dev = nullptr; c->marg_scratch = nullptr; c->has_marg = false;
+    c->marg_k_h.clear();
+    return PAYNE_OK;
+  };
+  if (!per_star) return drop();
+  const int S = c->n_stars;
+  std::vector<int> kk(S);
+  std::vector<double> cc(S, 0.0);
+  int with = 0;
+  for (int k = 0; k < S; ++k) {
+    const PayneContMarg& m = per_star[k];
+    const std::string who = "continuum marginalisation, star " + std::to_string(k) + ": ";
+    if (m.n_coef < 0 || m.n_coef > PAYNE_MAX_POLY)
+      return fail(PAYNE_E_INVALID, who + "n_coef " + std::to_string(m.n_coef) + " outside [1, " + std::to_string(PAYNE_MAX_POLY) + "]");
+    kk[k] = m.n_coef;
+    if (m.n_coef == 0) continue;
+    ++with;
+    const int np = c->star_lay_h.empty() ? (c->lay.modpoly_bool ? c->lay.n_poly : 0) : c->star_lay_h[k].n_poly;
+    if (np > 0) return fail(PAYNE_E_INVALID, who + "its layout samples pc_k as well (modpoly_bool with n_poly > 0)");
+    for (int i = 0; i < m.n_coef; ++i) {
+      if (!(std::isfinite(m.lo[i]) && std::isfinite(m.hi[i]) && m.lo[i] < m.hi[i]))
+        return fail(PAYNE_E_INVALID, who + "the box of coefficient " + std::to_string(i) + " must be finite with lo < hi");
+      cc[k] += 0.5 * std::log(2.0 * 3.141592653589793) - std::log(m.hi[i] - m.lo[i]);
+    }
+  }
+  if (with == 0) return fail(PAYNE_E_INVALID, "continuum marginalisation: n_coef outside [1, " + std::to_string(PAYNE_MAX_POLY) + "] for every star");
+  if (with != S)
+    return fail(PAYNE_E_UNSUPPORTED, "continuum marginalisation: some stars have the setting and others (n_coef 0) do not");
+  int rc = marg_unsupported(c);
+  if (rc) return rc;
+  int occ = 0;
+  if (!payne::probe_tail_fast_marg(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
+    return fail(PAYNE_E_UNSUPPORTED, "continuum marginalisation tail kernel does not fit on an SM");
+  rc = drop();
+  if (rc) return rc;
+  c->marg_grid = std::min(occ * c->sm_count, c->tail_grid_fast);   // the split kernel's scratch lines exist for these
+  rc = upload(&c->marg_k_dev, kk.data(), (size_t)S);
+  if (rc) return rc;
+  rc = upload(&c->marg_c_dev, cc.data(), (size_t)S);
+  if (rc) return rc;
+  CU_TRY(cudaMalloc((void**)&c->marg_scratch, (size_t)c->marg_grid * c->n_obs_max * sizeof(double)));
+  c->marg_k_h = kk;
+  c->has_marg = true;
+  return PAYNE_OK;
+}
+
+int payne_cont_batch_stars(PayneCtx* c, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
+                           double* coef_dev, int64_t ld_coef, double* chol_dev, int64_t ld_chol, double* chi2_dev,
+                           double* lnl_dev, void* stream) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B == 0) return PAYNE_OK;
+  if (!theta_dev) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  int rc = need_marg(c, false, coef_dev ? ld_coef : INT64_MAX, chol_dev ? ld_chol : INT64_MAX);
+  if (rc) return rc;
+  rc = need_star_array(c, star_dev, "payne_cont_batch_stars");
+  if (rc) return rc;
+  return run_batch(c, theta_dev, star_dev, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, nullptr, chi2_dev, 1,
+                   false, nullptr, coef_dev, ld_coef, chol_dev, ld_chol);
+}
+
+int payne_cont_batch_targets(PayneCtx* c, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
+                             double* coef_dev, int64_t ld_coef, double* chol_dev, int64_t ld_chol, double* chi2_dev,
+                             int64_t ld_chi2, double* lnl_dev, void* stream) {
+  if (!c) return fail(PAYNE_E_INVALID, "null argument");
+  if (B == 0) return PAYNE_OK;
+  if (!theta_dev || !target_dev) return fail(PAYNE_E_INVALID, "null argument");
+  DeviceGuard dg(c->device);
+  int rc = need_targets(c);
+  if (rc) return rc;
+  rc = need_marg(c, true, coef_dev ? ld_coef : INT64_MAX, chol_dev ? ld_chol : INT64_MAX);
+  if (rc) return rc;
+  if (chi2_dev && ld_chi2 < c->tgt_kmax) return fail(PAYNE_E_INVALID, "ld_chi2 < the largest member count");
+  return run_batch(c, theta_dev, nullptr, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, target_dev, chi2_dev,
+                   ld_chi2, false, nullptr, coef_dev, ld_coef, chol_dev, ld_chol);
+}
+
 int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) {
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   DeviceGuard dg(c->device);
@@ -1418,6 +1567,7 @@ int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) 
     c->tfirst_dev = nullptr; c->n_targets = 0; c->tgt_kmax = 0; c->tgt_nobs_max = 0;
     c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
     c->tgt_instr_col.clear();
+    c->tfirst_h.clear();
     return PAYNE_OK;
   }
   if (!c->has_spec) return fail(PAYNE_E_UNSUPPORTED, "targets need the spectrum emulator");
@@ -1473,6 +1623,7 @@ int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) 
     c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
   }
   c->n_targets = n_targets; c->tgt_kmax = kmax; c->tgt_nobs_max = nobs_max; c->tgt_instr_col = instr_col;
+  c->tfirst_h.assign(first, first + n_targets + 1);
   return PAYNE_OK;
 }
 
@@ -1594,6 +1745,7 @@ void payne_ctx_destroy(PayneCtx* c) {
   drop(c->theta_stage); drop(c->lnl_stage); drop(c->star_stage);
   drop(c->tfirst_dev); drop(c->tgt_points); drop(c->tgt_star);
   drop(c->binary_dev); drop(c->bin_scratch); drop(c->bin_par);
+  drop(c->marg_k_dev); drop(c->marg_c_dev); drop(c->marg_scratch);
   if (c->star_pin) cudaFreeHost(c->star_pin);
   for (int r = 0; r < 16; ++r)
     if (c->g_opened[r]) { cudaIpcCloseMemHandle(c->g_peer_buf[r]); cudaIpcCloseMemHandle(c->g_peer_flag[r]); }
@@ -1932,6 +2084,7 @@ int64_t payne_ctx_query(PayneCtx* c, const char* key) {
   if (k == "n_stars") return c->n_stars;
   if (k == "n_targets") return c->n_targets;
   if (k == "binary") return c->has_binary ? 1 : 0;
+  if (k == "cont_marg") return c->has_marg ? 1 : 0;
   if (k == "n_obs_total") return c->n_obs_total;
   if (k == "nfft1") return c->has_spec ? (1LL << c->tail.log2N1) : 0;
   if (k == "launches") return c->launches;

@@ -112,6 +112,15 @@ struct TailParams {
   double* bin_scratch;               // [grid, bin_ld] a_1 of the CTA's current point
   long long bin_ld;
   double* comp_out;                  // [B, 2, ld_flux] a_1 and a_2, or null
+  // Continuum marginalisation (payne_ctx_set_cont_marg; fast tail only): star k's K = marg_k[k] coefficients are
+  // integrated out, C = marg_c[k] = sum_k (ln 2 pi / 2 - ln w_k).  bin_scratch / bin_ld hold a_j of the CTA's current point,
+  // chi2_out / ld_chi2 every point's (or member's) Q.  Null marg_k: off.
+  const int* marg_k;
+  const double* marg_c;
+  double* coef_out;                  // [B, ld_coef] c-hat (a target's members back to back), or null
+  long long ld_coef;
+  double* chol_out;                  // [B, ld_chol] L, packed lower triangles K (K + 1) / 2 each, or null
+  long long ld_chol;
 };
 
 // lnL of point p: local result and, with the fused gather on, the copy in every peer's buffer

@@ -259,10 +259,46 @@ __device__ __forceinline__ double final_pass_poly(const TailParams& P, const Fas
   return acc;
 }
 
+// The residual pass of continuum marginalisation (marg_point) with an instrumental stage: final_pass_poly's thread
+// mapping, order and residual arithmetic, with m = a_j read from the CTA's scratch (by the thread that wrote it in
+// final_pass_bin<1>) and the star's own nk coefficients.  A separate function on purpose: a template switch inside
+// final_pass_poly changed the spills of the 65536-sample target kernel.
+__device__ __forceinline__ double final_pass_marg(const TailParams& P, const PointSetup& S, const FastSetup& FS, int tid,
+                                                  int p, int moff, int nk) {
+  const int off = FS.obs.off, jend = FS.obs.off + FS.obs.n;
+  const double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  double* mrow = P.model_out ? P.model_out + (long long)p * P.ld_flux + moff : nullptr;
+  double acc = 0.0;
+  constexpr int U = 4;
+#pragma unroll 1
+  for (int j0 = off + tid; j0 < jend; j0 += U * kNT) {
+    double is[U], ot[U], x[U], cv[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const bool in = j0 + u * kNT < jend;
+      is[u] = in ? __ldcg(P.obs_inv_s + j0 + u * kNT) : 0.0;
+      ot[u] = in ? __ldcg(P.obs_ot + j0 + u * kNT) : 0.0;
+      x[u] = in ? __ldcg(P.obs_x + j0 + u * kNT) : 0.0;
+    }
+    chebval_dev4(x, S.poly, nk, cv);
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      if (j0 + u * kNT < jend) {
+        const double m = scr[j0 + u * kNT - off] * cv[u];
+        if (mrow) mrow[j0 + u * kNT - off] = m;
+        const double r = fma(m, is[u], -ot[u]);
+        acc = fma(r, r, acc);
+      }
+    }
+  }
+  return acc;
+}
+
 // Binaries (payne_ctx_set_binary): the point's pixels with final_pass_poly's thread mapping and order.  BM = 1 (component
-// 1): a_1 = 1 + d (NaN outside the grid) into the CTA's scratch and comp row 0.  BM = 2 (component 2): a_2, a_1 read
-// back from the scratch (by the thread that wrote it), m = (a_1 + k a_2) / (1 + k) with the blackbody flux ratio k, the
-// continuum, chi2; a_2 into comp row 1 and m into the model row.  At k = 0 and a finite a_2, m is a_1 and the chi2 has
+// 1, and the first pass of continuum marginalisation): a_1 = 1 + d (NaN outside the grid) into the CTA's scratch and
+// comp row 0 (when given).  BM = 2 (component 2): a_2, a_1 read back from the scratch (by the thread that wrote it),
+// m = (a_1 + k a_2) / (1 + k) with the blackbody flux ratio k, the continuum, chi2; a_2 into comp row 1 and m into the
+// model row.  At k = 0 and a finite a_2, m is a_1 and the chi2 has
 // the bits of final_pass_poly.
 constexpr double kC2 = 1.438776877e8;   // second radiation constant hc / k_B, AA K
 
@@ -281,8 +317,12 @@ __device__ __forceinline__ double final_pass_bin(const TailParams& P, const Fast
   double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
   double* crow = P.comp_out ? P.comp_out + ((long long)p * 2 + (BM - 1)) * P.ld_flux : nullptr;
   double* mrow = (BM == 2 && P.model_out) ? P.model_out + (long long)p * P.ld_flux : nullptr;
-  const double t1 = __ldg(P.bin_par + 3LL * p), t2 = __ldg(P.bin_par + 3LL * p + 1), rr = __ldg(P.bin_par + 3LL * p + 2);
-  const double rr2 = rr * rr;
+  double t1 = 0.0, t2 = 0.0, rr2 = 0.0;
+  if constexpr (BM == 2) {
+    t1 = __ldg(P.bin_par + 3LL * p); t2 = __ldg(P.bin_par + 3LL * p + 1);
+    const double rr = __ldg(P.bin_par + 3LL * p + 2);
+    rr2 = rr * rr;
+  }
   double acc = 0.0;
   constexpr int U = 4;
 #pragma unroll 1
@@ -360,8 +400,12 @@ __device__ __forceinline__ double plain_pass_bin(const TailParams& P, const Poin
   double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
   double* crow = P.comp_out ? P.comp_out + ((long long)p * 2 + (BM - 1)) * P.ld_flux : nullptr;
   double* mrow = (BM == 2 && P.model_out) ? P.model_out + (long long)p * P.ld_flux : nullptr;
-  const double t1 = __ldg(P.bin_par + 3LL * p), t2 = __ldg(P.bin_par + 3LL * p + 1), rr = __ldg(P.bin_par + 3LL * p + 2);
-  const double rr2 = rr * rr;
+  double t1 = 0.0, t2 = 0.0, rr2 = 0.0;
+  if constexpr (BM == 2) {
+    t1 = __ldg(P.bin_par + 3LL * p); t2 = __ldg(P.bin_par + 3LL * p + 1);
+    const double rr = __ldg(P.bin_par + 3LL * p + 2);
+    rr2 = rr * rr;
+  }
   double acc = 0.0;
   for (int j = off + tid; j < jend; j += kNT) {
     const double x = __ldg(P.obs_w + j);
@@ -387,6 +431,41 @@ __device__ __forceinline__ double plain_pass_bin(const TailParams& P, const Poin
       const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
       acc += r * r;
     }
+  }
+  return acc;
+}
+
+// No instrumental profile: plain np.interp (predictspec.py:288-289), continuum, residuals.  MARG: the residual pass of
+// continuum marginalisation (marg_point), m = a_j from the CTA's scratch and nk coefficients, with this loop's own
+// arithmetic, thread mapping and order.
+template <bool STARS, bool MARG = false>
+__device__ __forceinline__ double plain_pass(const TailParams& P, const PointSetup& S, const FastSetup& FS,
+                                             const float* row, int tid, int p, int moff, int nk = 0) {
+  const double nan = CUDART_NAN;
+  const bool is_depth = true;   // this kernel is only launched on line-depth rows (f - 1)
+  const int npoly = MARG ? nk : P.n_poly;
+  const double* scr = MARG ? P.bin_scratch + (long long)blockIdx.x * P.bin_ld : nullptr;
+  double acc = 0.0;
+  const int n = P.n;
+  const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
+  const int off = obs_lo<STARS>(FS.obs), jend = obs_hi<STARS>(P, FS.obs);
+  for (int j = off + tid; j < jend; j += kNT) {
+    const double x = __ldg(P.obs_w + j);
+    double m;
+    if constexpr (MARG) m = scr[j - off];
+    else if (!(x >= wlo && x <= whi)) m = nan;
+    else {
+      const int g = (int)((__ldg(P.obs_lnw + j) - S.lnD - P.lnw0) * P.inv_dlnw);
+      const int jj = locate(P.w, S.D, x, g, 0, n - 2);
+      const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
+      const double a = (double)depth_of(row[jj], is_depth, false);
+      const double b = (double)depth_of(row[jj + 1], is_depth, false);
+      m = 1.0 + np_interp_pair(x, wa, wb, a, b);
+    }
+    if (npoly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, npoly);
+    if (P.model_out) P.model_out[(long long)p * P.ld_flux + moff + (j - off)] = m;
+    const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
+    acc += r * r;
   }
   return acc;
 }
@@ -460,7 +539,6 @@ __device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid
   constexpr bool kSplit = LOG2N1 >= 16;
   constexpr int LOG2MH = kSplit ? LOG2N1 - 2 : 8;
   const double nan = CUDART_NAN;
-  const bool is_depth = true;   // this kernel is only launched on line-depth rows (f - 1)
   double acc = 0.0;
   if (S.use_inst) {
     // ---------------- stage 2: mask, regrid, Gaussian broadening
@@ -500,29 +578,159 @@ __device__ __forceinline__ double point_chi2(const TailParams& P, const FastGrid
   } else if constexpr (BM != 0) {
     acc = plain_pass_bin<BM>(P, S, FS, row, tid, p);
   } else {
-    // ---------------- no instrumental profile: plain np.interp (predictspec.py:288-289)
-    const int n = P.n;
-    const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
-    const int off = obs_lo<STARS>(FS.obs), jend = obs_hi<STARS>(P, FS.obs);
-    for (int j = off + tid; j < jend; j += kNT) {
-      const double x = __ldg(P.obs_w + j);
-      double m;
-      if (!(x >= wlo && x <= whi)) m = nan;
-      else {
-        const int g = (int)((__ldg(P.obs_lnw + j) - S.lnD - P.lnw0) * P.inv_dlnw);
-        const int jj = locate(P.w, S.D, x, g, 0, n - 2);
-        const double wa = __ldg(P.w + jj) * S.D, wb = __ldg(P.w + jj + 1) * S.D;
-        const double a = (double)depth_of(row[jj], is_depth, false);
-        const double b = (double)depth_of(row[jj + 1], is_depth, false);
-        m = 1.0 + np_interp_pair(x, wa, wb, a, b);
-      }
-      if (P.n_poly) m *= chebval_dev(__ldg(P.obs_x + j), S.poly, P.n_poly);
-      if (P.model_out) P.model_out[(long long)p * P.ld_flux + moff + (j - off)] = m;
-      const double r = m * __ldg(P.obs_inv_s + j) - __ldg(P.obs_ot + j);
-      acc += r * r;
-    }
+    acc = plain_pass<STARS>(P, S, FS, row, tid, p, moff);
   }
   return acc;
+}
+
+// ---- continuum marginalisation (payne_ctx_set_cont_marg) ------------------------------------------------------------
+// Column pair (a, b), a >= b, of entry e of the lower triangle of [B | y]^T [B | y] without y.y (K + 1 columns: the
+// star's K Chebyshev columns b_jk = a_j T_k(x_j) / s_j, then y_j = o_j / s_j): G below column K, h = row K.
+__device__ __forceinline__ void marg_entry(int e, int& a, int& b) {
+  a = 0;
+  while (e > a) { e -= a + 1; ++a; }
+  b = e;
+}
+
+// NaN coefficients and Cholesky factor of star k's K coefficients at columns cofs / lofs of row p
+__device__ __forceinline__ void marg_nan_out(const TailParams& P, int p, int K, int cofs, int lofs, int tid) {
+  const double nan = CUDART_NAN;
+  for (int i = tid; P.coef_out && i < K; i += kNT) P.coef_out[(long long)p * P.ld_coef + cofs + i] = nan;
+  for (int i = tid; P.chol_out && i < K * (K + 1) / 2; i += kNT) P.chol_out[(long long)p * P.ld_chol + lofs + i] = nan;
+}
+
+// One point against star k with its continuum integrated out.  Returns this thread's partial Q (the chi2 at c-hat, with
+// final_pass_poly's or plain_pass's thread mapping and order, so the warp and CTA reduction of the caller gives Q the bits
+// of -2 lnL of a context that samples the coefficients); thread 0 gets M = -sum ln L_kk + C_k in `M`.
+//  1. stage 2 and the final pass of a binary's component 1 (point_chi2 BM = 1): a_j into the CTA's scratch;
+//  2. G and h in fp64 over chunks of pixels staged in the (dead) transform buffer: thread (e, r) sums entry e over
+//     pixels r, r + R, ... of every chunk in four accumulators, then thread e adds its R partials in order -- a fixed
+//     pixel-to-thread mapping and order that depends on K and the transform size only;
+//  3. warp 0: Cholesky G = L L^T, L z = h, L^T c = z; c-hat into S.poly (NaN with a pivot at or below 1e-10 of its diagonal entry: status bit 3
+//     when G is finite);
+//  4. the residual pass at c-hat on the scratch.
+template <int LOG2N1>
+__device__ __forceinline__ double marg_point(const TailParams& P, const FastGrid& F, PointSetup& S, const FastSetup& FS,
+                                             float2* z, const ZSmem& zs, const ZSplit& zp, float* gline, const TwTab& tw,
+                                             const float* row, int tid, int p, int moff, int k, int cofs, int lofs,
+                                             double& M) {
+  constexpr int kBufD = (LOG2N1 >= 16 ? (1 << LOG2N1) / 2 : (1 << LOG2N1)) / 2;   // doubles of the transform buffer
+  constexpr int kG = PAYNE_MAX_POLY + 1;                                           // row stride of G / L
+  const double nan = CUDART_NAN;
+  point_chi2<LOG2N1, true, true, 1>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, 0);
+  __syncthreads();                                        // a_j in the scratch; the transform buffer is free
+  const int K = __ldg(P.marg_k + k);
+  const int off = FS.obs.off, n = FS.obs.n;
+  const double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  double* sm = reinterpret_cast<double*>(z);
+  const int nc = K + 1, nent = nc * (nc + 1) / 2 - 1;
+  const int R = kNT / nent;
+  const int C = (kBufD - kNT) / nc;                       // pixels per chunk; the last kNT doubles take the partials
+  const bool act = tid < nent * R;
+  int ea = 0, eb = 0;
+  if (act) marg_entry(tid / R, ea, eb);
+  const int r = act ? tid % R : 0;
+  double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
+  for (int c0 = 0; c0 < n; c0 += C) {
+    const int cn = min(C, n - c0);
+    for (int i = tid; i < cn; i += kNT) {
+      const int j = off + c0 + i;
+      const double as = scr[c0 + i] * __ldg(P.obs_inv_s + j);
+      const double x = __ldg(P.obs_x + j);
+      double t0 = 1.0, t1 = x;
+      sm[i] = as;
+      for (int q = 1; q < K; ++q) {
+        sm[q * C + i] = as * t1;
+        const double t2 = 2.0 * x * t1 - t0;
+        t0 = t1; t1 = t2;
+      }
+      sm[K * C + i] = __ldg(P.obs_ot + j);
+    }
+    __syncthreads();
+    if (act) {
+      const double* ba = sm + ea * C;
+      const double* bb = sm + eb * C;
+      int i = r;
+      for (; i + 3 * R < cn; i += 4 * R) {
+        s0 = fma(ba[i], bb[i], s0);
+        s1 = fma(ba[i + R], bb[i + R], s1);
+        s2 = fma(ba[i + 2 * R], bb[i + 2 * R], s2);
+        s3 = fma(ba[i + 3 * R], bb[i + 3 * R], s3);
+      }
+      for (; i < cn; i += R) s0 = fma(ba[i], bb[i], s0);
+    }
+    __syncthreads();
+  }
+  double* part = sm + (kBufD - kNT);
+  if (act) part[tid] = ((s0 + s1) + s2) + s3;
+  __syncthreads();
+  double g = 0.0;
+  if (tid < nent) {
+    for (int q = 0; q < R; ++q) g += part[tid * R + q];
+    marg_entry(tid, ea, eb);
+  }
+  __syncthreads();                                        // G overlaps the partials of the smallest buffers
+  double* G = sm;                                         // G[a * kG + b], a >= b; h_b = G[K * kG + b]
+  if (tid < nent) G[ea * kG + eb] = g;
+  __syncthreads();
+  if (tid < 32) {
+    const unsigned full = 0xffffffffu;
+    const int lane = tid;
+    bool fin = true;
+    for (int e = lane; e < nent; e += 32) {
+      int a, b;
+      marg_entry(e, a, b);
+      fin = fin && isfinite(G[a * kG + b]);
+    }
+    fin = __all_sync(full, fin);
+    bool ok = true;
+    double* L = G;                                        // in place, column by column
+    for (int jc = 0; jc < K; ++jc) {
+      double v = 0.0, g0 = 0.0;
+      if (lane >= jc && lane < K) {
+        v = g0 = G[lane * kG + jc];
+        for (int q = 0; q < jc; ++q) v = fma(-L[lane * kG + q], L[jc * kG + q], v);
+      }
+      // a rank-deficient G leaves pivots of rounding size and either sign: fail at or below 1e-10 of the diagonal entry
+      const double d = __shfl_sync(full, v, jc), gd = __shfl_sync(full, g0, jc);
+      ok = ok && d > 1e-10 * gd;
+      const double ljj = sqrt(d);
+      if (lane > jc && lane < K) L[lane * kG + jc] = v / ljj;
+      if (lane == jc) L[jc * kG + jc] = ljj;
+      __syncwarp();
+    }
+    double v = lane < K ? G[K * kG + lane] : 0.0;         // L z = h
+    for (int i = 0; i < K; ++i) {
+      const double zi = __shfl_sync(full, v, i) / L[i * kG + i];
+      if (lane == i) v = zi;
+      else if (lane > i && lane < K) v = fma(-L[lane * kG + i], zi, v);
+    }
+    for (int i = K - 1; i >= 0; --i) {                    // L^T c = z
+      const double ci = __shfl_sync(full, v, i) / L[i * kG + i];
+      if (lane == i) v = ci;
+      else if (lane < i) v = fma(-L[i * kG + lane], ci, v);
+    }
+    if (!ok) v = nan;
+    if (lane < K) {
+      S.poly[lane] = v;
+      if (P.coef_out) P.coef_out[(long long)p * P.ld_coef + cofs + lane] = v;
+    }
+    if (P.chol_out)
+      for (int e = lane; e < K * (K + 1) / 2; e += 32) {
+        int a, b;
+        marg_entry(e, a, b);
+        P.chol_out[(long long)p * P.ld_chol + lofs + e] = ok ? L[a * kG + b] : nan;
+      }
+    if (lane == 0) {
+      double lsum = 0.0;
+      for (int i = 0; i < K; ++i) lsum += log(L[i * kG + i]);
+      M = ok ? __ldg(P.marg_c + k) - lsum : nan;
+      if (!ok && fin) atomicOr(P.status, 8);
+    }
+  }
+  __syncthreads();                                        // c-hat in S.poly
+  if (S.use_inst) return final_pass_marg(P, S, FS, tid, p, moff, K);
+  return plain_pass<true, true>(P, S, FS, row, tid, p, moff, K);
 }
 
 // Stage 1 of tail_fast_kernel (rotational broadening on the full emulator grid) for a binary's component: writes back
@@ -569,8 +777,10 @@ __device__ __forceinline__ void rot_stage(const TailParams& P, const FastGrid& F
 // and the final pass once per member against that member's record, and lnL is the members' chi2 summed in member order.
 // BIN: every point is a binary (TailParams::binary; POLY and STARS are then true): component 1's record and row, stage 1,
 // stage 2 and a final pass that keeps a_1; then component 2's, whose final pass combines the two (final_pass_bin).
+// MARG: continuum marginalisation (TailParams::marg_k; POLY and STARS are then true): every point, or every member of a
+// target, through marg_point, and lnL = -0.5 (Q + chi2_sed) + M (members: Q and M each summed in member order).
 // (3 CTAs/SM, 80 registers with a few spills, measured at C2 0.76 ms against 0.84 ms with 2 CTAs/SM and no spills)
-template <int LOG2N1, bool POLY, bool STARS, bool TGT = false, bool BIN = false>
+template <int LOG2N1, bool POLY, bool STARS, bool TGT = false, bool BIN = false, bool MARG = false>
 __global__ void __launch_bounds__(kNT, LOG2N1 <= 14 ? 3 : 1)
 tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -685,6 +895,11 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
     if (TGT ? K == 0 : S.bad) {
       if (P.model_out)
         for (int j = tid; j < obs_hi<STARS>(P, FS.obs) - obs_lo<STARS>(FS.obs); j += kNT) P.model_out[(long long)p * P.ld_flux + j] = nan;
+      if constexpr (MARG && !TGT) {
+        const int k = star_of(P.star, P.n_stars, p);
+        if (k >= 0) marg_nan_out(P, p, __ldg(P.marg_k + k), 0, 0, tid);
+        if (tid == 0 && P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2] = nan;
+      }
       if (tid == 0 && P.lnl) store_lnl(P, p, nan);
       __syncthreads();
       continue;
@@ -721,7 +936,23 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
       __syncthreads();
     }
 
-    if constexpr (!TGT) {
+    if constexpr (!TGT && MARG) {
+      double M = 0.0;
+      double acc = marg_point<LOG2N1>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, 0, star_of(P.star, P.n_stars, p), 0,
+                                      0, M);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+      if ((tid & 31) == 0) red[tid >> 5] = acc;
+      __syncthreads();
+      if (tid == 0) {
+        double c2 = 0.0;
+#pragma unroll
+        for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
+        if (P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2] = c2;
+        if (P.chi2_sed) c2 += P.chi2_sed[p];
+        if (P.lnl) store_lnl(P, p, -0.5 * c2 + M);
+      }
+    } else if constexpr (!TGT) {
       double acc = point_chi2<LOG2N1, POLY, STARS>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, 0);
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
@@ -739,6 +970,8 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
       // those of members 0 .. m-1 (the members' observations lie back to back in the set's arrays).
       const int off0 = FS.obs.off;
       double tot = 0.0;                                   // thread 0: chi2 of members 0 .. m, summed in that order
+      double mtot = 0.0;                                  // MARG, thread 0: M of members 0 .. m, likewise
+      int cofs = 0, lofs = 0;                             // MARG: the member's first coefficient / Cholesky column
       for (int m = 0; m < K; ++m) {
         if (m > 0) {
           __syncthreads();                                // member m-1's record, transform buffer and red[] are free
@@ -749,9 +982,22 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
         const bool bad = S.bad != 0;
         const int moff = FS.obs.off - off0;
         double acc = 0.0;
-        if (!bad) acc = point_chi2<LOG2N1, POLY, true>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, moff);
-        else if (P.model_out)
-          for (int j = tid; j < FS.obs.n; j += kNT) P.model_out[(long long)p * P.ld_flux + moff + j] = nan;
+        double M = 0.0;                                   // MARG: the member's M (thread 0)
+        int km = 0;                                       // MARG: the member's coefficients
+        if constexpr (MARG) {
+          const int k = __ldg(P.tfirst + __ldg(P.target + p)) + m;
+          km = __ldg(P.marg_k + k);
+          if (!bad) acc = marg_point<LOG2N1>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, moff, k, cofs, lofs, M);
+          else {
+            if (P.model_out)
+              for (int j = tid; j < FS.obs.n; j += kNT) P.model_out[(long long)p * P.ld_flux + moff + j] = nan;
+            marg_nan_out(P, p, km, cofs, lofs, tid);
+          }
+        } else {
+          if (!bad) acc = point_chi2<LOG2N1, POLY, true>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, moff);
+          else if (P.model_out)
+            for (int j = tid; j < FS.obs.n; j += kNT) P.model_out[(long long)p * P.ld_flux + moff + j] = nan;
+        }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
         if ((tid & 31) == 0) red[tid >> 5] = acc;
@@ -763,11 +1009,14 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
           if (bad) c2 = nan;
           if (P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2 + m] = c2;
           tot = m == 0 ? c2 : tot + c2;
+          if constexpr (MARG) mtot = m == 0 ? M : mtot + M;
         }
+        if constexpr (MARG) { cofs += km; lofs += km * (km + 1) / 2; }
       }
       if (tid == 0 && P.lnl) {
         if (P.chi2_sed) tot += P.chi2_sed[p];
-        store_lnl(P, p, -0.5 * tot);
+        if constexpr (MARG) store_lnl(P, p, -0.5 * tot + mtot);
+        else store_lnl(P, p, -0.5 * tot);
       }
     }
     // The row is scratch and fully consumed: L2 is told to drop its lines instead of writing them back

@@ -19,6 +19,9 @@ the member's LSF vector), resampling, continuum and chi2.
 
 ``binary=True`` models every spectrum as a double-lined binary: the flux-weighted sum of two stars (``set_binary``).
 
+``cont_box=[(lo, hi), ...]`` (per star, or for the single star) integrates the continuum polynomial out instead of
+sampling its coefficients (``set_cont_marg``).
+
 A fixed ``Inst_R`` that is a 1-D array is an LSF vector, the dispersion (AA) at every observed pixel,
 as in the reference (genmod.py:82-85 passes a non-float inst_R on to getspec's LSF branch,
 predictspec.py:265-286).
@@ -145,14 +148,16 @@ def _specnet_struct(spec, keep):
 class Engine:
     def __init__(self, spec=None, phot=None, obs_wave=None, obs_flux=None, obs_eflux=None,
                  obs_phot=None, fitpars_i=(), fixedpars=None, runbools=(True, False, False, False, False),
-                 precision='parity', device=None, stars=None, targets=None, binary=False):
+                 precision='parity', device=None, stars=None, targets=None, binary=False, cont_box=None):
         """``stars``: instead of ``obs_wave``, ``obs_flux``, ``obs_eflux`` and ``obs_phot``, a list of
         ``{'wave', 'flux', 'eflux', 'phot': {band: (mag, err)}}``, one per star; ``lnlike_batch`` and
         ``model_batch`` then take the star index of every row.  A star may also carry
           ``'fixedpars'``: its fixed parameter values, in place of the shared ``fixedpars``;
           ``'bands'``: the order of its magnitudes (its SED chi2 is summed in that order, likelihood.py:109-112);
           ``'fitpars_i'`` / ``'runbools'``: its own free parameters in its theta order (``pc_k`` among them) and
-          run booleans, in place of the shared ones.
+          run booleans, in place of the shared ones;
+          ``'cont_box'``: the box [(lo, hi), ...] of its continuum coefficients, which are then integrated out
+          (``set_cont_marg``).
         Its ``'phot'`` keys may be any subset of the photometry net's bands; without ``'bands'`` they go in the
         net's order.  In a photometry engine a star without ``'phot'`` is a star without photometry.  A fixed
         ``Inst_R`` that is a 1-D array is the star's LSF vector (one dispersion per observed pixel); every star
@@ -165,9 +170,13 @@ class Engine:
 
         ``binary``: every spectrum is a double-lined binary, read from ``fitpars_i`` / ``fixedpars`` under the names
         ``Teff_sec``, ``log(g)_sec``, ``[Fe/H]_sec``, ``[a/Fe]_sec``, ``Vmic_sec``, ``Vrad_sec``, ``Vrot_sec`` and
-        ``Rratio`` (see ``set_binary``)."""
+        ``Rratio`` (see ``set_binary``).
+
+        ``cont_box``: a single-star engine's ``'cont_box'``."""
         if stars is None:
-            stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot}]
+            stars = [{'wave': obs_wave, 'flux': obs_flux, 'eflux': obs_eflux, 'phot': obs_phot, 'cont_box': cont_box}]
+        elif cont_box is not None:
+            raise ValueError("with stars=[...], give every star its own 'cont_box'")
         elif any(v is not None for v in (obs_wave, obs_flux, obs_eflux, obs_phot)):
             raise ValueError('give either stars=[...] or obs_wave / obs_flux / obs_eflux / obs_phot, not both')
         stars = list(stars)
@@ -291,6 +300,10 @@ class Engine:
         self.binary = False
         if binary:
             self.set_binary()
+        self.cont_k = None
+        boxes = [st.get('cont_box') for st in stars]
+        if any(b is not None for b in boxes):
+            self.set_cont_marg(boxes)
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -368,6 +381,85 @@ class Engine:
                     dict(self.fixedpars if fixedpars is None else fixedpars))
         _lib.check(self.lib.payne_ctx_set_binary(self._ctx, C.byref(b)))
         self.binary = True
+
+    def set_cont_marg(self, boxes):
+        """Integrate every star's continuum polynomial out (include/payne_b200.h, PayneContMarg): ``boxes[k]`` is star
+        k's [(lo, hi), ...], one pair per coefficient, whose widths normalise the flat prior of the integral; None for
+        every star removes the setting.  lnL is then -0.5 (Q + chi2_sed) + M, Q the chi2 at the best-fitting
+        coefficients and M the log of the Gaussian integral over them, and the model rows are at those coefficients.
+        A star with the setting has no ``pc_k`` among its free parameters."""
+        if boxes is None or all(b is None for b in boxes):
+            _lib.check(self.lib.payne_ctx_set_cont_marg(self._ctx, None))
+            self.cont_k = None
+            return
+        if len(boxes) != self.n_stars:
+            raise ValueError('set_cont_marg: one box list per star (%d)' % self.n_stars)
+        arr = (_lib.PayneContMarg * self.n_stars)()
+        for k, b in enumerate(boxes):
+            b = [] if b is None else [tuple(map(float, lh)) for lh in b]
+            if len(b) > _lib.MAX_POLY:
+                raise ValueError('star %d: at most %d continuum coefficients' % (k, _lib.MAX_POLY))
+            arr[k].n_coef = len(b)
+            for i, (lo, hi) in enumerate(b):
+                arr[k].lo[i], arr[k].hi[i] = lo, hi
+        _lib.check(self.lib.payne_ctx_set_cont_marg(self._ctx, arr))
+        self.cont_k = [int(arr[k].n_coef) for k in range(self.n_stars)]
+
+    @staticmethod
+    def _cont_outputs(B, kc, kl, dev, nchi2=None):
+        nan = float('nan')
+        coef = torch.full((B, kc), nan, dtype=torch.float64, device=dev)
+        chol = torch.full((B, kl), nan, dtype=torch.float64, device=dev)
+        chi2 = torch.full((B,) if nchi2 is None else (B, nchi2), nan, dtype=torch.float64, device=dev)
+        lnl = torch.empty(B, dtype=torch.float64, device=dev)
+        return coef, chol, chi2, lnl
+
+    def cont_batch(self, theta, star=None):
+        """With the continuum integrated out: the best-fitting coefficients [B, K] (K the largest star's; a row's
+        columns beyond its star's K stay NaN), the Cholesky factor L of G = L L^T as packed lower triangles
+        [B, K(K+1)/2] (row by row), Q (the chi2 at those coefficients) [B] and lnL [B], as CUDA float64 tensors.  A
+        draw of the coefficients' conditional posterior is coef + L^-T z, z ~ N(0, I)."""
+        if self.cont_k is None:
+            raise ValueError('no continuum marginalisation: set_cont_marg first')
+        dev = torch.device('cuda', self.device)
+        if not isinstance(theta, torch.Tensor):
+            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
+        th = self._theta_dev(theta.to(dev))
+        B = th.shape[0]
+        if star is not None and not isinstance(star, torch.Tensor):
+            star = torch.from_numpy(np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind')))
+        sv = self._star_dev(star.to(dev) if star is not None else None, B, dev)
+        kc = max(self.cont_k)
+        coef, chol, chi2, lnl = self._cont_outputs(B, kc, kc * (kc + 1) // 2, dev)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(self.lib.payne_cont_batch_stars(
+            self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None, B, th.shape[1],
+            coef.data_ptr(), coef.shape[1], chol.data_ptr(), chol.shape[1], chi2.data_ptr(), lnl.data_ptr(), st))
+        return coef, chol, chi2, lnl
+
+    def cont_batch_targets(self, theta, target):
+        """``cont_batch`` for targets: the members' coefficients and Cholesky factors back to back in member order,
+        and Q [B, target_kmax] per member."""
+        if self.cont_k is None:
+            raise ValueError('no continuum marginalisation: set_cont_marg first')
+        if not self.n_targets:
+            raise ValueError('no targets: set_targets first')
+        dev = torch.device('cuda', self.device)
+        if not isinstance(theta, torch.Tensor):
+            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
+        th = self._theta_dev(theta.to(dev))
+        B = th.shape[0]
+        if not isinstance(target, torch.Tensor):
+            target = torch.from_numpy(np.ascontiguousarray(np.asarray(target).astype(np.int32, casting='same_kind')))
+        tv = self._star_dev(target.to(dev), B, dev)
+        kc = max(sum(self.cont_k[k] for k in m) for m in self.target_members)
+        kl = max(sum(self.cont_k[k] * (self.cont_k[k] + 1) // 2 for k in m) for m in self.target_members)
+        coef, chol, chi2, lnl = self._cont_outputs(B, kc, kl, dev, self.target_kmax)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(self.lib.payne_cont_batch_targets(
+            self._ctx, th.data_ptr(), tv.data_ptr(), B, th.shape[1], coef.data_ptr(), kc, chol.data_ptr(), kl,
+            chi2.data_ptr(), self.target_kmax, lnl.data_ptr(), st))
+        return coef, chol, chi2, lnl
 
     def lnlike_batch_binary(self, theta, star=None):
         """lnL of every row as a binary, ``theta`` and ``star`` as in ``lnlike_batch`` (None: star 0)."""

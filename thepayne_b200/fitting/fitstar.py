@@ -26,7 +26,13 @@ What differs, on purpose:
   * ``inputdict['binary'] = True`` with a single ``spec`` fits a double-lined binary (``binary.BinaryLikelihood``): the
     secondary's ``Teff_sec``, ``log(g)_sec``, ``Vrad_sec`` and ``Vrot_sec`` and the radius ratio ``Rratio`` follow the
     reference parameters (before ``pc_k``); ``[Fe/H]_sec``, ``[a/Fe]_sec`` and ``Vmic_sec`` get a column only when
-    ``priordict`` names them, and are the primary's otherwise.  ``{'fixed': v}`` fixes any of them.
+    ``priordict`` names them, and are the primary's otherwise.  ``{'fixed': v}`` fixes any of them;
+  * ``spec['modpoly_marginal'] = True`` (beside ``modpoly``; with a list-valued ``spec`` in every spectrum or in none)
+    integrates the continuum coefficients out per likelihood call instead of sampling them (``Engine.set_cont_marg``):
+    the sampler has K fewer dimensions per spectrum, and the coefficients' flat prior boxes are the ones a sampled
+    ``pc_k`` would get (``prior.pc_box``).  The output file keeps its ``pc`` columns: every written row holds a draw
+    c-hat + L^-T z, z ~ N(0, I), of the coefficients' conditional posterior at that row's parameters, seeded from the
+    sampler seed.
 """
 from __future__ import annotations
 
@@ -100,6 +106,8 @@ class FitPayne(object):
                 on.append('Vmic')
             for pp in on:
                 self.fitpars_bool[pp] = True
+            if sp.get('modpoly_marginal', False) and not sp.get('modpoly', False):
+                raise ValueError("spec['modpoly_marginal'] needs spec['modpoly']")
             if sp.get('modpoly', False):                                   # fitstar.py:110-147
                 self.modpoly_bool = True
                 if 'blaze_coeff' in self.priordict:
@@ -112,9 +120,13 @@ class FitPayne(object):
                 self.priordict['blaze_coeff'] = self.polycoefarr
                 self.polyorder = len(self.polycoefarr)
                 fa['norm_polyorder'] = self.polyorder
-                for ii in range(self.polyorder):
-                    self.fitpars.append('pc_{}'.format(ii))
-                    self.fitpars_bool['pc_{}'.format(ii)] = True
+                if sp.get('modpoly_marginal', False):
+                    fa['cont_names'] = ['pc_{}'.format(ii) for ii in range(self.polyorder)]
+                    fa['cont_box'] = [self.prior.pc_box(ii, self.polycoefarr) for ii in range(self.polyorder)]
+                else:
+                    for ii in range(self.polyorder):
+                        self.fitpars.append('pc_{}'.format(ii))
+                        self.fitpars_bool['pc_{}'.format(ii)] = True
 
         if 'phot' in inputdict:                                            # fitstar.py:157-190
             self.phot_bool = True
@@ -182,7 +194,14 @@ class FitPayne(object):
             self.fitpars_bool['Inst_R_%d' % s] = True
         if len({bool(sp.get('modpoly', False)) for sp in specs}) > 1:
             raise ValueError('every spectrum has a continuum polynomial (modpoly) or none does')
+        if len({bool(sp.get('modpoly_marginal', False)) for sp in specs}) > 1:
+            raise ValueError('every spectrum sets modpoly_marginal or none does')
         self.modpoly_bool = bool(specs[0].get('modpoly', False))
+        marginal = bool(specs[0].get('modpoly_marginal', False))
+        if marginal and not self.modpoly_bool:
+            raise ValueError("spec['modpoly_marginal'] needs spec['modpoly']")
+        if marginal:
+            fa['cont_names'] = []
         for s, sp in enumerate(specs):
             if not self.modpoly_bool:
                 break
@@ -192,7 +211,12 @@ class FitPayne(object):
                     self.priordict[key] = [[0.0, sp.get('polysigma', 1.0)] for _ in range(sp['polyorder'] + 1)]
                 else:
                     self.priordict[key] = [[0.0, 1.0] for _ in range(3)]
-            for k in range(len(self.priordict[key])):
+            K = len(self.priordict[key])
+            if marginal:
+                fa['spectra'][s]['cont_box'] = [self.prior.pc_box(k, self.priordict[key]) for k in range(K)]
+                fa['cont_names'] += ['pc_%d_%d' % (s, k) for k in range(K)]
+                continue
+            for k in range(K):
                 self.fitpars.append('pc_%d_%d' % (s, k))
                 self.fitpars_bool['pc_%d_%d' % (s, k)] = True
 
@@ -234,13 +258,40 @@ class FitPayne(object):
         self.outff.write('log(lk) log(vol) log(wt) h nc log(z) delta(log(z))')
         self.outff.write('\n')
 
-    def _writerow(self, it, vstar, parnames, tail):
+    def _writerow(self, it, vstar, parnames, tail, cont=None):
         pd = {pp: vv for pp, vv in zip(self.likeobj.fitpars_i, vstar)}
+        if cont is not None:
+            pd.update(zip(self.fitargs['cont_names'], cont))
         pd.update(self.likeobj.fixedpars)
         self.outff.write('{0} '.format(it))
         self.outff.write(' '.join([str(pd[q]) for q in parnames]))
         self.outff.write(' {0} {1} {2} {3} {4} {5} {6} '.format(*tail))
         self.outff.write('\n')
+
+    def _cont_boxes(self):
+        """The boxes of the marginalised coefficients in ``cont_names`` order, and every spectrum's count."""
+        fa = self.fitargs
+        per = [sp['cont_box'] for sp in fa['spectra']] if 'spectra' in fa else [fa['cont_box']]
+        return [b for p in per for b in p], [len(p) for p in per]
+
+    def _cont_draws(self, V):
+        """A draw c-hat + L^-T z, z ~ N(0, I), of the marginalised coefficients at every row of V (one batched call);
+        counts the rows whose c-hat leaves its box."""
+        coef, chol = self.likeobj.cont_batch(V)
+        boxes, orders = self._cont_boxes()
+        lo, hi = np.array([b[0] for b in boxes]), np.array([b[1] for b in boxes])
+        self._cont_outside += int(np.sum(np.any((coef[:, :len(boxes)] < lo) | (coef[:, :len(boxes)] > hi), axis=1)))
+        out = np.empty((len(V), len(boxes)))
+        c0 = l0 = 0
+        for K in orders:
+            L = np.zeros((len(V), K, K))
+            i, j = np.tril_indices(K)
+            L[:, i, j] = chol[:, l0:l0 + K * (K + 1) // 2]
+            z = self._cont_rng.standard_normal((len(V), K, 1))
+            out[:, c0:c0 + K] = coef[:, c0:c0 + K] + np.linalg.solve(np.transpose(L, (0, 2, 1)), z)[..., 0]
+            c0 += K
+            l0 += K * (K + 1) // 2
+        return out
 
     def _runsampler(self, samplerdict):
         npoints = samplerdict.get('npoints', 200)
@@ -264,18 +315,38 @@ class FitPayne(object):
                                        reflective=reflective, seed=samplerdict.get('seed', None))
         # several spectra: an LSF vector (one value per pixel, the same in every row) gets no column
         multi = 'spectra' in self.fitargs
-        parnames = list(self.likeobj.fitpars_i) + [kk for kk, vv in self.likeobj.fixedpars.items()
-                                                    if not (multi and np.ndim(vv) > 0)]
+        cont_names = self.fitargs.get('cont_names')
+        parnames = list(self.likeobj.fitpars_i) + list(cont_names or []) + \
+            [kk for kk, vv in self.likeobj.fixedpars.items() if not (multi and np.ndim(vv) > 0)]
         self._initoutput(parnames)
+        # marginalised continuum: rows wait for one batched call per flush that draws their coefficients
+        pending = []
+        self._cont_rng = np.random.default_rng(samplerdict.get('seed', None))
+        self._cont_outside = 0
+
+        def write(it, vstar, tail):
+            if cont_names is None:
+                self._writerow(it, vstar, parnames, tail)
+            else:
+                pending.append((it, vstar, tail))
+
+        def flush():
+            if pending:
+                draws = self._cont_draws(np.array([r[1] for r in pending], dtype=np.float64))
+                for (it, vstar, tail), c in zip(pending, draws):
+                    self._writerow(it, vstar, parnames, tail, c)
+                del pending[:]
+            self.outff.flush()
+
         ncall, nit = 0, 0
         for it, res in enumerate(sampler.sample(dlogz=delta_logz_final, maxiter=maxiter, maxcall=maxcall)):
             (worst, ustar, vstar, loglstar, logvol, logwt, logz, logzvar, h, nc, worst_it, propidx, propiter, eff,
              delta_logz) = res
-            self._writerow(it, vstar, parnames, (loglstar, logvol, logwt, h, nc, logz, delta_logz))
+            write(it, vstar, (loglstar, logvol, logwt, h, nc, logz, delta_logz))
             ncall += nc
             nit = it
             if (it % flushnum) == 0 or it == maxiter:
-                self.outff.flush()
+                flush()
                 if self.verbose and (it % (50 * flushnum)) == 0:
                     logzerr = np.sqrt(logzvar) if logzvar > 0.0 else np.nan
                     sys.stdout.write('iter: {0:d} | nc: {1:d} | ncall: {2:d} | eff(%): {3:6.3f} | logz: {4:6.3f} +/- '
@@ -288,8 +359,12 @@ class FitPayne(object):
         for it2, res in enumerate(sampler.add_live_points()):
             (worst, ustar, vstar, loglstar, logvol, logwt, logz, logzvar, h, nc, worst_it, boundidx, bounditer, eff,
              delta_logz) = res
-            self._writerow(nit + it2, vstar, parnames, (loglstar, logvol, logwt, h, nc, logz, delta_logz))
+            write(nit + it2, vstar, (loglstar, logvol, logwt, h, nc, logz, delta_logz))
+        flush()
         self.outff.close()
+        if self.verbose and cont_names is not None:
+            print('{0} written rows have a best-fitting continuum coefficient outside its box'.format(
+                self._cont_outside))
         if self.verbose:
             print('RUN TIME: {0}  ({1} likelihood evaluations in {2} batched calls)'.format(
                 datetime.now() - starttime, sampler.ncall, len(sampler.batch_sizes)))

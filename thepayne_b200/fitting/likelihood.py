@@ -8,6 +8,9 @@ expects (fitstar.py:342-348).
 A fixed ``Inst_R`` that is a 1-D array is the LSF vector of the observation (one dispersion per observed
 pixel), as in the reference: lnlikefn passes it on to genspec, which hands a non-float ``inst_R`` to getspec's
 LSF branch (genmod.py:82-85, predictspec.py:265-286).
+
+``fitargs['cont_box']`` (``FitPayne`` with ``spec['modpoly_marginal']``) integrates the continuum coefficients out
+(``Engine.set_cont_marg``); ``cont_batch`` gives their best-fitting values and Cholesky factors.
 """
 from __future__ import annotations
 
@@ -49,7 +52,7 @@ class likelihood(object):
             obs_eflux=fitargs.get('obs_eflux_fit'), obs_phot=fitargs.get('obs_phot'),
             fitpars_i=self.fitpars_i, fixedpars=self.fixedpars,
             runbools=[self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
-            precision=self.precision, device=kwargs.get('device'))
+            precision=self.precision, device=kwargs.get('device'), cont_box=fitargs.get('cont_box'))
         self._explicit = None
 
     # ------------------------------------------------------------------ reference entry points
@@ -99,6 +102,11 @@ class likelihood(object):
                          precision=self.precision)
             self._explicit = (key, eng)
         return float(self._explicit[1].lnlike_batch(np.array([vals], dtype=np.float64))[0])
+
+    def cont_batch(self, theta):
+        """Marginalised continuum: c-hat [B, K] and the packed Cholesky factors [B, K(K+1)/2] (numpy)."""
+        coef, chol, _, _ = self.engine.cont_batch(theta)
+        return coef.cpu().numpy(), chol.cpu().numpy()
 
     # ------------------------------------------------------------------ batched entry point
     def lnlike_batch(self, theta):

@@ -9,6 +9,9 @@ spectrum's layout reads its own columns under the reference's names (``Inst_R_<s
 of spectrum s gives.  ``fitargs['spectra']`` is the list of ``{'obs_wave_fit', 'obs_flux_fit', 'obs_eflux_fit'}``
 (``FitPayne`` builds it from a list-valued ``inputdict['spec']``).
 
+``fitargs['spectra'][s]['cont_box']`` (``FitPayne`` with ``modpoly_marginal``) integrates spectrum s's continuum
+coefficients out (``Engine.set_cont_marg``); ``cont_batch`` gives every spectrum's best-fitting values back to back.
+
 A fixed ``Inst_R_<s>`` that is a 1-D array is spectrum s's LSF vector, one dispersion (AA) per fitted pixel of that
 spectrum, as a fixed ``Inst_R`` array is in the single-spectrum ``likelihood``.  Every spectrum has one or none does.
 """
@@ -74,7 +77,8 @@ class MultiSpecLikelihood(object):
             poly = any(p.startswith('pc_') for p in fit)
             st = {'wave': sp['obs_wave_fit'], 'flux': sp['obs_flux_fit'], 'eflux': sp['obs_eflux_fit'],
                   'fitpars_i': fit, 'fixedpars': fixed,
-                  'runbools': [True, bool(self.phot_bool) and s == 0, poly, bool(self.photscale_bool)]}
+                  'runbools': [True, bool(self.phot_bool) and s == 0, poly, bool(self.photscale_bool)],
+                  'cont_box': sp.get('cont_box')}
             if self.phot_bool and s == 0:
                 st['phot'] = fitargs['obs_phot']
             stars.append(st)
@@ -95,6 +99,11 @@ class MultiSpecLikelihood(object):
         self._set_parsdict(pars)
         th = np.asarray(pars, dtype=np.float64).reshape(1, self.ndim)
         return float(self.engine.lnlike_batch_targets(th, np.zeros(1, np.int32))[0])
+
+    def cont_batch(self, theta):
+        """Marginalised continua: every spectrum's c-hat and packed Cholesky factor back to back (numpy)."""
+        coef, chol, _, _ = self.engine.cont_batch_targets(theta, np.zeros(len(theta), np.int32))
+        return coef.cpu().numpy(), chol.cpu().numpy()
 
     def lnlike_batch(self, theta):
         """theta [B, ndim] (CUDA float64 tensor, or numpy) -> lnL [B] of the same kind."""

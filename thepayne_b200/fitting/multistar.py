@@ -106,7 +106,8 @@ class StarSetLikelihood(object):
         stars = [{'wave': fa.get('obs_wave_fit'), 'flux': fa.get('obs_flux_fit'), 'eflux': fa.get('obs_eflux_fit'),
                   'phot': fa.get('obs_phot') if rb[1] else None,
                   'bands': list(fa['obs_phot'].keys()) if rb[1] else None,
-                  'fixedpars': dict(fa.get('fixedpars', {}))} for fa, rb in zip(fitargs_list, rb_list)]
+                  'fixedpars': dict(fa.get('fixedpars', {})), 'cont_box': fa.get('cont_box')}
+                 for fa, rb in zip(fitargs_list, rb_list)]
         if any(free != free0 for free in free_list) or any(rb != rb0 for rb in rb_list):
             for st, free, rb in zip(stars, free_list, rb_list):     # each star's own layout
                 st['fitpars_i'], st['runbools'] = free, rb
@@ -119,11 +120,19 @@ class StarSetLikelihood(object):
         self.star_fitpars_i, self.star_ndim = self.engine.star_fitpars_i, self.engine.star_ndim
         self.ndim = self.engine.ndim                      # the largest star's: the width of a batch row
         self.ncalls = 0                                   # lnlike_batch calls made on the engine
+        self._lock = threading.Lock()                     # the samplers' threads share the engine
 
     def lnlike_batch(self, theta, star):
         """theta [B, ndim] and star [B] (CUDA tensors or numpy, as ``Engine.lnlike_batch``) -> lnL [B]."""
-        self.ncalls += 1
-        return self.engine.lnlike_batch(theta, star)
+        with self._lock:
+            self.ncalls += 1
+            return self.engine.lnlike_batch(theta, star)
+
+    def cont_batch(self, theta, star):
+        """Marginalised continua (a star's ``cont_box``): c-hat and packed Cholesky factors of every row (numpy)."""
+        with self._lock:
+            coef, chol, _, _ = self.engine.cont_batch(theta, star)
+            return coef.cpu().numpy(), chol.cpu().numpy()
 
     def star(self, k):
         """Star k with the interface of ``likelihood.likelihood``."""
@@ -181,6 +190,10 @@ class StarView(object):
         self._set_parsdict(pars)
         th = np.asarray(pars, dtype=np.float64).reshape(1, self.ndim)
         return float(self._lnlike(th)[0])
+
+    def cont_batch(self, theta):
+        theta = self._pad(np.asarray(theta, dtype=np.float64))
+        return self.owner.cont_batch(theta, np.full(len(theta), self.k, dtype=np.int32))
 
     def lnlike_batch(self, theta):
         out = self._lnlike(theta)

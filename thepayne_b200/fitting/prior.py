@@ -66,6 +66,14 @@ class prior(object):
         self.defaultpars.update({p + '_sec': self.defaultpars[p] for p in _SPEC[:6]})
 
     # ------------------------------------------------------------------ unit cube -> parameters
+    @staticmethod
+    def pc_box(k, polycoefarr):
+        """(lo, hi) of continuum coefficient k (prior.py:187-197): [0.75, 1.25] for k = 0, blaze_coeff[k]'s mean +- 5
+        sigma otherwise.  The uniform prior of a sampled ``pc_k`` and the box of a marginalised one."""
+        if k == 0:
+            return 0.75, 1.25
+        return polycoefarr[k][0] - 5.0 * polycoefarr[k][1], polycoefarr[k][0] + 5.0 * polycoefarr[k][1]
+
     def _transform(self, name, u, iso):
         """One named parameter, scalar or array ``u`` (prior.py:150-176 / :226-268)."""
         pd = self.priordict
@@ -97,20 +105,12 @@ class prior(object):
             if m.group(1) == 'Inst_R' and m.group(3) is None:
                 return self._transform(name, u, iso=False)
             if m.group(1) == 'pc' and m.group(3) is not None:
-                k = int(m.group(3))
-                if k == 0:
-                    return (1.25 - 0.75) * u + 0.75
-                c = self.spectrum_polycoef[int(m.group(2))][k]
-                pcmax, pcmin = c[0] + 5.0 * c[1], c[0] - 5.0 * c[1]
+                pcmin, pcmax = self.pc_box(int(m.group(3)), self.spectrum_polycoef[int(m.group(2))])
                 return (pcmax - pcmin) * u + pcmin
         if 'pc' in name:
             if not self.spec_bool:
                 raise KeyError(name)
-            if name == 'pc_0':
-                return (1.25 - 0.75) * u + 0.75
-            k = int(name.split('_')[-1])
-            pcmax = self.polycoefarr[k][0] + 5.0 * self.polycoefarr[k][1]
-            pcmin = self.polycoefarr[k][0] - 5.0 * self.polycoefarr[k][1]
+            pcmin, pcmax = self.pc_box(int(name.split('_')[-1]), self.polycoefarr)
             return (pcmax - pcmin) * u + pcmin
         if self.spec_bool and (name in _SPEC or name in _BINARY):
             return self._transform(name, u, iso=False)
