@@ -337,6 +337,21 @@ def test_old_entries_unchanged_by_a_binary():
     binr.close()
 
 
+def test_removing_marginalisation_keeps_the_binary():
+    """binaries and continuum marginalisation share the per-CTA a_j scratch: clearing the one that is off keeps it"""
+    spec = _emulator(13)
+    eng = _engine(spec, 2)
+    th = _theta(300, 4, 2)
+    lnl = eng.lnlike_batch_binary(th)
+    flux, comp, lm = _np(*eng.model_batch_binary(th))
+    eng.set_cont_marg(None)
+    assert np.array_equal(eng.lnlike_batch_binary(th), lnl, equal_nan=True)
+    f2, c2, l2 = _np(*eng.model_batch_binary(th))
+    assert np.array_equal(f2, flux, equal_nan=True) and np.array_equal(c2, comp, equal_nan=True)
+    assert np.array_equal(l2, lm, equal_nan=True) and np.isfinite(lnl).any()
+    eng.close()
+
+
 # ------------------------------------------------------------------ the likelihood and a fit
 TRUTH = {'Teff': 5900.0, 'log(g)': 4.3, '[Fe/H]': 0.0, '[a/Fe]': 0.0, 'Vrad': -15.0, 'Vrot': 4.0, 'Inst_R': 32000.0,
          'Teff_sec': 4700.0, 'log(g)_sec': 4.6, 'Vrad_sec': 35.0, 'Vrot_sec': 2.0, 'Rratio': 0.8, 'pc_0': 1.0}

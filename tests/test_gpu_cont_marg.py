@@ -356,6 +356,21 @@ def test_failures_and_refusals():
     assert code(lambda: nonlog.set_cont_marg([_box(2)])) == _UNSUPPORTED              # grid without the fast tail
 
 
+def test_removing_binaries_keeps_marginalisation():
+    """binaries and continuum marginalisation share the per-CTA a_j scratch: clearing the one that is off keeps it"""
+    spec = _emulator(13)
+    marg, samp = _pair(spec, 3, 'free', _obs(spec, seed=4))
+    th = _rows(300, marg.ndim, seed=4)
+    lnl = marg.lnlike_batch(th)
+    cont = [_np(t) for t in marg.cont_batch(th)]
+    marg.set_binary(False)
+    assert np.array_equal(marg.lnlike_batch(th), lnl, equal_nan=True) and np.isfinite(lnl).any()
+    for a, b in zip(marg.cont_batch(th), cont):
+        assert np.array_equal(_np(a), b, equal_nan=True)
+    marg.close()
+    samp.close()
+
+
 # ------------------------------------------------------------------ FitPayne, sampled against marginal coefficients
 
 TRUTH = {'Teff': 5770.0, 'log(g)': 4.44, '[Fe/H]': 0.0, '[a/Fe]': 0.0, 'Vrad': 0.5, 'Vrot': 3.0, 'Inst_R': 32000.0}

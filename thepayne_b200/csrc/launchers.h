@@ -40,43 +40,25 @@ int tc_run_scaled_layer_x(const TcWeights& w, const float* bias, const float* h,
 int tc_gemm_test_x(const float* dA, int M, int N, int K, int precision, TcActs& a, const TcWeights& w,
                    const float* dbias, float* dC, int sm_count);
 
-// ---- tail_fast_tu.cu: fused tail on log-uniform grids (tail_fast.cuh)
-// sets the dynamic shared-memory opt-in of tail_fast_kernel<l2> on the current device and reports the
-// resident CTAs per SM; false when the kernel does not exist for l2 or the query fails
-// (two instantiations per size, in two translation units: without / with continuum polynomial or model output
-// in the final pass; the probe covers both and reports the smaller occupancy)
-bool probe_tail_fast(int l2, size_t smem_bytes, int* ctas_per_sm);
-int launch_tail_fast(int l2, bool poly, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
+// ---- tail_fast_tu.cu / tail_fast_poly_tu.cu: fused tail on log-uniform grids (tail_fast.cuh)
+// One form of tail_fast_kernel per kind of batch: points naming stars, targets (payne_ctx_set_targets), binaries
+// (payne_ctx_set_binary) and continuum marginalisation (payne_ctx_set_cont_marg, for points or targets).  Each size
+// has a form's instantiations in two translation units: without (tail_fast_tu.cu) and with (tail_fast_poly_tu.cu)
+// continuum polynomial or model output in the final pass; Binary and Marg exist with them only.
+enum class FastForm { Point, Target, Binary, Marg };
+// sets the dynamic shared-memory opt-in of every instantiation `form` may launch at 2^l2 samples on the current device
+// and reports the smallest of their resident CTAs per SM; false when the kernel does not exist for l2 or a query fails
+bool probe_tail_fast(int l2, FastForm form, size_t smem_bytes, int* ctas_per_sm);
+// the instantiation follows from T: polynomial or model output (T.n_poly, T.model_out), several stars (Point,
+// T.n_stars > 1) or targets (Marg, T.target)
+int launch_tail_fast(int l2, FastForm form, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
+// the per-point setup of a slab of nb points: one item per point, per (point, member) of a target (Target, or Marg
+// with T.target) or per (point, component) of a binary
+int launch_tail_setup(FastForm form, int nb, cudaStream_t st, const TailParams& T, const FastGrid& F);
 // copies the first-pass constants into the translation units' __constant__ memory on the current device
 // (call once per context, before the first launch)
 int init_tail_fast(const TwConst& tc);
-int init_tail_fast_plain(const TwConst& tc);
-int init_tail_fast_poly(const TwConst& tc);
 int init_tail_cluster(const TwConst& tc);
-bool probe_tail_fast_plain(int l2, size_t smem_bytes, int* ctas_per_sm);
-bool probe_tail_fast_poly(int l2, size_t smem_bytes, int* ctas_per_sm);
-int launch_tail_fast_plain(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
-int launch_tail_fast_poly(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
-int launch_tail_setup(int nb, cudaStream_t st, const TailParams& T, const FastGrid& F);
-// targets (payne_ctx_set_targets): the TGT instantiations of tail_fast_kernel and the per-(point, member) setup
-bool probe_tail_fast_targets(int l2, size_t smem_bytes, int* ctas_per_sm);
-bool probe_tail_fast_targets_plain(int l2, size_t smem_bytes, int* ctas_per_sm);
-bool probe_tail_fast_targets_poly(int l2, size_t smem_bytes, int* ctas_per_sm);
-int launch_tail_fast_targets(int l2, bool poly, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T,
-                             const FastGrid& F);
-int launch_tail_fast_targets_plain(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
-int launch_tail_fast_targets_poly(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
-int launch_tail_setup_targets(long long items, cudaStream_t st, const TailParams& T, const FastGrid& F);
-// binaries (payne_ctx_set_binary): the BIN instantiation of tail_fast_kernel (tail_fast_poly_tu.cu) and the
-// per-(point, component) setup of a slab of nb points
-bool probe_tail_fast_binary(int l2, size_t smem_bytes, int* ctas_per_sm);
-int launch_tail_fast_binary(int l2, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
-int launch_tail_setup_binary(int nb, cudaStream_t st, const TailParams& T, const FastGrid& F);
-// continuum marginalisation (payne_ctx_set_cont_marg): the MARG instantiations of tail_fast_kernel (tail_fast_poly_tu.cu),
-// for points naming stars and (targets = true) targets; their setup is launch_tail_setup / launch_tail_setup_targets
-bool probe_tail_fast_marg(int l2, size_t smem_bytes, int* ctas_per_sm);
-int launch_tail_fast_marg(int l2, bool targets, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T,
-                          const FastGrid& F);
 
 // ---- tail_cluster_tu.cu: the same tail with one transform spread over a cluster of four CTAs (tail_cluster.cuh;
 // emulator grids above 16384 pixels).  max_clusters = co-resident clusters on the device.

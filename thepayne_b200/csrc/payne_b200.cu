@@ -147,7 +147,8 @@ struct PayneCtx {
   payne::FastGrid fast{};
   size_t tail_smem = 0;
   size_t fast_smem = 0;      // tail_smem + rotation-table window (fast kernels)
-  int tail_grid = 0, tail_grid_fast = 0;
+  int tail_grid = 0;
+  int fast_grid[4] = {0, 0, 0, 0};   // CTAs of the fast tail of every payne::FastForm (form_grid), 0 until probed
   int grid_loguniform = 0;
   int use_fast = 0;        // analytic-regrid tail selected (log-uniform emulator grid)
   int allow_fast = 1;
@@ -177,29 +178,27 @@ struct PayneCtx {
   std::vector<double> star_fixed_h;     // host copies of star_fixed_dev / star_lay_dev (empty without them)
   std::vector<payne::StarLayout> star_lay_h;
   // targets (payne_ctx_set_targets): runs of consecutive stars that describe one physical star
-  int n_targets = 0, tgt_kmax = 0, tgt_grid = 0;   // tgt_grid: CTAs of the fast target kernel, 0 until it is probed
+  int n_targets = 0, tgt_kmax = 0;
   bool tgt_lsf_probed = false;          // the LSF target kernel's shared-memory opt-in is set
   std::string tgt_instr_col;            // the first member with an Inst_R column (refused beside LSF vectors), or empty
   long long tgt_nobs_max = 0;           // the largest sum of the members' n_obs (model row of a target)
   int* tfirst_dev = nullptr;            // [n_targets + 1]
   std::vector<int> tfirst_h;            // its host copy
-  payne::FastPoint* tgt_points = nullptr;   // [tgt_rows * tgt_kmax] per-(point, member) records (fast tail only)
-  int* tgt_star = nullptr;              // [tgt_rows] first member's star of every point of a slab
-  long long tgt_rows = 0, tgt_rec_alloc = 0;
-  // binaries (payne_ctx_set_binary): the secondary's description, the binary tail's grid and its workspace
+  // per-mode buffers (resize_buffer; *_n: elements allocated)
+  payne::FastPoint* tgt_points = nullptr;   // [rows * tgt_kmax] per-(point, member) records of a slab (fast tail only)
+  int* tgt_star = nullptr;              // [rows] first member's star of every point of a slab
+  double* bin_par = nullptr;            // [rows, 3] Teff_1, Teff_2, Rratio of the points of a slab (binaries)
+  double* aj_scratch = nullptr;         // [grid, n_obs_max] a_j of every CTA's current point (binaries or continuum
+                                        // marginalisation, which never go together; grid: that form's)
+  long long tgt_points_n = 0, tgt_star_n = 0, bin_par_n = 0, aj_scratch_n = 0;
+  // binaries (payne_ctx_set_binary): the secondary's description
   bool has_binary = false;
   PayneBinary* binary_dev = nullptr;
-  int bin_grid = 0;
-  double* bin_scratch = nullptr;        // [bin_grid, n_obs_max] a_1 of every CTA's current point
-  double* bin_par = nullptr;            // [bin_rows, 3] Teff_1, Teff_2, Rratio of the points of a slab
-  long long bin_rows = 0;
-  // continuum marginalisation (payne_ctx_set_cont_marg): every star's K and C, the MARG kernels' grid and their scratch
+  // continuum marginalisation (payne_ctx_set_cont_marg): every star's K and C
   bool has_marg = false;
   std::vector<int> marg_k_h;            // [n_stars] K of every star
   int* marg_k_dev = nullptr;
   double* marg_c_dev = nullptr;         // [n_stars] sum_k (ln(2 pi) / 2 - ln w_k)
-  int marg_grid = 0;
-  double* marg_scratch = nullptr;       // [marg_grid, n_obs_max] a_j of every CTA's current point
   // photometry
   bool has_phot = false;
   payne::PhotParams phot{};
@@ -495,7 +494,7 @@ int build_tail(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs) {
     // costs one wavefront instead of one per touched line).  Take the largest slice that does not
     // cost a resident CTA.
     int occf = 0;
-    auto probe = [&](size_t bytes, int* occ) { return payne::probe_tail_fast(l2, bytes, occ); };
+    auto probe = [&](size_t bytes, int* occ) { return payne::probe_tail_fast(l2, payne::FastForm::Point, bytes, occ); };
     int occ0 = 0;
     const bool ok0 = probe(c->tail_smem, &occ0);
     size_t win = 0;
@@ -510,7 +509,7 @@ int build_tail(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs) {
     c->fast_smem = c->tail_smem + win;
     c->fast.win_floats = (int)(win / 4);
     probe(c->fast_smem, &occf);
-    c->tail_grid_fast = occf * c->sm_count;
+    c->fast_grid[(int)payne::FastForm::Point] = occf * c->sm_count;
     {
       const char* denv = getenv("PAYNE_TAIL_DYNAMIC");       // "0": static round robin of points over the CTAs
       if (!(denv && denv[0] == '0')) {
@@ -523,7 +522,7 @@ int build_tail(PayneCtx* c, const PayneSpecNet* s, const PayneObs* obs) {
     }
     if (c->use_fast && l2 >= 16) {
       float* sc = nullptr;
-      CU_TRY(cudaMalloc((void**)&sc, (size_t)c->tail_grid_fast * (N1 / 2) * sizeof(float)));
+      CU_TRY(cudaMalloc((void**)&sc, (size_t)c->fast_grid[(int)payne::FastForm::Point] * (N1 / 2) * sizeof(float)));
       c->owned.push_back(sc);
       c->fast.scratch = sc;
     }
@@ -934,100 +933,129 @@ __global__ void target_star_kernel(const int* target, const int* tfirst, int n_t
 // members up inside the kernel and has no records.
 constexpr long long kTargetRecords = 65536;
 
-int ensure_target_workspace(PayneCtx* c, long long rows, bool records) {
-  const long long rec = records ? rows * c->tgt_kmax : 0;
-  if (rows <= c->tgt_rows && rec <= c->tgt_rec_alloc) return PAYNE_OK;
-  CU_TRY(cudaDeviceSynchronize());                       // earlier calls may still read the records
-  if (c->tgt_points) cudaFree(c->tgt_points);
-  if (c->tgt_star) cudaFree(c->tgt_star);
-  c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
-  if (rec) {
-    CU_TRY(cudaMalloc((void**)&c->tgt_points, (size_t)rec * sizeof(payne::FastPoint)));
-    CU_TRY(cudaMemset(c->tgt_points, 0, (size_t)rec * sizeof(payne::FastPoint)));
-  }
-  CU_TRY(cudaMalloc((void**)&c->tgt_star, (size_t)rows * sizeof(int)));
+// Grows the per-mode buffer *p to at least n zeroed elements, or frees it (n = 0); *have counts what it holds.  Earlier
+// calls may still read the old buffer, so the device is synchronised before it is freed.
+template <class T>
+int resize_buffer(T** p, long long* have, long long n) {
+  if (n > 0 ? n <= *have : !*p) return PAYNE_OK;
   CU_TRY(cudaDeviceSynchronize());
-  c->tgt_rows = rows; c->tgt_rec_alloc = rec;
+  if (*p) cudaFree(*p);
+  *p = nullptr; *have = 0;
+  if (n > 0) {
+    CU_TRY(cudaMalloc((void**)p, (size_t)n * sizeof(T)));
+    CU_TRY(cudaMemset(*p, 0, (size_t)n * sizeof(T)));
+    CU_TRY(cudaDeviceSynchronize());
+    *have = n;
+  }
   return PAYNE_OK;
 }
 
-// Binaries: Teff_1, Teff_2 and Rratio of the points of a slab of `rows` points
-int ensure_binary_workspace(PayneCtx* c, long long rows) {
-  if (rows <= c->bin_rows) return PAYNE_OK;
-  CU_TRY(cudaDeviceSynchronize());                       // earlier calls may still read them
-  if (c->bin_par) cudaFree(c->bin_par);
-  c->bin_par = nullptr; c->bin_rows = 0;
-  CU_TRY(cudaMalloc((void**)&c->bin_par, (size_t)rows * 3 * sizeof(double)));
-  c->bin_rows = rows;
+// CTAs of the fast tail of `form`: the Point grid from build_tail, the others probed when first needed and capped at
+// it (the split kernel's scratch lines exist for that many CTAs).
+int form_grid(PayneCtx* c, payne::FastForm form, int* grid) {
+  int& g = c->fast_grid[(int)form];
+  if (g == 0 && form != payne::FastForm::Point) {
+    static const char* const what[] = {"", "target", "binary", "continuum marginalisation"};
+    int occ = 0;
+    if (!payne::probe_tail_fast(c->tail.log2N1, form, c->fast_smem, &occ) || occ < 1)
+      return fail(PAYNE_E_UNSUPPORTED, std::string(what[(int)form]) + " tail kernel does not fit on an SM");
+    g = std::min(occ * c->sm_count, c->fast_grid[(int)payne::FastForm::Point]);
+  }
+  *grid = g;
   return PAYNE_OK;
 }
 
-// star: [B] star index of every point (null: star 0); flux_out rows are ld_flux apart.  target: see above; chi2_out
-// [B, ld_chi2] the chi2 of every member (targets only).  binary: every point is a binary (payne_ctx_set_binary), the
-// emulator runs 2 nb rows per slab of nb points; comp_out [B, 2, ld_flux] its components' spectra.
+// One call's points and outputs, as an extern "C" entry passes them.
+//   star: [B] star index of every point (null: star 0); target: [B] target of every point instead (payne_ctx_set_targets;
+//   star is then unused).  binary: every point is a binary (payne_ctx_set_binary): the emulator runs 2 nb rows per slab
+//   of nb points.
+//   Outputs (null: not wanted): flux [B, ld_flux] model rows; mags; chi2 [B, ld_chi2] the chi2 of every member
+//   (targets), or every point's Q (continuum marginalisation, ld_chi2 = 1 for points naming stars); comp [B, 2, ld_flux]
+//   a binary's components' spectra; coef [B, ld_coef] c-hat and chol [B, ld_chol] the packed Cholesky factor of every
+//   point (payne_ctx_set_cont_marg).
+struct Batch {
+  const double* theta = nullptr; long long B = 0, ld = 0;
+  double* lnl = nullptr;
+  const int* star = nullptr;
+  const int* target = nullptr;
+  bool binary = false;
+  double* flux = nullptr; long long ld_flux = 0;
+  double* mags = nullptr;
+  double* chi2 = nullptr; long long ld_chi2 = 0;
+  double* comp = nullptr;
+  double* coef = nullptr; long long ld_coef = 0;
+  double* chol = nullptr; long long ld_chol = 0;
+};
+
 int marg_unsupported(PayneCtx* c);
 
-// coef_out / chol_out (continuum marginalisation, payne_ctx_set_cont_marg): [B, ld_coef] c-hat and [B, ld_chol] the
-// packed Cholesky factor of every point; chi2_out is then every point's Q (ld_chi2 = 1 for points naming stars).
-int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, long long ld, double* flux_out,
-              long long ld_flux, double* mags_out, double* lnl, cudaStream_t st, const int* target = nullptr,
-              double* chi2_out = nullptr, long long ld_chi2 = 0, bool binary = false, double* comp_out = nullptr,
-              double* coef_out = nullptr, long long ld_coef = 0, double* chol_out = nullptr, long long ld_chol = 0) {
+int run_batch(PayneCtx* c, const Batch& q, cudaStream_t st) {
   using namespace payne;
+  const long long B = q.B, ld = q.ld;
   if (B <= 0) return PAYNE_OK;
   const bool marg = c->has_marg;
   if (marg) { int rc = marg_unsupported(c); if (rc) return rc; }
   if (ld < c->ndim_max) return fail(PAYNE_E_INVALID, "ld < ndim (the largest star's with per-star layouts)");
-  if (!target && flux_out && c->has_spec && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
-  const bool records = target && !c->lsf_on;             // the fast target tail's per-(point, member) records
+  if (!q.target && q.flux && c->has_spec && q.ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
+  const bool records = q.target && !c->lsf_on;           // the fast target tail's per-(point, member) records
   const long long slab = records ? std::min(c->slab, std::max(1LL, kTargetRecords / c->tgt_kmax))
-                       : binary ? std::max(1LL, c->slab / 2) : c->slab;
-  int rc = ensure_workspace(c, binary ? 2 * B : B);
+                       : q.binary ? std::max(1LL, c->slab / 2) : c->slab;
+  const long long rows = std::min(B, slab);
+  int rc = ensure_workspace(c, q.binary ? 2 * B : B);
+  if (!rc && q.target) rc = resize_buffer(&c->tgt_star, &c->tgt_star_n, rows);
+  if (!rc && records) rc = resize_buffer(&c->tgt_points, &c->tgt_points_n, rows * c->tgt_kmax);
+  if (!rc && q.binary) rc = resize_buffer(&c->bin_par, &c->bin_par_n, rows * 3);
   if (rc) return rc;
-  if (target) { rc = ensure_target_workspace(c, std::min(B, slab), records); if (rc) return rc; }
-  if (binary) { rc = ensure_binary_workspace(c, std::min(B, slab)); if (rc) return rc; }
+  // The tail: the LSF-vector tail, else the fast tail in the batch's form (points naming stars may run it
+  // cluster-distributed) on line-depth rows, else the general-grid tail (points naming stars only).
+  const bool fast_tail = c->has_spec && c->use_fast && c->allow_fast && !c->lsf_on;
+  const FastForm form = marg ? FastForm::Marg : q.target ? FastForm::Target : q.binary ? FastForm::Binary : FastForm::Point;
+  const bool cluster = form == FastForm::Point && c->use_cluster && c->allow_cluster;
+  int fgrid = 0;
+  if (fast_tail) { rc = form_grid(c, form, &fgrid); if (rc) return rc; }
   rc = order_after_previous(c, st);
   if (rc) return rc;
   if (c->timing) { c->ms_acc[0] = c->ms_acc[1] = c->ms_acc[2] = 0; c->ms_valid = false; c->pending.clear(); }
   for (long long p0 = 0; p0 < B; p0 += slab) {
     const int nb = (int)std::min(slab, B - p0);
-    if (target) {
+    if (q.target) {
       // the emulators and the photometry see every point as its target's first member
-      target_star_kernel<<<(nb + 255) / 256, 256, 0, st>>>(target + p0, c->tfirst_dev, c->n_targets, c->tgt_star, nb);
+      target_star_kernel<<<(nb + 255) / 256, 256, 0, st>>>(q.target + p0, c->tfirst_dev, c->n_targets, c->tgt_star, nb);
       c->launches++;
     }
-    const int* star_s = target ? c->tgt_star : star ? star + p0 : nullptr;   // this slab's star of every point
-    const double* th = theta + p0 * ld;
+    const int* star_s = q.target ? c->tgt_star : q.star ? q.star + p0 : nullptr;   // this slab's star of every point
+    const double* th = q.theta + p0 * ld;
     std::array<cudaEvent_t, 4> evs{};
     if (c->timing) {
       for (auto& e : evs) CU_TRY(cudaEventCreate(&e));
       CU_TRY(cudaEventRecord(evs[0], st));
     }
     int is_depth = 0;
-    const bool fast_tail = c->has_spec && c->use_fast && c->allow_fast && !c->lsf_on;
     TailParams T = c->tail;
+    FastGrid F = c->fast;                                 // the fast tail's, for this slab
     const bool gather_here = c->g_active && c->g_fuse && fast_tail;
     if (c->has_spec) {
       T.theta = th; T.ld = ld; T.flux = c->flux; T.ldf = c->ldf; T.B = nb;
       T.chi2_sed = c->has_phot ? c->chi2_sed : nullptr;
-      T.lnl = lnl ? lnl + p0 : nullptr;
-      T.model_out = flux_out ? flux_out + p0 * ld_flux : nullptr;
-      T.ld_flux = ld_flux;
+      T.lnl = q.lnl ? q.lnl + p0 : nullptr;
+      T.model_out = q.flux ? q.flux + p0 * q.ld_flux : nullptr;
+      T.ld_flux = q.ld_flux;
       T.star = star_s;
       T.status = c->status;
-      if (target) {
-        T.target = target + p0; T.tfirst = c->tfirst_dev; T.n_targets = c->n_targets; T.kmax = c->tgt_kmax;
-        T.chi2_out = chi2_out ? chi2_out + p0 * ld_chi2 : nullptr; T.ld_chi2 = ld_chi2;
+      if (q.target) {
+        T.target = q.target + p0; T.tfirst = c->tfirst_dev; T.n_targets = c->n_targets; T.kmax = c->tgt_kmax;
+        T.chi2_out = q.chi2 ? q.chi2 + p0 * q.ld_chi2 : nullptr; T.ld_chi2 = q.ld_chi2;
       }
-      if (binary) {
-        T.binary = c->binary_dev; T.bin_par = c->bin_par; T.bin_scratch = c->bin_scratch; T.bin_ld = c->n_obs_max;
-        T.comp_out = comp_out ? comp_out + p0 * 2 * ld_flux : nullptr;
+      if (q.binary || marg) { T.aj_scratch = c->aj_scratch; T.aj_ld = c->n_obs_max; }
+      if (q.binary) {
+        T.binary = c->binary_dev; T.bin_par = c->bin_par;
+        T.comp_out = q.comp ? q.comp + p0 * 2 * q.ld_flux : nullptr;
       }
       if (marg) {
-        T.marg_k = c->marg_k_dev; T.marg_c = c->marg_c_dev; T.bin_scratch = c->marg_scratch; T.bin_ld = c->n_obs_max;
-        T.chi2_out = chi2_out ? chi2_out + p0 * ld_chi2 : nullptr; T.ld_chi2 = ld_chi2;
-        T.coef_out = coef_out ? coef_out + p0 * ld_coef : nullptr; T.ld_coef = ld_coef;
-        T.chol_out = chol_out ? chol_out + p0 * ld_chol : nullptr; T.ld_chol = ld_chol;
+        T.marg_k = c->marg_k_dev; T.marg_c = c->marg_c_dev;
+        T.chi2_out = q.chi2 ? q.chi2 + p0 * q.ld_chi2 : nullptr; T.ld_chi2 = q.ld_chi2;
+        T.coef_out = q.coef ? q.coef + p0 * q.ld_coef : nullptr; T.ld_coef = q.ld_coef;
+        T.chol_out = q.chol ? q.chol + p0 * q.ld_chol : nullptr; T.ld_chol = q.ld_chol;
       }
       if (gather_here) {
         // all-gather fused into the tail (tail.cuh store_lnl / gather_exit): this slab's slice of every peer's buffer
@@ -1039,30 +1067,16 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         T.g_raise = (p0 + c->slab >= B) ? c->g_raise_to : 0ull;
       }
       if (fast_tail) {
+        // the single-CTA forms other than Point's run the split kernel at 65536 samples (the cluster tail has none)
+        F.work_start = cluster ? (int)std::min<long long>(c->cluster_n, nb) : std::min(fgrid, nb);
+        if (c->grid_cap > 0) F.work_start = std::min(F.work_start, c->grid_cap);
+        if (form != FastForm::Point) F.cluster = 0;
+        if (q.target) F.points = c->tgt_points;
+        if (cluster) F.win_floats = c->cluster_win_floats;
         // per-point setup depends only on theta: fork it beside the emulator GEMMs, join before the tail
         CU_TRY(cudaEventRecord(c->ev_fork, st));
         CU_TRY(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-        c->fast.work_start = marg ? std::min(c->marg_grid, nb) : target ? std::min(c->tgt_grid, nb)
-                           : binary ? std::min(c->bin_grid, nb)
-                           : (c->use_cluster && c->allow_cluster) ? (int)std::min<long long>(c->cluster_n, nb)
-                                                                  : std::min(c->tail_grid_fast, nb);
-        if (c->grid_cap > 0) c->fast.work_start = std::min(c->fast.work_start, c->grid_cap);
-        if (target) {
-          FastGrid FT = c->fast;
-          FT.points = c->tgt_points; FT.cluster = 0;
-          if (payne::launch_tail_setup_targets((long long)nb * c->tgt_kmax, c->side, T, FT))
-            return fail(PAYNE_E_CUDA, "tail_setup launch");
-        } else if (binary) {
-          FastGrid FB = c->fast;
-          FB.cluster = 0;
-          if (payne::launch_tail_setup_binary(nb, c->side, T, FB)) return fail(PAYNE_E_CUDA, "tail_setup launch");
-        } else if (marg) {
-          FastGrid FM = c->fast;
-          FM.cluster = 0;
-          if (payne::launch_tail_setup(nb, c->side, T, FM)) return fail(PAYNE_E_CUDA, "tail_setup launch");
-        } else if (payne::launch_tail_setup(nb, c->side, T, c->fast)) {
-          return fail(PAYNE_E_CUDA, "tail_setup launch");
-        }
+        if (payne::launch_tail_setup(form, nb, c->side, T, F)) return fail(PAYNE_E_CUDA, "tail_setup launch");
         if (gather_here && p0 == 0 && c->g_wait_for)
           // the buffer the tail is about to write on the peers is free once every rank's previous step has landed here;
           // waited for on the side stream, beside the emulator GEMMs
@@ -1072,8 +1086,8 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
       }
       EncodeParams E = c->enc;
       E.star = star_s;
-      if (binary) { E.binary = c->binary_dev; E.half = nb; }   // rows [nb, 2 nb): the secondaries
-      rc = run_mlp(c, E, th, ld, binary ? 2 * nb : nb, c->flux, c->ldf, true, &is_depth, st);
+      if (q.binary) { E.binary = c->binary_dev; E.half = nb; }   // rows [nb, 2 nb): the secondaries
+      rc = run_mlp(c, E, th, ld, q.binary ? 2 * nb : nb, c->flux, c->ldf, true, &is_depth, st);
       if (rc) return rc;
       if (c->cont) {
         // modspec *= np.interp(modwave, modcontwave, normalised F_lambda continuum) (predictspec.py:208-226)
@@ -1098,7 +1112,7 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
     if (c->has_phot) {
       PhotParams P = c->phot;
       P.theta = th; P.ld = ld; P.B = nb; P.chi2_sed = c->chi2_sed;
-      P.mags_out = mags_out ? mags_out + p0 * P.nb : nullptr;
+      P.mags_out = q.mags ? q.mags + p0 * P.nb : nullptr;
       P.star = star_s;
       P.status = c->status;
       if (P.band_slot)
@@ -1118,52 +1132,25 @@ int run_batch(PayneCtx* c, const double* theta, const int* star, long long B, lo
         // ... a star's own fixed Inst_R and a per-star layout's Inst_R column too: Rs = NaN, no scalar-R stage
         TL.inst_scale = std::numeric_limits<double>::quiet_NaN();
         const int grid = std::min(c->lsf_grid, nb);
-        if (target ? payne::launch_tail_lsf_targets(grid, c->lsf_smem, st, TL, c->lsf)
-                   : payne::launch_tail_lsf(grid, c->lsf_smem, st, TL, c->lsf))
+        if (q.target ? payne::launch_tail_lsf_targets(grid, c->lsf_smem, st, TL, c->lsf)
+                     : payne::launch_tail_lsf(grid, c->lsf_smem, st, TL, c->lsf))
           return fail(PAYNE_E_CUDA, "tail launch");
-      } else if (marg) {
-        // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no such form)
-        if (!(fast_tail && is_depth))
-          return fail(PAYNE_E_UNSUPPORTED, "continuum marginalisation needs the fast tail on line-depth rows");
-        FastGrid FM = c->fast;
-        FM.cluster = 0;
-        if (target) FM.points = c->tgt_points;
-        if (payne::launch_tail_fast_marg(T.log2N1, target != nullptr, c->fast.work_start, c->fast_smem, st, T, FM))
-          return fail(PAYNE_E_CUDA, "tail launch");
-      } else if (binary) {
-        // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no binary form)
-        if (!(fast_tail && is_depth)) return fail(PAYNE_E_UNSUPPORTED, "binaries need the fast tail on line-depth rows");
-        FastGrid FB = c->fast;
-        FB.cluster = 0;
-        if (payne::launch_tail_fast_binary(T.log2N1, c->fast.work_start, c->fast_smem, st, T, FB))
-          return fail(PAYNE_E_CUDA, "tail launch");
-      } else if (target) {
-        // 65536-sample transforms included: the single-CTA split kernel (the cluster tail has no target form)
-        if (!(fast_tail && is_depth)) return fail(PAYNE_E_UNSUPPORTED, "targets need the fast tail on line-depth rows");
-        FastGrid FT = c->fast;
-        FT.points = c->tgt_points; FT.cluster = 0;
-        const bool poly = T.n_poly != 0 || T.model_out != nullptr;
-        if (payne::launch_tail_fast_targets(T.log2N1, poly, c->fast.work_start, c->fast_smem, st, T, FT))
-          return fail(PAYNE_E_CUDA, "tail launch");
-      } else if (fast_tail && is_depth && c->use_cluster && c->allow_cluster) {
-        payne::FastGrid FC = c->fast;
-        FC.win_floats = c->cluster_win_floats;
-        if (payne::launch_tail_cluster(T.log2N1, c->fast.work_start, c->cluster_smem, st, T, FC))
-          return fail(PAYNE_E_CUDA, "tail launch");
-        if (gather_here && T.g_raise) c->g_fused = true;
       } else if (fast_tail && is_depth) {
-        const int grid = c->fast.work_start;
-        const bool poly = T.n_poly != 0 || T.model_out != nullptr;
-        if (payne::launch_tail_fast(T.log2N1, poly, grid, c->fast_smem, st, T, c->fast)) return fail(PAYNE_E_CUDA, "tail launch");
+        if (cluster ? payne::launch_tail_cluster(T.log2N1, F.work_start, c->cluster_smem, st, T, F)
+                    : payne::launch_tail_fast(T.log2N1, form, F.work_start, c->fast_smem, st, T, F))
+          return fail(PAYNE_E_CUDA, "tail launch");
         if (gather_here && T.g_raise) c->g_fused = true;
+      } else if (form != FastForm::Point) {
+        static const char* const what[] = {"", "targets need", "binaries need", "continuum marginalisation needs"};
+        return fail(PAYNE_E_UNSUPPORTED, std::string(what[(int)form]) + " the fast tail on line-depth rows");
       } else {
         if (c->tail.log2N1 > 15) return fail(PAYNE_E_UNSUPPORTED, "general-grid tail is limited to 32768-point transforms");
         const int grid = std::min(c->tail_grid, nb);
         if (payne::launch_tail_general(T.log2N1, grid, c->tail_smem, st, T, c->fast.twc)) return fail(PAYNE_E_CUDA, "tail launch");
       }
       c->launches++;
-    } else if (lnl) {
-      lnl_from_sed_kernel<<<(nb + 255) / 256, 256, 0, st>>>(c->chi2_sed, lnl + p0, nb);
+    } else if (q.lnl) {
+      lnl_from_sed_kernel<<<(nb + 255) / 256, 256, 0, st>>>(c->chi2_sed, q.lnl + p0, nb);
       c->launches++;
     }
     if (c->timing) { CU_TRY(cudaEventRecord(evs[3], st)); c->pending.push_back(evs); }
@@ -1256,12 +1243,8 @@ int probe_targets(PayneCtx* c) {
     c->tgt_lsf_probed = true;
     return PAYNE_OK;
   }
-  if (c->tgt_grid > 0) return PAYNE_OK;
-  if (!payne::probe_tail_fast_targets(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
-    return fail(PAYNE_E_UNSUPPORTED, "target tail kernel does not fit on an SM");
-  // the split kernel's scratch lines exist for tail_grid_fast CTAs
-  c->tgt_grid = std::min(occ * c->sm_count, c->tail_grid_fast);
-  return PAYNE_OK;
+  int grid = 0;
+  return form_grid(c, payne::FastForm::Target, &grid);
 }
 
 // The target entries: targets set, and the context still runs a tail they can use (a one-star context may have
@@ -1275,10 +1258,14 @@ int need_targets(PayneCtx* c) {
   return probe_targets(c);
 }
 
-// The host-buffer entries: idx_host is every point's star, or its target (targets = true), or null (star 0).
-int lnlike_host(PayneCtx* c, const double* theta_host, const int32_t* star_host, int64_t B, int64_t ld, double* lnl_host,
-                bool targets, bool binary = false) {
+// The host-buffer entries: q names host buffers (theta, lnl, and every point's star or target, or neither: star 0),
+// which are staged through pinned and device buffers.
+int lnlike_host(PayneCtx* c, Batch q) {
   int rc;
+  const long long B = q.B, ld = q.ld;
+  const bool targets = q.target != nullptr;
+  const int32_t* star_host = targets ? q.target : q.star;
+  double* lnl_host = q.lnl;
   const int n_idx = targets ? c->n_targets : c->n_stars;
   if (star_host)
     for (int64_t i = 0; i < B; ++i)
@@ -1312,16 +1299,17 @@ int lnlike_host(PayneCtx* c, const double* theta_host, const int32_t* star_host,
     c->lnl_map = (!(zenv && zenv[0] == '0') && cudaHostGetDevicePointer(&dp, c->lnl_pin, 0) == cudaSuccess) ? (double*)dp : nullptr;
     cudaGetLastError();
   }
-  std::memcpy(c->theta_pin, theta_host, (size_t)B * ld * sizeof(double));
+  std::memcpy(c->theta_pin, q.theta, (size_t)B * ld * sizeof(double));
   CU_TRY(cudaMemcpyAsync(c->theta_stage, c->theta_pin, (size_t)B * ld * sizeof(double),
                          cudaMemcpyHostToDevice, c->stream));
   if (star_host) {
     std::memcpy(c->star_pin, star_host, (size_t)B * sizeof(int));
     CU_TRY(cudaMemcpyAsync(c->star_stage, c->star_pin, (size_t)B * sizeof(int), cudaMemcpyHostToDevice, c->stream));
   }
-  const int* idx = star_host ? c->star_stage : nullptr;
-  rc = run_batch(c, c->theta_stage, targets ? nullptr : idx, B, ld, nullptr, 0, nullptr,
-                 c->lnl_map ? c->lnl_map : c->lnl_stage, c->stream, targets ? idx : nullptr, nullptr, 0, binary);
+  q.theta = c->theta_stage;
+  (targets ? q.target : q.star) = star_host ? c->star_stage : nullptr;
+  q.lnl = c->lnl_map ? c->lnl_map : c->lnl_stage;
+  rc = run_batch(c, q, c->stream);
   if (rc) return rc;
   if (!c->lnl_map)
     CU_TRY(cudaMemcpyAsync(c->lnl_pin, c->lnl_stage, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost,
@@ -1395,11 +1383,11 @@ int payne_ctx_set_binary(PayneCtx* c, const PayneBinary* b) {
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
   DeviceGuard dg(c->device);
   auto drop = [&]() -> int {
-    CU_TRY(cudaDeviceSynchronize());                     // earlier calls may still read them
+    CU_TRY(cudaDeviceSynchronize());                     // earlier calls may still read it
     if (c->binary_dev) cudaFree(c->binary_dev);
-    if (c->bin_scratch) cudaFree(c->bin_scratch);
-    c->binary_dev = nullptr; c->bin_scratch = nullptr; c->has_binary = false;
-    return PAYNE_OK;
+    c->binary_dev = nullptr; c->has_binary = false;
+    // the a_j scratch is continuum marginalisation's while that is on
+    return c->has_marg ? PAYNE_OK : resize_buffer(&c->aj_scratch, &c->aj_scratch_n, 0);
   };
   if (!b) return drop();
   int rc = binary_unsupported(c);
@@ -1422,15 +1410,15 @@ int payne_ctx_set_binary(PayneCtx* c, const PayneBinary* b) {
                 std::to_string(ndim) + ")");
   if (b->rratio_col < 0 && !std::isfinite(b->rratio_fixed))
     return fail(PAYNE_E_INVALID, "binary: Rratio needs a theta column or a finite fixed value");
-  int occ = 0;
-  if (!payne::probe_tail_fast_binary(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
-    return fail(PAYNE_E_UNSUPPORTED, "binary tail kernel does not fit on an SM");
+  int grid = 0;
+  rc = form_grid(c, payne::FastForm::Binary, &grid);
+  if (rc) return rc;
   rc = drop();
   if (rc) return rc;
-  c->bin_grid = std::min(occ * c->sm_count, c->tail_grid_fast);   // the split kernel's scratch lines exist for these
   rc = upload(&c->binary_dev, b, 1);
   if (rc) return rc;
-  CU_TRY(cudaMalloc((void**)&c->bin_scratch, (size_t)c->bin_grid * c->n_obs_max * sizeof(double)));
+  rc = resize_buffer(&c->aj_scratch, &c->aj_scratch_n, (long long)grid * c->n_obs_max);
+  if (rc) return rc;
   c->has_binary = true;
   return PAYNE_OK;
 }
@@ -1443,8 +1431,9 @@ int payne_lnlike_batch_binary(PayneCtx* c, const double* theta_dev, const int32_
   DeviceGuard dg(c->device);
   int rc = need_binary(c);
   if (rc) return rc;
-  return run_batch(c, theta_dev, star_dev, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, nullptr, nullptr, 0,
-                   true);
+  Batch q{theta_dev, B, ld, lnl_dev, star_dev};
+  q.binary = true;
+  return run_batch(c, q, (cudaStream_t)stream);
 }
 
 int payne_lnlike_batch_binary_host(PayneCtx* c, const double* theta_host, const int32_t* star_host, int64_t B, int64_t ld,
@@ -1455,7 +1444,9 @@ int payne_lnlike_batch_binary_host(PayneCtx* c, const double* theta_host, const 
   DeviceGuard dg(c->device);
   int rc = need_binary(c);
   if (rc) return rc;
-  return lnlike_host(c, theta_host, star_host, B, ld, lnl_host, false, true);
+  Batch q{theta_host, B, ld, lnl_host, star_host};
+  q.binary = true;
+  return lnlike_host(c, q);
 }
 
 int payne_model_batch_binary(PayneCtx* c, const double* theta_dev, const int32_t* star_dev, int64_t B, int64_t ld,
@@ -1467,8 +1458,10 @@ int payne_model_batch_binary(PayneCtx* c, const double* theta_dev, const int32_t
   int rc = need_binary(c);
   if (rc) return rc;
   if ((flux_dev || comp_dev) && ld_flux < c->n_obs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest n_obs");
-  return run_batch(c, theta_dev, star_dev, B, ld, flux_dev, ld_flux, nullptr, lnl_dev, (cudaStream_t)stream, nullptr,
-                   nullptr, 0, true, comp_dev);
+  Batch q{theta_dev, B, ld, lnl_dev, star_dev};
+  q.binary = true;
+  q.flux = flux_dev; q.ld_flux = ld_flux; q.comp = comp_dev;
+  return run_batch(c, q, (cudaStream_t)stream);
 }
 
 int payne_ctx_set_cont_marg(PayneCtx* c, const PayneContMarg* per_star) {
@@ -1478,10 +1471,10 @@ int payne_ctx_set_cont_marg(PayneCtx* c, const PayneContMarg* per_star) {
     CU_TRY(cudaDeviceSynchronize());                     // earlier calls may still read them
     if (c->marg_k_dev) cudaFree(c->marg_k_dev);
     if (c->marg_c_dev) cudaFree(c->marg_c_dev);
-    if (c->marg_scratch) cudaFree(c->marg_scratch);
-    c->marg_k_dev = nullptr; c->marg_c_dev = nullptr; c->marg_scratch = nullptr; c->has_marg = false;
+    c->marg_k_dev = nullptr; c->marg_c_dev = nullptr; c->has_marg = false;
     c->marg_k_h.clear();
-    return PAYNE_OK;
+    // the a_j scratch is the binary tail's while binaries are on
+    return c->has_binary ? PAYNE_OK : resize_buffer(&c->aj_scratch, &c->aj_scratch_n, 0);
   };
   if (!per_star) return drop();
   const int S = c->n_stars;
@@ -1509,17 +1502,17 @@ int payne_ctx_set_cont_marg(PayneCtx* c, const PayneContMarg* per_star) {
     return fail(PAYNE_E_UNSUPPORTED, "continuum marginalisation: some stars have the setting and others (n_coef 0) do not");
   int rc = marg_unsupported(c);
   if (rc) return rc;
-  int occ = 0;
-  if (!payne::probe_tail_fast_marg(c->tail.log2N1, c->fast_smem, &occ) || occ < 1)
-    return fail(PAYNE_E_UNSUPPORTED, "continuum marginalisation tail kernel does not fit on an SM");
+  int grid = 0;
+  rc = form_grid(c, payne::FastForm::Marg, &grid);
+  if (rc) return rc;
   rc = drop();
   if (rc) return rc;
-  c->marg_grid = std::min(occ * c->sm_count, c->tail_grid_fast);   // the split kernel's scratch lines exist for these
   rc = upload(&c->marg_k_dev, kk.data(), (size_t)S);
   if (rc) return rc;
   rc = upload(&c->marg_c_dev, cc.data(), (size_t)S);
   if (rc) return rc;
-  CU_TRY(cudaMalloc((void**)&c->marg_scratch, (size_t)c->marg_grid * c->n_obs_max * sizeof(double)));
+  rc = resize_buffer(&c->aj_scratch, &c->aj_scratch_n, (long long)grid * c->n_obs_max);
+  if (rc) return rc;
   c->marg_k_h = kk;
   c->has_marg = true;
   return PAYNE_OK;
@@ -1536,8 +1529,10 @@ int payne_cont_batch_stars(PayneCtx* c, const double* theta_dev, const int32_t* 
   if (rc) return rc;
   rc = need_star_array(c, star_dev, "payne_cont_batch_stars");
   if (rc) return rc;
-  return run_batch(c, theta_dev, star_dev, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, nullptr, chi2_dev, 1,
-                   false, nullptr, coef_dev, ld_coef, chol_dev, ld_chol);
+  Batch q{theta_dev, B, ld, lnl_dev, star_dev};
+  q.chi2 = chi2_dev; q.ld_chi2 = 1;
+  q.coef = coef_dev; q.ld_coef = ld_coef; q.chol = chol_dev; q.ld_chol = ld_chol;
+  return run_batch(c, q, (cudaStream_t)stream);
 }
 
 int payne_cont_batch_targets(PayneCtx* c, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
@@ -1552,8 +1547,11 @@ int payne_cont_batch_targets(PayneCtx* c, const double* theta_dev, const int32_t
   rc = need_marg(c, true, coef_dev ? ld_coef : INT64_MAX, chol_dev ? ld_chol : INT64_MAX);
   if (rc) return rc;
   if (chi2_dev && ld_chi2 < c->tgt_kmax) return fail(PAYNE_E_INVALID, "ld_chi2 < the largest member count");
-  return run_batch(c, theta_dev, nullptr, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, target_dev, chi2_dev,
-                   ld_chi2, false, nullptr, coef_dev, ld_coef, chol_dev, ld_chol);
+  Batch q{theta_dev, B, ld, lnl_dev};
+  q.target = target_dev;
+  q.chi2 = chi2_dev; q.ld_chi2 = ld_chi2;
+  q.coef = coef_dev; q.ld_coef = ld_coef; q.chol = chol_dev; q.ld_chol = ld_chol;
+  return run_batch(c, q, (cudaStream_t)stream);
 }
 
 int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) {
@@ -1562,10 +1560,10 @@ int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) 
   if (!first) {
     CU_TRY(cudaDeviceSynchronize());                     // earlier calls may still read the table
     if (c->tfirst_dev) cudaFree(c->tfirst_dev);
-    if (c->tgt_points) cudaFree(c->tgt_points);
-    if (c->tgt_star) cudaFree(c->tgt_star);
     c->tfirst_dev = nullptr; c->n_targets = 0; c->tgt_kmax = 0; c->tgt_nobs_max = 0;
-    c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
+    int rc = resize_buffer(&c->tgt_points, &c->tgt_points_n, 0);
+    if (!rc) rc = resize_buffer(&c->tgt_star, &c->tgt_star_n, 0);
+    if (rc) return rc;
     c->tgt_instr_col.clear();
     c->tfirst_h.clear();
     return PAYNE_OK;
@@ -1609,7 +1607,7 @@ int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) 
     }
   }
   if (c->lsf_on && !instr_col.empty()) return fail(PAYNE_E_INVALID, instr_col);
-  c->tgt_grid = 0; c->tgt_lsf_probed = false;           // probed again for this context's current tail
+  c->tgt_lsf_probed = false;                            // probed again for this context's current tail
   int rc = probe_targets(c);
   if (rc) return rc;
   CU_TRY(cudaDeviceSynchronize());
@@ -1618,9 +1616,8 @@ int payne_ctx_set_targets(PayneCtx* c, const int32_t* first, int32_t n_targets) 
   rc = upload(&c->tfirst_dev, first, (size_t)n_targets + 1);
   if (rc) return rc;
   if (c->tgt_kmax != kmax) {                             // the record stride changes: reallocate at the next call
-    if (c->tgt_points) cudaFree(c->tgt_points);
-    if (c->tgt_star) cudaFree(c->tgt_star);
-    c->tgt_points = nullptr; c->tgt_star = nullptr; c->tgt_rows = c->tgt_rec_alloc = 0;
+    rc = resize_buffer(&c->tgt_points, &c->tgt_points_n, 0);
+    if (rc) return rc;
   }
   c->n_targets = n_targets; c->tgt_kmax = kmax; c->tgt_nobs_max = nobs_max; c->tgt_instr_col = instr_col;
   c->tfirst_h.assign(first, first + n_targets + 1);
@@ -1635,7 +1632,9 @@ int payne_lnlike_batch_targets(PayneCtx* c, const double* theta_dev, const int32
   DeviceGuard dg(c->device);
   int rc = need_targets(c);
   if (rc) return rc;
-  return run_batch(c, theta_dev, nullptr, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream, target_dev);
+  Batch q{theta_dev, B, ld, lnl_dev};
+  q.target = target_dev;
+  return run_batch(c, q, (cudaStream_t)stream);
 }
 
 int payne_model_batch_targets(PayneCtx* c, const double* theta_dev, const int32_t* target_dev, int64_t B, int64_t ld,
@@ -1649,8 +1648,10 @@ int payne_model_batch_targets(PayneCtx* c, const double* theta_dev, const int32_
   if (rc) return rc;
   if (flux_dev && ld_flux < c->tgt_nobs_max) return fail(PAYNE_E_INVALID, "ld_flux < the largest target's pixels (all members)");
   if (chi2_dev && ld_chi2 < c->tgt_kmax) return fail(PAYNE_E_INVALID, "ld_chi2 < the largest member count");
-  return run_batch(c, theta_dev, nullptr, B, ld, flux_dev, ld_flux, mags_dev, lnl_dev, (cudaStream_t)stream, target_dev,
-                   chi2_dev, ld_chi2);
+  Batch q{theta_dev, B, ld, lnl_dev};
+  q.target = target_dev;
+  q.flux = flux_dev; q.ld_flux = ld_flux; q.mags = mags_dev; q.chi2 = chi2_dev; q.ld_chi2 = ld_chi2;
+  return run_batch(c, q, (cudaStream_t)stream);
 }
 
 int payne_abi_version(void) { return PAYNE_ABI_VERSION; }
@@ -1743,9 +1744,8 @@ void payne_ctx_destroy(PayneCtx* c) {
   c->fast.points = nullptr; drop(c->status);
   payne::tc_free_acts_x(&c->actA); payne::tc_free_acts_x(&c->actB);
   drop(c->theta_stage); drop(c->lnl_stage); drop(c->star_stage);
-  drop(c->tfirst_dev); drop(c->tgt_points); drop(c->tgt_star);
-  drop(c->binary_dev); drop(c->bin_scratch); drop(c->bin_par);
-  drop(c->marg_k_dev); drop(c->marg_c_dev); drop(c->marg_scratch);
+  drop(c->tfirst_dev); drop(c->tgt_points); drop(c->tgt_star); drop(c->bin_par); drop(c->aj_scratch);
+  drop(c->binary_dev); drop(c->marg_k_dev); drop(c->marg_c_dev);
   if (c->star_pin) cudaFreeHost(c->star_pin);
   for (int r = 0; r < 16; ++r)
     if (c->g_opened[r]) { cudaIpcCloseMemHandle(c->g_peer_buf[r]); cudaIpcCloseMemHandle(c->g_peer_flag[r]); }
@@ -1774,7 +1774,7 @@ int payne_lnlike_batch_stars(PayneCtx* c, const double* theta_dev, const int32_t
   int rc = need_star_array(c, star_dev, "payne_lnlike_batch_stars");
   if (rc) return rc;
   DeviceGuard dg(c->device);
-  return run_batch(c, theta_dev, star_dev, B, ld, nullptr, 0, nullptr, lnl_dev, (cudaStream_t)stream);
+  return run_batch(c, Batch{theta_dev, B, ld, lnl_dev, star_dev}, (cudaStream_t)stream);
 }
 
 int payne_model_batch(PayneCtx* c, const double* theta_dev, int64_t B, int64_t ld, double* flux_dev,
@@ -1790,7 +1790,9 @@ int payne_model_batch_stars(PayneCtx* c, const double* theta_dev, const int32_t*
   int rc = need_star_array(c, star_dev, "payne_model_batch_stars");
   if (rc) return rc;
   DeviceGuard dg(c->device);
-  return run_batch(c, theta_dev, star_dev, B, ld, flux_dev, ld_flux, mags_dev, lnl_dev, (cudaStream_t)stream);
+  Batch q{theta_dev, B, ld, lnl_dev, star_dev};
+  q.flux = flux_dev; q.ld_flux = ld_flux; q.mags = mags_dev;
+  return run_batch(c, q, (cudaStream_t)stream);
 }
 
 int payne_lnlike_batch_host(PayneCtx* c, const double* theta_host, int64_t B, int64_t ld, double* lnl_host) {
@@ -1800,12 +1802,11 @@ int payne_lnlike_batch_host(PayneCtx* c, const double* theta_host, int64_t B, in
 int payne_lnlike_batch_stars_host(PayneCtx* c, const double* theta_host, const int32_t* star_host, int64_t B, int64_t ld,
                                   double* lnl_host) {
   if (!c) return fail(PAYNE_E_INVALID, "null argument");
-  if (B == 0) return PAYNE_OK;
-  if (!theta_host || !lnl_host) return fail(PAYNE_E_INVALID, "null argument");
   if (B <= 0) return PAYNE_OK;
+  if (!theta_host || !lnl_host) return fail(PAYNE_E_INVALID, "null argument");
   int rc = need_star_array(c, star_host, "payne_lnlike_batch_stars_host");
   if (rc) return rc;
-  return lnlike_host(c, theta_host, star_host, B, ld, lnl_host, false);
+  return lnlike_host(c, Batch{theta_host, B, ld, lnl_host, star_host});
 }
 
 int payne_lnlike_batch_targets_host(PayneCtx* c, const double* theta_host, const int32_t* target_host, int64_t B,
@@ -1816,7 +1817,9 @@ int payne_lnlike_batch_targets_host(PayneCtx* c, const double* theta_host, const
   DeviceGuard dg(c->device);                             // (need_targets may probe a target kernel)
   int rc = need_targets(c);
   if (rc) return rc;
-  return lnlike_host(c, theta_host, target_host, B, ld, lnl_host, true);
+  Batch q{theta_host, B, ld, lnl_host};
+  q.target = target_host;
+  return lnlike_host(c, q);
 }
 
 }  // extern "C"
@@ -1951,7 +1954,7 @@ int payne_lnlike_batch_gather(PayneCtx* c, const double* theta_dev, int64_t B, i
   c->g_active = true; c->g_fused = false;
   c->g_wait_for = (unsigned long long)s; c->g_raise_to = (unsigned long long)(s + 1);
   c->g_bufoff = (size_t)(s % 3) * per;
-  int rc = run_batch(c, theta_dev, nullptr, B, ld, nullptr, 0, nullptr, mine, st);
+  int rc = run_batch(c, Batch{theta_dev, B, ld, mine}, st);
   c->g_active = false;
   if (rc) return rc;
   if (gathered_prev) *gathered_prev = s > 0 ? c->g_buf + (size_t)((s - 1) % 3) * per : nullptr;

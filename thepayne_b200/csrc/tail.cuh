@@ -109,11 +109,11 @@ struct TailParams {
   // record c * B + p.  Null binary: no binary.
   const PayneBinary* binary;         // device copy
   double* bin_par;                   // [B, 3] Teff_1, Teff_2, Rratio of every point (tail_setup_binary_kernel)
-  double* bin_scratch;               // [grid, bin_ld] a_1 of the CTA's current point
-  long long bin_ld;
+  double* aj_scratch;                // [grid, aj_ld] a_1 (binaries) or a_j (marginalisation) of the CTA's current point
+  long long aj_ld;
   double* comp_out;                  // [B, 2, ld_flux] a_1 and a_2, or null
   // Continuum marginalisation (payne_ctx_set_cont_marg; fast tail only): star k's K = marg_k[k] coefficients are
-  // integrated out, C = marg_c[k] = sum_k (ln 2 pi / 2 - ln w_k).  bin_scratch / bin_ld hold a_j of the CTA's current point,
+  // integrated out, C = marg_c[k] = sum_k (ln 2 pi / 2 - ln w_k).  aj_scratch / aj_ld hold a_j of the CTA's current point,
   // chi2_out / ld_chi2 every point's (or member's) Q.  Null marg_k: off.
   const int* marg_k;
   const double* marg_c;

@@ -266,7 +266,7 @@ __device__ __forceinline__ double final_pass_poly(const TailParams& P, const Fas
 __device__ __forceinline__ double final_pass_marg(const TailParams& P, const PointSetup& S, const FastSetup& FS, int tid,
                                                   int p, int moff, int nk) {
   const int off = FS.obs.off, jend = FS.obs.off + FS.obs.n;
-  const double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  const double* scr = P.aj_scratch + (long long)blockIdx.x * P.aj_ld;
   double* mrow = P.model_out ? P.model_out + (long long)p * P.ld_flux + moff : nullptr;
   double acc = 0.0;
   constexpr int U = 4;
@@ -314,7 +314,7 @@ __device__ __forceinline__ double final_pass_bin(const TailParams& P, const Fast
   const float hdu = S.hdu;
   const double q0 = FS.q0, scale = FS.scale;
   const int off = FS.obs.off, jend = FS.obs.off + FS.obs.n;
-  double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  double* scr = P.aj_scratch + (long long)blockIdx.x * P.aj_ld;
   double* crow = P.comp_out ? P.comp_out + ((long long)p * 2 + (BM - 1)) * P.ld_flux : nullptr;
   double* mrow = (BM == 2 && P.model_out) ? P.model_out + (long long)p * P.ld_flux : nullptr;
   double t1 = 0.0, t2 = 0.0, rr2 = 0.0;
@@ -397,7 +397,7 @@ __device__ __forceinline__ double plain_pass_bin(const TailParams& P, const Poin
   const int n = P.n;
   const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
   const int off = FS.obs.off, jend = FS.obs.off + FS.obs.n;
-  double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  double* scr = P.aj_scratch + (long long)blockIdx.x * P.aj_ld;
   double* crow = P.comp_out ? P.comp_out + ((long long)p * 2 + (BM - 1)) * P.ld_flux : nullptr;
   double* mrow = (BM == 2 && P.model_out) ? P.model_out + (long long)p * P.ld_flux : nullptr;
   double t1 = 0.0, t2 = 0.0, rr2 = 0.0;
@@ -444,7 +444,7 @@ __device__ __forceinline__ double plain_pass(const TailParams& P, const PointSet
   const double nan = CUDART_NAN;
   const bool is_depth = true;   // this kernel is only launched on line-depth rows (f - 1)
   const int npoly = MARG ? nk : P.n_poly;
-  const double* scr = MARG ? P.bin_scratch + (long long)blockIdx.x * P.bin_ld : nullptr;
+  const double* scr = MARG ? P.aj_scratch + (long long)blockIdx.x * P.aj_ld : nullptr;
   double acc = 0.0;
   const int n = P.n;
   const double wlo = __ldg(P.w) * S.D, whi = __ldg(P.w + n - 1) * S.D;
@@ -621,7 +621,7 @@ __device__ __forceinline__ double marg_point(const TailParams& P, const FastGrid
   __syncthreads();                                        // a_j in the scratch; the transform buffer is free
   const int K = __ldg(P.marg_k + k);
   const int off = FS.obs.off, n = FS.obs.n;
-  const double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+  const double* scr = P.aj_scratch + (long long)blockIdx.x * P.aj_ld;
   double* sm = reinterpret_cast<double*>(z);
   const int nc = K + 1, nent = nc * (nc + 1) / 2 - 1;
   const int R = kNT / nent;
@@ -859,7 +859,7 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
         }
         if (S.bad) {                                      // NaN a_c: the model and lnL of the point are NaN
           bad = true;
-          double* scr = P.bin_scratch + (long long)blockIdx.x * P.bin_ld;
+          double* scr = P.aj_scratch + (long long)blockIdx.x * P.aj_ld;
           for (int j = tid; j < FS.obs.n; j += kNT) {
             if (c == 0) scr[j] = nan;
             if (P.comp_out) P.comp_out[((long long)p * 2 + c) * P.ld_flux + j] = nan;

@@ -53,6 +53,19 @@ def _pd(a):
     return a.ctypes.data_as(C.POINTER(C.c_double))
 
 
+def _i32(a):
+    return np.ascontiguousarray(np.asarray(a).astype(np.int32, casting='same_kind'))
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def _nan(want, shape, dev):
+    """A NaN-filled float64 output on ``dev``, or None when not wanted."""
+    return torch.full(shape, float('nan'), dtype=torch.float64, device=dev) if want else None
+
+
 # the secondary's own parameters of a binary (``Engine(binary=True)``) and the primary's parameter each one replaces
 # (names ending in ``_<digit>`` already mean "spectrum s" in the multi-spectrum fit)
 BINARY_PARS = {'Teff_sec': 'Teff', 'log(g)_sec': 'log(g)', '[Fe/H]_sec': '[Fe/H]', '[a/Fe]_sec': '[a/Fe]',
@@ -405,15 +418,6 @@ class Engine:
         _lib.check(self.lib.payne_ctx_set_cont_marg(self._ctx, arr))
         self.cont_k = [int(arr[k].n_coef) for k in range(self.n_stars)]
 
-    @staticmethod
-    def _cont_outputs(B, kc, kl, dev, nchi2=None):
-        nan = float('nan')
-        coef = torch.full((B, kc), nan, dtype=torch.float64, device=dev)
-        chol = torch.full((B, kl), nan, dtype=torch.float64, device=dev)
-        chi2 = torch.full((B,) if nchi2 is None else (B, nchi2), nan, dtype=torch.float64, device=dev)
-        lnl = torch.empty(B, dtype=torch.float64, device=dev)
-        return coef, chol, chi2, lnl
-
     def cont_batch(self, theta, star=None):
         """With the continuum integrated out: the best-fitting coefficients [B, K] (K the largest star's; a row's
         columns beyond its star's K stay NaN), the Cholesky factor L of G = L L^T as packed lower triangles
@@ -421,19 +425,12 @@ class Engine:
         draw of the coefficients' conditional posterior is coef + L^-T z, z ~ N(0, I)."""
         if self.cont_k is None:
             raise ValueError('no continuum marginalisation: set_cont_marg first')
-        dev = torch.device('cuda', self.device)
-        if not isinstance(theta, torch.Tensor):
-            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
-        th = self._theta_dev(theta.to(dev))
-        B = th.shape[0]
-        if star is not None and not isinstance(star, torch.Tensor):
-            star = torch.from_numpy(np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind')))
-        sv = self._star_dev(star.to(dev) if star is not None else None, B, dev)
+        th, sv, lnl, st = self._dev_args(theta, star, copy=True)
+        B, dev = th.shape[0], th.device
         kc = max(self.cont_k)
-        coef, chol, chi2, lnl = self._cont_outputs(B, kc, kc * (kc + 1) // 2, dev)
-        st = torch.cuda.current_stream(dev).cuda_stream
+        coef, chol, chi2 = _nan(True, (B, kc), dev), _nan(True, (B, kc * (kc + 1) // 2), dev), _nan(True, (B,), dev)
         _lib.check(self.lib.payne_cont_batch_stars(
-            self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None, B, th.shape[1],
+            self._ctx, th.data_ptr(), _ptr(sv), B, th.shape[1],
             coef.data_ptr(), coef.shape[1], chol.data_ptr(), chol.shape[1], chi2.data_ptr(), lnl.data_ptr(), st))
         return coef, chol, chi2, lnl
 
@@ -444,68 +441,34 @@ class Engine:
             raise ValueError('no continuum marginalisation: set_cont_marg first')
         if not self.n_targets:
             raise ValueError('no targets: set_targets first')
-        dev = torch.device('cuda', self.device)
-        if not isinstance(theta, torch.Tensor):
-            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
-        th = self._theta_dev(theta.to(dev))
-        B = th.shape[0]
-        if not isinstance(target, torch.Tensor):
-            target = torch.from_numpy(np.ascontiguousarray(np.asarray(target).astype(np.int32, casting='same_kind')))
-        tv = self._star_dev(target.to(dev), B, dev)
+        th, tv, lnl, st = self._dev_args(theta, target, copy=True)
+        B, dev = th.shape[0], th.device
         kc = max(sum(self.cont_k[k] for k in m) for m in self.target_members)
         kl = max(sum(self.cont_k[k] * (self.cont_k[k] + 1) // 2 for k in m) for m in self.target_members)
-        coef, chol, chi2, lnl = self._cont_outputs(B, kc, kl, dev, self.target_kmax)
-        st = torch.cuda.current_stream(dev).cuda_stream
+        coef, chol, chi2 = _nan(True, (B, kc), dev), _nan(True, (B, kl), dev), _nan(True, (B, self.target_kmax), dev)
         _lib.check(self.lib.payne_cont_batch_targets(
-            self._ctx, th.data_ptr(), tv.data_ptr(), B, th.shape[1], coef.data_ptr(), kc, chol.data_ptr(), kl,
+            self._ctx, th.data_ptr(), _ptr(tv), B, th.shape[1], coef.data_ptr(), kc, chol.data_ptr(), kl,
             chi2.data_ptr(), self.target_kmax, lnl.data_ptr(), st))
         return coef, chol, chi2, lnl
 
     def lnlike_batch_binary(self, theta, star=None):
         """lnL of every row as a binary, ``theta`` and ``star`` as in ``lnlike_batch`` (None: star 0)."""
         if isinstance(theta, torch.Tensor) and theta.is_cuda:
-            th = self._theta_dev(theta)
-            sv = self._star_dev(star, th.shape[0], th.device)
-            out = torch.empty(th.shape[0], dtype=torch.float64, device=th.device)
-            st = torch.cuda.current_stream(th.device).cuda_stream
-            _lib.check(self.lib.payne_lnlike_batch_binary(self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None,
-                                                          th.shape[0], th.shape[1], out.data_ptr(), st))
-            return out
-        th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
-        if th.ndim != 2 or th.shape[1] != self.ndim:
-            raise ValueError('theta must be [B, %d]' % self.ndim)
-        sv = None
-        if star is not None:
-            if isinstance(star, torch.Tensor):
-                star = star.cpu().numpy()
-            sv = np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind'))
-            if sv.shape != (th.shape[0],):
-                raise ValueError('star must be [%d]' % th.shape[0])
-        out = np.empty(th.shape[0], dtype=np.float64)
-        _lib.check(self.lib.payne_lnlike_batch_binary_host(self._ctx, th.ctypes.data,
-                                                           sv.ctypes.data if sv is not None else None,
-                                                           th.shape[0], th.shape[1], out.ctypes.data))
-        return out
+            th, sv, lnl, st = self._dev_args(theta, star, copy=False)
+            _lib.check(self.lib.payne_lnlike_batch_binary(self._ctx, th.data_ptr(), _ptr(sv), th.shape[0], th.shape[1],
+                                                          lnl.data_ptr(), st))
+            return lnl
+        return self._host_lnlike(self.lib.payne_lnlike_batch_binary_host, theta, star, 'star')
 
     def model_batch_binary(self, theta, star=None, want_flux=True, want_comp=True):
         """Model spectra [B, n_obs], the components' spectra before the continuum [B, 2, n_obs] and lnL [B] of every
         row as a binary, as CUDA float64 tensors (the pixels beyond a row's star stay NaN)."""
-        dev = torch.device('cuda', self.device)
-        if not isinstance(theta, torch.Tensor):
-            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
-        th = self._theta_dev(theta.to(dev))
-        B = th.shape[0]
-        if star is not None and not isinstance(star, torch.Tensor):
-            star = torch.from_numpy(np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind')))
-        sv = self._star_dev(star.to(dev) if star is not None else None, B, dev)
-        flux = torch.full((B, self.n_obs), float('nan'), dtype=torch.float64, device=dev) if want_flux else None
-        comp = torch.full((B, 2, self.n_obs), float('nan'), dtype=torch.float64, device=dev) if want_comp else None
-        lnl = torch.empty(B, dtype=torch.float64, device=dev)
-        st = torch.cuda.current_stream(dev).cuda_stream
+        th, sv, lnl, st = self._dev_args(theta, star, copy=True)
+        B, dev = th.shape[0], th.device
+        flux = _nan(want_flux, (B, self.n_obs), dev)
+        comp = _nan(want_comp, (B, 2, self.n_obs), dev)
         _lib.check(self.lib.payne_model_batch_binary(
-            self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None, B, th.shape[1],
-            flux.data_ptr() if flux is not None else None, self.n_obs,
-            comp.data_ptr() if comp is not None else None, lnl.data_ptr(), st))
+            self._ctx, th.data_ptr(), _ptr(sv), B, th.shape[1], _ptr(flux), self.n_obs, _ptr(comp), lnl.data_ptr(), st))
         return flux, comp, lnl
 
     def lnlike_batch_targets(self, theta, target):
@@ -515,25 +478,11 @@ class Engine:
         if not self.n_targets:
             raise ValueError('no targets: set_targets first')
         if isinstance(theta, torch.Tensor) and theta.is_cuda:
-            th = self._theta_dev(theta)
-            tv = self._star_dev(target, th.shape[0], th.device)
-            out = torch.empty(th.shape[0], dtype=torch.float64, device=th.device)
-            st = torch.cuda.current_stream(th.device).cuda_stream
-            _lib.check(self.lib.payne_lnlike_batch_targets(self._ctx, th.data_ptr(), tv.data_ptr(), th.shape[0],
-                                                           th.shape[1], out.data_ptr(), st))
-            return out
-        th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
-        if th.ndim != 2 or th.shape[1] != self.ndim:
-            raise ValueError('theta must be [B, %d]' % self.ndim)
-        if isinstance(target, torch.Tensor):
-            target = target.cpu().numpy()
-        tv = np.ascontiguousarray(np.asarray(target).astype(np.int32, casting='same_kind'))
-        if tv.shape != (th.shape[0],):
-            raise ValueError('target must be [%d]' % th.shape[0])
-        out = np.empty(th.shape[0], dtype=np.float64)
-        _lib.check(self.lib.payne_lnlike_batch_targets_host(self._ctx, th.ctypes.data, tv.ctypes.data, th.shape[0],
-                                                            th.shape[1], out.ctypes.data))
-        return out
+            th, tv, lnl, st = self._dev_args(theta, target, copy=False)
+            _lib.check(self.lib.payne_lnlike_batch_targets(self._ctx, th.data_ptr(), _ptr(tv), th.shape[0],
+                                                           th.shape[1], lnl.data_ptr(), st))
+            return lnl
+        return self._host_lnlike(self.lib.payne_lnlike_batch_targets_host, theta, target, 'target')
 
     def model_batch_targets(self, theta, target, want_flux=True, want_chi2=True, want_mags=True):
         """Model spectra [B, max target_n_obs] (row p: its members' spectra back to back in member order, the rest
@@ -541,25 +490,15 @@ class Engine:
         lnL [B], as CUDA float64 tensors."""
         if not self.n_targets:
             raise ValueError('no targets: set_targets first')
-        dev = torch.device('cuda', self.device)
-        if not isinstance(theta, torch.Tensor):
-            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
-        th = self._theta_dev(theta.to(dev))
-        B = th.shape[0]
-        if not isinstance(target, torch.Tensor):
-            target = torch.from_numpy(np.ascontiguousarray(np.asarray(target).astype(np.int32, casting='same_kind')))
-        tv = self._star_dev(target.to(dev), B, dev)
+        th, tv, lnl, st = self._dev_args(theta, target, copy=True)
+        B, dev = th.shape[0], th.device
         nf = max(self.target_n_obs)
-        flux = torch.full((B, nf), float('nan'), dtype=torch.float64, device=dev) if want_flux else None
-        chi2 = torch.full((B, self.target_kmax), float('nan'), dtype=torch.float64, device=dev) if want_chi2 else None
-        mags = torch.full((B, self.nb), float('nan'), dtype=torch.float64, device=dev) if (want_mags and self.nb) else None
-        lnl = torch.empty(B, dtype=torch.float64, device=dev)
-        st = torch.cuda.current_stream(dev).cuda_stream
+        flux = _nan(want_flux, (B, nf), dev)
+        chi2 = _nan(want_chi2, (B, self.target_kmax), dev)
+        mags = _nan(want_mags and self.nb, (B, self.nb), dev)
         _lib.check(self.lib.payne_model_batch_targets(
-            self._ctx, th.data_ptr(), tv.data_ptr(), B, th.shape[1],
-            flux.data_ptr() if flux is not None else None, nf,
-            chi2.data_ptr() if chi2 is not None else None, self.target_kmax,
-            mags.data_ptr() if mags is not None else None, lnl.data_ptr(), st))
+            self._ctx, th.data_ptr(), _ptr(tv), B, th.shape[1], _ptr(flux), nf, _ptr(chi2), self.target_kmax,
+            _ptr(mags), lnl.data_ptr(), st))
         return flux, chi2, mags, lnl
 
     def last_ms(self, which):
@@ -573,14 +512,41 @@ class Engine:
             raise ValueError('theta has %d columns, layout expects %d' % (theta.shape[1], self.ndim))
         return theta.contiguous()
 
-    def _star_dev(self, star, B, dev):
-        if star is None:
-            return None
-        if not (isinstance(star, torch.Tensor) and star.is_cuda and star.dtype == torch.int32):
-            raise ValueError('with a CUDA theta, star must be an int32 CUDA tensor')
-        if star.shape != (B,) or star.device != dev:
-            raise ValueError('star must be [%d] on %s' % (B, dev))
-        return star.contiguous()
+    def _dev_args(self, theta, idx, copy):
+        """A device entry's inputs: theta [B, ndim] and idx [B] (every row's star or target; None: star 0) as CUDA
+        tensors, an empty float64 lnL [B] on their device and that device's current stream.  ``copy``: numpy and CPU
+        inputs are copied to the engine's device first; else theta must be a CUDA tensor and idx an int32 CUDA
+        tensor on its device."""
+        if copy:
+            theta = theta if isinstance(theta, torch.Tensor) else torch.from_numpy(_f64(theta))
+            theta = theta.to(torch.device('cuda', self.device))
+        th = self._theta_dev(theta)
+        B, dev = th.shape[0], th.device
+        if idx is not None:
+            if copy:
+                idx = (idx if isinstance(idx, torch.Tensor) else torch.from_numpy(_i32(idx))).to(dev)
+            if not (isinstance(idx, torch.Tensor) and idx.is_cuda and idx.dtype == torch.int32):
+                raise ValueError('with a CUDA theta, star must be an int32 CUDA tensor')
+            if idx.shape != (B,) or idx.device != dev:
+                raise ValueError('star must be [%d] on %s' % (B, dev))
+            idx = idx.contiguous()
+        return th, idx, torch.empty(B, dtype=torch.float64, device=dev), torch.cuda.current_stream(dev).cuda_stream
+
+    def _host_lnlike(self, entry, theta, idx, what):
+        """lnL [B] (numpy) through the host-buffer entry ``entry``: theta [B, ndim] and idx [B] (every row's star or
+        target, ``what``; None: star 0) as anything numpy takes."""
+        th = _f64(theta)
+        if th.ndim != 2 or th.shape[1] != self.ndim:
+            raise ValueError('theta must be [B, %d]' % self.ndim)
+        iv = None
+        if idx is not None:
+            iv = _i32(idx.cpu().numpy() if isinstance(idx, torch.Tensor) else idx)
+            if iv.shape != (th.shape[0],):
+                raise ValueError('%s must be [%d]' % (what, th.shape[0]))
+        out = np.empty(th.shape[0], dtype=np.float64)
+        _lib.check(entry(self._ctx, th.ctypes.data, iv.ctypes.data if iv is not None else None, th.shape[0], th.shape[1],
+                         out.ctypes.data))
+        return out
 
     def lnlike_batch(self, theta, star=None):
         """theta: [B, ndim] float64.  CUDA tensor -> CUDA tensor [B] (stream-ordered, no sync);
@@ -589,51 +555,22 @@ class Engine:
         which only a single-star engine accepts).  On the device a row with an index outside
         [0, n_stars) gets NaN and sets status bit 2; the host path refuses such an index."""
         if isinstance(theta, torch.Tensor) and theta.is_cuda:
-            th = self._theta_dev(theta)
-            sv = self._star_dev(star, th.shape[0], th.device)
-            out = torch.empty(th.shape[0], dtype=torch.float64, device=th.device)
-            st = torch.cuda.current_stream(th.device).cuda_stream
-            _lib.check(self.lib.payne_lnlike_batch_stars(self._ctx, th.data_ptr(),
-                                                         sv.data_ptr() if sv is not None else None,
-                                                         th.shape[0], th.shape[1], out.data_ptr(), st))
-            return out
-        th = np.ascontiguousarray(np.asarray(theta, dtype=np.float64))
-        if th.ndim != 2 or th.shape[1] != self.ndim:
-            raise ValueError('theta must be [B, %d]' % self.ndim)
-        sv = None
-        if star is not None:
-            if isinstance(star, torch.Tensor):
-                star = star.cpu().numpy()
-            sv = np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind'))
-            if sv.shape != (th.shape[0],):
-                raise ValueError('star must be [%d]' % th.shape[0])
-        out = np.empty(th.shape[0], dtype=np.float64)
-        _lib.check(self.lib.payne_lnlike_batch_stars_host(self._ctx, th.ctypes.data,
-                                                          sv.ctypes.data if sv is not None else None,
-                                                          th.shape[0], th.shape[1], out.ctypes.data))
-        return out
+            th, sv, lnl, st = self._dev_args(theta, star, copy=False)
+            _lib.check(self.lib.payne_lnlike_batch_stars(self._ctx, th.data_ptr(), _ptr(sv), th.shape[0], th.shape[1],
+                                                         lnl.data_ptr(), st))
+            return lnl
+        return self._host_lnlike(self.lib.payne_lnlike_batch_stars_host, theta, star, 'star')
 
     def model_batch(self, theta, star=None, want_flux=True, want_mags=True):
         """Model spectra [B, n_obs], magnitudes [B, nb] and lnL [B] as CUDA float64 tensors.  With several
         stars, n_obs is the largest star's: row p holds the first ``n_obs_star[star[p]]`` pixels, the rest
         stay NaN; likewise row p of the magnitudes holds its star's ``star_bands[star[p]]``, the rest NaN.  ``star`` as in ``lnlike_batch`` (numpy is copied to the device)."""
-        dev = torch.device('cuda', self.device)
-        if not isinstance(theta, torch.Tensor):
-            theta = torch.from_numpy(np.ascontiguousarray(np.asarray(theta, dtype=np.float64)))
-        th = self._theta_dev(theta.to(dev))
-        B = th.shape[0]
-        if star is not None and not isinstance(star, torch.Tensor):
-            star = torch.from_numpy(np.ascontiguousarray(np.asarray(star).astype(np.int32, casting='same_kind')))
-        sv = self._star_dev(star.to(dev) if star is not None else None, B, dev)
-        flux = torch.full((B, self.n_obs), float('nan'), dtype=torch.float64, device=dev) \
-            if (want_flux and self.n_obs) else None
-        mags = torch.full((B, self.nb), float('nan'), dtype=torch.float64, device=dev) if (want_mags and self.nb) else None
-        lnl = torch.empty(B, dtype=torch.float64, device=dev)
-        st = torch.cuda.current_stream(dev).cuda_stream
+        th, sv, lnl, st = self._dev_args(theta, star, copy=True)
+        B, dev = th.shape[0], th.device
+        flux = _nan(want_flux and self.n_obs, (B, self.n_obs), dev)
+        mags = _nan(want_mags and self.nb, (B, self.nb), dev)
         _lib.check(self.lib.payne_model_batch_stars(
-            self._ctx, th.data_ptr(), sv.data_ptr() if sv is not None else None, B, th.shape[1],
-            flux.data_ptr() if flux is not None else None, self.n_obs,
-            mags.data_ptr() if mags is not None else None, lnl.data_ptr(), st))
+            self._ctx, th.data_ptr(), _ptr(sv), B, th.shape[1], _ptr(flux), self.n_obs, _ptr(mags), lnl.data_ptr(), st))
         return flux, mags, lnl
 
     def ann_eval(self, x):
