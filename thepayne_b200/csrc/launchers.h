@@ -44,7 +44,8 @@ int tc_gemm_test_x(const float* dA, int M, int N, int K, int precision, TcActs& 
 // One form of tail_fast_kernel per kind of batch: points naming stars, targets (payne_ctx_set_targets), binaries
 // (payne_ctx_set_binary) and continuum marginalisation (payne_ctx_set_cont_marg, for points or targets).  Each size
 // has a form's instantiations in two translation units: without (tail_fast_tu.cu) and with (tail_fast_poly_tu.cu)
-// continuum polynomial or model output in the final pass; Binary and Marg exist with them only.
+// continuum polynomial or model output in the final pass; Binary and Marg exist with them only.  tail_fast_tu.inl maps a
+// form (and the second of its pair: several stars, or targets under Marg) to the kernel's point body, FastBody.
 enum class FastForm { Point, Target, Binary, Marg };
 // sets the dynamic shared-memory opt-in of every instantiation `form` may launch at 2^l2 samples on the current device
 // and reports the smallest of their resident CTAs per SM; false when the kernel does not exist for l2 or a query fails
@@ -52,8 +53,8 @@ bool probe_tail_fast(int l2, FastForm form, size_t smem_bytes, int* ctas_per_sm)
 // the instantiation follows from T: polynomial or model output (T.n_poly, T.model_out), several stars (Point,
 // T.n_stars > 1) or targets (Marg, T.target)
 int launch_tail_fast(int l2, FastForm form, int grid, size_t smem_bytes, cudaStream_t st, const TailParams& T, const FastGrid& F);
-// the per-point setup of a slab of nb points: one item per point, per (point, member) of a target (Target, or Marg
-// with T.target) or per (point, component) of a binary
+// the per-point setup of a slab of nb points (tail_setup_kernel<BODY>): one item per point, per (point, member) of a
+// target (Target, or Marg with T.target) or per (point, component) of a binary
 int launch_tail_setup(FastForm form, int nb, cudaStream_t st, const TailParams& T, const FastGrid& F);
 // copies the first-pass constants into the translation units' __constant__ memory on the current device
 // (call once per context, before the first launch)

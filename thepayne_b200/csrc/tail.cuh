@@ -108,7 +108,7 @@ struct TailParams {
   // Binaries (payne_ctx_set_binary; fast tail only): point p's component c has emulator row c * B + p and FastPoint
   // record c * B + p.  Null binary: no binary.
   const PayneBinary* binary;         // device copy
-  double* bin_par;                   // [B, 3] Teff_1, Teff_2, Rratio of every point (tail_setup_binary_kernel)
+  double* bin_par;                   // [B, 3] Teff_1, Teff_2, Rratio of every point (tail_setup_kernel)
   double* aj_scratch;                // [grid, aj_ld] a_1 (binaries) or a_j (marginalisation) of the CTA's current point
   long long aj_ld;
   double* comp_out;                  // [B, 2, ld_flux] a_1 and a_2, or null
@@ -138,6 +138,35 @@ __device__ __forceinline__ void gather_exit(const TailParams& P, unsigned nctas)
     __threadfence_system();
     for (int r = 0; r < P.g_world; ++r) *reinterpret_cast<volatile unsigned long long*>(P.g_flag[r]) = P.g_raise;
   }
+}
+
+// The CTA's sum of every thread's acc, complete in thread 0 (0 elsewhere): warp shuffles, then the warps' partials in
+// warp order, so the bits do not depend on scheduling.  red: kTailThreads / 32 doubles of shared memory, written before
+// the barrier this ends with.
+__device__ __forceinline__ double cta_sum(double acc, double* red, int tid) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if ((tid & 31) == 0) red[tid >> 5] = acc;
+  __syncthreads();
+  double c2 = 0.0;
+  if (tid == 0) {
+#pragma unroll
+    for (int w = 0; w < kTailThreads / 32; ++w) c2 += red[w];
+  }
+  return c2;
+}
+
+// NaN into the n model pixels of a bad point (or member) from column moff of row p; nothing without model output
+__device__ __forceinline__ void model_nan(const TailParams& P, int p, int moff, int n, int tid) {
+  if (P.model_out)
+    for (int j = tid; j < n; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + moff + j] = CUDART_NAN;
+}
+
+// A per-point record into shared memory, as int4 by threads 0 .. sizeof(T) / 16 - 1; the caller's barrier publishes it
+template <class T>
+__device__ __forceinline__ void load_record(T& dst, const T* src, int tid) {
+  static_assert(sizeof(T) % 16 == 0, "records are copied as int4");
+  if (tid < (int)(sizeof(T) / 16)) reinterpret_cast<int4*>(&dst)[tid] = __ldg(reinterpret_cast<const int4*>(src) + tid);
 }
 
 struct PointSetup {
@@ -241,6 +270,21 @@ struct RotHT {
   }
 };
 using RotH = RotHT<0>;
+
+// Stage 1's transfer function at N1 samples, with the rotation table's first intervals staged in the CTA's shared-memory
+// window `win` (win_floats floats, 4 per interval).  The point can touch the entries [0, vsini_scale * N1/2 + 3]; a point
+// whose range is longer keeps its first win_floats/4 intervals there and reads the rest from the global table.  The
+// window holds the first intervals of the one table, so the win_have intervals an earlier point of the CTA staged stay
+// valid.  The caller's next barrier publishes the new entries.
+__device__ __forceinline__ RotHT<2> rot_window(const TailParams& P, const PointSetup& S, int N1, float* win, int win_floats,
+                                               int& win_have, int tid) {
+  const double xt_max = S.vsini_scale * (double)(N1 >> 1);
+  float4* win4 = reinterpret_cast<float4*>(win);
+  const int nwin = (int)fmin(fmin(xt_max + 2.0, (double)(win_floats >> 2)), (double)P.ntab);
+  for (int i = win_have + tid; i < nwin; i += kTailThreads) win4[i] = __ldg(P.sbtab + i);
+  win_have = max(win_have, nwin);
+  return RotHT<2>{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, 1.0f / (float)(N1 >> 1), P.ntab, RotHT<2>::fix40(S.vsini_scale)};
+}
 
 // Gaussian taper exp(-2 pi^2 sigma^2 ss^2) (smoothing.py:598-600), ss = k / (N dv).
 struct GaussH {

@@ -348,6 +348,9 @@ __device__ __forceinline__ double final_pass_part(const TailParams& P, const Fas
 
 // One cluster of four CTAs owns one live point at a time.  LOG2N1 in {15, 16}; every CTA holds N1/8 complex
 // points (32 / 64 KB) plus its own copy of the rotation-table window.
+// (It keeps its own copies of the record load, the NaN model row, the window staging and the CTA reduction of tail.cuh:
+// with those helpers the code of all four instantiations changed -- rot_window alone changed it for STARS -- and the
+// 65536-sample single-star kernel's stack and spills went from 144 / 184 / 72 to 136 / 176 / 64 bytes.)
 template <int LOG2N1, bool STARS>
 __global__ void __launch_bounds__(kNT, 3)
 tail_cluster_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {

@@ -53,12 +53,11 @@ struct FastSetup {
 };
 
 // Per-point setup, computed by tail_setup_kernel (one thread per point) ahead of the tail so that
-// no CTA of the tail idles behind a single thread's fp64 logarithms.
+// no CTA of the tail idles behind a single thread's fp64 logarithms.  Copied into shared memory as int4 (load_record).
 struct alignas(16) FastPoint {
   PointSetup S;
   FastSetup FS;
 };
-static_assert(sizeof(FastPoint) % 16 == 0, "FastPoint is copied as int4");
 
 template <class T>
 __device__ __forceinline__ void divmod_init(int tid, int num, int den, int& j, int& rem) {
@@ -733,80 +732,250 @@ __device__ __forceinline__ double marg_point(const TailParams& P, const FastGrid
   return plain_pass<true, true>(P, S, FS, row, tid, p, moff, K);
 }
 
-// Stage 1 of tail_fast_kernel (rotational broadening on the full emulator grid) for a binary's component: writes back
-// the row's pixels [blo, bhi] and ends with a barrier.  win / win_have: the CTA's shared-memory window of the rotation
-// table.  (The kernel's other instantiations keep their own copy: moving theirs into this function cost the 4096- and
-// 8192-sample plain kernels 92 bytes of spills.)
+// The point body a tail_fast_kernel runs per point, its form (tail_fast_tu.inl maps the host's FastForm to it):
+//  OneStar      a single-star context, whose pixel bounds are the kernel parameters' (obs_lo / obs_hi);
+//  Stars        a context of several stars: the point's star;
+//  Target       every point names a target (TailParams::target): stage 1 runs once on the row, then stage 2 and the final
+//               pass once per member against that member's record, and lnL is the members' chi2 summed in member order;
+//  Binary       every point is a binary (TailParams::binary): component 1's record and row, stage 1, stage 2 and a final
+//               pass that keeps a_1; then component 2's, whose final pass combines the two (final_pass_bin);
+//  MargStars /  continuum marginalisation (TailParams::marg_k) of a point or of every member of a target, through
+//  MargTargets  marg_point: lnL = -0.5 (Q + chi2_sed) + M (members: Q and M each summed in member order).
+// Binary and Marg* have the polynomial / model-output final pass only (POLY).
+enum class FastBody { OneStar, Stars, Target, Binary, MargStars, MargTargets };
+
+__host__ __device__ constexpr bool body_target(FastBody b) { return b == FastBody::Target || b == FastBody::MargTargets; }
+__host__ __device__ constexpr bool body_marg(FastBody b) { return b == FastBody::MargStars || b == FastBody::MargTargets; }
+
+// What a point body needs of its kernel: the transform buffer and its views, the rotation-table window, the reduction
+// slots
+struct FastCta {
+  float2* z;
+  ZSmem zs;
+  ZSplit zp;
+  float* gline;
+  TwTab tw;
+  float* win;
+  int win_have;                                           // table intervals already in the window
+  double* red;
+  int tid;
+};
+
+// Stage 1 (rotational broadening on the full emulator grid): writes back the row's pixels [blo, bhi] (those stage 2
+// reads) and ends with a barrier.
 template <int LOG2N1>
-__device__ __forceinline__ void rot_stage(const TailParams& P, const FastGrid& F, const PointSetup& S, float2* z,
-                                          const ZSmem& zs, const ZSplit& zp, float* gline, const TwTab& tw, float* win,
-                                          int& win_have, float* row, int tid, int blo, int bhi) {
+__device__ __forceinline__ void rot_stage(const TailParams& P, const FastGrid& F, const PointSetup& S, FastCta& c,
+                                          float* row, int blo, int bhi) {
   constexpr int N1 = 1 << LOG2N1;
   constexpr bool kSplit = LOG2N1 >= 16;
   constexpr int LOG2MH = kSplit ? LOG2N1 - 2 : 8;          // complex points per half (split only)
-  const int n = P.n;
-  // the table entries this point can touch: [0, vsini_scale * N1/2 + 3]; staged in shared
-  // memory when they fit (the barrier after the regrid below publishes them)
-  const double xt_max = S.vsini_scale * (double)(N1 >> 1);
-  // (a point whose range is longer keeps its first win_floats/4 intervals there and reads the rest
-  // from the global table)
-  float4* win4 = reinterpret_cast<float4*>(win);
-  const int nwin = (int)fmin(fmin(xt_max + 2.0, (double)(F.win_floats >> 2)), (double)P.ntab);
-  // (the window holds the first intervals of the one table: what an earlier point of this CTA staged stays valid)
-  for (int i = win_have + tid; i < nwin; i += kNT) win4[i] = __ldg(P.sbtab + i);
-  win_have = max(win_have, nwin);
-  const RotHT<2> H{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, 1.0f / (float)(N1 >> 1), P.ntab, RotHT<2>::fix40(S.vsini_scale)};
+  const int n = P.n, tid = c.tid;
+  // (the barrier after the regrid below publishes the window)
+  const RotHT<2> H = rot_window(P, S, N1, c.win, F.win_floats, c.win_have, tid);
   if constexpr (!kSplit) {
     // regrid fused into the first FFT pass (measured against the separate regrid: tail -5 %)
-    ct_convolve_regrid<LOG2N1 - 1>(z, tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
-    regrid_back(row, zs, F, tid, n, N1, blo, bhi);
+    ct_convolve_regrid<LOG2N1 - 1>(c.z, c.tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
+    regrid_back(row, c.zs, F, tid, n, N1, blo, bhi);
   } else {
-    stage_regrid(S, row, zp, tid, N1, F.f_num, F.f_den, 0, F.f_invden, F.c_native, F.f_incj, F.f_incr);
+    stage_regrid(S, row, c.zp, tid, N1, F.f_num, F.f_den, 0, F.f_invden, F.c_native, F.f_incj, F.f_incr);
     __syncthreads();
-    ct_convolve_split<LOG2MH>(z, reinterpret_cast<float2*>(gline), tw, F.twc, H, tid);
-    regrid_back(row, zp, F, tid, n, N1, blo, bhi);
+    ct_convolve_split<LOG2MH>(c.z, reinterpret_cast<float2*>(c.gline), c.tw, F.twc, H, tid);
+    regrid_back(row, c.zp, F, tid, n, N1, blo, bhi);
   }
   __syncthreads();
+}
+
+// A point against its star (OneStar, Stars, MargStars; not a bad one): stage 1, then point_chi2 or marg_point, and lnL.
+template <int LOG2N1, bool POLY, FastBody BODY>
+__device__ __forceinline__ void star_point(const TailParams& P, const FastGrid& F, PointSetup& S, const FastSetup& FS,
+                                           FastCta& c, float* row, int p) {
+  constexpr bool STARS = BODY != FastBody::OneStar;
+  const int tid = c.tid;
+  if (POLY && !body_marg(BODY) && S.do_rot) {
+    rot_stage<LOG2N1>(P, F, S, c, row, S.use_inst ? max(S.i0 - 1, 0) : 0, S.use_inst ? min(S.i1 + 1, P.n - 1) : P.n - 1);
+  } else if (S.do_rot) {
+    // The plain kernels (the sampler's hot path) and MargStars keep their own copy of stage 1 and of its window
+    // staging: calling rot_stage cost the 4096- and 8192-sample plain kernels 92 to 124 bytes of spills and the
+    // MargStars kernels of those sizes 72 / 84 and 92 / 104 bytes of spill stores / loads, and rot_window alone
+    // changed the code of every plain kernel.
+    constexpr int N1 = 1 << LOG2N1;
+    constexpr bool kSplit = LOG2N1 >= 16;
+    constexpr int LOG2MH = kSplit ? LOG2N1 - 2 : 8;
+    const int n = P.n;
+    // the table entries this point can touch: [0, vsini_scale * N1/2 + 3]; staged in shared memory when they fit (the
+    // barrier after the regrid below publishes them)
+    const double xt_max = S.vsini_scale * (double)(N1 >> 1);
+    float4* win4 = reinterpret_cast<float4*>(c.win);
+    const int nwin = (int)fmin(fmin(xt_max + 2.0, (double)(F.win_floats >> 2)), (double)P.ntab);
+    for (int i = c.win_have + tid; i < nwin; i += kNT) win4[i] = __ldg(P.sbtab + i);
+    c.win_have = max(c.win_have, nwin);
+    const RotHT<2> H{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, 1.0f / (float)(N1 >> 1), P.ntab, RotHT<2>::fix40(S.vsini_scale)};
+    // pixels stage 2 will read: its mask [i0, i1] (one more on each side keeps the edge patch exact)
+    const int blo = S.use_inst ? max(S.i0 - 1, 0) : 0;
+    const int bhi = S.use_inst ? min(S.i1 + 1, n - 1) : n - 1;
+    if constexpr (!kSplit) {
+      ct_convolve_regrid<LOG2N1 - 1>(c.z, c.tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
+      regrid_back(row, c.zs, F, tid, n, N1, blo, bhi);
+    } else {
+      stage_regrid(S, row, c.zp, tid, N1, F.f_num, F.f_den, 0, F.f_invden, F.c_native, F.f_incj, F.f_incr);
+      __syncthreads();
+      ct_convolve_split<LOG2MH>(c.z, reinterpret_cast<float2*>(c.gline), c.tw, F.twc, H, tid);
+      regrid_back(row, c.zp, F, tid, n, N1, blo, bhi);
+    }
+    __syncthreads();
+  }
+  if constexpr (body_marg(BODY)) {
+    double M = 0.0;
+    double c2 = cta_sum(marg_point<LOG2N1>(P, F, S, FS, c.z, c.zs, c.zp, c.gline, c.tw, row, tid, p, 0,
+                                           star_of(P.star, P.n_stars, p), 0, 0, M), c.red, tid);
+    if (tid == 0) {
+      if (P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2] = c2;
+      if (P.chi2_sed) c2 += P.chi2_sed[p];
+      if (P.lnl) store_lnl(P, p, -0.5 * c2 + M);
+    }
+  } else {
+    // (the CTA reduction of cta_sum written out, the warps' sum taken only where lnL is stored: cta_sum here changed
+    // the code of the plain kernels and the stack and spills of the 2048-sample polynomial one)
+    double acc = point_chi2<LOG2N1, POLY, STARS>(P, F, S, FS, c.z, c.zs, c.zp, c.gline, c.tw, row, tid, p, 0);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if ((tid & 31) == 0) c.red[tid >> 5] = acc;
+    __syncthreads();
+    if (tid == 0 && P.lnl) {
+      double c2 = 0.0;
+#pragma unroll
+      for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += c.red[wdx];
+      if (P.chi2_sed) c2 += P.chi2_sed[p];
+      store_lnl(P, p, -0.5 * c2);
+    }
+  }
+}
+
+// A point naming a target (Target, MargTargets) of K > 0 members, whose records rec[0, K) the kernel loaded from rec[0]
+// on: stage 1 once on the row's pixels tu = the union of the members' windows, then every member against its own
+// record; the row is read-only from there on.
+template <int LOG2N1, bool POLY, FastBody BODY>
+__device__ __forceinline__ void target_point(const TailParams& P, const FastGrid& F, FastPoint& SP, FastCta& c,
+                                             float* row, int p, const FastPoint* rec, int K, int2 tu) {
+  PointSetup& S = SP.S;
+  const FastSetup& FS = SP.FS;
+  const int tid = c.tid;
+  // the labels and Vrot of every member are the first member's (payne_ctx_set_targets), so its do_rot, vsini_scale
+  // and clean hold for the row; skipped when every member is bad
+  if (S.do_rot && tu.x <= tu.y) rot_stage<LOG2N1>(P, F, S, c, row, tu.x, tu.y);
+  // Member m's model pixels follow those of members 0 .. m-1 (the members' observations lie back to back in the set's
+  // arrays).
+  const int off0 = FS.obs.off;
+  double tot = 0.0;                                       // thread 0: chi2 of members 0 .. m, summed in that order
+  double mtot = 0.0;                                      // Marg, thread 0: M of members 0 .. m, likewise
+  int cofs = 0, lofs = 0;                                 // Marg: the member's first coefficient / Cholesky column
+  for (int m = 0; m < K; ++m) {
+    if (m > 0) {
+      __syncthreads();                                    // member m-1's record, transform buffer and red[] are free
+      load_record(SP, rec + m, tid);
+      __syncthreads();
+    }
+    const bool bad = S.bad != 0;
+    const int moff = FS.obs.off - off0;
+    double acc = 0.0;
+    double M = 0.0;                                       // Marg: the member's M (thread 0)
+    int km = 0;                                           // Marg: the member's coefficients
+    if constexpr (body_marg(BODY)) {
+      const int k = __ldg(P.tfirst + __ldg(P.target + p)) + m;
+      km = __ldg(P.marg_k + k);
+      if (!bad) acc = marg_point<LOG2N1>(P, F, S, FS, c.z, c.zs, c.zp, c.gline, c.tw, row, tid, p, moff, k, cofs, lofs, M);
+      else {
+        model_nan(P, p, moff, FS.obs.n, tid);
+        marg_nan_out(P, p, km, cofs, lofs, tid);
+      }
+    } else {
+      if (!bad) acc = point_chi2<LOG2N1, POLY, true>(P, F, S, FS, c.z, c.zs, c.zp, c.gline, c.tw, row, tid, p, moff);
+      else model_nan(P, p, moff, FS.obs.n, tid);
+    }
+    double c2 = cta_sum(acc, c.red, tid);
+    if (tid == 0) {
+      if (bad) c2 = CUDART_NAN;
+      if (P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2 + m] = c2;
+      tot = m == 0 ? c2 : tot + c2;
+      if constexpr (body_marg(BODY)) mtot = m == 0 ? M : mtot + M;
+    }
+    if constexpr (body_marg(BODY)) { cofs += km; lofs += km * (km + 1) / 2; }
+  }
+  if (tid == 0 && P.lnl) {
+    if (P.chi2_sed) tot += P.chi2_sed[p];
+    if constexpr (body_marg(BODY)) store_lnl(P, p, -0.5 * tot + mtot);
+    else store_lnl(P, p, -0.5 * tot);
+  }
+}
+
+// A binary: component c's record c * B + p (component 0's loaded by the kernel) on its row c * B + p, stage 1, stage 2
+// and final_pass_bin<c + 1>.  A bad component makes a_c, the model and lnL NaN.
+template <int LOG2N1>
+__device__ __forceinline__ void binary_point(const TailParams& P, const FastGrid& F, FastPoint& SP, FastCta& c,
+                                             float* row, int p, const FastPoint* points) {
+  PointSetup& S = SP.S;
+  const FastSetup& FS = SP.FS;
+  const int tid = c.tid;
+  double acc = 0.0;
+  bool bad = false;
+  for (int cc = 0; cc < 2; ++cc) {
+    float* rowc = row + (long long)cc * P.B * P.ldf;
+    if (cc == 1) {
+      __syncthreads();                                    // component 1's record and transform buffer are free
+      load_record(SP, points + P.B + p, tid);
+      __syncthreads();
+    }
+    if (S.bad) {
+      bad = true;
+      // (a_c, the component row and the model row in one loop: model_nan in its place changed the spills of the
+      // 16384- and 65536-sample binary kernels)
+      double* scr = P.aj_scratch + (long long)blockIdx.x * P.aj_ld;
+      for (int j = tid; j < FS.obs.n; j += kNT) {
+        if (cc == 0) scr[j] = CUDART_NAN;
+        if (P.comp_out) P.comp_out[((long long)p * 2 + cc) * P.ld_flux + j] = CUDART_NAN;
+        if (cc == 1 && P.model_out) P.model_out[(long long)p * P.ld_flux + j] = CUDART_NAN;
+      }
+      continue;
+    }
+    if (S.do_rot) {
+      const int blo = S.use_inst ? max(S.i0 - 1, 0) : 0;
+      const int bhi = S.use_inst ? min(S.i1 + 1, P.n - 1) : P.n - 1;
+      rot_stage<LOG2N1>(P, F, S, c, rowc, blo, bhi);
+    }
+    if (cc == 0) point_chi2<LOG2N1, true, true, 1>(P, F, S, FS, c.z, c.zs, c.zp, c.gline, c.tw, rowc, tid, p, 0);
+    else acc = point_chi2<LOG2N1, true, true, 2>(P, F, S, FS, c.z, c.zs, c.zp, c.gline, c.tw, rowc, tid, p, 0);
+  }
+  const double c2 = cta_sum(acc, c.red, tid);
+  if (tid == 0 && P.lnl) store_lnl(P, p, bad ? CUDART_NAN : -0.5 * c2);
 }
 
 // LOG2N1 <= 15: the whole transform sits in shared memory (3 CTAs/SM up to 2^14).
 // LOG2N1 == 16: split transform, half in shared memory (128 KB), half in the scratch line.
 // POLY: continuum polynomial and / or model output in the final pass (the host picks the instantiation).
-// STARS: a context of several stars (obs_lo / obs_hi).
-// TGT: every point names a target (TailParams::target; STARS is then true): stage 1 runs once on the row, then stage 2
-// and the final pass once per member against that member's record, and lnL is the members' chi2 summed in member order.
-// BIN: every point is a binary (TailParams::binary; POLY and STARS are then true): component 1's record and row, stage 1,
-// stage 2 and a final pass that keeps a_1; then component 2's, whose final pass combines the two (final_pass_bin).
-// MARG: continuum marginalisation (TailParams::marg_k; POLY and STARS are then true): every point, or every member of a
-// target, through marg_point, and lnL = -0.5 (Q + chi2_sed) + M (members: Q and M each summed in member order).
+// BODY: what a point is (FastBody).
 // (3 CTAs/SM, 80 registers with a few spills, measured at C2 0.76 ms against 0.84 ms with 2 CTAs/SM and no spills)
-template <int LOG2N1, bool POLY, bool STARS, bool TGT = false, bool BIN = false, bool MARG = false>
+template <int LOG2N1, bool POLY, FastBody BODY>
 __global__ void __launch_bounds__(kNT, LOG2N1 <= 14 ? 3 : 1)
 tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
+  static_assert(POLY || !(BODY == FastBody::Binary || body_marg(BODY)), "Binary and Marg* have the POLY final pass only");
+  constexpr bool STARS = BODY != FastBody::OneStar;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  float2* z = reinterpret_cast<float2*>(smem_raw);
   float* zf = reinterpret_cast<float*>(smem_raw);
   __shared__ FastPoint SP;
   __shared__ double red[kNT / 32];
-  PointSetup& S = SP.S;
-  FastSetup& FS = SP.FS;
   const int tid = threadIdx.x;
-  const TwTab tw{P.tw, P.log2tw, P.twpass};
-  const double nan = CUDART_NAN;
   constexpr int N1 = 1 << LOG2N1;
   constexpr bool kSplit = LOG2N1 >= 16;
-  constexpr int LOG2MH = kSplit ? LOG2N1 - 2 : 8;          // complex points per half (split only)
   float* gline = kSplit ? F.scratch + (size_t)blockIdx.x * (N1 / 2) : nullptr;
-  const ZSmem zs{zf};
-  const ZSplit zp{zf, gline, N1 / 2};
-  float* win = zf + (kSplit ? N1 / 2 : N1);               // rotation-table window behind the transform buffer
+  // (the rotation-table window lies behind the transform buffer)
+  FastCta c{reinterpret_cast<float2*>(smem_raw), ZSmem{zf}, ZSplit{zf, gline, N1 / 2}, gline,
+            TwTab{P.tw, P.log2tw, P.twpass}, zf + (kSplit ? N1 / 2 : N1), 0, red, tid};
   const FastPoint* points = reinterpret_cast<const FastPoint*>(F.points);
 
   // (lives in red[0], which is dead between the end of one point and the reduction of the next: 16 more bytes of
   // static shared memory would come out of every point's rotation-table window)
   int& s_next = *reinterpret_cast<int*>(&red[0]);
   int pn;
-  int win_have = 0;                                       // table intervals already in the window
   for (int p = blockIdx.x; p < P.B; p = pn) {
     float* row = P.flux + (long long)p * P.ldf;
     // the next point is claimed now (its latency hides under this point) and read after the barrier below; thread 0
@@ -814,7 +983,7 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
     if (tid == 0) s_next = F.work_counter ? atomicAdd(F.work_counter, 1) : p + (int)gridDim.x;
     const FastPoint* rec = points + p;
     int K = 1;                                            // members (targets; 0: no such target)
-    if constexpr (TGT) {
+    if constexpr (body_target(BODY)) {
       const int t = __ldg(P.target + p);
       K = (t >= 0 && t < P.n_targets) ? __ldg(P.tfirst + t + 1) - __ldg(P.tfirst + t) : 0;
       rec = points + (long long)p * P.kmax;
@@ -836,195 +1005,43 @@ tail_fast_kernel(const __grid_constant__ TailParams P, const __grid_constant__ F
         if (tid == 32) *reinterpret_cast<int2*>(&red[1]) = make_int2(lo, hi);
       }
     }
-    if (tid < (int)(sizeof(FastPoint) / 16))
-      reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(rec) + tid);
+    load_record(SP, rec, tid);
     __syncthreads();
     pn = s_next;
     int2 tu = make_int2(0, -1);
-    if constexpr (TGT) {
+    if constexpr (body_target(BODY)) {
       tu = *reinterpret_cast<const int2*>(&red[1]);
       __syncthreads();                                    // red[1] is read everywhere before a member's reduction
     }
-    if constexpr (BIN) {
-      // component c: record c * B + p, row c * B + p
-      double acc = 0.0;
-      bool bad = false;
-      for (int c = 0; c < 2; ++c) {
-        float* rowc = row + (long long)c * P.B * P.ldf;
-        if (c == 1) {
-          __syncthreads();                                // component 1's record and transform buffer are free
-          if (tid < (int)(sizeof(FastPoint) / 16))
-            reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(points + P.B + p) + tid);
-          __syncthreads();
-        }
-        if (S.bad) {                                      // NaN a_c: the model and lnL of the point are NaN
-          bad = true;
-          double* scr = P.aj_scratch + (long long)blockIdx.x * P.aj_ld;
-          for (int j = tid; j < FS.obs.n; j += kNT) {
-            if (c == 0) scr[j] = nan;
-            if (P.comp_out) P.comp_out[((long long)p * 2 + c) * P.ld_flux + j] = nan;
-            if (c == 1 && P.model_out) P.model_out[(long long)p * P.ld_flux + j] = nan;
-          }
-          continue;
-        }
-        if (S.do_rot) {
-          const int blo = S.use_inst ? max(S.i0 - 1, 0) : 0;
-          const int bhi = S.use_inst ? min(S.i1 + 1, P.n - 1) : P.n - 1;
-          rot_stage<LOG2N1>(P, F, S, z, zs, zp, gline, tw, win, win_have, rowc, tid, blo, bhi);
-        }
-        if (c == 0) point_chi2<LOG2N1, true, true, 1>(P, F, S, FS, z, zs, zp, gline, tw, rowc, tid, p, 0);
-        else acc = point_chi2<LOG2N1, true, true, 2>(P, F, S, FS, z, zs, zp, gline, tw, rowc, tid, p, 0);
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-      if ((tid & 31) == 0) red[tid >> 5] = acc;
-      __syncthreads();
-      if (tid == 0 && P.lnl) {
-        double c2 = 0.0;
-#pragma unroll
-        for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
-        store_lnl(P, p, bad ? nan : -0.5 * c2);
-      }
-      if (P.discard_rows) {
-        discard_lines(row, P.n, tid);
-        discard_lines(row + (long long)P.B * P.ldf, P.n, tid);
-      }
-      __syncthreads();
-      continue;
-    }
-    if (TGT ? K == 0 : S.bad) {
-      if (P.model_out)
-        for (int j = tid; j < obs_hi<STARS>(P, FS.obs) - obs_lo<STARS>(FS.obs); j += kNT) P.model_out[(long long)p * P.ld_flux + j] = nan;
-      if constexpr (MARG && !TGT) {
-        const int k = star_of(P.star, P.n_stars, p);
-        if (k >= 0) marg_nan_out(P, p, __ldg(P.marg_k + k), 0, 0, tid);
-        if (tid == 0 && P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2] = nan;
-      }
-      if (tid == 0 && P.lnl) store_lnl(P, p, nan);
-      __syncthreads();
-      continue;
-    }
-    // ---------------- stage 1: rotational broadening on the full emulator grid
-    // (a target: the labels and Vrot of every member are the first member's -- payne_ctx_set_targets -- so its
-    // do_rot, vsini_scale and clean hold for the row; skipped when every member is bad)
-    if (TGT ? (S.do_rot && tu.x <= tu.y) : S.do_rot) {
-      const int n = P.n;
-      // the table entries this point can touch: [0, vsini_scale * N1/2 + 3]; staged in shared
-      // memory when they fit (the barrier after the regrid below publishes them)
-      const double xt_max = S.vsini_scale * (double)(N1 >> 1);
-      // (a point whose range is longer keeps its first win_floats/4 intervals there and reads the rest
-      // from the global table)
-      float4* win4 = reinterpret_cast<float4*>(win);
-      const int nwin = (int)fmin(fmin(xt_max + 2.0, (double)(F.win_floats >> 2)), (double)P.ntab);
-      // (the window holds the first intervals of the one table: what an earlier point of this CTA staged stays valid)
-      for (int i = win_have + tid; i < nwin; i += kNT) win4[i] = __ldg(P.sbtab + i);
-      win_have = max(win_have, nwin);
-      const RotHT<2> H{P.sbtab, win4, nwin, S.vsini_scale, P.sb_h, 1.0f / (float)(N1 >> 1), P.ntab, RotHT<2>::fix40(S.vsini_scale)};
-      // pixels stage 2 will read: its mask [i0, i1] (one more on each side keeps the edge patch exact)
-      const int blo = TGT ? tu.x : S.use_inst ? max(S.i0 - 1, 0) : 0;
-      const int bhi = TGT ? tu.y : S.use_inst ? min(S.i1 + 1, n - 1) : n - 1;
-      if constexpr (!kSplit) {
-        // regrid fused into the first FFT pass (measured against the separate regrid: tail -5 %)
-        ct_convolve_regrid<LOG2N1 - 1>(z, tw, F.twc, H, tid, row, F.f_num, F.f_den, F.f_invden, F.c_native, S.clean != 0);
-        regrid_back(row, zs, F, tid, n, N1, blo, bhi);
-      } else {
-        stage_regrid(S, row, zp, tid, N1, F.f_num, F.f_den, 0, F.f_invden, F.c_native, F.f_incj, F.f_incr);
-        __syncthreads();
-        ct_convolve_split<LOG2MH>(z, reinterpret_cast<float2*>(gline), tw, F.twc, H, tid);
-        regrid_back(row, zp, F, tid, n, N1, blo, bhi);
-      }
-      __syncthreads();
-    }
-
-    if constexpr (!TGT && MARG) {
-      double M = 0.0;
-      double acc = marg_point<LOG2N1>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, 0, star_of(P.star, P.n_stars, p), 0,
-                                      0, M);
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-      if ((tid & 31) == 0) red[tid >> 5] = acc;
-      __syncthreads();
-      if (tid == 0) {
-        double c2 = 0.0;
-#pragma unroll
-        for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
-        if (P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2] = c2;
-        if (P.chi2_sed) c2 += P.chi2_sed[p];
-        if (P.lnl) store_lnl(P, p, -0.5 * c2 + M);
-      }
-    } else if constexpr (!TGT) {
-      double acc = point_chi2<LOG2N1, POLY, STARS>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, 0);
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-      if ((tid & 31) == 0) red[tid >> 5] = acc;
-      __syncthreads();
-      if (tid == 0 && P.lnl) {
-        double c2 = 0.0;
-#pragma unroll
-        for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
-        if (P.chi2_sed) c2 += P.chi2_sed[p];
-        store_lnl(P, p, -0.5 * c2);
-      }
+    if constexpr (BODY == FastBody::Binary) {
+      binary_point<LOG2N1>(P, F, SP, c, row, p, points);
     } else {
-      // every member against its own record: the row is read-only from here on.  Member m's model pixels follow
-      // those of members 0 .. m-1 (the members' observations lie back to back in the set's arrays).
-      const int off0 = FS.obs.off;
-      double tot = 0.0;                                   // thread 0: chi2 of members 0 .. m, summed in that order
-      double mtot = 0.0;                                  // MARG, thread 0: M of members 0 .. m, likewise
-      int cofs = 0, lofs = 0;                             // MARG: the member's first coefficient / Cholesky column
-      for (int m = 0; m < K; ++m) {
-        if (m > 0) {
-          __syncthreads();                                // member m-1's record, transform buffer and red[] are free
-          if (tid < (int)(sizeof(FastPoint) / 16))
-            reinterpret_cast<int4*>(&SP)[tid] = __ldg(reinterpret_cast<const int4*>(rec + m) + tid);
-          __syncthreads();
+      if (body_target(BODY) ? K == 0 : SP.S.bad) {        // NaN lnL and model row; the row is not read
+        // (the model row's NaN fill written out: model_nan here changed the code of the plain kernels)
+        if (P.model_out)
+          for (int j = tid; j < obs_hi<STARS>(P, SP.FS.obs) - obs_lo<STARS>(SP.FS.obs); j += kNT)
+            P.model_out[(long long)p * P.ld_flux + j] = CUDART_NAN;
+        if constexpr (BODY == FastBody::MargStars) {
+          const int k = star_of(P.star, P.n_stars, p);
+          if (k >= 0) marg_nan_out(P, p, __ldg(P.marg_k + k), 0, 0, tid);
+          if (tid == 0 && P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2] = CUDART_NAN;
         }
-        const bool bad = S.bad != 0;
-        const int moff = FS.obs.off - off0;
-        double acc = 0.0;
-        double M = 0.0;                                   // MARG: the member's M (thread 0)
-        int km = 0;                                       // MARG: the member's coefficients
-        if constexpr (MARG) {
-          const int k = __ldg(P.tfirst + __ldg(P.target + p)) + m;
-          km = __ldg(P.marg_k + k);
-          if (!bad) acc = marg_point<LOG2N1>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, moff, k, cofs, lofs, M);
-          else {
-            if (P.model_out)
-              for (int j = tid; j < FS.obs.n; j += kNT) P.model_out[(long long)p * P.ld_flux + moff + j] = nan;
-            marg_nan_out(P, p, km, cofs, lofs, tid);
-          }
-        } else {
-          if (!bad) acc = point_chi2<LOG2N1, POLY, true>(P, F, S, FS, z, zs, zp, gline, tw, row, tid, p, moff);
-          else if (P.model_out)
-            for (int j = tid; j < FS.obs.n; j += kNT) P.model_out[(long long)p * P.ld_flux + moff + j] = nan;
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-        if ((tid & 31) == 0) red[tid >> 5] = acc;
+        if (tid == 0 && P.lnl) store_lnl(P, p, CUDART_NAN);
         __syncthreads();
-        if (tid == 0) {
-          double c2 = 0.0;
-#pragma unroll
-          for (int wdx = 0; wdx < kNT / 32; ++wdx) c2 += red[wdx];
-          if (bad) c2 = nan;
-          if (P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2 + m] = c2;
-          tot = m == 0 ? c2 : tot + c2;
-          if constexpr (MARG) mtot = m == 0 ? M : mtot + M;
-        }
-        if constexpr (MARG) { cofs += km; lofs += km * (km + 1) / 2; }
+        continue;
       }
-      if (tid == 0 && P.lnl) {
-        if (P.chi2_sed) tot += P.chi2_sed[p];
-        if constexpr (MARG) store_lnl(P, p, -0.5 * tot + mtot);
-        else store_lnl(P, p, -0.5 * tot);
-      }
+      if constexpr (body_target(BODY)) target_point<LOG2N1, POLY, BODY>(P, F, SP, c, row, p, rec, K, tu);
+      else star_point<LOG2N1, POLY, BODY>(P, F, SP.S, SP.FS, c, row, p);
     }
     // The row is scratch and fully consumed: L2 is told to drop its lines instead of writing them back
     // (discard.global.L2).  Without this every row crosses HBM three times (the emulator's write is evicted --
     // the slab is larger than L2 --, the tail reads it, and the in-place rewrite after the rotation stage is
     // evicted again): measured DRAM traffic of the tail 456 MB = 2.0x the algorithmic bytes, 254 MB = 1.09x
     // with the discard, for +1.4 % of kernel time.  Only lines that lie wholly inside this row are dropped.
-    if (P.discard_rows) discard_lines(row, P.n, tid);
+    if (P.discard_rows) {
+      discard_lines(row, P.n, tid);
+      if constexpr (BODY == FastBody::Binary) discard_lines(row + (long long)P.B * P.ldf, P.n, tid);
+    }
     __syncthreads();
   }
   if (tid == 0) gather_exit(P, gridDim.x);
@@ -1042,21 +1059,47 @@ __device__ __forceinline__ void stage2_setup(const FastGrid& F, const PointSetup
   FS.q0 = (double)S.i0 + S.lnD * F.inv_dlnw;
 }
 
-// One thread per point: mask limits, transform sizes, Doppler factor, taper constant, and the
-// stage-2 / final regrid ratios (the serial prologue of the tail, done for the whole slab at once).
-template <int kUnused = 0>
+// One thread per setup item (the serial prologue of the tail, done for the whole slab at once): mask limits, transform
+// sizes, Doppler factor, taper constant and the stage-2 / final regrid ratios of FastPoint record `item`.  The item of
+// tail_fast_kernel<BODY>'s point p:
+//  - a point of one star (OneStar, Stars, MargStars; launched as Stars): item p;
+//  - a target's member m (Target, MargTargets; launched as Target): item p * kmax + m.  The items of members a target
+//    does not have are not written; a point whose target lies outside [0, n_targets) gets a bad record at p * kmax;
+//  - a binary's component c (Binary): item c * B + p, the secondary's labels, Vrad and Vrot through P.binary, and from
+//    component 0's thread the point's Teff_1, Teff_2 and Rratio.
+template <FastBody BODY>
 __global__ void __launch_bounds__(64)
 tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= P.B) return;
-  FastPoint* out = reinterpret_cast<FastPoint*>(F.points) + p;
-  if (p == 0 && F.work_counter) *F.work_counter = F.work_start;
+  constexpr bool TGT = body_target(BODY), BIN = BODY == FastBody::Binary;
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long long)P.B * (TGT ? P.kmax : BIN ? 2 : 1)) return;
+  if (i == 0 && F.work_counter) *F.work_counter = F.work_start;
+  int p, k, c = 0;                                        // point, star, component
+  if constexpr (TGT) {
+    p = (int)(i / P.kmax);
+    const int m = (int)(i - (long long)p * P.kmax);
+    const int t = P.target[p];
+    k = -1;
+    if (t >= 0 && t < P.n_targets) {
+      const int f = P.tfirst[t];
+      if (m >= P.tfirst[t + 1] - f) return;
+      k = f + m;
+    } else if (m > 0) {
+      return;
+    }
+  } else {
+    if constexpr (BIN) c = (int)(i / P.B);
+    p = (int)(i - (long long)c * P.B);
+    k = star_of(P.star, P.n_stars, p);
+  }
+  const double* th = P.theta + (long long)p * P.ld;
   PointSetup S{};
   FastSetup FS{};
-  tail_setup(P, P.theta + (long long)p * P.ld, p, S, FS.obs);
+  tail_setup_star(P, th, k, S, FS.obs, c ? P.binary : nullptr);
   if (!S.bad && S.use_inst) {
     stage2_setup(F, S, FS);
-    if (F.cluster && P.stars[star_of(P.star, P.n_stars, p)].sorted) {
+    // (F.cluster is set for batches of points naming stars only)
+    if (F.cluster && P.stars[k].sorted) {
       // tail_cluster.cuh: CTA r of the cluster serves the observed pixels whose position falls into quarter r
       for (int r = 0; r < 3; ++r) {
         const double thr = (double)((long long)(r + 1) << (S.log2N2 - 2));
@@ -1071,56 +1114,10 @@ tail_setup_kernel(const __grid_constant__ TailParams P, const __grid_constant__ 
       FS.jcut[0] = -1;
     }
   }
-  out->S = S;
-  out->FS = FS;
-}
-
-// Targets: one thread per (point, member) item, item i = p * kmax + m (the items of members a target does not have
-// are not written).  A point whose target lies outside [0, n_targets) gets a bad record at item p * kmax.
-template <int kUnused = 0>
-__global__ void __launch_bounds__(64)
-tail_setup_targets_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= (long long)P.B * P.kmax) return;
-  if (i == 0 && F.work_counter) *F.work_counter = F.work_start;
-  const int p = (int)(i / P.kmax), m = (int)(i - (long long)p * P.kmax);
-  const int t = P.target[p];
-  int k = -1;
-  if (t >= 0 && t < P.n_targets) {
-    const int f = P.tfirst[t];
-    if (m >= P.tfirst[t + 1] - f) return;
-    k = f + m;
-  } else if (m > 0) {
-    return;
-  }
-  PointSetup S{};
-  FastSetup FS{};
-  tail_setup_star(P, P.theta + (long long)p * P.ld, k, S, FS.obs);
-  if (!S.bad && S.use_inst) stage2_setup(F, S, FS);
   FastPoint* out = reinterpret_cast<FastPoint*>(F.points) + i;
   out->S = S;
   out->FS = FS;
-}
-
-// Binaries: one thread per (point, component) item, item i = c * B + p: component c's record i (the secondary's
-// labels, Vrad and Vrot through P.binary) and, from component 1's thread, the point's Teff_1, Teff_2 and Rratio.
-template <int kUnused = 0>
-__global__ void __launch_bounds__(64)
-tail_setup_binary_kernel(const __grid_constant__ TailParams P, const __grid_constant__ FastGrid F) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 2LL * P.B) return;
-  if (i == 0 && F.work_counter) *F.work_counter = F.work_start;
-  const int c = (int)(i / P.B), p = (int)(i - (long long)c * P.B);
-  const double* th = P.theta + (long long)p * P.ld;
-  const int k = star_of(P.star, P.n_stars, p);
-  PointSetup S{};
-  FastSetup FS{};
-  tail_setup_star(P, th, k, S, FS.obs, c ? P.binary : nullptr);
-  if (!S.bad && S.use_inst) stage2_setup(F, S, FS);
-  FastPoint* out = reinterpret_cast<FastPoint*>(F.points) + i;
-  out->S = S;
-  out->FS = FS;
-  if (c == 0) {
+  if (BIN && c == 0) {
     const double t1 = get_par(P, th, PAYNE_P_TEFF, k);
     const PayneBinary& b = *P.binary;
     P.bin_par[3LL * p] = t1;

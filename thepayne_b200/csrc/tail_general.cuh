@@ -45,8 +45,7 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
     if (tid == 0) tail_setup(P, th, p, S, SL);
     __syncthreads();
     if (S.bad) {
-      if (P.model_out)
-        for (int j = tid; j < SL.n; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
+      model_nan(P, p, 0, SL.n, tid);
       if (tid == 0 && P.lnl) P.lnl[p] = nan;
       __syncthreads();
       continue;
@@ -140,14 +139,8 @@ tail_general_kernel(const __grid_constant__ TailParams P, const __grid_constant_
       }
     }
     // ---------------- block reduction -> one lnL per live point (likelihood.py:117)
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if ((tid & 31) == 0) red[tid >> 5] = acc;
-    __syncthreads();
+    double c2 = cta_sum(acc, red, tid);
     if (tid == 0 && P.lnl) {
-      double c2 = 0.0;
-#pragma unroll
-      for (int wdx = 0; wdx < kTailThreads / 32; ++wdx) c2 += red[wdx];
       if (P.chi2_sed) c2 += P.chi2_sed[p];
       P.lnl[p] = -0.5 * c2;
     }

@@ -156,8 +156,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
       const int i0 = sh_i0, i1 = sh_i1, nM = i1 - i0 + 1;
       const int off = so.off, no = so.n;
       if (S.bad || nM < 17) {
-        if (P.model_out)
-          for (int j = tid; j < no; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
+        model_nan(P, p, 0, no, tid);
         if (tid == 0 && P.lnl) P.lnl[p] = nan;
         __syncthreads();
         continue;
@@ -244,8 +243,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
       const int log2nx = (Nf == Nf && Nf > 0.0 && Nf < 1e9) ? (int)ceil(log2(Nf)) : -1;
       if (log2nx < 1 || log2nx > L.log2nx_max) {               // nx = 1: the reference's irfft raises (DESIGN §5)
         if (tid == 0) { if (log2nx > L.log2nx_max) atomicOr(P.status, 1); if (P.lnl) P.lnl[p] = nan; }
-        if (P.model_out)
-          for (int j = tid; j < no; j += kTailThreads) P.model_out[(long long)p * P.ld_flux + j] = nan;
+        model_nan(P, p, 0, no, tid);
         __syncthreads();
         continue;
       }
@@ -291,14 +289,8 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
           acc += r * r;
         }
       }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-      if ((tid & 31) == 0) red[tid >> 5] = acc;
-      __syncthreads();
+      double c2 = cta_sum(acc, red, tid);
       if (tid == 0 && P.lnl) {
-        double c2 = 0.0;
-#pragma unroll
-        for (int wdx = 0; wdx < kTailThreads / 32; ++wdx) c2 += red[wdx];
         if (P.chi2_sed) c2 += P.chi2_sed[p];
         P.lnl[p] = -0.5 * c2;
       }
@@ -437,20 +429,6 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
       return true;
     };
 
-    // chi2 of the CTA: the warps' shares summed in warp order (thread 0)
-    auto reduce = [&](double acc) {
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-      if ((tid & 31) == 0) red[tid >> 5] = acc;
-      __syncthreads();
-      double c2 = 0.0;
-      if (tid == 0) {
-#pragma unroll
-        for (int wdx = 0; wdx < kTailThreads / 32; ++wdx) c2 += red[wdx];
-      }
-      return c2;
-    };
-
     for (int p = blockIdx.x; p < P.B; p += gridDim.x) {
       const double* th = P.theta + (long long)p * P.ld;
       float* row = P.flux + (long long)p * P.ldf;
@@ -484,7 +462,7 @@ tail_lsf_kernel(const __grid_constant__ TailParams P, const __grid_constant__ Ls
         } else if (mrow_m) {
           for (int j = tid; j < so.n; j += kTailThreads) mrow_m[j] = nan;
         }
-        double c2 = reduce(acc);                         // (its barrier also frees S, so and the scratch)
+        double c2 = cta_sum(acc, red, tid);              // (its barrier also frees S, so and the scratch)
         if (tid == 0) {
           if (!ok) c2 = nan;
           if (valid && P.chi2_out) P.chi2_out[(long long)p * P.ld_chi2 + m] = c2;

@@ -15,7 +15,7 @@ B = 'thepayne_b200/csrc/_build/'
 for obj, pat, marks in [(B + 'gemm_tu.o', 'tc_gemm_kernelILi128ELi2ELi0EE', ['UTCHMMA', 'UTMALDG', 'UTMASTG', 'LDTM']),
                         (B + 'gemm_tu.o', 'tc_gemm_kernelILi64ELi2ELi1EE', ['UTCHMMA', 'LDTM']),
                         (B + 'gemm_tu.o', 'tc_hidden_stack_kernel', ['UTCHMMA', 'UCGABAR_ARV', 'UTMALDG']),
-                        (B + 'tail_fast_tu.o', 'tail_fast_kernelILi14ELb0E', ['FADD2', 'LDS.128', 'CCTL', 'CALL']),
+                        (B + 'tail_fast_tu.o', 'tail_fast_kernelILi14ELb0ELNS_8FastBodyE0EE', ['FADD2', 'LDS.128', 'CCTL', 'CALL']),
                         (B + 'tail_cluster_tu.o', 'tail_cluster_kernelILi16E', ['UCGABAR_ARV', 'MAPA', 'ST.E.64', 'LD.E.64'])]:
     f = funcs(sass(obj))
     name = [k for k in f if pat in k][0]
