@@ -453,12 +453,8 @@ class Engine:
 
     def lnlike_batch_binary(self, theta, star=None):
         """lnL of every row as a binary, ``theta`` and ``star`` as in ``lnlike_batch`` (None: star 0)."""
-        if isinstance(theta, torch.Tensor) and theta.is_cuda:
-            th, sv, lnl, st = self._dev_args(theta, star, copy=False)
-            _lib.check(self.lib.payne_lnlike_batch_binary(self._ctx, th.data_ptr(), _ptr(sv), th.shape[0], th.shape[1],
-                                                          lnl.data_ptr(), st))
-            return lnl
-        return self._host_lnlike(self.lib.payne_lnlike_batch_binary_host, theta, star, 'star')
+        return self._lnlike(self.lib.payne_lnlike_batch_binary, self.lib.payne_lnlike_batch_binary_host, theta, star,
+                            'star')
 
     def model_batch_binary(self, theta, star=None, want_flux=True, want_comp=True):
         """Model spectra [B, n_obs], the components' spectra before the continuum [B, 2, n_obs] and lnL [B] of every
@@ -477,12 +473,8 @@ class Engine:
         through the host entry, which refuses such an index)."""
         if not self.n_targets:
             raise ValueError('no targets: set_targets first')
-        if isinstance(theta, torch.Tensor) and theta.is_cuda:
-            th, tv, lnl, st = self._dev_args(theta, target, copy=False)
-            _lib.check(self.lib.payne_lnlike_batch_targets(self._ctx, th.data_ptr(), _ptr(tv), th.shape[0],
-                                                           th.shape[1], lnl.data_ptr(), st))
-            return lnl
-        return self._host_lnlike(self.lib.payne_lnlike_batch_targets_host, theta, target, 'target')
+        return self._lnlike(self.lib.payne_lnlike_batch_targets, self.lib.payne_lnlike_batch_targets_host, theta,
+                            target, 'target')
 
     def model_batch_targets(self, theta, target, want_flux=True, want_chi2=True, want_mags=True):
         """Model spectra [B, max target_n_obs] (row p: its members' spectra back to back in member order, the rest
@@ -532,9 +524,14 @@ class Engine:
             idx = idx.contiguous()
         return th, idx, torch.empty(B, dtype=torch.float64, device=dev), torch.cuda.current_stream(dev).cuda_stream
 
-    def _host_lnlike(self, entry, theta, idx, what):
-        """lnL [B] (numpy) through the host-buffer entry ``entry``: theta [B, ndim] and idx [B] (every row's star or
-        target, ``what``; None: star 0) as anything numpy takes."""
+    def _lnlike(self, dev_entry, host_entry, theta, idx, what):
+        """lnL [B] of theta [B, ndim] and idx [B] (every row's star or target, ``what``; None: star 0): with a CUDA
+        theta a CUDA tensor from the device entry ``dev_entry``, else numpy from the host-buffer entry ``host_entry``,
+        theta and idx then as anything numpy takes."""
+        if isinstance(theta, torch.Tensor) and theta.is_cuda:
+            th, iv, lnl, st = self._dev_args(theta, idx, copy=False)
+            _lib.check(dev_entry(self._ctx, th.data_ptr(), _ptr(iv), th.shape[0], th.shape[1], lnl.data_ptr(), st))
+            return lnl
         th = _f64(theta)
         if th.ndim != 2 or th.shape[1] != self.ndim:
             raise ValueError('theta must be [B, %d]' % self.ndim)
@@ -544,8 +541,8 @@ class Engine:
             if iv.shape != (th.shape[0],):
                 raise ValueError('%s must be [%d]' % (what, th.shape[0]))
         out = np.empty(th.shape[0], dtype=np.float64)
-        _lib.check(entry(self._ctx, th.ctypes.data, iv.ctypes.data if iv is not None else None, th.shape[0], th.shape[1],
-                         out.ctypes.data))
+        _lib.check(host_entry(self._ctx, th.ctypes.data, iv.ctypes.data if iv is not None else None, th.shape[0],
+                              th.shape[1], out.ctypes.data))
         return out
 
     def lnlike_batch(self, theta, star=None):
@@ -554,12 +551,8 @@ class Engine:
         every row, an int32 CUDA tensor with a CUDA theta, anything numpy takes otherwise (None: star 0,
         which only a single-star engine accepts).  On the device a row with an index outside
         [0, n_stars) gets NaN and sets status bit 2; the host path refuses such an index."""
-        if isinstance(theta, torch.Tensor) and theta.is_cuda:
-            th, sv, lnl, st = self._dev_args(theta, star, copy=False)
-            _lib.check(self.lib.payne_lnlike_batch_stars(self._ctx, th.data_ptr(), _ptr(sv), th.shape[0], th.shape[1],
-                                                         lnl.data_ptr(), st))
-            return lnl
-        return self._host_lnlike(self.lib.payne_lnlike_batch_stars_host, theta, star, 'star')
+        return self._lnlike(self.lib.payne_lnlike_batch_stars, self.lib.payne_lnlike_batch_stars_host, theta, star,
+                            'star')
 
     def model_batch(self, theta, star=None, want_flux=True, want_mags=True):
         """Model spectra [B, n_obs], magnitudes [B, nb] and lnL [B] as CUDA float64 tensors.  With several

@@ -52,6 +52,15 @@ _BINARY = ['Teff_sec', 'log(g)_sec', '[Fe/H]_sec', '[a/Fe]_sec', 'Vrad_sec', 'Vr
 _BINARY_ON = ['Teff_sec', 'log(g)_sec', 'Vrad_sec', 'Vrot_sec', 'Rratio']
 
 
+def _fitted(sp, sel):
+    """A spectrum dictionary's fitted observation: wave, flux and eflux at ``sel`` as float64, the wavelengths in
+    vacuum unless ``convertair`` is False."""
+    fit = {'obs_%s_fit' % k: np.asarray(sp['obs_' + k], dtype=np.float64)[sel] for k in ['wave', 'flux', 'eflux']}
+    if sp.get('convertair', True):
+        fit['obs_wave_fit'] = airtovacuum(fit['obs_wave_fit'])
+    return fit
+
+
 class FitPayne(object):
     def __init__(self, **kwargs):
         from .likelihood import likelihood
@@ -85,48 +94,29 @@ class FitPayne(object):
             raise NotImplementedError('binary with several spectra (a list-valued spec)')
         if self.binary_bool and 'phot' in inputdict:
             raise NotImplementedError('binary with photometry: the SED of two stars is not modelled')
-        if isinstance(inputdict.get('spec'), (list, tuple)):
-            self._setup_spectra(inputdict)
-        elif 'spec' in inputdict:                                          # fitstar.py:70-154
-            sp = inputdict['spec']
+        if 'spec' in inputdict:                                            # fitstar.py:70-154
             self.spec_bool = True
-            fa['obs_wave'], fa['obs_flux'], fa['obs_eflux'] = sp['obs_wave'], sp['obs_flux'], sp['obs_eflux']
             fa['specANNpath'] = inputdict.get('specANNpath', None)
             fa['NNtype'] = inputdict.get('NNtype', 'LinNet')
+            for pp in ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot', 'Inst_R'] + \
+                    (['Vmic'] if fa['NNtype'] == 'YST2' else []):
+                self.fitpars_bool[pp] = True
+        if isinstance(inputdict.get('spec'), (list, tuple)):
+            self._setup_spectra(inputdict)
+        elif 'spec' in inputdict:
+            sp = inputdict['spec']
+            fa['obs_wave'], fa['obs_flux'], fa['obs_eflux'] = sp['obs_wave'], sp['obs_flux'], sp['obs_eflux']
             sel = slice(None)
-            if 'wave_minmax' in sp:
+            if 'wave_minmax' in sp:                    # the wavelengths as given: float32 ones compare in float32
                 fa['wave_minmax'] = sp['wave_minmax']
                 sel = (np.asarray(fa['obs_wave']) >= sp['wave_minmax'][0]) & (np.asarray(fa['obs_wave']) <= sp['wave_minmax'][1])
-            for k in ['wave', 'flux', 'eflux']:
-                fa['obs_%s_fit' % k] = np.asarray(fa['obs_' + k], dtype=np.float64)[sel]
-            if sp.get('convertair', True):
-                fa['obs_wave_fit'] = airtovacuum(fa['obs_wave_fit'])
-            on = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot', 'Inst_R']
-            if fa['NNtype'] == 'YST2':
-                on.append('Vmic')
-            for pp in on:
-                self.fitpars_bool[pp] = True
-            if sp.get('modpoly_marginal', False) and not sp.get('modpoly', False):
-                raise ValueError("spec['modpoly_marginal'] needs spec['modpoly']")
-            if sp.get('modpoly', False):                                   # fitstar.py:110-147
-                self.modpoly_bool = True
-                if 'blaze_coeff' in self.priordict:
-                    self.polycoefarr = self.priordict['blaze_coeff']
-                elif 'polyorder' in sp:
-                    sig = sp.get('polysigma', 1.0)
-                    self.polycoefarr = [[0.0, sig] for _ in range(sp['polyorder'] + 1)]
-                else:
-                    self.polycoefarr = [[0.0, 1.0] for _ in range(3)]
-                self.priordict['blaze_coeff'] = self.polycoefarr
-                self.polyorder = len(self.polycoefarr)
+            fa.update(_fitted(sp, sel))
+            coef, box = self._setup_continuum(sp, 'blaze_coeff', 'pc_{}')
+            if coef is not None:
+                self.polycoefarr, self.polyorder = coef, len(coef)
                 fa['norm_polyorder'] = self.polyorder
-                if sp.get('modpoly_marginal', False):
-                    fa['cont_names'] = ['pc_{}'.format(ii) for ii in range(self.polyorder)]
-                    fa['cont_box'] = [self.prior.pc_box(ii, self.polycoefarr) for ii in range(self.polyorder)]
-                else:
-                    for ii in range(self.polyorder):
-                        self.fitpars.append('pc_{}'.format(ii))
-                        self.fitpars_bool['pc_{}'.format(ii)] = True
+                if box is not None:
+                    fa['cont_box'] = box
 
         if 'phot' in inputdict:                                            # fitstar.py:157-190
             self.phot_bool = True
@@ -163,30 +153,21 @@ class FitPayne(object):
                 'runbools': [self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool]}
 
     def _setup_spectra(self, inputdict):
-        """A list-valued ``spec``: every spectrum's observation as the single one's (wave_minmax, convertair), the
-        shared spectral parameters once, ``Inst_R_<s>`` and ``pc_<s>_<k>`` per spectrum."""
+        """A list-valued ``spec``: every spectrum's observation as the single one's (wave_minmax, convertair), and
+        ``Inst_R_<s>`` in place of ``Inst_R`` and ``pc_<s>_<k>`` per spectrum."""
         specs = list(inputdict['spec'])
         if not specs:
             raise ValueError("inputdict['spec'] is an empty list")
         if any('Vrad' in sp for sp in specs) or any(k.startswith('Vrad_') for k in self.priordict):
             raise NotImplementedError('a Vrad per spectrum: FitPayne fits one Vrad shared by every spectrum')
         fa = self.fitargs
-        self.spec_bool = True
-        fa['specANNpath'] = inputdict.get('specANNpath', None)
-        fa['NNtype'] = inputdict.get('NNtype', 'LinNet')
         fa['spectra'] = []
         for sp in specs:
             w = np.asarray(sp['obs_wave'], dtype=np.float64)
             sel = slice(None)
             if 'wave_minmax' in sp:
                 sel = (w >= sp['wave_minmax'][0]) & (w <= sp['wave_minmax'][1])
-            one = {'obs_%s_fit' % k: np.asarray(sp['obs_' + k], dtype=np.float64)[sel] for k in ['wave', 'flux', 'eflux']}
-            if sp.get('convertair', True):
-                one['obs_wave_fit'] = airtovacuum(one['obs_wave_fit'])
-            fa['spectra'].append(one)
-        on = ['Teff', 'log(g)', '[Fe/H]', '[a/Fe]', 'Vrad', 'Vrot'] + (['Vmic'] if fa['NNtype'] == 'YST2' else [])
-        for pp in on:
-            self.fitpars_bool[pp] = True
+            fa['spectra'].append(_fitted(sp, sel))
         self.fitpars.remove('Inst_R')
         self.fitpars_bool.pop('Inst_R')
         for s in range(len(specs)):
@@ -196,29 +177,36 @@ class FitPayne(object):
             raise ValueError('every spectrum has a continuum polynomial (modpoly) or none does')
         if len({bool(sp.get('modpoly_marginal', False)) for sp in specs}) > 1:
             raise ValueError('every spectrum sets modpoly_marginal or none does')
-        self.modpoly_bool = bool(specs[0].get('modpoly', False))
-        marginal = bool(specs[0].get('modpoly_marginal', False))
-        if marginal and not self.modpoly_bool:
+        for s, sp in enumerate(specs):                                     # as fitstar.py:110-147 per spectrum
+            box = self._setup_continuum(sp, 'blaze_coeff_%d' % s, 'pc_%d_{}' % s)[1]
+            if box is not None:
+                fa['spectra'][s]['cont_box'] = box
+
+    def _setup_continuum(self, sp, key, name):
+        """The continuum polynomial of a spectrum dictionary with ``modpoly`` (fitstar.py:110-147): the prior
+        ``priordict[key]`` of its coefficients (default: ``polyorder`` + 1 of width ``polysigma``, else three of width
+        1), named ``name.format(k)``.  Sampled, they join the free parameters; with ``modpoly_marginal`` they join
+        ``cont_names`` and get the boxes of a sampled ``pc_k``.  Returns the prior and the boxes (None when sampled);
+        (None, None) without ``modpoly``."""
+        if sp.get('modpoly_marginal', False) and not sp.get('modpoly', False):
             raise ValueError("spec['modpoly_marginal'] needs spec['modpoly']")
-        if marginal:
-            fa['cont_names'] = []
-        for s, sp in enumerate(specs):
-            if not self.modpoly_bool:
-                break
-            key = 'blaze_coeff_%d' % s
-            if key not in self.priordict:                                  # as fitstar.py:110-147 per spectrum
-                if 'polyorder' in sp:
-                    self.priordict[key] = [[0.0, sp.get('polysigma', 1.0)] for _ in range(sp['polyorder'] + 1)]
-                else:
-                    self.priordict[key] = [[0.0, 1.0] for _ in range(3)]
-            K = len(self.priordict[key])
-            if marginal:
-                fa['spectra'][s]['cont_box'] = [self.prior.pc_box(k, self.priordict[key]) for k in range(K)]
-                fa['cont_names'] += ['pc_%d_%d' % (s, k) for k in range(K)]
-                continue
-            for k in range(K):
-                self.fitpars.append('pc_%d_%d' % (s, k))
-                self.fitpars_bool['pc_%d_%d' % (s, k)] = True
+        if not sp.get('modpoly', False):
+            return None, None
+        self.modpoly_bool = True
+        if key not in self.priordict:
+            if 'polyorder' in sp:
+                self.priordict[key] = [[0.0, sp.get('polysigma', 1.0)] for _ in range(sp['polyorder'] + 1)]
+            else:
+                self.priordict[key] = [[0.0, 1.0] for _ in range(3)]
+        coef = self.priordict[key]
+        names = [name.format(k) for k in range(len(coef))]
+        if not sp.get('modpoly_marginal', False):
+            for pp in names:
+                self.fitpars.append(pp)
+                self.fitpars_bool[pp] = True
+            return coef, None
+        self.fitargs.setdefault('cont_names', []).extend(names)
+        return coef, [self.prior.pc_box(k, coef) for k in range(len(coef))]
 
     def __call__(self, indicts):
         return self.run_dynesty(indicts)

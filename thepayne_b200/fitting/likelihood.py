@@ -27,35 +27,34 @@ def free_parameters(fitpars):
     return [pp for pp in fitpars[0] if fitpars[1][pp]]
 
 
-class likelihood(object):
-    def __init__(self, fitargs, fitpars, runbools, **kwargs):
-        self.verbose = kwargs.get('verbose', True)
-        self.fitargs = fitargs
-        self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool = runbools[:5]
-        if self.carbon_bool:
-            raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
-        self.fixedpars = self.fitargs['fixedpars']
-        self.precision = kwargs.get('precision', 'parity')
-        self.GM = GenMod(precision=self.precision)
-        if self.spec_bool:
-            self.GM._initspecnn(nnpath=fitargs['specANNpath'], NNtype=self.fitargs.get('NNtype', 'LinNet'),
-                                carbon_bool=self.carbon_bool)
-        if self.phot_bool:
-            self.GM._initphotnn(self.fitargs['obs_phot'].keys(), nnpath=fitargs['photANNpath'])
-        self.fitpars_i = free_parameters(fitpars)
-        self.ndim = len(self.fitpars_i)
-        self.parsdict = {}
-        self.engine = Engine(
-            spec=self.GM.PP.anns.model if self.spec_bool else None,
-            phot=self.GM.fppsed.net if self.phot_bool else None,
-            obs_wave=fitargs.get('obs_wave_fit'), obs_flux=fitargs.get('obs_flux_fit'),
-            obs_eflux=fitargs.get('obs_eflux_fit'), obs_phot=fitargs.get('obs_phot'),
-            fitpars_i=self.fitpars_i, fixedpars=self.fixedpars,
-            runbools=[self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
-            precision=self.precision, device=kwargs.get('device'), cont_box=fitargs.get('cont_box'))
-        self._explicit = None
+def _genmod(fitargs, runbools, precision, bands=None):
+    """The run booleans (spec, phot, modpoly, photscale, carbon) and the emulators (``GenMod``) of a fit: the spectrum
+    net of ``specANNpath`` / ``NNtype`` with spectra, the photometry net of ``photANNpath`` for ``bands`` (default:
+    the ``obs_phot`` bands) with photometry."""
+    runbools = tuple(runbools[:5])
+    if runbools[4]:
+        raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
+    GM = GenMod(precision=precision)
+    if runbools[0]:
+        GM._initspecnn(nnpath=fitargs['specANNpath'], NNtype=fitargs.get('NNtype', 'LinNet'))
+    if runbools[1]:
+        GM._initphotnn(fitargs['obs_phot'].keys() if bands is None else bands, nnpath=fitargs['photANNpath'])
+    return runbools, GM
 
-    # ------------------------------------------------------------------ reference entry points
+
+class _Likelihood(object):
+    """The interface every kind of fit gives its sampler: ``fitpars_i`` (the sampled parameters in theta order),
+    ``ndim``, ``fixedpars``, ``parsdict`` (the last row evaluated, fixed values included), ``lnlikefn`` for one row
+    and ``lnlike_batch`` for many.  A kind of fit supplies ``_lnlike(theta)``: lnL of rows [B, ndim] (CUDA float64
+    tensor, or numpy) of the same kind; ``_lnlike_batch`` may route the batched calls elsewhere.  With continuum
+    marginalisation it supplies ``_cont(theta)`` too: ``Engine.cont_batch``'s outputs for the rows."""
+
+    def __init__(self, fitpars_i, fixedpars):
+        self.fitpars_i = fitpars_i
+        self.ndim = len(fitpars_i)
+        self.fixedpars = fixedpars
+        self.parsdict = {}
+
     def _set_parsdict(self, pars):
         self.parsdict = {pp: vv for pp, vv in zip(self.fitpars_i, pars)}
         for kk in self.fixedpars.keys():
@@ -65,7 +64,55 @@ class likelihood(object):
         """One parameter vector -> float (likelihood.py:42-82)."""
         self._set_parsdict(pars)
         th = np.asarray(pars, dtype=np.float64).reshape(1, self.ndim)
-        return float(self.engine.lnlike_batch(th)[0])
+        return float(self._lnlike(th)[0])
+
+    def lnlike_batch(self, theta):
+        """theta [B, ndim] (CUDA float64 tensor, or numpy) -> lnL [B] of the same kind."""
+        out = self._lnlike_batch(theta)
+        last = theta[-1]
+        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
+        return out
+
+    def _lnlike_batch(self, theta):
+        return self._lnlike(theta)
+
+    def cont_batch(self, theta):
+        """Marginalised continuum: c-hat [B, K] and the packed Cholesky factors [B, K(K+1)/2] (numpy)."""
+        coef, chol, _, _ = self._cont(theta)
+        return coef.cpu().numpy(), chol.cpu().numpy()
+
+    def _cont(self, theta):
+        raise NotImplementedError('%s integrates no continuum out' % type(self).__name__)
+
+
+class likelihood(_Likelihood):
+    def __init__(self, fitargs, fitpars, runbools, **kwargs):
+        self.verbose = kwargs.get('verbose', True)
+        self.fitargs = fitargs
+        self.precision = kwargs.get('precision', 'parity')
+        (self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool), self.GM = \
+            _genmod(fitargs, runbools, self.precision)
+        super().__init__(free_parameters(fitpars), fitargs['fixedpars'])
+        self.engine = self._engine(self.fitpars_i, self.fixedpars, device=kwargs.get('device'),
+                                   cont_box=fitargs.get('cont_box'))
+        self._explicit = None
+
+    def _engine(self, fitpars_i, fixedpars, **kwargs):
+        """An engine on this fit's observation and emulators for the layout ``fitpars_i`` / ``fixedpars``."""
+        fa = self.fitargs
+        return Engine(spec=self.GM.PP.anns.model if self.spec_bool else None,
+                      phot=self.GM.fppsed.net if self.phot_bool else None,
+                      obs_wave=fa.get('obs_wave_fit'), obs_flux=fa.get('obs_flux_fit'),
+                      obs_eflux=fa.get('obs_eflux_fit'), obs_phot=fa.get('obs_phot'),
+                      fitpars_i=fitpars_i, fixedpars=fixedpars,
+                      runbools=[self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
+                      precision=self.precision, **kwargs)
+
+    def _lnlike(self, theta):
+        return self.engine.lnlike_batch(theta)
+
+    def _cont(self, theta):
+        return self.engine.cont_batch(theta)
 
     def lnlike(self, specpars=None, photpars=None):
         """Explicit ``specpars`` / ``photpars`` lists as built by lnlikefn (likelihood.py:84-117)."""
@@ -92,26 +139,5 @@ class likelihood(object):
         if self._explicit is None or self._explicit[0] != key:
             if self._explicit is not None:
                 self._explicit[1].close()
-            fa = self.fitargs
-            eng = Engine(spec=self.GM.PP.anns.model if self.spec_bool else None,
-                         phot=self.GM.fppsed.net if self.phot_bool else None,
-                         obs_wave=fa.get('obs_wave_fit'), obs_flux=fa.get('obs_flux_fit'),
-                         obs_eflux=fa.get('obs_eflux_fit'), obs_phot=fa.get('obs_phot'), fitpars_i=names,
-                         fixedpars=None if lsf is None else {'Inst_R': lsf},
-                         runbools=[self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
-                         precision=self.precision)
-            self._explicit = (key, eng)
+            self._explicit = (key, self._engine(names, None if lsf is None else {'Inst_R': lsf}))
         return float(self._explicit[1].lnlike_batch(np.array([vals], dtype=np.float64))[0])
-
-    def cont_batch(self, theta):
-        """Marginalised continuum: c-hat [B, K] and the packed Cholesky factors [B, K(K+1)/2] (numpy)."""
-        coef, chol, _, _ = self.engine.cont_batch(theta)
-        return coef.cpu().numpy(), chol.cpu().numpy()
-
-    # ------------------------------------------------------------------ batched entry point
-    def lnlike_batch(self, theta):
-        """theta [B, ndim] (CUDA float64 tensor, or numpy) -> lnL [B] of the same kind."""
-        out = self.engine.lnlike_batch(theta)
-        last = theta[-1]
-        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
-        return out

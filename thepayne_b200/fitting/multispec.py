@@ -1,5 +1,4 @@
-"""``MultiSpecLikelihood``: one star observed in several spectra (echelle orders, spectrograph arms), the
-``likelihood`` interface (``lnlikefn``, ``lnlike_batch``, ``parsdict``, ``fitpars_i``, ``ndim``, ``fixedpars``).
+"""``MultiSpecLikelihood``: one star observed in several spectra (echelle orders, spectrograph arms).
 
 The spectra are the members of one target of an observation set (``Engine(stars=[...], targets=[S])``): the labels,
 ``Vrad`` and ``Vrot`` are shared, spectrum s has its own resolving power ``Inst_R_<s>`` and continuum coefficients
@@ -23,8 +22,7 @@ import numpy as np
 import torch
 
 from ..engine import Engine
-from .genmod import GenMod
-from .likelihood import free_parameters
+from .likelihood import _genmod, _Likelihood, free_parameters
 
 _PHOT = ['log(R)', 'Dist', 'log(A)', 'Av', 'Rv']
 
@@ -40,29 +38,22 @@ def spectrum_name(name, s):
     return name
 
 
-class MultiSpecLikelihood(object):
+class MultiSpecLikelihood(_Likelihood):
     def __init__(self, fitargs, fitpars, runbools, **kwargs):
         self.fitargs = fitargs
-        self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool = runbools[:5]
-        if not self.spec_bool:
+        if not runbools[0]:
             raise ValueError('MultiSpecLikelihood needs spectra')
-        if self.carbon_bool:
-            raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
-        self.fixedpars = fitargs['fixedpars']
+        fixedpars = fitargs['fixedpars']
         spectra = fitargs['spectra']
-        lsf = [np.ndim(self.fixedpars.get('Inst_R_%d' % s, 0.0)) == 1 for s in range(len(spectra))]
+        lsf = [np.ndim(fixedpars.get('Inst_R_%d' % s, 0.0)) == 1 for s in range(len(spectra))]
         if any(lsf) and not all(lsf):
             raise ValueError('spectra %s have an LSF vector (a fixed Inst_R_<s> array) and spectra %s do not: every '
                              'spectrum has one or none does' % ([s for s, v in enumerate(lsf) if v],
                                                                 [s for s, v in enumerate(lsf) if not v]))
         self.precision = kwargs.get('precision', 'parity')
-        self.GM = GenMod(precision=self.precision)
-        self.GM._initspecnn(nnpath=fitargs['specANNpath'], NNtype=fitargs.get('NNtype', 'LinNet'))
-        if self.phot_bool:
-            self.GM._initphotnn(fitargs['obs_phot'].keys(), nnpath=fitargs['photANNpath'])
-        self.fitpars_i = free_parameters(fitpars)
-        self.ndim = len(self.fitpars_i)
-        self.parsdict = {}
+        (self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool), self.GM = \
+            _genmod(fitargs, runbools, self.precision)
+        super().__init__(free_parameters(fitpars), fixedpars)
         stars = []
         for s, sp in enumerate(spectra):
             fit = [spectrum_name(p, s) for p in self.fitpars_i]
@@ -89,29 +80,12 @@ class MultiSpecLikelihood(object):
                              runbools=[True, self.phot_bool, self.modpoly_bool, self.photscale_bool, False],
                              precision=self.precision, device=kwargs.get('device'))
 
-    def _set_parsdict(self, pars):
-        self.parsdict = {pp: vv for pp, vv in zip(self.fitpars_i, pars)}
-        for kk in self.fixedpars.keys():
-            self.parsdict[kk] = self.fixedpars[kk]
-
-    def lnlikefn(self, pars):
-        """One parameter vector -> float."""
-        self._set_parsdict(pars)
-        th = np.asarray(pars, dtype=np.float64).reshape(1, self.ndim)
-        return float(self.engine.lnlike_batch_targets(th, np.zeros(1, np.int32))[0])
-
-    def cont_batch(self, theta):
-        """Marginalised continua: every spectrum's c-hat and packed Cholesky factor back to back (numpy)."""
-        coef, chol, _, _ = self.engine.cont_batch_targets(theta, np.zeros(len(theta), np.int32))
-        return coef.cpu().numpy(), chol.cpu().numpy()
-
-    def lnlike_batch(self, theta):
-        """theta [B, ndim] (CUDA float64 tensor, or numpy) -> lnL [B] of the same kind."""
+    def _lnlike(self, theta):
         if isinstance(theta, torch.Tensor) and theta.is_cuda:
             target = torch.zeros(theta.shape[0], dtype=torch.int32, device=theta.device)
         else:
             target = np.zeros(len(theta), np.int32)
-        out = self.engine.lnlike_batch_targets(theta, target)
-        last = theta[-1]
-        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
-        return out
+        return self.engine.lnlike_batch_targets(theta, target)
+
+    def _cont(self, theta):
+        return self.engine.cont_batch_targets(theta, np.zeros(len(theta), np.int32))

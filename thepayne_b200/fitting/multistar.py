@@ -27,8 +27,7 @@ import numpy as np
 
 from ..engine import Engine
 from .fitstar import FitPayne
-from .genmod import GenMod
-from .likelihood import free_parameters
+from .likelihood import _genmod, _Likelihood, free_parameters
 
 
 def _same(a, b):
@@ -66,8 +65,6 @@ class StarSetLikelihood(object):
         rb_list = [[bool(b) for b in rb[:5]] for rb in rb_list]
         free_list = [free_parameters(fp) for fp in fp_list]
         fa0, free0, rb0 = fitargs_list[0], free_list[0], rb_list[0]
-        if any(rb[4] for rb in rb_list):
-            raise NotImplementedError('carbon_bool is hard-wired off in the reference (fitstar.py:150-154)')
         phot_stars = [k for k in range(S) if rb_list[k][1]]
         for k in range(1, S):
             fa = fitargs_list[k]
@@ -89,20 +86,17 @@ class StarSetLikelihood(object):
         for k in phot_stars[1:]:
             if not _same(fitargs_list[k].get('photANNpath'), fitargs_list[phot_stars[0]].get('photANNpath')):
                 raise ValueError('star %d: photANNpath differs from star %d' % (k, phot_stars[0]))
-        self.spec_bool, _, self.modpoly_bool, self.photscale_bool, self.carbon_bool = rb0
-        self.phot_bool = bool(phot_stars)
+        self.bands = []
+        for k in phot_stars:
+            self.bands += [b for b in fitargs_list[k]['obs_phot'].keys() if b not in self.bands]
+        # star 0's spectrum net (every star names the same), the photometry net of the first star with photometry
+        nets = dict(fa0, photANNpath=fitargs_list[phot_stars[0]]['photANNpath']) if phot_stars else fa0
+        (self.spec_bool, self.phot_bool, self.modpoly_bool, self.photscale_bool, self.carbon_bool), self.GM = _genmod(
+            nets, [rb0[0], bool(phot_stars), rb0[2], rb0[3], any(rb[4] for rb in rb_list)], precision, self.bands)
         self.n_stars = S
         self.fitargs_list = fitargs_list
         self.fixedpars = fa0['fixedpars']
         self.precision = precision
-        self.GM = GenMod(precision=precision)            # the emulators, as likelihood.__init__ loads them
-        if self.spec_bool:
-            self.GM._initspecnn(nnpath=fa0['specANNpath'], NNtype=fa0.get('NNtype', 'LinNet'), carbon_bool=False)
-        self.bands = []
-        if self.phot_bool:
-            for k in phot_stars:
-                self.bands += [b for b in fitargs_list[k]['obs_phot'].keys() if b not in self.bands]
-            self.GM._initphotnn(self.bands, nnpath=fitargs_list[phot_stars[0]]['photANNpath'])
         stars = [{'wave': fa.get('obs_wave_fit'), 'flux': fa.get('obs_flux_fit'), 'eflux': fa.get('obs_eflux_fit'),
                   'phot': fa.get('obs_phot') if rb[1] else None,
                   'bands': list(fa['obs_phot'].keys()) if rb[1] else None,
@@ -130,9 +124,12 @@ class StarSetLikelihood(object):
 
     def cont_batch(self, theta, star):
         """Marginalised continua (a star's ``cont_box``): c-hat and packed Cholesky factors of every row (numpy)."""
+        coef, chol, _, _ = self._cont(theta, star)
+        return coef.cpu().numpy(), chol.cpu().numpy()
+
+    def _cont(self, theta, star):
         with self._lock:
-            coef, chol, _, _ = self.engine.cont_batch(theta, star)
-            return coef.cpu().numpy(), chol.cpu().numpy()
+            return self.engine.cont_batch(theta, star)
 
     def star(self, k):
         """Star k with the interface of ``likelihood.likelihood``."""
@@ -147,19 +144,15 @@ def _is_per_star(fitpars, S):
                                      for f in fitpars)
 
 
-class StarView(object):
-    """One star of a ``StarSetLikelihood``: ``lnlikefn``, ``lnlike_batch(theta)``, ``parsdict``, ``fitpars_i``,
-    ``ndim``, ``fixedpars`` (the star's own) as in ``likelihood.likelihood``.  Its rows [B, ndim] are padded to the
-    engine's width before they are posted."""
+class StarView(_Likelihood):
+    """One star of a ``StarSetLikelihood`` with the interface of ``likelihood.likelihood`` and the star's own
+    ``fixedpars``.  Its rows [B, ndim] are padded to the engine's width before they are posted."""
 
     def __init__(self, owner, k):
         self.owner, self.k = owner, int(k)
         own = getattr(owner, 'star_fitpars_i', None)        # an owner without it has one layout for all stars
-        self.fitpars_i = own[self.k] if own is not None else owner.fitpars_i
-        self.ndim = len(self.fitpars_i)
         self.fitargs = owner.fitargs_list[self.k]
-        self.fixedpars = self.fitargs.get('fixedpars', {})
-        self.parsdict = {}
+        super().__init__(own[self.k] if own is not None else owner.fitpars_i, self.fitargs.get('fixedpars', {}))
 
     def _pad(self, theta):
         # columns beyond the star's ndim are never read (NaN keeps a wrong read visible)
@@ -172,11 +165,6 @@ class StarView(object):
         theta = np.asarray(theta, dtype=np.float64)
         return np.concatenate([theta, np.full((len(theta), w), np.nan)], axis=1)
 
-    def _set_parsdict(self, pars):
-        self.parsdict = {pp: vv for pp, vv in zip(self.fitpars_i, pars)}
-        for kk in self.fixedpars.keys():
-            self.parsdict[kk] = self.fixedpars[kk]
-
     def _lnlike(self, theta):
         theta = self._pad(theta)
         if hasattr(theta, 'is_cuda') and theta.is_cuda:
@@ -186,20 +174,9 @@ class StarView(object):
             star = np.full(len(theta), self.k, dtype=np.int32)
         return self.owner.lnlike_batch(theta, star)
 
-    def lnlikefn(self, pars):
-        self._set_parsdict(pars)
-        th = np.asarray(pars, dtype=np.float64).reshape(1, self.ndim)
-        return float(self._lnlike(th)[0])
-
-    def cont_batch(self, theta):
+    def _cont(self, theta):
         theta = self._pad(np.asarray(theta, dtype=np.float64))
-        return self.owner.cont_batch(theta, np.full(len(theta), self.k, dtype=np.int32))
-
-    def lnlike_batch(self, theta):
-        out = self._lnlike(theta)
-        last = theta[-1]
-        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
-        return out
+        return self.owner._cont(theta, np.full(len(theta), self.k, dtype=np.int32))
 
 
 class _Released(Exception):
@@ -270,17 +247,15 @@ class LockstepBatcher(object):
 
 
 class _BatchedStarView(StarView):
-    """A star's view whose batched calls go through the lock-step batcher."""
+    """A star's view whose batched calls go through the lock-step batcher.  ``lnlikefn`` goes straight to the owner:
+    one row through the barrier would wait for every other sampler."""
 
     def __init__(self, owner, k, batcher):
         super().__init__(owner, k)
         self.batcher = batcher
 
-    def lnlike_batch(self, theta):
-        out = self.batcher.call(self.k, self._pad(theta))
-        last = theta[-1]
-        self._set_parsdict([float(v) for v in (last.tolist() if hasattr(last, 'tolist') else last)])
-        return out
+    def _lnlike_batch(self, theta):
+        return self.batcher.call(self.k, self._pad(theta))
 
 
 class FitPayneMany(object):
